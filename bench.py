@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — encode+decode megapixels/s of the pixlzr hot path on N B200s (one process per GPU).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W
 
@@ -21,6 +21,10 @@ The same line carries the two sharded configurations of BASELINE.json, measured 
              (pxz_shrink_batch / pxz_expand_batch: one launch per stage over a stack of frames);
 and, at N >= 2, "nccl_parity": the sharded result of a small frame equals the single-GPU result, including ranks
 without rows and a rank that fails before the exchange.  Prints ONE JSON line on rank 0.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step gave its caller for the frames whose decodes
+are still in the output buffers (one per stream) as DIR/<name>.npy (see dump_outputs).  The inputs depend on the
+arguments only, so two builds run with the same arguments can be compared file for file.
 """
 from __future__ import annotations
 
@@ -283,6 +287,42 @@ def timed_region(torch, dist, world, device, fn, reps):
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     return float(ms.item()), mine
+
+
+DUMP_BYTES = 64 << 20  # --dump-outputs writes at most this much in all
+DUMP_SEED = 0x44554D50
+
+
+def dump_outputs(out_dir: str, decoded: list, descs: list, payloads: list) -> int:
+    """Writes the encode + decode results of F frames as out_dir/<name>.npy and returns the bytes written:
+      block_offset (float64), block_value / block_width / block_height (float32)   [F, blocks]  every descriptor
+      payload_bytes (float64) [F]                                                   payload size of each frame
+      payload_sample (float32) [F, Q]       Q payload bytes at seeded positions (the same ones for equal sizes)
+      decoded_sample (float32) [F, P, C]    P decoded pixels at seeded positions (the same ones in every frame)
+    An 8K RGBA frame is 133 MB, so P and Q are chosen to keep the files within DUMP_BYTES."""
+    n = len(decoded)
+    h, w, c = decoded[0].shape
+    npx = h * w
+    n_pix = min(npx, (DUMP_BYTES // 2) // (4 * c * n))
+    n_pay = min([p.size for p in payloads] + [(DUMP_BYTES // 4) // (4 * n)])
+    pix_idx = np.sort(np.random.default_rng(DUMP_SEED).choice(npx, n_pix, replace=False))
+    arrays = {
+        "block_offset": np.stack([d["offset"] for d in descs]).astype(np.float64),
+        "block_value": np.stack([d["value"] for d in descs]).astype(np.float32),
+        "block_width": np.stack([d["w"] for d in descs]).astype(np.float32),
+        "block_height": np.stack([d["h"] for d in descs]).astype(np.float32),
+        "payload_bytes": np.array([p.size for p in payloads], np.float64),
+        "payload_sample": np.stack([p[np.sort(np.random.default_rng(DUMP_SEED).choice(p.size, n_pay, replace=False))]
+                                    for p in payloads]).astype(np.float32),
+        "decoded_sample": np.stack([img.reshape(npx, c)[pix_idx] for img in decoded]).astype(np.float32),
+    }
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes of outputs exceed {DUMP_BYTES}")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
 
 
 def run_sharded_c4(torch, dist, N, S, args, rank, world, local_rank, device):
@@ -618,6 +658,26 @@ def run_b200(args, rank: int, world: int, local_rank: int):
         elapsed_ms = ev0.elapsed_time(ev1)
         launches = captured_launches if graph is not None else sum(c.launch_count() for c in ctxs) - launches0
         clocks = sampler.stop(t_wall0, t_wall1)
+
+        # ---- --dump-outputs: the last timed step's results, before the passes below overwrite the output buffers --------
+        if args.dump_outputs and rank == 0:
+            decoded, descs_k, payloads = [], [], []
+            for k in range(n_streams):
+                i = k + (batch - 1 - k) // n_streams * n_streams  # the step's last frame on stream k: its decode is in outs[k]
+                got = outs[k].cpu().numpy()
+                # the step freed its payloads: encode the same frame again (the encode is deterministic) and require it to
+                # decode to what the timed step decoded
+                pl = wrapped[0][i % distinct].shrink(BS, BS, N.METRIC_OKLAB_MAD, FACTOR, FILTER_DOWN, 0)
+                descs, px = pl.download()
+                again = pl.expand(FILTER_UP)
+                pl.free()
+                if not np.array_equal(again, got):
+                    raise RuntimeError(f"--dump-outputs: frame {i} encoded again does not decode to the timed step's result")
+                decoded.append(got)
+                descs_k.append(descs)
+                payloads.append(px)
+            dump_outputs(args.dump_outputs, decoded, descs_k, payloads)
+            del decoded, descs_k, payloads
 
         # per-kernel durations without cross-stream overlap: the same frames on the launching stream only, CUDA events
         # around every launch (pxz_profile_*).  This pass is what the roofline of the dominant kernel is computed from.
@@ -973,7 +1033,12 @@ def main():
     ap.add_argument("--c5-images", type=int, default=4096)
     ap.add_argument("--c5-stack", type=int, default=64, help="frames per pxz_shrink_batch call")
     ap.add_argument("--extra-reps", type=int, default=2, help="timed repetitions of the C4 / C5 passes")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's results as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the b200 implementation")
     args.warmup = max(args.warmup, 0)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

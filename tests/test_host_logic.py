@@ -357,3 +357,47 @@ def test_bench_device_frames_do_not_depend_on_the_shard_layout():
             assert np.array_equal(local, S.gather_block_rows(whole, 64, idx))
             S.scatter_block_rows(local, back, 64, idx)
         assert np.array_equal(back, whole)
+
+
+def test_bench_dump_outputs_is_a_fixed_sample_within_the_budget(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 / float64 files within the byte budget, every descriptor, and pixels sampled at the
+    same positions in every frame and in every run, so that two builds can be compared file for file."""
+    import sys
+
+    if ROOT not in sys.path:
+        sys.path.insert(0, ROOT)
+    import bench
+
+    h, w, n = 96, 160, 3
+    pos = np.arange(h * w)
+    # pixel p of frame f is (p mod 256, p div 256, f, 255): a sampled pixel tells where it came from
+    frames = [np.stack([pos % 256, pos // 256, np.full(h * w, f), np.full(h * w, 255)], -1).astype(np.uint8).reshape(h, w, 4)
+              for f in range(n)]
+    rng = np.random.default_rng(6)
+    descs = []
+    for _ in range(n):
+        d = np.zeros(15, N.DESC_DTYPE)
+        d["offset"], d["value"] = np.cumsum(rng.integers(1, 1 << 20, 15)), rng.random(15, dtype=np.float32)
+        d["w"], d["h"] = rng.integers(1, 65, 15), rng.integers(1, 65, 15)
+        descs.append(d)
+    payloads = [rng.integers(0, 256, size, dtype=np.uint8) for size in (5000, 7000, 6000)]
+    monkeypatch.setattr(bench, "DUMP_BYTES", 1 << 16)
+    total = bench.dump_outputs(str(tmp_path / "a"), frames, descs, payloads)
+    bench.dump_outputs(str(tmp_path / "b"), frames, descs, payloads)
+    names = sorted(os.listdir(tmp_path / "a"))
+    assert names == sorted(os.listdir(tmp_path / "b")) and len(names) == 7
+    out = {}
+    for name in names:
+        a, b = np.load(tmp_path / "a" / name), np.load(tmp_path / "b" / name)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b), name
+        out[name[:-4]] = a
+    assert sum(a.nbytes for a in out.values()) == total <= 1 << 16
+    for field, name in (("offset", "block_offset"), ("value", "block_value"), ("w", "block_width"), ("h", "block_height")):
+        assert np.array_equal(out[name], np.stack([d[field] for d in descs]).astype(out[name].dtype)), name
+    assert out["payload_bytes"].tolist() == [5000, 7000, 6000]
+    assert out["payload_sample"].shape[0] == n and 0 < out["payload_sample"].shape[1] <= 5000
+    dec = out["decoded_sample"]
+    assert dec.shape[0] == n and 0 < dec.shape[1] < h * w and dec.shape[2] == 4
+    where = dec[..., 0] + 256 * dec[..., 1]
+    assert (np.diff(where[0]) > 0).all() and (where == where[0]).all()
+    assert (dec[..., 2] == np.arange(n)[:, None]).all() and (dec[..., 3] == 255).all()
