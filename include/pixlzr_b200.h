@@ -262,6 +262,38 @@ pxz_status pxz_payload_to_container(pxz_ctx* ctx, const pxz_payload* p, uint32_t
                                     size_t cap, uint64_t* bytes_out);
 pxz_status pxz_payload_from_container(pxz_ctx* ctx, const uint8_t* data, size_t len, int32_t* filter_byte, pxz_payload** out);
 
+/* ---- random access (EXTENSION: the reference always decodes whole images) ------------------------------------------
+ * A block's expand depends only on its descriptor, its pixels and its tile size, so a block-aligned window of an image is
+ * an ordinary pixlzr image (same trailing-tile rule at its right and bottom edges), and the container's line table lets a
+ * reader jump to any block row.  Regions are bit-identical to the same rectangle of the whole decode (DESIGN.md §3).
+ *
+ * The blocks of columns [c0, c0+nc) x rows [r0, r0+nr) of p, as a payload of the sub-image they tile: width
+ * min(W, (c0+nc)*bw) - c0*bw, height likewise, same block size and channels.  Descriptors (value, w, h) are copied, block
+ * pixels copied and re-packed densely in row-major window order; per-block expand filters (strategy) and resize tables are
+ * kept.  The result is an ordinary payload, independent of p: every call that takes a payload takes it.
+ * PXZ_E_ARG: empty or out-of-grid window.  PXZ_E_UNSUPPORTED: a batch payload. */
+pxz_status pxz_payload_window(pxz_ctx* ctx, const pxz_payload* p, uint32_t c0, uint32_t r0, uint32_t nc, uint32_t nr,
+                              pxz_payload** out);
+/* Pixels [x, x+w) x [y, y+h) of the decoded image, bit-identical to that rectangle of pxz_expand_to_image(p, filter_up)
+ * (with pxz_ctx_set_fast_resample(1): within +-1 LSB, since a small window may run the other resample kernel family);
+ * only the blocks the rectangle touches are read and resampled.  out: w x h, p's channels, not a batch.
+ * PXZ_E_ARG: empty rectangle, rectangle outside the image, output geometry mismatch.  PXZ_E_UNSUPPORTED: a batch payload. */
+pxz_status pxz_expand_region(pxz_ctx* ctx, const pxz_payload* p, pxz_filter filter_up, uint32_t x, uint32_t y, uint32_t w,
+                             uint32_t h, pxz_image* out);
+/* Header only: dimensions, block size, filter byte (-1 if absent); checks the line table against len.  O(rows). */
+pxz_status pxz_container_header(const uint8_t* data, size_t len, uint32_t* w, uint32_t* h, uint32_t* bw, uint32_t* bh,
+                                int32_t* filter_byte);
+/* The .pxlzr file of the block window (c0, r0, nc, nr) of the image in `data`, without decoding: header with the window's
+ * size, a new line table, the window's block records copied verbatim.  Reads the header, the line table and the block
+ * headers of rows r0 .. r0+nr-1 only; every record of those rows is checked as pxz_container_decode checks it, and each
+ * row against its line-table entry.  Consequence: a file that is corrupt only outside the window still crops (and its
+ * crop decodes), while pxz_container_decode refuses the whole file.  cap >= len always suffices; out == NULL writes
+ * nothing and returns the size of the cropped file.  Byte-identical to the file of the same window written from a payload
+ * (pxz_payload_window + pxz_payload_to_container).  Returns the bytes written, or a negative pxz_status: PXZ_E_ARG for an
+ * empty or out-of-grid window or a too small `cap`, PXZ_E_FORMAT / PXZ_E_UNSUPPORTED as pxz_container_decode. */
+int64_t pxz_container_crop(const uint8_t* data, size_t len, uint32_t c0, uint32_t r0, uint32_t nc, uint32_t nr, uint8_t* out,
+                           size_t cap);
+
 #ifdef __cplusplus
 }
 #endif

@@ -82,6 +82,10 @@ SYMBOLS = {
     "pxz_payload_from_container": (_i, [_vp, _vp, _sz, _P(C.c_int32), _P(_vp)]),
     "pxz_container_decode": (_i, [_vp, _sz, _P(_u32), _P(_u32), _P(_u32), _P(_u32), _P(C.c_int32), _P(_u32),
                                   _P(_u64), _vp, _vp]),
+    "pxz_payload_window": (_i, [_vp, _vp, _u32, _u32, _u32, _u32, _P(_vp)]),
+    "pxz_expand_region": (_i, [_vp, _vp, _i, _u32, _u32, _u32, _u32, _vp]),
+    "pxz_container_header": (_i, [_vp, _sz, _P(_u32), _P(_u32), _P(_u32), _P(_u32), _P(C.c_int32)]),
+    "pxz_container_crop": (C.c_int64, [_vp, _sz, _u32, _u32, _u32, _u32, _vp, _sz]),
 }
 
 
@@ -427,6 +431,26 @@ class Payload:
     def expand_to_image(self, filter_up: int, out: Image):
         self.ctx.check(lib().pxz_expand_to_image(self.ctx.handle, self._h, int(filter_up), out.handle))
 
+    # ---- random access (extension) -----------------------------------------------------------------------
+    def window(self, c0: int, r0: int, nc: int, nr: int) -> "Payload":
+        """The blocks of columns [c0, c0+nc) x rows [r0, r0+nr) as a payload of their own (pxz_payload_window)."""
+        h = C.c_void_p()
+        self.ctx.check(lib().pxz_payload_window(self.ctx.handle, self._h, c0, r0, nc, nr, C.byref(h)))
+        return Payload(self.ctx, h)
+
+    def expand_region_to_image(self, filter_up: int, x: int, y: int, w: int, h: int, out: Image):
+        """Pixels [x, x+w) x [y, y+h) of the decoded image into `out` (w x h), e.g. an image_wrap'ped torch tensor."""
+        self.ctx.check(lib().pxz_expand_region(self.ctx.handle, self._h, int(filter_up), x, y, w, h, out.handle))
+
+    def expand_region(self, filter_up: int, x: int, y: int, w: int, h: int) -> np.ndarray:
+        """[h, w, c]: pixels [x, x+w) x [y, y+h) of expand(filter_up), resampling only the blocks they touch."""
+        img = self.ctx.image_alloc(w, h, self.info()["channels"])  # an empty rectangle fails here with PXZ_E_ARG
+        try:
+            self.expand_region_to_image(filter_up, x, y, w, h, img)
+            return img.download()
+        finally:
+            img.free()
+
     def free(self):
         if self._h:
             lib().pxz_payload_free(self._h)
@@ -514,3 +538,29 @@ def container_decode(data: bytes):
         raise PixlzrError(st, "malformed .pxlzr container")
     hdr = dict(w=w.value, h=h.value, bw=bw.value, bh=bh.value, filter=filt.value, channels=ch.value)
     return hdr, descs, pixels[:nbytes.value]
+
+
+def container_header(data) -> dict:
+    """{w, h, bw, bh, filter} of a .pxlzr file without reading its blocks (pxz_container_header).  `data`: any buffer
+    (bytes, mmap, ...); only the header and the line table are read."""
+    buf = np.frombuffer(data, np.uint8)
+    w, h, bw, bh = (C.c_uint32() for _ in range(4))
+    filt = C.c_int32()
+    st = lib().pxz_container_header(ptr(buf), buf.size, C.byref(w), C.byref(h), C.byref(bw), C.byref(bh), C.byref(filt))
+    if st != OK:
+        raise PixlzrError(st, "malformed .pxlzr container")
+    return dict(w=w.value, h=h.value, bw=bw.value, bh=bh.value, filter=filt.value)
+
+
+def container_crop(data, c0: int, r0: int, nc: int, nr: int) -> bytes:
+    """The .pxlzr file of the block window (c0, r0, nc, nr) of the file in `data` (any buffer: an mmap of a large file is
+    read only in the header, the line table and the window's block rows), without decoding (pxz_container_crop)."""
+    buf = np.frombuffer(data, np.uint8)
+    n = lib().pxz_container_crop(ptr(buf), buf.size, c0, r0, nc, nr, None, 0)
+    if n < 0:
+        raise PixlzrError(int(n), "pxz_container_crop")
+    out = np.empty(max(1, n), np.uint8)
+    n = lib().pxz_container_crop(ptr(buf), buf.size, c0, r0, nc, nr, ptr(out), out.size)
+    if n < 0:
+        raise PixlzrError(int(n), "pxz_container_crop")
+    return out[:n].tobytes()

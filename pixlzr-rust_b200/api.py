@@ -109,6 +109,20 @@ def _check_image(image: np.ndarray) -> np.ndarray:
     return np.ascontiguousarray(image)
 
 
+def _check_rect(width: int, height: int, x: int, y: int, w: int, h: int) -> None:
+    """The rectangle errors of pxz_expand_region, raised before anything is read or uploaded."""
+    if w <= 0 or h <= 0:
+        raise N.PixlzrError(N.E_ARG, "empty rectangle")
+    if x < 0 or y < 0 or x + w > width or y + h > height:
+        raise N.PixlzrError(N.E_ARG, "rectangle outside the image")
+
+
+def _touched_blocks(bw: int, bh: int, x: int, y: int, w: int, h: int) -> Tuple[int, int, int, int]:
+    """(c0, r0, nc, nr): the block window a pixel rectangle touches."""
+    c0, r0 = x // bw, y // bh
+    return c0, r0, (x + w - 1) // bw - c0 + 1, (y + h - 1) // bh - r0 + 1
+
+
 @dataclass
 class Strategy:
     """(down, up) filter per value bucket of width 1/64 (pxz_strategy, include/pixlzr_b200.h).  The bucket of a block
@@ -359,6 +373,28 @@ class Pixlzr:
         finally:
             pl.free()
 
+    def to_image_region(self, filter: FilterType, x: int, y: int, w: int, h: int) -> np.ndarray:
+        """EXTENSION (random access): to_image(filter)[y:y+h, x:x+w], bit for bit; only the blocks the rectangle touches
+        are uploaded and resampled."""
+        _check_rect(self.width, self.height, x, y, w, h)
+        if self._image is not None:
+            return self._image[y:y + h, x:x + w].copy()
+        c0, r0, nc, nr = _touched_blocks(self.block_width, self.block_height, x, y, w, h)
+        cols = self.block_grid_width()
+        idx = ((r0 + np.arange(nr))[:, None] * cols + (c0 + np.arange(nc))[None, :]).reshape(-1)
+        descs = self._descs[idx].copy()
+        sizes = descs["w"].astype(np.int64) * descs["h"] * self._channels
+        descs["offset"] = np.concatenate([[0], np.cumsum(sizes)[:-1]])
+        pixels = np.concatenate([self._pixels[o:o + n] for o, n in zip(self._descs["offset"][idx].tolist(), sizes.tolist())])
+        x0, y0 = c0 * self.block_width, r0 * self.block_height
+        ww = min(self.width, (c0 + nc) * self.block_width) - x0
+        wh = min(self.height, (r0 + nr) * self.block_height) - y0
+        pl = self._ctx().payload_upload(ww, wh, self.block_width, self.block_height, self._channels, descs, pixels)
+        try:
+            return pl.expand_region(int(filter), x - x0, y - y0, w, h)
+        finally:
+            pl.free()
+
     def expand(self, filter: FilterType) -> "Pixlzr":
         """Pixlzr::expand (pixlzr.rs:77-122): every block resized to its full tile size."""
         out = Pixlzr.from_image(self.to_image(filter), self.block_width, self.block_height, self.ctx)
@@ -413,6 +449,22 @@ class Pixlzr:
         pl, _ = ctx.payload_from_container(data)
         try:
             return pl.expand(int(filter))
+        finally:
+            pl.free()
+
+    @staticmethod
+    def decode_vec_region_to_image(data, filter: FilterType, x: int, y: int, w: int, h: int,
+                                   ctx: Optional[N.Context] = None) -> np.ndarray:
+        """EXTENSION (random access): pixels [x, x+w) x [y, y+h) of decode_vec_to_image(data, filter), bit for bit.  Only
+        the block rows the rectangle touches are read; the touched blocks are cut out of the file without decoding
+        (pxz_container_crop), and only that file crosses PCIe.  `data`: bytes or any buffer, e.g. an mmap of the file."""
+        hdr = N.container_header(data)
+        _check_rect(hdr["w"], hdr["h"], x, y, w, h)
+        c0, r0, nc, nr = _touched_blocks(hdr["bw"], hdr["bh"], x, y, w, h)
+        ctx = ctx or default_context()
+        pl, _ = ctx.payload_from_container(N.container_crop(data, c0, r0, nc, nr))
+        try:
+            return pl.expand_region(int(filter), x - c0 * hdr["bw"], y - r0 * hdr["bh"], w, h)
         finally:
             pl.free()
 

@@ -36,7 +36,29 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("-d", "--direction-wise", type=lambda s: {"true": True, "false": False}[s.lower()], default=None,
                    metavar="true|false", help="Direction-wise scan")
     p.add_argument("--force", action="store_true", help="If image-2-image, force shrinking?")
+    # extension (random access): not a flag of the reference
+    p.add_argument("--region", type=parse_region, default=None, metavar="X,Y,W,H",
+                   help="Decode only this pixel rectangle (.pix / .pixlzr -> image only)")
     return p
+
+
+def parse_region(s: str) -> Tuple[int, int, int, int]:
+    parts = s.split(",")
+    try:
+        x, y, w, h = (int(v) for v in parts)
+    except ValueError:
+        raise argparse.ArgumentTypeError(f"expected X,Y,W,H (four integers), got {s!r}") from None
+    if x < 0 or y < 0 or w <= 0 or h <= 0:
+        raise argparse.ArgumentTypeError(f"expected X, Y >= 0 and W, H > 0, got {s!r}")
+    return x, y, w, h
+
+
+def region_error(args) -> Optional[str]:
+    """Why --region does not apply to this conversion, or None."""
+    if args.region is not None and operation(args.input, args.output) != ("pix", "image"):
+        return "--region decodes a rectangle of a .pix / .pixlzr file into an image: the input must be a container and the " \
+               "output an image"
+    return None
 
 
 def parse_args(argv: Optional[List[str]] = None):
@@ -93,6 +115,13 @@ def run(args) -> None:
     filt = FILTERS[args.filter]
     shrink_by = api.parse_shrinking_factor(args.shrinking_factor)
     src, dst = operation(args.input, args.output)
+    err = region_error(args)
+    if err:
+        raise ValueError(err)
+    if args.region is not None and not (args.force and args.direction_wise):
+        with open(args.input, "rb") as f:
+            _save_image(args.output, api.Pixlzr.decode_vec_region_to_image(f.read(), filt, *args.region))
+        return
     # the two plain conversions run with the container stage on the device (same bytes / pixels as the general path)
     if src == "image" and dst == "pix" and args.force:
         with open(args.output, "wb") as f:
@@ -114,12 +143,18 @@ def run(args) -> None:
     _maybe_shrink(pix, args, shrink_by)
     if dst == "pix":
         pix.save(args.output)
+    elif args.region is not None:
+        _save_image(args.output, pix.to_image_region(filt, *args.region))
     else:
         _save_image(args.output, pix.to_image(filt))
 
 
 def main(argv: Optional[List[str]] = None) -> int:
     args = parse_args(argv)
+    err = region_error(args)
+    if err:
+        print(f"pixlzr: {err}", file=sys.stderr)
+        return 2
     try:
         run(args)
     except FileNotFoundError as e:

@@ -45,10 +45,12 @@ struct TabSet {  // device copy of the axis tables of one (spec, filter, directi
 
 using TabKey = std::tuple<std::vector<uint32_t>, std::vector<uint32_t>, int, int>;
 
-enum KernelId { K_MAD_FAST = 0, K_MAD_EXACT, K_SOBEL, K_MINMAX, K_PLAN, K_RESAMPLE_DOWN, K_RESAMPLE_UP, K_QOI_ENCODE, K_QOI_DECODE, K_COUNT };
-const char* const kKernelNames[K_COUNT] = {"analyze_mad_fast", "mad_exact",     "analyze_sobel", "minmax",
-                                           "plan",             "resample_down", "resample_up",   "qoi_encode",
-                                           "qoi_decode"};
+// K_REGION_COPY times the device-to-device copy of pxz_expand_region out of its staging image (not a kernel)
+enum KernelId { K_MAD_FAST = 0, K_MAD_EXACT, K_SOBEL, K_MINMAX, K_PLAN, K_RESAMPLE_DOWN, K_RESAMPLE_UP, K_QOI_ENCODE, K_QOI_DECODE,
+                K_PAYLOAD_WINDOW, K_REGION_COPY, K_COUNT };
+const char* const kKernelNames[K_COUNT] = {"analyze_mad_fast", "mad_exact",      "analyze_sobel", "minmax",
+                                           "plan",             "resample_down",  "resample_up",   "qoi_encode",
+                                           "qoi_decode",       "payload_window", "region_copy"};
 struct ProfRec {
   int id;
   cudaEvent_t a, b;
@@ -214,7 +216,8 @@ void dev_free(pxz_ctx* ctx, void* p) {
   if (p) cudaFreeAsync(p, ctx->stream);
 }
 
-pxz_status ensure_scratch(pxz_ctx* ctx, uint32_t nblocks) {
+// scan_bytes: the scan state the next plan / window launch needs (0: launch_plan's for nblocks)
+pxz_status ensure_scratch(pxz_ctx* ctx, uint32_t nblocks, size_t scan_bytes = 0) {
   if (ctx->values_cap < nblocks) {
     dev_free(ctx, ctx->d_vx);
     dev_free(ctx, ctx->d_vy);
@@ -231,7 +234,7 @@ pxz_status ensure_scratch(pxz_ctx* ctx, uint32_t nblocks) {
     if ((st = dev_alloc(ctx, (void**)&ctx->d_list, ((size_t)nblocks + 1) * 4)) != PXZ_OK) return st;
     ctx->values_cap = nblocks;
   }
-  const size_t need = plan_scan_state_bytes(nblocks);
+  const size_t need = scan_bytes ? scan_bytes : plan_scan_state_bytes(nblocks);
   if (ctx->scan_cap < need) {
     dev_free(ctx, ctx->d_scan);
     ctx->d_scan = nullptr;
@@ -857,8 +860,11 @@ static pxz_status payload_rechannel(pxz_ctx* ctx, const pxz_payload* src, uint32
   const uint32_t sc = g.C;
   g.C = dc;
   const uint32_t nblocks = g.cols * g.rows;
+  // k_payload_convert writes each block at offset / sc * dc.  Uploaded payloads may hold blocks larger than their tiles, so
+  // W * H * dc does not bound that; every block lies inside src->capacity (payload_from_descs checks it).
+  const uint64_t cap = std::max<uint64_t>((uint64_t)g.W * g.H * dc * g.nimg, (src->capacity + sc - 1) / sc * dc);
   pxz_payload* p = nullptr;
-  pxz_status st = payload_new(ctx, g, (uint64_t)g.W * g.H * dc * g.nimg, &p);
+  pxz_status st = payload_new(ctx, g, cap, &p);
   if (st != PXZ_OK) return st;
   p->spec = src->spec;
   p->strategy = src->strategy;
@@ -1383,6 +1389,89 @@ pxz_status pxz_expand(pxz_ctx* ctx, const pxz_payload* p, pxz_filter filter_up, 
   st = pxz_expand_to_image(ctx, p, filter_up, im);
   if (st == PXZ_OK) st = pxz_image_download(ctx, im, host_out, host_pitch);
   pxz_image_free(im);
+  return st;
+}
+
+// ---- random access (extension) ------------------------------------------------------------------------------------
+// A block's expand reads only its descriptor, its pixels and its tile size, so the blocks of a window, given the tile
+// sizes they have in the whole image, are an ordinary payload whose expand is that window of the whole expand.
+pxz_status pxz_payload_window(pxz_ctx* ctx, const pxz_payload* p, uint32_t c0, uint32_t r0, uint32_t nc, uint32_t nr,
+                              pxz_payload** out) {
+  if (!ctx || !p || !out) return PXZ_E_ARG;
+  *out = nullptr;
+  cudaSetDevice(ctx->device);
+  const Geom& pg = p->g;
+  if (pg.nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "windows of a batch payload are not supported");
+  if (nc == 0 || nr == 0 || c0 >= pg.cols || r0 >= pg.rows || nc > pg.cols - c0 || nr > pg.rows - r0)
+    return fail(ctx, PXZ_E_ARG, "empty or out-of-grid window");
+  const uint32_t w = (uint32_t)(std::min<uint64_t>(pg.W, (uint64_t)(c0 + nc) * pg.bw) - (uint64_t)c0 * pg.bw);
+  const uint32_t h = (uint32_t)(std::min<uint64_t>(pg.H, (uint64_t)(r0 + nr) * pg.bh) - (uint64_t)r0 * pg.bh);
+  Geom g;
+  pxz_status st = make_geom(ctx, w, h, pg.C, pg.bw, pg.bh, &g);
+  if (st != PXZ_OK) return st;
+  const uint32_t nblocks = nc * nr;
+  if ((st = ensure_scratch(ctx, nblocks, window_scan_state_bytes(nblocks))) != PXZ_OK) return st;
+  // max_small_px bounds every block of p, whatever made it (uploads may hold blocks larger than their tiles); the parent's
+  // capacity alone could be the whole gigapixel frame
+  const uint64_t capacity = std::min<uint64_t>(p->capacity, (uint64_t)nblocks * p->max_small_px * pg.C);
+  pxz_payload* wp = nullptr;
+  if ((st = payload_new(ctx, g, capacity, &wp)) != PXZ_OK) return st;
+  // the window's table indices are the parent's: same spec, same bounds, same kernel family
+  wp->spec = p->spec;
+  wp->strategy = p->strategy;
+  wp->max_small_px = p->max_small_px; wp->max_small_dim = p->max_small_dim;
+  wp->max_tmp_down = p->max_tmp_down; wp->max_tmp_up = p->max_tmp_up;
+  cudaError_t e;
+  {
+    ProfScope prof(ctx, K_PAYLOAD_WINDOW);
+    e = launch_payload_window(p->d_descs, p->d_tabidx, (uint32_t)p->nblocks_cap, p->d_pixels, pg.cols, c0, r0, g, p->strategy == 1,
+                              wp->d_descs, wp->d_tabidx, (uint32_t)wp->nblocks_cap, wp->d_pixels, wp->d_total, ctx->d_scan, ctx->stream,
+                              &ctx->launches);
+  }
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    payload_release(wp);
+    return fail(ctx, PXZ_E_CUDA, std::string("payload window: ") + cudaGetErrorString(e));
+  }
+  *out = wp;
+  return PXZ_OK;
+}
+
+pxz_status pxz_expand_region(pxz_ctx* ctx, const pxz_payload* p, pxz_filter filter_up, uint32_t x, uint32_t y, uint32_t w,
+                             uint32_t h, pxz_image* out) {
+  if (!ctx || !p || !out) return PXZ_E_ARG;
+  cudaSetDevice(ctx->device);
+  const Geom& pg = p->g;
+  if (pg.nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "regions of a batch payload are not supported");
+  if ((int)filter_up < 0 || (int)filter_up > 4) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (w == 0 || h == 0) return fail(ctx, PXZ_E_ARG, "empty rectangle");
+  if (x >= pg.W || y >= pg.H || w > pg.W - x || h > pg.H - y) return fail(ctx, PXZ_E_ARG, "rectangle outside the image");
+  if (out->w != w || out->h != h || out->c != pg.C || out->nimg != 1) return fail(ctx, PXZ_E_ARG, "output image geometry mismatch");
+  if (x == 0 && y == 0 && w == pg.W && h == pg.H) return pxz_expand_to_image(ctx, p, filter_up, out);
+  const uint32_t c0 = x / pg.bw, r0 = y / pg.bh;
+  const uint32_t nc = (x + w - 1) / pg.bw - c0 + 1, nr = (y + h - 1) / pg.bh - r0 + 1;
+  pxz_payload* wp = nullptr;
+  pxz_status st = pxz_payload_window(ctx, p, c0, r0, nc, nr, &wp);
+  if (st != PXZ_OK) return st;
+  const uint32_t dx = x - c0 * pg.bw, dy = y - r0 * pg.bh;
+  if (dx == 0 && dy == 0 && w == wp->g.W && h == wp->g.H) {
+    st = pxz_expand_to_image(ctx, wp, filter_up, out);  // the rectangle is the window: no staging
+  } else {
+    pxz_image* stage = nullptr;
+    st = pxz_image_alloc(ctx, wp->g.W, wp->g.H, pg.C, &stage);
+    if (st == PXZ_OK) st = pxz_expand_to_image(ctx, wp, filter_up, stage);
+    if (st == PXZ_OK) {
+      ProfScope prof(ctx, K_REGION_COPY);
+      const cudaError_t e = cudaMemcpy2DAsync(out->d, out->pitch, stage->d + (size_t)dy * stage->pitch + (size_t)dx * pg.C, stage->pitch,
+                                              (size_t)w * pg.C, h, cudaMemcpyDeviceToDevice, ctx->stream);
+      if (e != cudaSuccess) {
+        cudaGetLastError();
+        st = fail(ctx, PXZ_E_CUDA, std::string("region copy: ") + cudaGetErrorString(e));
+      }
+    }
+    pxz_image_free(stage);  // stream-ordered: the copy queued above keeps it
+  }
+  payload_release(wp);
   return st;
 }
 

@@ -153,6 +153,71 @@ inline uint32_t grid_f32(uint32_t n, uint32_t b) {  // pixlzr.rs:37-42, encoding
 constexpr size_t kHeader = 26;      // constants.rs:19-20
 constexpr size_t kBlockHeader = 13; // "block" + f32 + u32
 
+struct FileHeader {
+  uint32_t w, h, bw, bh, cols, rows;
+  int32_t filt;       // -1 if absent
+  size_t line_table;  // offset of the line table
+  size_t body;        // offset of the first block record
+};
+
+// The file header and the line table's total (encoding/mod.rs:95-141): O(rows), no block record is read.
+pxz_status read_header(const uint8_t* data, size_t len, FileHeader* hd) {
+  if (len < 9 || memcmp(data, "PIXLZR", 6) != 0) return PXZ_E_FORMAT;  // encoding/mod.rs:99-104
+  const uint32_t version = (uint32_t)data[6] << 16 | (uint32_t)data[7] << 8 | data[8];
+  size_t p = 9;
+  hd->filt = -1;
+  if (version >= 1) {  // "filter" since 0.0.1 (encoding/mod.rs:16-19,109-111)
+    if (len < p + 1) return PXZ_E_FORMAT;
+    hd->filt = data[p++];
+  }
+  if (version < 2) return PXZ_E_UNSUPPORTED;  // "line-sizes" since 0.0.2; the reference cannot read older files either
+  if (len < p + 16) return PXZ_E_FORMAT;
+  hd->w = rd32(data + p); hd->h = rd32(data + p + 4); hd->bw = rd32(data + p + 8); hd->bh = rd32(data + p + 12);
+  p += 16;
+  if (hd->bw == 0 || hd->bh == 0 || hd->w == 0 || hd->h == 0) return PXZ_E_FORMAT;
+  hd->cols = grid_f32(hd->w, hd->bw);
+  hd->rows = grid_f32(hd->h, hd->bh);
+  // the reference sizes the grid in f32 (encoding/mod.rs:118-119), the device side in integers: the two agree below
+  // 2^24; a file for which they differ is refused instead of being walked with two different block counts
+  if ((uint64_t)hd->cols != ((uint64_t)hd->w + hd->bw - 1) / hd->bw || (uint64_t)hd->rows != ((uint64_t)hd->h + hd->bh - 1) / hd->bh)
+    return PXZ_E_UNSUPPORTED;
+  if ((uint64_t)hd->cols * hd->rows > 0x7FFFFFFFull) return PXZ_E_UNSUPPORTED;
+  if (len < p + (size_t)hd->rows * 4) return PXZ_E_FORMAT;
+  hd->line_table = p;
+  uint64_t body = 0;
+  for (uint32_t r = 0; r < hd->rows; ++r) body += rd32(data + p + (size_t)r * 4);
+  hd->body = p + (size_t)hd->rows * 4;
+  if (hd->body + body != len) return PXZ_E_FORMAT;  // assert_eq!(reader.data.len(), ...), encoding/mod.rs:141
+  return PXZ_OK;
+}
+
+struct BlockRecord {
+  float value;
+  uint32_t qlen, qw, qh;  // QOI body length (after the 13-byte record header) and size
+};
+
+// Checks the block record at data[p] ("block" | value | qoi_len | QOI stream minus its magic): magic, lengths, the QOI
+// header and hostile sizes.  *ch: the file's channel count, 0 until the first record sets it.
+pxz_status read_block_record(const uint8_t* data, size_t len, size_t p, uint32_t* ch, BlockRecord* rec) {
+  if (p + kBlockHeader + 10 > len || memcmp(data + p, "block", 5) != 0) return PXZ_E_FORMAT;
+  const uint32_t bits = rd32(data + p + 5);
+  memcpy(&rec->value, &bits, 4);
+  rec->qlen = rd32(data + p + 9);
+  p += kBlockHeader;
+  if (p + rec->qlen > len || rec->qlen < 18) return PXZ_E_FORMAT;
+  rec->qw = rd32(data + p);
+  rec->qh = rd32(data + p + 4);
+  const uint32_t qc = data[p + 8];
+  if (qc != 3 && qc != 4) return PXZ_E_FORMAT;
+  if (*ch == 0) *ch = qc;
+  if (qc != *ch) return PXZ_E_UNSUPPORTED;  // mixed RGB / RGBA blocks in one file
+  if (rec->qw > 65535 || rec->qh > 65535 || rec->qw == 0 || rec->qh == 0) return PXZ_E_UNSUPPORTED;
+  // hostile headers: the qoi crate refuses more than 400 M pixels, and an op byte yields at most 62 pixels (a run),
+  // so a stream of qlen bytes cannot fill more than 62 * qlen of them — checked before anything is allocated
+  if ((uint64_t)rec->qw * rec->qh > 400000000ull || (uint64_t)rec->qw * rec->qh > 62ull * rec->qlen) return PXZ_E_FORMAT;
+  return PXZ_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -227,69 +292,95 @@ pxz_status pxz_container_decode(const uint8_t* data, size_t len, uint32_t* w, ui
                                 int32_t* filter_byte, uint32_t* channels, uint64_t* payload_bytes, pxz_block_desc* descs,
                                 uint8_t* pixels) {
   if (!data || !w || !h || !bw || !bh || !channels || !payload_bytes) return PXZ_E_ARG;
-  if (len < 9 || memcmp(data, "PIXLZR", 6) != 0) return PXZ_E_FORMAT;  // encoding/mod.rs:99-104
-  const uint32_t version = (uint32_t)data[6] << 16 | (uint32_t)data[7] << 8 | data[8];
-  size_t p = 9;
-  int32_t filt = -1;
-  if (version >= 1) {  // "filter" since 0.0.1 (encoding/mod.rs:16-19,109-111)
-    if (len < p + 1) return PXZ_E_FORMAT;
-    filt = data[p++];
-  }
-  if (version < 2) return PXZ_E_UNSUPPORTED;  // "line-sizes" since 0.0.2; the reference cannot read older files either
-  if (len < p + 16) return PXZ_E_FORMAT;
-  *w = rd32(data + p); *h = rd32(data + p + 4); *bw = rd32(data + p + 8); *bh = rd32(data + p + 12);
-  p += 16;
-  if (filter_byte) *filter_byte = filt;
-  if (*bw == 0 || *bh == 0 || *w == 0 || *h == 0) return PXZ_E_FORMAT;
-  const uint32_t cols = grid_f32(*w, *bw), rows = grid_f32(*h, *bh);
-  // the reference sizes the grid in f32 (encoding/mod.rs:118-119), the device side in integers: the two agree below
-  // 2^24; a file for which they differ is refused instead of being walked with two different block counts
-  if ((uint64_t)cols != ((uint64_t)*w + *bw - 1) / *bw || (uint64_t)rows != ((uint64_t)*h + *bh - 1) / *bh) return PXZ_E_UNSUPPORTED;
-  if ((uint64_t)cols * rows > 0x7FFFFFFFull) return PXZ_E_UNSUPPORTED;
-  if (len < p + (size_t)rows * 4) return PXZ_E_FORMAT;
-  const size_t line_table = p;
-  uint64_t body = 0;
-  for (uint32_t r = 0; r < rows; ++r) body += rd32(data + p + (size_t)r * 4);
-  p += (size_t)rows * 4;
-  if (p + body != len) return PXZ_E_FORMAT;  // assert_eq!(reader.data.len(), ...), encoding/mod.rs:141
+  FileHeader hd;
+  pxz_status st = read_header(data, len, &hd);
+  if (st != PXZ_OK) return st;
+  *w = hd.w; *h = hd.h; *bw = hd.bw; *bh = hd.bh;
+  if (filter_byte) *filter_byte = hd.filt;
+  const uint32_t cols = hd.cols, rows = hd.rows;
+  size_t p = hd.body;
   uint64_t off = 0;
   uint32_t ch = 0;
   size_t row_start = p;
   for (size_t bi = 0; bi < (size_t)cols * rows; ++bi) {
     if (bi && bi % cols == 0) {
       // every block row fills exactly its entry of the line table (encoding/mod.rs:142-155 slices the rows by it)
-      if (p - row_start != rd32(data + line_table + (bi / cols - 1) * 4)) return PXZ_E_FORMAT;
+      if (p - row_start != rd32(data + hd.line_table + (bi / cols - 1) * 4)) return PXZ_E_FORMAT;
       row_start = p;
     }
-    if (p + kBlockHeader + 10 > len || memcmp(data + p, "block", 5) != 0) return PXZ_E_FORMAT;
-    uint32_t bits = rd32(data + p + 5);
-    float v;
-    memcpy(&v, &bits, 4);
-    const uint32_t qlen = rd32(data + p + 9);
+    BlockRecord rec;
+    if ((st = read_block_record(data, len, p, &ch, &rec)) != PXZ_OK) return st;
     p += kBlockHeader;
-    if (p + qlen > len || qlen < 18) return PXZ_E_FORMAT;
-    const uint32_t qw = rd32(data + p), qh = rd32(data + p + 4), qc = data[p + 8];
-    if (qc != 3 && qc != 4) return PXZ_E_FORMAT;
-    if (ch == 0) ch = qc;
-    if (qc != ch) return PXZ_E_UNSUPPORTED;  // mixed RGB / RGBA blocks in one file
-    if (qw > 65535 || qh > 65535 || qw == 0 || qh == 0) return PXZ_E_UNSUPPORTED;
-    // hostile headers: the qoi crate refuses more than 400 M pixels, and an op byte yields at most 62 pixels (a run),
-    // so a stream of qlen bytes cannot fill more than 62 * qlen of them — checked before anything is allocated
-    if ((uint64_t)qw * qh > 400000000ull || (uint64_t)qw * qh > 62ull * qlen) return PXZ_E_FORMAT;
     if (descs) {
       descs[bi].offset = off;
-      descs[bi].value = v;
-      descs[bi].w = (uint16_t)qw;
-      descs[bi].h = (uint16_t)qh;
-      if (pixels && !qoi_body_decode(data + p, qlen, ch, pixels + off, (size_t)qw * qh)) return PXZ_E_FORMAT;
+      descs[bi].value = rec.value;
+      descs[bi].w = (uint16_t)rec.qw;
+      descs[bi].h = (uint16_t)rec.qh;
+      if (pixels && !qoi_body_decode(data + p, rec.qlen, ch, pixels + off, (size_t)rec.qw * rec.qh)) return PXZ_E_FORMAT;
     }
-    off += (uint64_t)qw * qh * qc;
-    p += qlen;
+    off += (uint64_t)rec.qw * rec.qh * ch;
+    p += rec.qlen;
   }
-  if (p - row_start != rd32(data + line_table + (size_t)(rows - 1) * 4)) return PXZ_E_FORMAT;
+  if (p - row_start != rd32(data + hd.line_table + (size_t)(rows - 1) * 4)) return PXZ_E_FORMAT;
   *channels = ch;
   *payload_bytes = off;
   return PXZ_OK;
+}
+
+pxz_status pxz_container_header(const uint8_t* data, size_t len, uint32_t* w, uint32_t* h, uint32_t* bw, uint32_t* bh,
+                                int32_t* filter_byte) {
+  if (!data || !w || !h || !bw || !bh) return PXZ_E_ARG;
+  FileHeader hd;
+  const pxz_status st = read_header(data, len, &hd);
+  if (st != PXZ_OK) return st;
+  *w = hd.w; *h = hd.h; *bw = hd.bw; *bh = hd.bh;
+  if (filter_byte) *filter_byte = hd.filt;
+  return PXZ_OK;
+}
+
+int64_t pxz_container_crop(const uint8_t* data, size_t len, uint32_t c0, uint32_t r0, uint32_t nc, uint32_t nr, uint8_t* out,
+                           size_t cap) {
+  if (!data) return PXZ_E_ARG;
+  FileHeader hd;
+  pxz_status st = read_header(data, len, &hd);
+  if (st != PXZ_OK) return st;
+  if (nc == 0 || nr == 0 || c0 >= hd.cols || r0 >= hd.rows || nc > hd.cols - c0 || nr > hd.rows - r0) return PXZ_E_ARG;
+  // rows before the window are skipped by their line-table entries; the rows of the window are walked record by record
+  size_t p = hd.body;
+  for (uint32_t r = 0; r < r0; ++r) p += rd32(data + hd.line_table + (size_t)r * 4);
+  const size_t head = kHeader + (size_t)nr * 4;
+  if (out && head > cap) return PXZ_E_ARG;
+  size_t o = head;
+  uint32_t ch = 0;
+  for (uint32_t r = r0; r < r0 + nr; ++r) {
+    const size_t row_start = p;
+    size_t sel0 = p, sel1 = p;  // bytes of the records c0 .. c0 + nc - 1
+    for (uint32_t c = 0; c < hd.cols; ++c) {
+      if (c == c0) sel0 = p;
+      BlockRecord rec;
+      if ((st = read_block_record(data, len, p, &ch, &rec)) != PXZ_OK) return st;
+      p += kBlockHeader + rec.qlen;
+      if (c + 1 == c0 + nc) sel1 = p;
+    }
+    if (p - row_start != rd32(data + hd.line_table + (size_t)r * 4)) return PXZ_E_FORMAT;
+    const size_t n = sel1 - sel0;
+    if (out) {
+      if (o + n > cap) return PXZ_E_ARG;
+      memcpy(out + o, data + sel0, n);
+      be32(out + kHeader + (size_t)(r - r0) * 4, (uint32_t)n);
+    }
+    o += n;
+  }
+  if (out) {
+    memcpy(out, "PIXLZR", 6);
+    out[6] = 0; out[7] = 0; out[8] = 2;
+    out[9] = (uint8_t)hd.filt;  // present from version 0.0.1 on
+    be32(out + 10, (uint32_t)(std::min<uint64_t>(hd.w, (uint64_t)(c0 + nc) * hd.bw) - (uint64_t)c0 * hd.bw));
+    be32(out + 14, (uint32_t)(std::min<uint64_t>(hd.h, (uint64_t)(r0 + nr) * hd.bh) - (uint64_t)r0 * hd.bh));
+    be32(out + 18, hd.bw);
+    be32(out + 22, hd.bh);
+  }
+  return (int64_t)o;
 }
 
 }  // extern "C"

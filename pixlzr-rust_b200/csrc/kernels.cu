@@ -1077,6 +1077,48 @@ struct ScanState {
   unsigned long long status[1];  // [num_tiles]: flag << 62 | value ; flag 1 = aggregate, 2 = inclusive prefix
 };
 
+// Decoupled look-back for tile `tile` (tiles taken in ticket order) whose own sum is `agg`; called by all 32 lanes of one
+// warp, returns the tile's exclusive prefix to every lane and publishes its inclusive prefix.  One window of 32
+// predecessors per step: every lane waits for its own predecessor's status, the window is summed back to the nearest
+// inclusive prefix (tiles are ticket-ordered, so predecessors always arrive).
+__device__ __forceinline__ unsigned long long lookback_prefix(ScanState* st, uint32_t tile, unsigned long long agg, int lane) {
+  constexpr unsigned long long kValue = (1ull << 62) - 1;
+  unsigned long long prefix = 0;
+  volatile unsigned long long* status = st->status;
+  if (tile == 0) {
+    if (lane == 0) {
+      __threadfence();
+      status[0] = (2ull << 62) | agg;
+    }
+  } else {
+    if (lane == 0) {
+      status[tile] = (1ull << 62) | agg;
+      __threadfence();
+    }
+    int base = (int)tile - 1;
+    while (true) {
+      const int idx = base - lane;
+      unsigned long long sv = 2ull << 62;  // before tile 0: an inclusive prefix of zero
+      if (idx >= 0) {
+        do { sv = status[idx]; } while ((sv >> 62) == 0ull);
+      }
+      const unsigned incl = __ballot_sync(0xffffffffu, (sv >> 62) == 2ull);
+      const int stop = incl ? __ffs((int)incl) - 1 : 31;  // nearest inclusive prefix in this window
+      unsigned long long v = lane <= stop ? (sv & kValue) : 0ull;
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+      prefix += v;
+      if (incl) break;
+      base -= 32;
+    }
+    if (lane == 0) {
+      __threadfence();
+      status[tile] = (2ull << 62) | (prefix + agg);
+    }
+  }
+  return prefix;
+}
+
 template <bool STRATEGY>
 __global__ void __launch_bounds__(kThreads) k_plan(const float* __restrict__ vx, const float* __restrict__ vy, Geom g,
                                                    ValueMap vm, const float* __restrict__ minmax, LevelThresholds thr,
@@ -1171,42 +1213,7 @@ __global__ void __launch_bounds__(kThreads) k_plan(const float* __restrict__ vx,
   unsigned long long excl = wbase + inc - tsum;
 
   if (warp == 0) {
-    // decoupled look-back, one window of 32 predecessors per step: every lane waits for its own predecessor's status,
-    // the window is summed back to the nearest inclusive prefix (tiles are ticket-ordered, so predecessors always arrive)
-    constexpr unsigned long long kValue = (1ull << 62) - 1;
-    unsigned long long prefix = 0;
-    volatile unsigned long long* status = st->status;
-    if (tile == 0) {
-      if (lane == 0) {
-        __threadfence();
-        status[0] = (2ull << 62) | agg;
-      }
-    } else {
-      if (lane == 0) {
-        status[tile] = (1ull << 62) | agg;
-        __threadfence();
-      }
-      int base = (int)tile - 1;
-      while (true) {
-        const int idx = base - lane;
-        unsigned long long sv = 2ull << 62;  // before tile 0: an inclusive prefix of zero
-        if (idx >= 0) {
-          do { sv = status[idx]; } while ((sv >> 62) == 0ull);
-        }
-        const unsigned incl = __ballot_sync(0xffffffffu, (sv >> 62) == 2ull);
-        const int stop = incl ? __ffs((int)incl) - 1 : 31;  // nearest inclusive prefix in this window
-        unsigned long long v = lane <= stop ? (sv & kValue) : 0ull;
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
-        prefix += v;
-        if (incl) break;
-        base -= 32;
-      }
-      if (lane == 0) {
-        __threadfence();
-        status[tile] = (2ull << 62) | (prefix + agg);
-      }
-    }
+    const unsigned long long prefix = lookback_prefix(st, tile, agg, lane);
     if (lane == 0) s_prefix = prefix;
     if ((tile + 1) * (uint32_t)kPlanTile >= nblocks) {
       if (lane == 0) *total = prefix + agg;
@@ -1232,6 +1239,112 @@ __global__ void __launch_bounds__(kThreads) k_plan(const float* __restrict__ vx,
       if (STRATEGY) tabidx_up[b] = tix_up[j];
       lists[(size_t)cls[j] * cap + s_base[cls[j]] + rank[j]] = b;
       excl += sz[j];
+    }
+  }
+  // the CTA that finishes last leaves ticket, status and cursors zeroed for the next launch on this stream
+  __shared__ bool s_last;
+  if (tid == 0) {
+    __threadfence();
+    s_last = atomicAdd(&st->done, 1u) == gridDim.x - 1;
+  }
+  __syncthreads();
+  if (s_last) {
+    for (uint32_t i = tid; i < gridDim.x; i += kThreads) st->status[i] = 0ull;
+    if (tid < 2 * kCostClasses) cursor[tid] = 0u;
+    if (tid == 0) { st->ticket = 0u; st->done = 0u; }
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// window of a payload (random access): the blocks of columns [c0, c0 + g.cols) x rows [r0, r0 + g.rows) of a parent payload
+// with `pcols` columns, as the payload of the sub-image they tile (geometry g).  One lane of warp 0 per window block takes
+// the parent's descriptor and table indices, the block sizes are scanned as in k_plan (same look-back, same work-order
+// lists; 32-block tiles, see window_scan_state_bytes), then every warp of the CTA copies whole blocks to their re-packed
+// offsets.  Tiles of 32 blocks rather than k_plan's 256: the copy, not the scan, is the work, and with 256 blocks per CTA
+// a window of a few hundred blocks ran on one or two SMs, each warp copying 32 blocks in turn (50 us for 256 blocks).  A
+// block's tile size in the window is its tile size in the parent, so the parent's table indices stay valid.
+// meta / pmeta: tabidx [cap] | order lists | expand-side indices [cap] (pxz_payload::d_tabidx); copy_up: take the latter too
+// ------------------------------------------------------------------------------------------------
+constexpr int kWindowTile = 32;  // window blocks per CTA: one warp scans them, all 8 warps copy them (4 blocks per warp)
+__global__ void __launch_bounds__(kThreads) k_payload_window(const pxz_block_desc* __restrict__ pdescs, const uint32_t* __restrict__ pmeta,
+                                                             uint32_t pcap, const uint8_t* __restrict__ ppx, uint32_t pcols, uint32_t c0,
+                                                             uint32_t r0, Geom g, int copy_up, pxz_block_desc* __restrict__ descs,
+                                                             uint32_t* __restrict__ meta, uint32_t cap, uint8_t* __restrict__ px,
+                                                             unsigned long long* __restrict__ total, ScanState* st, uint32_t* __restrict__ cursor) {
+  __shared__ unsigned int s_tile;
+  __shared__ uint32_t s_hist[kCostClasses], s_base[kCostClasses];
+  __shared__ unsigned long long s_src[kWindowTile], s_dst[kWindowTile];
+  __shared__ uint32_t s_len[kWindowTile];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (tid < kCostClasses) s_hist[tid] = 0;
+  if (tid == 0) s_tile = atomicAdd(&st->ticket, 1u);
+  __syncthreads();
+  const uint32_t tile = s_tile;
+  const uint32_t nblocks = g.cols * g.rows;
+  if (warp == 0) {
+    const uint32_t b = tile * kWindowTile + lane;
+    uint32_t pb = 0, cls = 0, rank = 0;
+    pxz_block_desc d = {};
+    unsigned long long sz = 0;
+    if (b < nblocks) {
+      const uint32_t j = b / g.cols, i = b - j * g.cols;
+      pb = (r0 + j) * pcols + c0 + i;
+      d = pdescs[pb];
+      sz = (unsigned long long)d.w * d.h * g.C;
+      const Tile t = tile_of(g, b);
+      cls = cost_class(d.w, d.h, t.tw, t.th);
+      rank = atomicAdd(&s_hist[cls], 1u);
+    }
+    __syncwarp();
+    if (lane < kCostClasses) {
+      s_base[lane] = s_hist[lane] ? atomicAdd(&cursor[lane], s_hist[lane]) : 0u;
+      __threadfence();  // reserved before this CTA's scan status is published (the last CTA reads the final cursors)
+    }
+    __syncwarp();
+    unsigned long long inc = sz;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+      unsigned long long n = __shfl_up_sync(0xffffffffu, inc, o);
+      if (lane >= o) inc += n;
+    }
+    const unsigned long long agg = __shfl_sync(0xffffffffu, inc, 31);
+    const unsigned long long prefix = lookback_prefix(st, tile, agg, lane);
+    if ((tile + 1) * (uint32_t)kWindowTile >= nblocks) {
+      if (lane == 0) *total = prefix + agg;
+      // every other CTA has published its status, hence reserved its slots: the cursors are final
+      __syncwarp();
+      __threadfence();
+      if (lane < kCostClasses) meta[(size_t)cap + (size_t)kCostClasses * cap + lane] = atomicAdd(&cursor[lane], 0u);
+    }
+    if (b < nblocks) {
+      const unsigned long long off = prefix + inc - sz;
+      s_src[lane] = d.offset;
+      s_dst[lane] = off;
+      s_len[lane] = (uint32_t)sz;
+      d.offset = off;
+      descs[b] = d;
+      meta[b] = pmeta[pb];
+      if (copy_up) meta[(size_t)cap + order_list_words(cap) + b] = pmeta[(size_t)pcap + order_list_words(pcap) + pb];
+      meta[(size_t)cap + (size_t)cls * cap + s_base[cls] + rank] = b;
+    }
+  }
+  __syncthreads();
+  // block pixels: a warp per block, in 16-byte words when both offsets and the length allow, else 4-byte words (every RGBA
+  // block), else bytes
+  const uint32_t nhere = min((uint32_t)kWindowTile, nblocks - min(nblocks, tile * (uint32_t)kWindowTile));
+  for (uint32_t k = (uint32_t)warp; k < nhere; k += kThreads / 32) {
+    const uint8_t* s = ppx + s_src[k];
+    uint8_t* o = px + s_dst[k];
+    const uint32_t n = s_len[k];
+    const unsigned long long a = s_src[k] | s_dst[k] | n;
+    if ((a & 15u) == 0) {
+#pragma unroll 4
+      for (uint32_t q = lane; q < n / 16; q += 32) reinterpret_cast<uint4*>(o)[q] = ldg_nc_v4(s + (size_t)q * 16);
+    } else if ((a & 3u) == 0) {
+#pragma unroll 4
+      for (uint32_t q = lane; q < n / 4; q += 32) reinterpret_cast<uint32_t*>(o)[q] = __ldg(reinterpret_cast<const uint32_t*>(s) + q);
+    } else {
+      for (uint32_t q = lane; q < n; q += 32) o[q] = __ldg(s + q);
     }
   }
   // the CTA that finishes last leaves ticket, status and cursors zeroed for the next launch on this stream
@@ -2366,6 +2479,24 @@ cudaError_t launch_plan(const float* vx, const float* vy, const Geom& g, const V
   if (adaptive) e = launch_pdl(k_plan<true>, tiles, kThreads, 0, s, vx, vy, g, vm, minmax, thr, mask, descs, tabidx, total, st, cursor, lists, cap, lut, tabidx_up);
   else e = launch_pdl(k_plan<false>, tiles, kThreads, 0, s, vx, vy, g, vm, minmax, thr, mask, descs, tabidx, total, st, cursor, lists, cap, lut, tabidx_up);
   return e != cudaSuccess ? e : cudaGetLastError();
+}
+
+size_t window_scan_state_bytes(uint32_t nblocks) {
+  const uint32_t tiles = (nblocks + kWindowTile - 1) / kWindowTile;
+  return kClassHistBytes + sizeof(ScanState) + (size_t)tiles * sizeof(unsigned long long);
+}
+
+cudaError_t launch_payload_window(const pxz_block_desc* pdescs, const uint32_t* pmeta, uint32_t pcap, const uint8_t* ppx, uint32_t pcols,
+                                  uint32_t c0, uint32_t r0, const Geom& g, bool copy_up, pxz_block_desc* descs, uint32_t* meta, uint32_t cap,
+                                  uint8_t* px, uint64_t* total_bytes, void* scan_state, cudaStream_t s, uint64_t* launches) {
+  const uint32_t nblocks = g.cols * g.rows;
+  uint32_t* cursor = reinterpret_cast<uint32_t*>(scan_state);  // zero on entry and on exit
+  ScanState* st = reinterpret_cast<ScanState*>(reinterpret_cast<uint8_t*>(scan_state) + kClassHistBytes);
+  ++*launches;
+  k_payload_window<<<(nblocks + kWindowTile - 1) / kWindowTile, kThreads, 0, s>>>(pdescs, pmeta, pcap, ppx, pcols, c0, r0, g, copy_up ? 1 : 0,
+                                                                            descs, meta, cap, px,
+                                                                            reinterpret_cast<unsigned long long*>(total_bytes), st, cursor);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_class_lists(const pxz_block_desc* descs, const Geom& g, void* scan_state, uint32_t* lists, uint32_t cap,

@@ -133,6 +133,14 @@ __host__ __device__
 inline size_t order_list_words(size_t cap) { return (size_t)kOrderClasses * cap + kOrderClasses; }
 cudaError_t launch_class_lists(const pxz_block_desc* descs, const Geom& g, void* scan_state, uint32_t* lists, uint32_t cap,
                                cudaStream_t s, uint64_t* launches);
+// The blocks of columns [c0, c0 + g.cols) x rows [r0, r0 + g.rows) of a payload with pcols columns (descs / meta / pixels of
+// capacity pcap) as the payload of geometry g: descriptors with re-packed offsets, table indices (and, with copy_up, the
+// expand-side indices), work-order lists, total and pixels, in one launch.  meta: pxz_payload::d_tabidx layout.
+// scan_state: window_scan_state_bytes(g.cols * g.rows), zero on entry and on exit (shared with launch_plan).
+size_t window_scan_state_bytes(uint32_t nblocks);
+cudaError_t launch_payload_window(const pxz_block_desc* pdescs, const uint32_t* pmeta, uint32_t pcap, const uint8_t* ppx, uint32_t pcols,
+                                  uint32_t c0, uint32_t r0, const Geom& g, bool copy_up, pxz_block_desc* descs, uint32_t* meta, uint32_t cap,
+                                  uint8_t* px, uint64_t* total_bytes, void* scan_state, cudaStream_t s, uint64_t* launches);
 // quadtree level (process/tree.rs:47-77): leaf[b] = active && ((v >= thr) ^ positive), recurse[b] = active && !that,
 // where active = recurse flag of the parent block one level up (NULL parent = every block is active)
 cudaError_t launch_tree_mask(const float* vx, const Geom& g, const uint8_t* parent_recurse, uint32_t parent_cols, float thr,
