@@ -180,6 +180,20 @@ pxz_status pxz_analyze(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t
 pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
                       pxz_filter filter_down, uint32_t flags, pxz_payload** out);
 
+/* EXTENSION (rate control; the reference takes the factor only, src/bin/main.rs `-k`).  k = the largest finite f32 > 0 for
+ * which pxz_shrink(ctx, img, bw, bh, metric, k, filter_down, flags) produces at most max_bytes payload bytes
+ * (pxz_payload_info's `bytes`; an RGB image counts 3 bytes per pixel).  *out is that payload, byte for byte what
+ * pxz_shrink returns for k (descriptors incl. stored values, pixels); *factor_out = k.  k = FLT_MAX when even that fits.
+ * The size is monotone in k, so one analysis pass is enough: the device evaluates the size for up to 256 factors per round
+ * from the block values alone, and the Oklab fast path checks the two sizes that bracket the budget in reference order
+ * (DESIGN.md §3).  Each round reads sizes back to the host, so this call synchronises the stream and cannot be captured
+ * in a CUDA graph.
+ * PXZ_E_ARG: max_bytes below the payload at the smallest positive factor (the message names that size),
+ *            PXZ_FLAG_AFTER_IDENTITY (the factor is unused), unknown filter / metric.
+ * PXZ_E_UNSUPPORTED: a batch image; PXZ_FLAG_NORMALISE_GLOBAL on a context with a communicator. */
+pxz_status pxz_shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_bytes,
+                              pxz_filter filter_down, uint32_t flags, float* factor_out, pxz_payload** out);
+
 /* Scalar part of reduce_image_section (operations.rs:128-156) on the host: (v0, v1) after `after`
  * -> parse_value -> level -> reduced size of a w x h block and the stored block value.  Uses the
  * same threshold table as the device plan kernel. */

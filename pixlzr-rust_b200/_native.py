@@ -63,6 +63,7 @@ SYMBOLS = {
     "pxz_grid": (_i, [_u32, _u32, _u32, _u32, _P(_u32), _P(_u32)]),
     "pxz_analyze": (_i, [_vp, _vp, _u32, _u32, _i, _u32, _vp, _vp]),
     "pxz_shrink": (_i, [_vp, _vp, _u32, _u32, _i, C.c_float, _i, _u32, _P(_vp)]),
+    "pxz_shrink_to_size": (_i, [_vp, _vp, _u32, _u32, _i, _u64, _i, _u32, _P(C.c_float), _P(_vp)]),
     "pxz_reduce_dims": (_i, [C.c_float, C.c_float, _u32, _u32, _P(_u32), _P(_u32), _P(C.c_float)]),
     "pxz_resample_table": (C.c_int32, [_u32, _u32, _i, _vp, _vp, _vp, _u32]),
     "pxz_payload_info": (_i, [_vp, _vp] + [_P(_u32)] * 7 + [_P(_u64)]),
@@ -349,6 +350,14 @@ class Image:
         self.ctx.check(lib().pxz_shrink(self.ctx.handle, self._h, bw, bh, metric, factor, int(filter_down), flags,
                                         C.byref(h)))
         return Payload(self.ctx, h)
+
+    def shrink_to_size(self, bw: int, bh: int, metric: int, max_bytes: int, filter_down: int, flags: int = 0):
+        """(Payload, k): the payload of shrink(..., k, ...) for the largest factor k whose payload has at most `max_bytes`
+        bytes (pxz_shrink_to_size; k = FLT_MAX when even that fits)."""
+        h, k = C.c_void_p(), C.c_float()
+        self.ctx.check(lib().pxz_shrink_to_size(self.ctx.handle, self._h, bw, bh, metric, int(max_bytes), int(filter_down), flags,
+                                                C.byref(k), C.byref(h)))
+        return Payload(self.ctx, h), float(k.value)
 
     def tree_process(self, threshold: float, bw: int, bh: int, min_bw: int, min_bh: int, filter_down: int, filter_up: int,
                      out: "Image"):

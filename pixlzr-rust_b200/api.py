@@ -305,6 +305,29 @@ class Pixlzr:
             return  # every block has block_value.is_some(): the reference clones them unchanged
         self._shrink(N.METRIC_OKLAB_MAD, filter_downscale, factor, N.FLAG_EXACT_VALUES if exact_values else 0)
 
+    def shrink_to_size(self, filter_downscale: FilterType, max_bytes: int, directionally: bool = False,
+                       exact_values: bool = False) -> float:
+        """EXTENSION (rate control): shrink_by (or shrink_directionally) with the largest factor whose payload has at most
+        `max_bytes` bytes; returns that factor (pxz_shrink_to_size).  shrink_by / shrink_directionally with the returned
+        factor give the same blocks.  Needs the source image: refused on a decoded or already shrunk Pixlzr."""
+        if self._image is None:
+            raise ValueError("shrink_to_size needs the source image (Pixlzr.from_image), not a decoded or already shrunk one")
+        ctx = self._ctx()
+        img = ctx.image_upload(self._image)
+        try:
+            metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
+            pl, k = img.shrink_to_size(self.block_width, self.block_height, metric, max_bytes, int(filter_downscale),
+                                       N.FLAG_EXACT_VALUES if exact_values else 0)
+            try:
+                self._descs, self._pixels = pl.download()
+            finally:
+                pl.free()
+        finally:
+            img.free()
+        self._values_present = True
+        self._image = None
+        return k
+
     def shrink_directionally(self, filter_downscale: FilterType, factor: float):
         """Pixlzr::shrink_directionally (pixlzr.rs:187-205)."""
         self._shrink(N.METRIC_SOBEL_DIR, filter_downscale, factor, 0)
@@ -437,6 +460,24 @@ class Pixlzr:
                             int(filter_downscale), 0)
             try:
                 return pl.to_container(0, True)  # from_image leaves `filter` unset: byte 0
+            finally:
+                pl.free()
+        finally:
+            img.free()
+
+    @staticmethod
+    def encode_image_to_vec_sized(image: np.ndarray, block_width: int, block_height: int, filter_downscale: FilterType,
+                                  max_bytes: int, directionally: bool = False, ctx: Optional[N.Context] = None) -> Tuple[bytes, float]:
+        """EXTENSION (rate control): encode_image_to_vec with the largest factor whose payload (not the file) has at most
+        `max_bytes` bytes.  Returns (file, factor); encode_image_to_vec with that factor writes the same file."""
+        image = _check_image(image)
+        ctx = ctx or default_context()
+        img = ctx.image_upload(image)
+        try:
+            pl, k = img.shrink_to_size(block_width, block_height, N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD,
+                                       max_bytes, int(filter_downscale), 0)
+            try:
+                return pl.to_container(0, True), k
             finally:
                 pl.free()
         finally:
@@ -585,6 +626,11 @@ def tree_process_custom(image: np.ndarray, threshold: float, block_size: Tuple[i
 def tree_process(image: np.ndarray, block_size: int, threshold: float, ctx: Optional[N.Context] = None) -> np.ndarray:
     """tree::process (process/tree.rs:89-109): Lanczos3 down, Nearest up, minimum block 4."""
     return tree_process_custom(image, threshold, (block_size, block_size), (4, 4), (FilterType.Lanczos3, FilterType.Nearest), ctx)
+
+
+def format_shrinking_factor(k: float) -> str:
+    """The shortest decimal that parse_shrinking_factor reads back to the same f32 (e.g. the factor shrink_to_size chose)."""
+    return str(np.float32(k))
 
 
 def parse_shrinking_factor(s: str) -> float:

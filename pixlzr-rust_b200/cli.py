@@ -39,7 +39,21 @@ def build_parser() -> argparse.ArgumentParser:
     # extension (random access): not a flag of the reference
     p.add_argument("--region", type=parse_region, default=None, metavar="X,Y,W,H",
                    help="Decode only this pixel rectangle (.pix / .pixlzr -> image only)")
+    # extension (rate control): not a flag of the reference
+    p.add_argument("--payload-bytes", type=parse_payload_bytes, default=None, metavar="N",
+                   help="Shrink with the largest factor whose block payload has at most N bytes, and print that factor "
+                        "(image input, with --force; replaces -k)")
     return p
+
+
+def parse_payload_bytes(s: str) -> int:
+    try:
+        n = int(s)
+    except ValueError:
+        raise argparse.ArgumentTypeError(f"expected a byte count, got {s!r}") from None
+    if n < 0:
+        raise argparse.ArgumentTypeError(f"expected a byte count >= 0, got {s!r}")
+    return n
 
 
 def parse_region(s: str) -> Tuple[int, int, int, int]:
@@ -61,18 +75,37 @@ def region_error(args) -> Optional[str]:
     return None
 
 
+def payload_bytes_error(args) -> Optional[str]:
+    """Why --payload-bytes does not apply to these arguments, or None."""
+    if args.payload_bytes is None:
+        return None
+    if operation(args.input, args.output)[0] != "image":
+        return "--payload-bytes chooses the factor of an encode: the input must be an image, not a container"
+    if not args.force:
+        return "--payload-bytes shrinks the blocks: it needs --force"
+    if getattr(args, "factor_given", False):
+        return "--payload-bytes chooses the shrinking factor: it cannot be combined with -k"
+    if args.region is not None:
+        return "--payload-bytes does not apply to a region decode"
+    return None
+
+
 def parse_args(argv: Optional[List[str]] = None):
     """`-k -1/2`: the reference's clap option has allow_hyphen_values (main.rs:28-33); argparse needs `--opt=value`."""
     argv = list(sys.argv[1:] if argv is None else argv)
-    out, i = [], 0
+    out, i, factor_given = [], 0, False
     while i < len(argv):
         if argv[i] in ("-k", "--shrinking-factor") and i + 1 < len(argv):
             out.append("--shrinking-factor=" + argv[i + 1])
+            factor_given = True
             i += 2
         else:
+            factor_given = factor_given or argv[i].startswith("--shrinking-factor=")
             out.append(argv[i])
             i += 1
-    return build_parser().parse_args(out)
+    args = build_parser().parse_args(out)
+    args.factor_given = factor_given  # --payload-bytes refuses an explicit -k, even `-k 1`
+    return args
 
 
 def kind_of(path: str, default: str) -> str:
@@ -115,9 +148,12 @@ def run(args) -> None:
     filt = FILTERS[args.filter]
     shrink_by = api.parse_shrinking_factor(args.shrinking_factor)
     src, dst = operation(args.input, args.output)
-    err = region_error(args)
+    err = region_error(args) or payload_bytes_error(args)
     if err:
         raise ValueError(err)
+    if args.payload_bytes is not None:
+        _run_sized(args, bw, bh, filt, src, dst)
+        return
     if args.region is not None and not (args.force and args.direction_wise):
         with open(args.input, "rb") as f:
             _save_image(args.output, api.Pixlzr.decode_vec_region_to_image(f.read(), filt, *args.region))
@@ -149,9 +185,23 @@ def run(args) -> None:
         _save_image(args.output, pix.to_image(filt))
 
 
+def _run_sized(args, bw: int, bh: int, filt, src: str, dst: str) -> None:
+    """image -> container / image with the factor chosen for --payload-bytes; prints the factor in a form -k reads back."""
+    image = _open_image(args.input)
+    if dst == "pix":
+        data, k = api.Pixlzr.encode_image_to_vec_sized(image, bw, bh, filt, args.payload_bytes, bool(args.direction_wise))
+        with open(args.output, "wb") as f:
+            f.write(data)
+    else:
+        pix = api.Pixlzr.from_image(image, bw, bh)
+        k = pix.shrink_to_size(filt, args.payload_bytes, bool(args.direction_wise))
+        _save_image(args.output, pix.to_image(filt))
+    print(f"shrinking factor: {api.format_shrinking_factor(k)}")
+
+
 def main(argv: Optional[List[str]] = None) -> int:
     args = parse_args(argv)
-    err = region_error(args)
+    err = region_error(args) or payload_bytes_error(args)
     if err:
         print(f"pixlzr: {err}", file=sys.stderr)
         return 2

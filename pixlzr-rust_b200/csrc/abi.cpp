@@ -13,6 +13,7 @@
 #include <string.h>
 
 #include <algorithm>
+#include <functional>
 #include <map>
 #include <memory>
 #include <new>
@@ -47,10 +48,10 @@ using TabKey = std::tuple<std::vector<uint32_t>, std::vector<uint32_t>, int, int
 
 // K_REGION_COPY times the device-to-device copy of pxz_expand_region out of its staging image (not a kernel)
 enum KernelId { K_MAD_FAST = 0, K_MAD_EXACT, K_SOBEL, K_MINMAX, K_PLAN, K_RESAMPLE_DOWN, K_RESAMPLE_UP, K_QOI_ENCODE, K_QOI_DECODE,
-                K_PAYLOAD_WINDOW, K_REGION_COPY, K_COUNT };
+                K_PAYLOAD_WINDOW, K_REGION_COPY, K_SIZE_CURVE, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"analyze_mad_fast", "mad_exact",      "analyze_sobel", "minmax",
                                            "plan",             "resample_down",  "resample_up",   "qoi_encode",
-                                           "qoi_decode",       "payload_window", "region_copy"};
+                                           "qoi_decode",       "payload_window", "region_copy",   "size_curve"};
 struct ProfRec {
   int id;
   cudaEvent_t a, b;
@@ -883,116 +884,94 @@ static pxz_status payload_rechannel(pxz_ctx* ctx, const pxz_payload* src, uint32
   return PXZ_OK;
 }
 
-pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
-                      pxz_filter filter_down, uint32_t flags, pxz_payload** out) {
-  if (!ctx || !img || !out) return PXZ_E_ARG;
-  *out = nullptr;
-  cudaSetDevice(ctx->device);
-  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
-    // widen to RGBA (alpha 255: its metric term is exactly +0 and the opaque resample path never touches it), run the
-    // 4-channel pipeline, narrow the payload back
-    pxz_image* wide = nullptr;
-    pxz_status st = pxz_image_alloc_batch(ctx, img->w, img->h, 4, img->nimg, &wide);
-    if (st != PXZ_OK) return st;
-    cudaError_t e = launch_rgb_widen(img->d, img->pitch, wide->d, wide->pitch, img->w, img->h * img->nimg, 1, ctx->stream, ctx->sm_count,
-                                     &ctx->launches);
-    pxz_payload* p4 = nullptr;
-    if (e != cudaSuccess) {
-      cudaGetLastError();
-      st = fail(ctx, PXZ_E_CUDA, std::string("rgb widen: ") + cudaGetErrorString(e));
-    } else {
-      st = pxz_shrink(ctx, wide, bw, bh, metric, factor, filter_down, flags, &p4);
-    }
-    pxz_image_free(wide);  // stream-ordered: the kernels queued above keep it
-    if (st != PXZ_OK) return st;
-    st = payload_rechannel(ctx, p4, 3, out);
-    payload_release(p4);
-    return st;
+// An RGB image on the RGBA fast kernels: widen it to RGBA (alpha 255: its metric term is exactly +0 and the opaque resample
+// path never touches it), run `encode` on the 4-channel image, narrow the payload back
+extern "C++" {  // a template inside the extern "C" block
+template <class F>
+static pxz_status encode_via_rgba(pxz_ctx* ctx, const pxz_image* img, F&& encode, pxz_payload** out) {
+  pxz_image* wide = nullptr;
+  pxz_status st = pxz_image_alloc_batch(ctx, img->w, img->h, 4, img->nimg, &wide);
+  if (st != PXZ_OK) return st;
+  cudaError_t e = launch_rgb_widen(img->d, img->pitch, wide->d, wide->pitch, img->w, img->h * img->nimg, 1, ctx->stream, ctx->sm_count,
+                                   &ctx->launches);
+  pxz_payload* p4 = nullptr;
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    st = fail(ctx, PXZ_E_CUDA, std::string("rgb widen: ") + cudaGetErrorString(e));
+  } else {
+    st = encode(wide, &p4);
   }
-  const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
-  // Every rank of a communicator must reach the min/max exchange, whatever happens to it before: a rank-local failure
-  // (an unknown filter, a trailing block the Sobel metric cannot take, no memory) joins with neutral values and an
-  // error flag instead of leaving its peers in the collective.
-  auto bail = [&](pxz_status why) -> pxz_status {
-    if (normalise && ctx->comm) {
-      const std::string msg = ctx->err;
-      bool peers_ok = true;
-      exchange_minmax(ctx, false, &peers_ok);
-      ctx->err = msg;
-    }
-    return why;
-  };
-  if ((int)filter_down < 0 || (int)filter_down > 4) return bail(fail(ctx, PXZ_E_ARG, "unknown filter"));
-  Geom g;
-  pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g, img->nimg);
-  if (st != PXZ_OK) return bail(st);
-  if (normalise && img->nimg > 1) return bail(fail(ctx, PXZ_E_UNSUPPORTED, "global normalisation is per image: not available on a batch"));
-  const uint32_t nblocks = g.cols * g.rows;
+  pxz_image_free(wide);  // stream-ordered: the kernels queued above keep it
+  if (st != PXZ_OK) return st;
+  st = payload_rechannel(ctx, p4, 3, out);
+  payload_release(p4);
+  return st;
+}
+}  // extern "C++"
 
+static ValueMap shrink_value_map(const pxz_ctx* ctx, pxz_metric metric, uint32_t flags, float factor) {
   ValueMap vm;
   vm.factor = factor;
   vm.mode = (metric == PXZ_METRIC_SOBEL_DIR) ? 2 : ((flags & PXZ_FLAG_AFTER_IDENTITY) ? 1 : 0);
-  vm.normalise = normalise ? 1 : 0;
+  vm.normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) ? 1 : 0;
   vm.extra_thr = NAN;
   if (ctx->strategy.on)
     for (int k = 1; k < kStrategyBuckets; ++k)
       if (ctx->strategy.down[k] != ctx->strategy.down[k - 1] || ctx->strategy.up[k] != ctx->strategy.up[k - 1])
         vm.bucket_edges |= 1ull << (k - 1);
+  return vm;
+}
 
-  // with global normalisation every value depends on the exact min and max, so the Oklab path
-  // runs in reference order for all blocks (DESIGN.md)
-  const bool exact_all = (flags & PXZ_FLAG_EXACT_VALUES) != 0;
-  // Global normalisation of the Oklab values on the fast path: the exact extremes come from the few tiles that can hold
-  // them, and the guard band (scaled by 1 / range) then decides as in the default mode which tiles need their
-  // reference-order value; with PXZ_FLAG_EXACT_VALUES every tile is computed in reference order as before.
-  const bool fast_norm = normalise && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
-  st = run_analysis(ctx, img, g, metric, exact_all, (metric == PXZ_METRIC_OKLAB_MAD && !exact_all && !normalise) ? &vm : nullptr);
-  if (st != PXZ_OK) return bail(st);
+// min / max of the values in ctx->d_vx (and d_vy) into ctx->d_minmax
+static pxz_status run_minmax(pxz_ctx* ctx, pxz_metric metric, uint32_t nblocks) {
+  ProfScope prof(ctx, K_MINMAX);
+  cudaError_t me = launch_minmax(ctx->d_vx, metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr, nblocks, ctx->d_minmax, ctx->stream,
+                                 &ctx->launches);
+  if (me != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ctx, PXZ_E_CUDA, std::string("minmax: ") + cudaGetErrorString(me));
+  }
+  return PXZ_OK;
+}
 
-  if (normalise) {
-    auto minmax = [&]() -> pxz_status {
-      ProfScope prof(ctx, K_MINMAX);
-      cudaError_t me = launch_minmax(ctx->d_vx, metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr, nblocks, ctx->d_minmax,
-                                     ctx->stream, &ctx->launches);
-      if (me != cudaSuccess) {
-        cudaGetLastError();
-        return fail(ctx, PXZ_E_CUDA, std::string("minmax: ") + cudaGetErrorString(me));
-      }
-      return PXZ_OK;
-    };
-    if ((st = minmax()) != PXZ_OK) return bail(st);
-    if (fast_norm) {
-      {
-        ProfScope prof(ctx, K_MAD_EXACT);
-        cudaError_t ee = launch_analyze_mad_exact(img->d, img->pitch, g, ctx->d_vx, ctx->d_vx, ctx->d_opaque, nullptr, &ctx->thr, &ctx->band,
-                                                  ctx->d_minmax, ctx->d_list, ctx->d_list + nblocks, ctx->stream, ctx->sm_count,
-                                                  &ctx->launches);
-        if (ee != cudaSuccess) {
-          cudaGetLastError();
-          return bail(fail(ctx, PXZ_E_CUDA, std::string("extremes: ") + cudaGetErrorString(ee)));
-        }
-      }
-      if ((st = minmax()) != PXZ_OK) return bail(st);  // over the patched values: the exact extremes
-    }
-    bool peers_ok = true;
-    st = exchange_minmax(ctx, true, &peers_ok);
-    if (st != PXZ_OK) return st;
-    if (!peers_ok) return fail(ctx, PXZ_E_NCCL, "another rank failed before the min/max exchange");
-    if (fast_norm) {
-      ProfScope prof(ctx, K_MAD_EXACT);
-      cudaError_t ee = cudaMemsetAsync(ctx->d_list + nblocks, 0, sizeof(uint32_t), ctx->stream);  // the list counter
-      if (ee == cudaSuccess)
-        ee = launch_analyze_mad_exact(img->d, img->pitch, g, ctx->d_vx, ctx->d_vx, ctx->d_opaque, &vm, &ctx->thr, &ctx->band, ctx->d_minmax,
-                                      ctx->d_list, ctx->d_list + nblocks, ctx->stream, ctx->sm_count, &ctx->launches);
-      if (ee != cudaSuccess) {
-        cudaGetLastError();
-        return fail(ctx, PXZ_E_CUDA, std::string("guard band: ") + cudaGetErrorString(ee));
-      }
+// Global normalisation on the fast Oklab path, first half: the exact extremes come from the few tiles that can hold them
+// (their reference-order values patched into ctx->d_vx), then a second min / max over the patched values
+static pxz_status run_exact_extremes(pxz_ctx* ctx, const pxz_image* img, const Geom& g, uint32_t nblocks) {
+  {
+    ProfScope prof(ctx, K_MAD_EXACT);
+    cudaError_t ee = launch_analyze_mad_exact(img->d, img->pitch, g, ctx->d_vx, ctx->d_vx, ctx->d_opaque, nullptr, &ctx->thr, &ctx->band,
+                                              ctx->d_minmax, ctx->d_list, ctx->d_list + nblocks, ctx->stream, ctx->sm_count,
+                                              &ctx->launches);
+    if (ee != cudaSuccess) {
+      cudaGetLastError();
+      return fail(ctx, PXZ_E_CUDA, std::string("extremes: ") + cudaGetErrorString(ee));
     }
   }
+  return run_minmax(ctx, PXZ_METRIC_OKLAB_MAD, nblocks);
+}
 
+// Guard band of the fast Oklab path for the factor of `vm`: the tiles listed from the fast values `vx_fast` get their
+// reference-order value in `vx` (in place when vx == vx_fast, as pxz_shrink does)
+static pxz_status run_guard_band(pxz_ctx* ctx, const pxz_image* img, const Geom& g, const ValueMap& vm, float* vx, const float* vx_fast) {
+  const uint32_t nblocks = g.cols * g.rows;
+  ProfScope prof(ctx, K_MAD_EXACT);
+  cudaError_t ee = cudaMemsetAsync(ctx->d_list + nblocks, 0, sizeof(uint32_t), ctx->stream);  // the list counter
+  if (ee == cudaSuccess)
+    ee = launch_analyze_mad_exact(img->d, img->pitch, g, vx, vx_fast, ctx->d_opaque, &vm, &ctx->thr, &ctx->band, ctx->d_minmax, ctx->d_list,
+                                  ctx->d_list + nblocks, ctx->stream, ctx->sm_count, &ctx->launches);
+  if (ee != cudaSuccess) {
+    cudaGetLastError();
+    return fail(ctx, PXZ_E_CUDA, std::string("guard band: ") + cudaGetErrorString(ee));
+  }
+  return PXZ_OK;
+}
+
+// The part of pxz_shrink after the analysis: plan (value -> level -> dims -> offsets) from ctx->d_vx / d_vy, then the
+// resample into a new payload
+static pxz_status plan_and_resample(pxz_ctx* ctx, const pxz_image* img, const Geom& g, pxz_metric metric, const ValueMap& vm,
+                                    pxz_filter filter_down, bool exact_all, pxz_payload** out) {
   pxz_payload* p = nullptr;
-  st = payload_new(ctx, g, (uint64_t)g.W * g.H * g.C * g.nimg, &p);
+  pxz_status st = payload_new(ctx, g, (uint64_t)g.W * g.H * g.C * g.nimg, &p);
   if (st != PXZ_OK) return st;
   p->spec = spec_for_geom(g);
   {
@@ -1037,6 +1016,188 @@ pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t 
   }
   *out = p;
   return PXZ_OK;
+}
+
+pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
+                      pxz_filter filter_down, uint32_t flags, pxz_payload** out) {
+  if (!ctx || !img || !out) return PXZ_E_ARG;
+  *out = nullptr;
+  cudaSetDevice(ctx->device);
+  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh))
+    return encode_via_rgba(
+        ctx, img, [&](const pxz_image* wide, pxz_payload** p4) { return pxz_shrink(ctx, wide, bw, bh, metric, factor, filter_down, flags, p4); },
+        out);
+  const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
+  // Every rank of a communicator must reach the min/max exchange, whatever happens to it before: a rank-local failure
+  // (an unknown filter, a trailing block the Sobel metric cannot take, no memory) joins with neutral values and an
+  // error flag instead of leaving its peers in the collective.
+  auto bail = [&](pxz_status why) -> pxz_status {
+    if (normalise && ctx->comm) {
+      const std::string msg = ctx->err;
+      bool peers_ok = true;
+      exchange_minmax(ctx, false, &peers_ok);
+      ctx->err = msg;
+    }
+    return why;
+  };
+  if ((int)filter_down < 0 || (int)filter_down > 4) return bail(fail(ctx, PXZ_E_ARG, "unknown filter"));
+  Geom g;
+  pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g, img->nimg);
+  if (st != PXZ_OK) return bail(st);
+  if (normalise && img->nimg > 1) return bail(fail(ctx, PXZ_E_UNSUPPORTED, "global normalisation is per image: not available on a batch"));
+  const uint32_t nblocks = g.cols * g.rows;
+
+  const ValueMap vm = shrink_value_map(ctx, metric, flags, factor);
+
+  // with global normalisation every value depends on the exact min and max, so the Oklab path
+  // runs in reference order for all blocks (DESIGN.md)
+  const bool exact_all = (flags & PXZ_FLAG_EXACT_VALUES) != 0;
+  // Global normalisation of the Oklab values on the fast path: the exact extremes come from the few tiles that can hold
+  // them, and the guard band (scaled by 1 / range) then decides as in the default mode which tiles need their
+  // reference-order value; with PXZ_FLAG_EXACT_VALUES every tile is computed in reference order as before.
+  const bool fast_norm = normalise && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
+  st = run_analysis(ctx, img, g, metric, exact_all, (metric == PXZ_METRIC_OKLAB_MAD && !exact_all && !normalise) ? &vm : nullptr);
+  if (st != PXZ_OK) return bail(st);
+
+  if (normalise) {
+    if ((st = run_minmax(ctx, metric, nblocks)) != PXZ_OK) return bail(st);
+    if (fast_norm && (st = run_exact_extremes(ctx, img, g, nblocks)) != PXZ_OK) return bail(st);
+    bool peers_ok = true;
+    st = exchange_minmax(ctx, true, &peers_ok);
+    if (st != PXZ_OK) return st;
+    if (!peers_ok) return fail(ctx, PXZ_E_NCCL, "another rank failed before the min/max exchange");
+    if (fast_norm && (st = run_guard_band(ctx, img, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
+  }
+  return plan_and_resample(ctx, img, g, metric, vm, filter_down, exact_all, out);
+}
+
+// Rate control (pxz_shrink_to_size).  bpp: bytes per pixel the budget counts (3 for an RGB image on the RGBA kernels).
+static pxz_status shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_bytes,
+                                 pxz_filter filter_down, uint32_t flags, uint32_t bpp, float* factor_out, pxz_payload** out) {
+  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh))
+    return encode_via_rgba(
+        ctx, img,
+        [&](const pxz_image* wide, pxz_payload** p4) {
+          return shrink_to_size(ctx, wide, bw, bh, metric, max_bytes, filter_down, flags, 3, factor_out, p4);
+        },
+        out);
+  if ((int)filter_down < 0 || (int)filter_down > 4) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (metric != PXZ_METRIC_OKLAB_MAD && metric != PXZ_METRIC_SOBEL_DIR) return fail(ctx, PXZ_E_ARG, "unknown metric");
+  if (flags & PXZ_FLAG_AFTER_IDENTITY) return fail(ctx, PXZ_E_ARG, "PXZ_FLAG_AFTER_IDENTITY ignores the factor: no size to choose");
+  if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "a size budget is per image: not available on a batch");
+  const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
+  if (normalise && ctx->comm)
+    return fail(ctx, PXZ_E_UNSUPPORTED, "a size budget with global normalisation over a communicator is not available");
+  Geom g;
+  pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g, img->nimg);
+  if (st != PXZ_OK) return st;
+  const uint32_t nblocks = g.cols * g.rows;
+  ValueMap vm = shrink_value_map(ctx, metric, flags, 1.0f);
+  const bool exact_all = (flags & PXZ_FLAG_EXACT_VALUES) != 0;
+  // fast Oklab values: sizes found on them are checked against the guard band before they are trusted
+  const bool fast = metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
+
+  // analysis as pxz_shrink runs it, without the guard band (it depends on the factor)
+  st = run_analysis(ctx, img, g, metric, exact_all, nullptr);
+  if (st != PXZ_OK) return st;
+  if (normalise) {
+    if ((st = run_minmax(ctx, metric, nblocks)) != PXZ_OK) return st;
+    if (fast && (st = run_exact_extremes(ctx, img, g, nblocks)) != PXZ_OK) return st;
+  }
+
+  // scratch: the sizes of one round, and on the fast path the copy of the values the search runs on
+  uint8_t* scratch = nullptr;
+  const size_t sizes_bytes = (size_t)kMaxSizeCandidates * sizeof(uint64_t);
+  if ((st = dev_alloc(ctx, (void**)&scratch, sizes_bytes + (fast ? (size_t)nblocks * 4 : 0))) != PXZ_OK) return st;
+  std::unique_ptr<uint8_t, std::function<void(uint8_t*)>> scratch_guard(scratch, [ctx](uint8_t* q) { dev_free(ctx, q); });
+  uint64_t* d_sizes = reinterpret_cast<uint64_t*>(scratch);
+  float* d_search = fast ? reinterpret_cast<float*>(scratch + sizes_bytes) : ctx->d_vx;
+  const float* d_search_y = metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr;
+  if (fast) PXZ_CUDA(ctx, cudaMemcpyAsync(d_search, ctx->d_vx, (size_t)nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+
+  constexpr uint32_t kMaxPattern = 0x7F7FFFFFu;  // FLT_MAX; patterns 1 .. kMaxPattern are the finite factors > 0
+  auto factor_of = [](uint32_t bits) {
+    float f;
+    memcpy(&f, &bits, 4);
+    return f;
+  };
+  uint64_t size_at_min = 0;  // payload at the smallest positive factor (pattern 1), once evaluated
+  std::vector<uint64_t> sizes(kMaxSizeCandidates);
+  auto evaluate = [&](const std::vector<uint32_t>& pats) -> pxz_status {
+    SizeCandidates cand;
+    cand.n = (uint32_t)pats.size();
+    for (size_t i = 0; i < pats.size(); ++i) cand.k[i] = factor_of(pats[i]);
+    {
+      ProfScope prof(ctx, K_SIZE_CURVE);
+      PXZ_CUDA(ctx, launch_size_curve(d_search, d_search_y, g, vm, ctx->d_minmax, ctx->thr, bpp, cand, d_sizes, ctx->stream, ctx->sm_count,
+                                      &ctx->launches));
+    }
+    PXZ_CUDA(ctx, cudaMemcpyAsync(sizes.data(), d_sizes, pats.size() * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+    PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    for (size_t i = 0; i < pats.size(); ++i)
+      if (pats[i] == 1u) size_at_min = sizes[i];
+    return PXZ_OK;
+  };
+  // The size is monotone in the factor (DESIGN.md §3), so the bit patterns that fit are a prefix of [1, kMaxPattern].
+  // lo fits (0: none known to), hi does not (kMaxPattern + 1: none known not to); each round evaluates up to 256 evenly
+  // spaced patterns strictly between them.
+  uint32_t k_bits = 0;
+  auto search = [&]() -> pxz_status {
+    uint32_t lo = 0, hi = kMaxPattern + 1;
+    while (hi - lo > 1) {
+      const uint32_t inner = hi - lo - 1;
+      const uint32_t n = std::min<uint32_t>(inner, kMaxSizeCandidates);
+      std::vector<uint32_t> pats(n);
+      for (uint32_t i = 0; i < n; ++i) pats[i] = lo + 1 + (n > 1 ? (uint32_t)((uint64_t)i * (inner - 1) / (n - 1)) : 0u);
+      if ((st = evaluate(pats)) != PXZ_OK) return st;
+      uint32_t new_lo = lo, new_hi = hi;
+      for (uint32_t i = 0; i < n; ++i) {
+        if (sizes[i] <= max_bytes) new_lo = pats[i];
+        else { new_hi = pats[i]; break; }
+      }
+      lo = new_lo;
+      hi = new_hi;
+    }
+    k_bits = lo;
+    return PXZ_OK;
+  };
+  for (;;) {
+    if ((st = search()) != PXZ_OK) return st;
+    if (!fast) break;
+    // The search ran on fast values.  Recompute, in reference order, the guard band of k and of the next factor up (band
+    // list from the untouched fast values, exact values into the search copy): both sizes are then exact.  When they do not
+    // bracket the budget, search again on the corrected copy — each failure replaced at least one value by its exact one.
+    std::vector<uint32_t> pats;
+    if (k_bits >= 1u) pats.push_back(k_bits);
+    if (k_bits < kMaxPattern) pats.push_back(k_bits + 1);
+    for (uint32_t bits : pats) {
+      ValueMap v = vm;
+      v.factor = factor_of(bits);
+      if ((st = run_guard_band(ctx, img, g, v, d_search, ctx->d_vx)) != PXZ_OK) return st;
+    }
+    if ((st = evaluate(pats)) != PXZ_OK) return st;
+    const bool fits = k_bits < 1u || sizes[0] <= max_bytes;
+    const bool next_over = k_bits >= kMaxPattern || sizes[pats.size() - 1] > max_bytes;
+    if (fits && next_over) break;
+  }
+  if (k_bits == 0)
+    return fail(ctx, PXZ_E_ARG, "max_bytes " + std::to_string(max_bytes) + " is below the payload at the smallest positive factor (" +
+                                    std::to_string(size_at_min) + " bytes)");
+  const float k = factor_of(k_bits);
+  // encode at k exactly as pxz_shrink does, from the fast values
+  vm.factor = k;
+  if (fast && (st = run_guard_band(ctx, img, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
+  st = plan_and_resample(ctx, img, g, metric, vm, filter_down, exact_all, out);
+  if (st == PXZ_OK) *factor_out = k;
+  return st;
+}
+
+pxz_status pxz_shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_bytes,
+                              pxz_filter filter_down, uint32_t flags, float* factor_out, pxz_payload** out) {
+  if (!ctx || !img || !out || !factor_out) return PXZ_E_ARG;
+  *out = nullptr;
+  cudaSetDevice(ctx->device);
+  return shrink_to_size(ctx, img, bw, bh, metric, max_bytes, filter_down, flags, img->c, factor_out, out);
 }
 
 // host restatement of the plan kernel's scalar path (same threshold table)

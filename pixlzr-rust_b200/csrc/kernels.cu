@@ -1256,6 +1256,69 @@ __global__ void __launch_bounds__(kThreads) k_plan(const float* __restrict__ vx,
 }
 
 // ------------------------------------------------------------------------------------------------
+// size curve (rate control, pxz_shrink_to_size): for each of M candidate factors, the payload size k_plan would compute
+// from one set of raw values, through the same value -> dims helpers (map_values, parse_value_dev, level_k, scaled_dim).  A thread keeps kSizeItems blocks' values and tile sizes in registers and walks the
+// candidates of its CTA (blockIdx.y splits them when the image has too few blocks to fill the device); per candidate a
+// warp sum, the warps' partial sums in shared memory, then one 64-bit atomicAdd per CTA and candidate.  Integer sums: the
+// result does not depend on the order of the additions.  bytes[] is zero on entry.
+// ------------------------------------------------------------------------------------------------
+constexpr int kSizeItems = 4;
+__global__ void __launch_bounds__(kThreads) k_size_curve(const float* __restrict__ vx, const float* __restrict__ vy, Geom g,
+                                                         ValueMap vm, const float* __restrict__ minmax, LevelThresholds thr,
+                                                         uint32_t bpp, SizeCandidates cand, unsigned long long* __restrict__ bytes) {
+  __shared__ float s_k[kMaxSizeCandidates];
+  __shared__ unsigned long long s_part[kThreads / 32][kMaxSizeCandidates];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t per = (cand.n + gridDim.y - 1) / gridDim.y;
+  const uint32_t c0 = blockIdx.y * per, c1 = min(cand.n, c0 + per);
+  for (uint32_t c = c0 + tid; c < c1; c += kThreads) s_k[c - c0] = cand.k[c];
+  float mm[4] = {0.f, 0.f, 0.f, 0.f};
+  if (vm.normalise)
+#pragma unroll
+    for (int i = 0; i < 4; ++i) mm[i] = minmax[i];
+  const uint32_t nblocks = g.cols * g.rows;
+  float rx[kSizeItems], ry[kSizeItems];
+  uint32_t tw[kSizeItems], th[kSizeItems];
+#pragma unroll
+  for (int j = 0; j < kSizeItems; ++j) {
+    const uint32_t b = (blockIdx.x * kSizeItems + j) * kThreads + tid;
+    tw[j] = th[j] = 0u;  // no block: contributes nothing
+    rx[j] = ry[j] = 0.f;
+    if (b < nblocks) {
+      const Tile t = tile_of(g, b);
+      tw[j] = t.tw;
+      th[j] = t.th;
+      rx[j] = vx[b];
+      ry[j] = vy ? vy[b] : rx[j];
+    }
+  }
+  __syncthreads();
+  for (uint32_t c = c0; c < c1; ++c) {
+    ValueMap v = vm;
+    v.factor = s_k[c - c0];
+    unsigned long long px = 0;
+#pragma unroll
+    for (int j = 0; j < kSizeItems; ++j) {
+      float v0, v1;
+      map_values(v, mm, rx[j], ry[j], v0, v1);
+      const uint32_t dw = scaled_dim(tw[j], level_k(parse_value_dev(v0), thr));
+      const uint32_t dh = scaled_dim(th[j], level_k(parse_value_dev(v1), thr));
+      if (tw[j] != 0u) px += (unsigned long long)dw * dh;
+    }
+#pragma unroll
+    for (int o = 16; o > 0; o >>= 1) px += __shfl_xor_sync(0xffffffffu, px, o);
+    if (lane == 0) s_part[warp][c - c0] = px;
+  }
+  __syncthreads();
+  for (uint32_t c = c0 + tid; c < c1; c += kThreads) {
+    unsigned long long s = 0;
+#pragma unroll
+    for (int w = 0; w < kThreads / 32; ++w) s += s_part[w][c - c0];
+    if (s != 0ull) atomicAdd(&bytes[c], s * bpp);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
 // window of a payload (random access): the blocks of columns [c0, c0 + g.cols) x rows [r0, r0 + g.rows) of a parent payload
 // with `pcols` columns, as the payload of the sub-image they tile (geometry g).  One lane of warp 0 per window block takes
 // the parent's descriptor and table indices, the block sizes are scanned as in k_plan (same look-back, same work-order
@@ -2479,6 +2542,21 @@ cudaError_t launch_plan(const float* vx, const float* vy, const Geom& g, const V
   if (adaptive) e = launch_pdl(k_plan<true>, tiles, kThreads, 0, s, vx, vy, g, vm, minmax, thr, mask, descs, tabidx, total, st, cursor, lists, cap, lut, tabidx_up);
   else e = launch_pdl(k_plan<false>, tiles, kThreads, 0, s, vx, vy, g, vm, minmax, thr, mask, descs, tabidx, total, st, cursor, lists, cap, lut, tabidx_up);
   return e != cudaSuccess ? e : cudaGetLastError();
+}
+
+cudaError_t launch_size_curve(const float* vx, const float* vy, const Geom& g, const ValueMap& vm, const float* minmax,
+                              const LevelThresholds& thr, uint32_t bpp, const SizeCandidates& cand, uint64_t* bytes, cudaStream_t s,
+                              int sm_count, uint64_t* launches) {
+  if (cand.n == 0 || cand.n > (uint32_t)kMaxSizeCandidates) return cudaErrorInvalidValue;
+  cudaError_t e = cudaMemsetAsync(bytes, 0, (size_t)cand.n * sizeof(uint64_t), s);
+  if (e != cudaSuccess) return e;
+  const uint32_t nblocks = g.cols * g.rows;
+  const int gx = clamp_grid(((long long)nblocks + kThreads * kSizeItems - 1) / (kThreads * kSizeItems), 1ll << 30);
+  // few blocks: split the candidates over more CTAs (at least 8 candidates per CTA) to fill the SMs
+  const int gy = clamp_grid(std::min<long long>((long long)sm_count * 2 / gx, cand.n / 8), 32);
+  ++*launches;
+  k_size_curve<<<dim3(gx, gy), kThreads, 0, s>>>(vx, vy, g, vm, minmax, thr, bpp, cand, reinterpret_cast<unsigned long long*>(bytes));
+  return cudaGetLastError();
 }
 
 size_t window_scan_state_bytes(uint32_t nblocks) {

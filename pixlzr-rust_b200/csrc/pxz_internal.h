@@ -123,6 +123,16 @@ cudaError_t launch_plan(const float* vx, const float* vy, const Geom& g, const V
                         const LevelThresholds& thr, const uint8_t* mask, pxz_block_desc* descs, uint32_t* tabidx,
                         uint64_t* total_bytes, void* scan_state, uint32_t* lists, uint32_t cap, cudaStream_t s,
                         uint64_t* launches, const StrategyLut* strategy = nullptr, uint32_t* tabidx_up = nullptr);
+// Payload sizes k_plan would compute (mask = NULL) for each of cand.n factors: bytes[i] = sum over blocks of w' * h' * bpp
+// with the factor vm.factor replaced by cand.k[i].  bpp: bytes per pixel counted (3 for an RGB image on the RGBA kernels).
+constexpr int kMaxSizeCandidates = 256;
+struct SizeCandidates {
+  uint32_t n;
+  float k[kMaxSizeCandidates];
+};
+cudaError_t launch_size_curve(const float* vx, const float* vy, const Geom& g, const ValueMap& vm, const float* minmax,
+                              const LevelThresholds& thr, uint32_t bpp, const SizeCandidates& cand, uint64_t* bytes, cudaStream_t s,
+                              int sm_count, uint64_t* launches);
 // Work order of the warp-per-tile resample kernels: lists[c * cap + i], c < 8, = the blocks of cost class c (0 = most
 // expensive), lists[8 * cap + c] = how many.  launch_plan fills them; this entry point does the same for descriptors
 // that came from the host.
