@@ -194,6 +194,37 @@ pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t 
 pxz_status pxz_shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_bytes,
                               pxz_filter filter_down, uint32_t flags, float* factor_out, pxz_payload** out);
 
+/* ---- decode error and strategy fit (EXTENSION: the reference has no error measure; its author's filter-pair experiment,
+ * strategies.txt, was run outside the crate) ---------------------------------------------------------------------------
+ * Per-block error between two images of one geometry (w, h, channels; not batches) on the block grid (bw, bh) of pxz_grid:
+ * sse[b] = sum over the tile's pixels and channels of (a - b)^2 (exact, u64), max[b] = max |a - b| over the same.  Integer
+ * arithmetic: the result does not depend on the order of the sums.  Each output may be NULL; *total_sse = sum of sse[b].
+ * Host arrays hold cols*rows entries in row-major order.  PSNR = 10 log10(255^2 * w * h * channels / total_sse).
+ * PXZ_E_ARG: geometry mismatch, block size 0.  PXZ_E_UNSUPPORTED: a batch image. */
+pxz_status pxz_image_error(pxz_ctx* ctx, const pxz_image* a, const pxz_image* b, uint32_t bw, uint32_t bh,
+                           uint64_t* host_block_sse, uint8_t* host_block_max, uint64_t* host_total_sse);
+
+#define PXZ_FILTER_PAIRS 25 /* pair index = down * 5 + up */
+/* For every (down, up) filter pair: the error of pxz_expand_to_image(pxz_shrink(img, bw, bh, metric, factor, down, flags), up)
+ * against img, summed per strategy bucket of the block's stored value.  host_sse[bucket * 25 + pair] (65 * 25 u64),
+ * host_blocks[bucket] (65 u32): filled, not accumulated.  A block's shrink + expand depends only on its tile, its dims and its
+ * filter pair, so the error of any per-bucket table is the sum of these entries.  The bucket of each block is the one its
+ * reference-order stored value gives, in every mode (every bucket edge is resolved in the guard band of the fast Oklab path),
+ * so flags 0 and PXZ_FLAG_EXACT_VALUES return identical reports.  The context's strategy is not used and is left installed.
+ * One analysis, 5 shrinks, 25 expands and error passes; only the report crosses to the host.
+ * PXZ_E_ARG as pxz_shrink (unknown metric, Sobel trailing tile, ...).  PXZ_E_UNSUPPORTED: a batch image,
+ * PXZ_FLAG_NORMALISE_GLOBAL on a context with a communicator. */
+pxz_status pxz_strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
+                                uint32_t flags, uint64_t* host_sse, uint32_t* host_blocks);
+/* Host: the table that minimises the summed error per bucket.  down[b], up[b] = the pair of least sse[b][*]; on a tie base's
+ * pair if it is among the least, else the lowest pair index; a bucket with blocks[b] == 0 keeps base's pair.  base == NULL
+ * means pxz_strategy_by_level.  Reports of several images can be added element-wise before this call.
+ * Installed with pxz_ctx_set_strategy in the default (reference-order) resample arithmetic, the table's pxz_shrink ->
+ * pxz_expand_to_image -> pxz_image_error total is exactly sum over b of sse[b][down[b] * 5 + up[b]], which is <= the total of
+ * every uniform pair and of base.  With pxz_ctx_set_fast_resample(1) pixels are within +-1 LSB and that equality does not hold.
+ * PXZ_E_ARG: a NULL sse / blocks / out, an unknown filter in base. */
+pxz_status pxz_strategy_choose(const uint64_t* sse, const uint32_t* blocks, const pxz_strategy* base, pxz_strategy* out);
+
 /* Scalar part of reduce_image_section (operations.rs:128-156) on the host: (v0, v1) after `after`
  * -> parse_value -> level -> reduced size of a w x h block and the stored block value.  Uses the
  * same threshold table as the device plan kernel. */

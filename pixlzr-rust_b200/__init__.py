@@ -8,16 +8,21 @@ Layout
   build.py     in-tree nvcc build
 """
 from .api import (  # noqa: F401
+    ErrorReport,
     FilterType,
     Pixlzr,
     PixlzrBlock,
     Strategy,
+    StrategyReport,
     get_block_variance,
     get_block_variance_directionally,
+    image_error,
     parse_shrinking_factor,
+    payload_error,
     process,
     process_by_strategy,
     process_custom,
+    psnr_of,
     reduce_image_section,
     tree_process,
     tree_process_custom,

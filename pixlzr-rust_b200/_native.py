@@ -87,6 +87,9 @@ SYMBOLS = {
     "pxz_expand_region": (_i, [_vp, _vp, _i, _u32, _u32, _u32, _u32, _vp]),
     "pxz_container_header": (_i, [_vp, _sz, _P(_u32), _P(_u32), _P(_u32), _P(_u32), _P(C.c_int32)]),
     "pxz_container_crop": (C.c_int64, [_vp, _sz, _u32, _u32, _u32, _u32, _vp, _sz]),
+    "pxz_image_error": (_i, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _P(_u64)]),
+    "pxz_strategy_measure": (_i, [_vp, _vp, _u32, _u32, _i, C.c_float, _u32, _vp, _vp]),
+    "pxz_strategy_choose": (_i, [_vp, _vp, _vp, _vp]),
 }
 
 
@@ -140,6 +143,29 @@ def strategy_by_level():
     if rc != 0:
         raise RuntimeError(f"pxz_strategy_by_level failed ({rc})")
     return buf[:STRATEGY_BUCKETS].copy(), buf[STRATEGY_BUCKETS:].copy()
+
+
+FILTER_PAIRS = 25  # pair index = down * 5 + up
+
+
+def strategy_choose(sse: np.ndarray, blocks: np.ndarray, base=None):
+    """(down, up) uint8[65]: per bucket the (down, up) pair of least summed error in a strategy_measure report (summed over
+    any number of images); ties keep base's pair, else the lowest pair index; empty buckets keep base's pair.  base: (down,
+    up) or None for strategy_by_level (pxz_strategy_choose)."""
+    sse = np.ascontiguousarray(sse, np.uint64)
+    blocks = np.ascontiguousarray(blocks, np.uint32)
+    if sse.size != STRATEGY_BUCKETS * FILTER_PAIRS or blocks.size != STRATEGY_BUCKETS:
+        raise ValueError(f"a report has {STRATEGY_BUCKETS} x {FILTER_PAIRS} sums and {STRATEGY_BUCKETS} counts")
+    basebuf = None
+    if base is not None:
+        basebuf = np.concatenate([np.asarray(base[0], np.uint8).reshape(-1), np.asarray(base[1], np.uint8).reshape(-1)])
+        if basebuf.size != 2 * STRATEGY_BUCKETS:
+            raise ValueError(f"a strategy has {STRATEGY_BUCKETS} entries per direction")
+    out = np.zeros(2 * STRATEGY_BUCKETS, np.uint8)
+    st = lib().pxz_strategy_choose(ptr(sse), ptr(blocks), ptr(basebuf), ptr(out))
+    if st != OK:
+        raise PixlzrError(st, "pxz_strategy_choose")
+    return out[:STRATEGY_BUCKETS].copy(), out[STRATEGY_BUCKETS:].copy()
 
 
 class PinnedBuffer:
@@ -359,6 +385,25 @@ class Image:
                                                 C.byref(k), C.byref(h)))
         return Payload(self.ctx, h), float(k.value)
 
+    def error(self, other: "Image", bw: int, bh: int):
+        """(block_sse uint64 [rows, cols], block_max uint8 [rows, cols], total_sse): the squared error and the largest
+        difference of every tile of the (bw, bh) grid between this image and `other` (pxz_image_error; exact)."""
+        cols, rows = grid(self.w, self.h, bw, bh)
+        sse = np.empty((rows, cols), np.uint64)
+        mx = np.empty((rows, cols), np.uint8)
+        total = C.c_uint64()
+        self.ctx.check(lib().pxz_image_error(self.ctx.handle, self._h, other.handle, bw, bh, ptr(sse), ptr(mx), C.byref(total)))
+        return sse, mx, int(total.value)
+
+    def strategy_measure(self, bw: int, bh: int, metric: int, factor: float, flags: int = 0):
+        """(sse uint64 [65, 25], blocks uint32 [65]): for every (down, up) pair (index down * 5 + up) the error of
+        expand(shrink(self, ..., down, flags), up) against this image, summed per strategy bucket of the stored block
+        values, and the block count per bucket (pxz_strategy_measure)."""
+        sse = np.zeros((STRATEGY_BUCKETS, FILTER_PAIRS), np.uint64)
+        blocks = np.zeros(STRATEGY_BUCKETS, np.uint32)
+        self.ctx.check(lib().pxz_strategy_measure(self.ctx.handle, self._h, bw, bh, metric, factor, flags, ptr(sse), ptr(blocks)))
+        return sse, blocks
+
     def tree_process(self, threshold: float, bw: int, bh: int, min_bw: int, min_bh: int, filter_down: int, filter_up: int,
                      out: "Image"):
         self.ctx.check(lib().pxz_tree_process(self.ctx.handle, self._h, threshold, bw, bh, min_bw, min_bh, int(filter_down),
@@ -439,6 +484,16 @@ class Payload:
 
     def expand_to_image(self, filter_up: int, out: Image):
         self.ctx.check(lib().pxz_expand_to_image(self.ctx.handle, self._h, int(filter_up), out.handle))
+
+    def error(self, source: Image, filter_up: int):
+        """Image.error of the decode (expand_to_image into a scratch image) against `source`, on this payload's block grid."""
+        i = self.info()
+        img = self.ctx.image_alloc(i["w"], i["h"], i["channels"])
+        try:
+            self.expand_to_image(filter_up, img)
+            return img.error(source, i["bw"], i["bh"])
+        finally:
+            img.free()
 
     # ---- random access (extension) -----------------------------------------------------------------------
     def window(self, c0: int, r0: int, nc: int, nr: int) -> "Payload":

@@ -143,6 +143,106 @@ class Strategy:
     def bucket(value: float) -> int:
         return N.strategy_bucket(value)
 
+    @classmethod
+    def fit(cls, images, block_width: int, block_height: int, factor: float, directionally: bool = False,
+            exact_values: bool = False, base: Optional["Strategy"] = None,
+            ctx: Optional[N.Context] = None) -> Tuple["Strategy", "StrategyReport"]:
+        """EXTENSION: the table of least summed error over `images` (numpy images) for shrink_by (or shrink_directionally)
+        with `factor` at this block size: every (down, up) pair is measured on the device per value bucket
+        (pxz_strategy_measure), the reports are added and each bucket takes its best pair (pxz_strategy_choose; ties and
+        empty buckets keep `base`'s pair, default by_level).  Returns the table and the summed report; report.total(table)
+        is the exact error of the table's decodes in the default resample arithmetic."""
+        ctx = ctx or default_context()
+        metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
+        flags = N.FLAG_EXACT_VALUES if exact_values else 0
+        sse = np.zeros((N.STRATEGY_BUCKETS, N.FILTER_PAIRS), np.uint64)
+        blocks = np.zeros(N.STRATEGY_BUCKETS, np.uint32)
+        for image in images:
+            img = ctx.image_upload(_check_image(image))
+            try:
+                s, b = img.strategy_measure(block_width, block_height, metric, factor, flags)
+            finally:
+                img.free()
+            sse += s
+            blocks += b
+        down, up = N.strategy_choose(sse, blocks, None if base is None else (base.down, base.up))
+        return cls(down, up), StrategyReport(sse, blocks)
+
+
+@dataclass
+class StrategyReport:
+    """What pxz_strategy_measure returns (summed over images): sse[bucket, down * 5 + up] = the squared error of the blocks
+    of that bucket when shrunk with `down` and expanded with `up`; blocks[bucket] = how many blocks the bucket holds."""
+    sse: np.ndarray     # uint64 [65, 25]
+    blocks: np.ndarray  # uint32 [65]
+
+    def total(self, strategy: Strategy) -> int:
+        """The squared error of a decode with `strategy` installed: the sum of each bucket's entry for its pair."""
+        pairs = strategy.down.astype(np.int64) * 5 + strategy.up.astype(np.int64)
+        return int(sum(int(self.sse[b, pairs[b]]) for b in range(N.STRATEGY_BUCKETS)))
+
+
+def psnr_of(total_sse: int, samples: int) -> float:
+    """10 log10(255^2 * samples / total_sse) in dB (samples = width * height * channels); inf for identical images."""
+    if total_sse == 0:
+        return float("inf")
+    return 10.0 * float(np.log10(255.0 * 255.0 * samples / float(total_sse)))
+
+
+@dataclass
+class ErrorReport:
+    """EXTENSION: the error of one image against another, per block of a grid (pxz_image_error)."""
+    block_sse: np.ndarray  # uint64 [rows, cols]: sum of (a - b)^2 over the tile's pixels and channels
+    block_max: np.ndarray  # uint8 [rows, cols]: max |a - b| over the same
+    total_sse: int
+    samples: int           # width * height * channels
+
+    @property
+    def mse(self) -> float:
+        return self.total_sse / self.samples
+
+    @property
+    def psnr(self) -> float:
+        return psnr_of(self.total_sse, self.samples)
+
+    @property
+    def max_error(self) -> int:
+        return int(self.block_max.max()) if self.block_max.size else 0
+
+
+def image_error(a, b, block_width: int, block_height: int, ctx: Optional[N.Context] = None) -> ErrorReport:
+    """EXTENSION: per-block squared error and largest difference of `a` against `b` (numpy images or device images of one
+    geometry), computed on the device in one streaming pass; only the per-block figures come back."""
+    ctx = ctx or (a.ctx if isinstance(a, N.Image) else default_context())
+    owned = []
+
+    def on_device(x):
+        if isinstance(x, N.Image):
+            return x
+        owned.append(ctx.image_upload(_check_image(x)))
+        return owned[-1]
+
+    try:
+        da, db = on_device(a), on_device(b)
+        sse, mx, total = da.error(db, block_width, block_height)
+        return ErrorReport(sse, mx, total, da.w * da.h * da.c)
+    finally:
+        for x in owned:
+            x.free()
+
+
+def payload_error(payload: N.Payload, source, filter_up: FilterType) -> ErrorReport:
+    """EXTENSION: the error of a payload's decode with `filter_up` against its source image (numpy or device image), on the
+    payload's block grid (Payload.error): the decode stays on the device."""
+    ctx = payload.ctx
+    src = source if isinstance(source, N.Image) else ctx.image_upload(_check_image(source))
+    try:
+        sse, mx, total = payload.error(src, int(filter_up))
+        return ErrorReport(sse, mx, total, src.w * src.h * src.c)
+    finally:
+        if src is not source:
+            src.free()
+
 
 class Pixlzr:
     """struct Pixlzr (pixlzr.rs:17-25).  Holds either the source image (blocks = tiles, no values) or

@@ -43,6 +43,10 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--payload-bytes", type=parse_payload_bytes, default=None, metavar="N",
                    help="Shrink with the largest factor whose block payload has at most N bytes, and print that factor "
                         "(image input, with --force; replaces -k)")
+    # extension (decode error): not a flag of the reference
+    p.add_argument("--psnr", action="store_true",
+                   help="Decode what was written (with -f), compare it with the input image on the device and print the PSNR "
+                        "and the largest difference (image input only)")
     return p
 
 
@@ -87,6 +91,13 @@ def payload_bytes_error(args) -> Optional[str]:
         return "--payload-bytes chooses the shrinking factor: it cannot be combined with -k"
     if args.region is not None:
         return "--payload-bytes does not apply to a region decode"
+    return None
+
+
+def psnr_error(args) -> Optional[str]:
+    """Why --psnr does not apply to these arguments, or None."""
+    if getattr(args, "psnr", False) and operation(args.input, args.output)[0] != "image":
+        return "--psnr compares the decoded output with the input image: the input must be an image, not a container"
     return None
 
 
@@ -148,7 +159,7 @@ def run(args) -> None:
     filt = FILTERS[args.filter]
     shrink_by = api.parse_shrinking_factor(args.shrinking_factor)
     src, dst = operation(args.input, args.output)
-    err = region_error(args) or payload_bytes_error(args)
+    err = region_error(args) or payload_bytes_error(args) or psnr_error(args)
     if err:
         raise ValueError(err)
     if args.payload_bytes is not None:
@@ -199,14 +210,38 @@ def _run_sized(args, bw: int, bh: int, filt, src: str, dst: str) -> None:
     print(f"shrinking factor: {api.format_shrinking_factor(k)}")
 
 
+def format_psnr(psnr: float) -> str:
+    return "inf" if psnr == float("inf") else f"{psnr:.6f}"
+
+
+def report_psnr(args) -> None:
+    """Decodes the written output with -f and prints its error against the input image (computed on the device)."""
+    bw = args.block_width
+    bh = args.block_height if args.block_height is not None else bw
+    source = _open_image(args.input)
+    if operation(args.input, args.output)[1] == "pix":
+        ctx = api.default_context()
+        with open(args.output, "rb") as f:
+            pl, _ = ctx.payload_from_container(f.read())
+        try:
+            rep = api.payload_error(pl, source, FILTERS[args.filter])
+        finally:
+            pl.free()
+    else:
+        rep = api.image_error(_open_image(args.output), source, bw, bh)
+    print(f"psnr: {format_psnr(rep.psnr)} dB, max error: {rep.max_error}")
+
+
 def main(argv: Optional[List[str]] = None) -> int:
     args = parse_args(argv)
-    err = region_error(args) or payload_bytes_error(args)
+    err = region_error(args) or payload_bytes_error(args) or psnr_error(args)
     if err:
         print(f"pixlzr: {err}", file=sys.stderr)
         return 2
     try:
         run(args)
+        if args.psnr:
+            report_psnr(args)
     except FileNotFoundError as e:
         print(f"Could not open the image [ {e.filename} ]", file=sys.stderr)
         return 1

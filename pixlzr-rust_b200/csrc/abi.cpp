@@ -48,10 +48,11 @@ using TabKey = std::tuple<std::vector<uint32_t>, std::vector<uint32_t>, int, int
 
 // K_REGION_COPY times the device-to-device copy of pxz_expand_region out of its staging image (not a kernel)
 enum KernelId { K_MAD_FAST = 0, K_MAD_EXACT, K_SOBEL, K_MINMAX, K_PLAN, K_RESAMPLE_DOWN, K_RESAMPLE_UP, K_QOI_ENCODE, K_QOI_DECODE,
-                K_PAYLOAD_WINDOW, K_REGION_COPY, K_SIZE_CURVE, K_COUNT };
+                K_PAYLOAD_WINDOW, K_REGION_COPY, K_SIZE_CURVE, K_BLOCK_ERROR, K_BUCKET_SUM, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"analyze_mad_fast", "mad_exact",      "analyze_sobel", "minmax",
                                            "plan",             "resample_down",  "resample_up",   "qoi_encode",
-                                           "qoi_decode",       "payload_window", "region_copy",   "size_curve"};
+                                           "qoi_decode",       "payload_window", "region_copy",   "size_curve",
+                                           "block_error",      "bucket_sum"};
 struct ProfRec {
   int id;
   cudaEvent_t a, b;
@@ -887,20 +888,26 @@ static pxz_status payload_rechannel(pxz_ctx* ctx, const pxz_payload* src, uint32
 // An RGB image on the RGBA fast kernels: widen it to RGBA (alpha 255: its metric term is exactly +0 and the opaque resample
 // path never touches it), run `encode` on the 4-channel image, narrow the payload back
 extern "C++" {  // a template inside the extern "C" block
+static pxz_status rgb_widened(pxz_ctx* ctx, const pxz_image* img, pxz_image** wide) {
+  pxz_status st = pxz_image_alloc_batch(ctx, img->w, img->h, 4, img->nimg, wide);
+  if (st != PXZ_OK) return st;
+  cudaError_t e = launch_rgb_widen(img->d, img->pitch, (*wide)->d, (*wide)->pitch, img->w, img->h * img->nimg, 1, ctx->stream, ctx->sm_count,
+                                   &ctx->launches);
+  if (e != cudaSuccess) {
+    cudaGetLastError();
+    pxz_image_free(*wide);
+    *wide = nullptr;
+    return fail(ctx, PXZ_E_CUDA, std::string("rgb widen: ") + cudaGetErrorString(e));
+  }
+  return PXZ_OK;
+}
 template <class F>
 static pxz_status encode_via_rgba(pxz_ctx* ctx, const pxz_image* img, F&& encode, pxz_payload** out) {
   pxz_image* wide = nullptr;
-  pxz_status st = pxz_image_alloc_batch(ctx, img->w, img->h, 4, img->nimg, &wide);
+  pxz_status st = rgb_widened(ctx, img, &wide);
   if (st != PXZ_OK) return st;
-  cudaError_t e = launch_rgb_widen(img->d, img->pitch, wide->d, wide->pitch, img->w, img->h * img->nimg, 1, ctx->stream, ctx->sm_count,
-                                   &ctx->launches);
   pxz_payload* p4 = nullptr;
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    st = fail(ctx, PXZ_E_CUDA, std::string("rgb widen: ") + cudaGetErrorString(e));
-  } else {
-    st = encode(wide, &p4);
-  }
+  st = encode(wide, &p4);
   pxz_image_free(wide);  // stream-ordered: the kernels queued above keep it
   if (st != PXZ_OK) return st;
   st = payload_rechannel(ctx, p4, 3, out);
@@ -1198,6 +1205,168 @@ pxz_status pxz_shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, u
   *out = nullptr;
   cudaSetDevice(ctx->device);
   return shrink_to_size(ctx, img, bw, bh, metric, max_bytes, filter_down, flags, img->c, factor_out, out);
+}
+
+// ---- decode error and strategy fit (extension) -------------------------------------------------------------------
+// per-block error of a against b on the grid g into d_sse (and d_max, if given): both cleared first
+static pxz_status run_block_error(pxz_ctx* ctx, const pxz_image* a, const pxz_image* b, const Geom& g, uint64_t* d_sse, uint32_t* d_max) {
+  const size_t nblocks = (size_t)g.cols * g.rows;
+  PXZ_CUDA(ctx, cudaMemsetAsync(d_sse, 0, nblocks * sizeof(uint64_t), ctx->stream));
+  if (d_max) PXZ_CUDA(ctx, cudaMemsetAsync(d_max, 0, nblocks * sizeof(uint32_t), ctx->stream));
+  ProfScope prof(ctx, K_BLOCK_ERROR);
+  PXZ_CUDA(ctx, launch_block_error(a->d, a->pitch, b->d, b->pitch, g, d_sse, d_max, ctx->stream, ctx->sm_count, &ctx->launches));
+  return PXZ_OK;
+}
+
+pxz_status pxz_image_error(pxz_ctx* ctx, const pxz_image* a, const pxz_image* b, uint32_t bw, uint32_t bh, uint64_t* host_block_sse,
+                           uint8_t* host_block_max, uint64_t* host_total_sse) {
+  if (!ctx || !a || !b) return PXZ_E_ARG;
+  cudaSetDevice(ctx->device);
+  if (a->nimg != 1 || b->nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "the error of a batch image is not supported");
+  if (a->w != b->w || a->h != b->h || a->c != b->c) return fail(ctx, PXZ_E_ARG, "image geometry mismatch");
+  Geom g;
+  pxz_status st = make_geom(ctx, a->w, a->h, a->c, bw, bh, &g);
+  if (st != PXZ_OK) return st;
+  const size_t nblocks = (size_t)g.cols * g.rows;
+  uint8_t* buf = nullptr;
+  if ((st = dev_alloc(ctx, (void**)&buf, nblocks * (sizeof(uint64_t) + sizeof(uint32_t)))) != PXZ_OK) return st;
+  std::unique_ptr<uint8_t, std::function<void(uint8_t*)>> buf_guard(buf, [ctx](uint8_t* q) { dev_free(ctx, q); });
+  uint64_t* d_sse = reinterpret_cast<uint64_t*>(buf);
+  uint32_t* d_max = reinterpret_cast<uint32_t*>(buf + nblocks * sizeof(uint64_t));
+  if ((st = run_block_error(ctx, a, b, g, d_sse, host_block_max ? d_max : nullptr)) != PXZ_OK) return st;
+  // the total is summed on the host from the block sums (cols * rows words; the grid is what the caller asked for)
+  std::vector<uint64_t> sse(nblocks);
+  std::vector<uint32_t> mx(host_block_max ? nblocks : 0);
+  PXZ_CUDA(ctx, cudaMemcpyAsync(sse.data(), d_sse, nblocks * sizeof(uint64_t), cudaMemcpyDeviceToHost, ctx->stream));
+  if (host_block_max) PXZ_CUDA(ctx, cudaMemcpyAsync(mx.data(), d_max, nblocks * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  uint64_t total = 0;
+  for (size_t i = 0; i < nblocks; ++i) total += sse[i];
+  if (host_block_sse) memcpy(host_block_sse, sse.data(), nblocks * sizeof(uint64_t));
+  if (host_block_max)
+    for (size_t i = 0; i < nblocks; ++i) host_block_max[i] = (uint8_t)mx[i];
+  if (host_total_sse) *host_total_sse = total;
+  return PXZ_OK;
+}
+
+// pxz_strategy_measure after the checks, with the context's strategy cleared: one analysis, then for each down filter the plan
+// + resample of pxz_shrink and for each up filter an expand into one scratch image and the error / bucket passes
+static pxz_status strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
+                                   uint32_t flags, uint64_t* host_sse, uint32_t* host_blocks) {
+  // An RGB image that pxz_shrink runs on the RGBA kernels is measured as its RGBA widening: the payloads are then the 4-channel
+  // payloads pxz_shrink narrows, and the decodes those pxz_expand_to_image narrows.  The alpha channel is 255 in the source and
+  // in every decode, so it adds 0 to every sum and the report equals that of the 3-channel image.
+  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
+    pxz_image* wide = nullptr;
+    pxz_status st = rgb_widened(ctx, img, &wide);
+    if (st != PXZ_OK) return st;
+    st = strategy_measure(ctx, wide, bw, bh, metric, factor, flags, host_sse, host_blocks);
+    pxz_image_free(wide);
+    return st;
+  }
+  Geom g;
+  pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g);
+  if (st != PXZ_OK) return st;
+  const uint32_t nblocks = g.cols * g.rows;
+  // Every bucket edge is resolved in the guard band, so the bucket of every block is the one its reference-order value gives
+  // (DESIGN.md §3); the dims are those of pxz_shrink in every mode
+  ValueMap vm = shrink_value_map(ctx, metric, flags, factor);
+  vm.bucket_edges = ~0ull;
+  const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
+  const bool exact_all = (flags & PXZ_FLAG_EXACT_VALUES) != 0;
+  const bool fast_norm = normalise && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
+  st = run_analysis(ctx, img, g, metric, exact_all, (metric == PXZ_METRIC_OKLAB_MAD && !exact_all && !normalise) ? &vm : nullptr);
+  if (st != PXZ_OK) return st;
+  if (normalise) {
+    if ((st = run_minmax(ctx, metric, nblocks)) != PXZ_OK) return st;
+    if (fast_norm && (st = run_exact_extremes(ctx, img, g, nblocks)) != PXZ_OK) return st;
+    if (fast_norm && (st = run_guard_band(ctx, img, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
+  }
+  // device scratch: the report (65 x 25 sums, 65 counts), the block errors of one pair
+  const size_t report_sse = (size_t)kStrategyBuckets * kFilterPairs * sizeof(uint64_t);
+  const size_t report_bytes = report_sse + kStrategyBuckets * sizeof(uint32_t);
+  const size_t block_sse_off = (report_bytes + 7) & ~(size_t)7;
+  uint8_t* buf = nullptr;
+  if ((st = dev_alloc(ctx, (void**)&buf, block_sse_off + (size_t)nblocks * sizeof(uint64_t))) != PXZ_OK) return st;
+  std::unique_ptr<uint8_t, std::function<void(uint8_t*)>> buf_guard(buf, [ctx](uint8_t* q) { dev_free(ctx, q); });
+  uint64_t* d_sse = reinterpret_cast<uint64_t*>(buf);
+  uint32_t* d_blocks = reinterpret_cast<uint32_t*>(buf + report_sse);
+  uint64_t* d_block_sse = reinterpret_cast<uint64_t*>(buf + block_sse_off);
+  PXZ_CUDA(ctx, cudaMemsetAsync(buf, 0, report_bytes, ctx->stream));
+  pxz_image* dec = nullptr;
+  if ((st = pxz_image_alloc(ctx, img->w, img->h, img->c, &dec)) != PXZ_OK) return st;
+  std::unique_ptr<pxz_image, void (*)(pxz_image*)> dec_guard(dec, pxz_image_free);
+  // down outer, up inner: one payload and one decode alive at a time.  The dims do not depend on the filter, so the five
+  // payloads have the same descriptors and the bucket of a block is the same in all 25 passes.
+  for (uint32_t down = 0; down < 5; ++down) {
+    pxz_payload* p = nullptr;
+    if ((st = plan_and_resample(ctx, img, g, metric, vm, (pxz_filter)down, exact_all, &p)) != PXZ_OK) return st;
+    for (uint32_t up = 0; up < 5 && st == PXZ_OK; ++up) {
+      const uint32_t pair = down * 5 + up;
+      st = pxz_expand_to_image(ctx, p, (pxz_filter)up, dec);
+      if (st == PXZ_OK) st = run_block_error(ctx, img, dec, g, d_block_sse, nullptr);
+      if (st == PXZ_OK) {
+        ProfScope prof(ctx, K_BUCKET_SUM);
+        const cudaError_t e = launch_bucket_sum(p->d_descs, d_block_sse, nblocks, pair, pair == 0, d_sse, d_blocks, ctx->stream, ctx->sm_count,
+                                                &ctx->launches);
+        if (e != cudaSuccess) {
+          cudaGetLastError();
+          st = fail(ctx, PXZ_E_CUDA, std::string("bucket sum: ") + cudaGetErrorString(e));
+        }
+      }
+    }
+    payload_release(p);
+    if (st != PXZ_OK) return st;
+  }
+  PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, d_sse, report_sse, cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaMemcpyAsync(host_blocks, d_blocks, kStrategyBuckets * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return PXZ_OK;
+}
+
+pxz_status pxz_strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
+                                uint32_t flags, uint64_t* host_sse, uint32_t* host_blocks) {
+  if (!ctx || !img || !host_sse || !host_blocks) return PXZ_E_ARG;
+  cudaSetDevice(ctx->device);
+  if (img->nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "a strategy measure is per image: not available on a batch");
+  if ((flags & PXZ_FLAG_NORMALISE_GLOBAL) && ctx->comm)
+    return fail(ctx, PXZ_E_UNSUPPORTED, "a strategy measure with global normalisation over a communicator is not available");
+  // the installed strategy would pick one pair per block: cleared for the call, restored on every return path
+  struct StrategyOff {
+    pxz_ctx* c;
+    StrategyLut saved;
+    explicit StrategyOff(pxz_ctx* cc) : c(cc), saved(cc->strategy) { c->strategy.on = 0; }
+    ~StrategyOff() { c->strategy = saved; }
+  } off(ctx);
+  return strategy_measure(ctx, img, bw, bh, metric, factor, flags, host_sse, host_blocks);
+}
+
+pxz_status pxz_strategy_choose(const uint64_t* sse, const uint32_t* blocks, const pxz_strategy* base, pxz_strategy* out) {
+  if (!sse || !blocks || !out) return PXZ_E_ARG;
+  pxz_strategy b;
+  if (base) {
+    for (int k = 0; k < PXZ_STRATEGY_BUCKETS; ++k)
+      if (base->down[k] > 4 || base->up[k] > 4) return PXZ_E_ARG;
+    b = *base;
+  } else {
+    pxz_strategy_by_level(&b);
+  }
+  for (int k = 0; k < PXZ_STRATEGY_BUCKETS; ++k) {
+    const uint64_t* row = sse + (size_t)k * PXZ_FILTER_PAIRS;
+    const uint32_t own = (uint32_t)b.down[k] * 5u + b.up[k];
+    uint32_t pick = own;
+    if (blocks[k] != 0) {
+      uint64_t least = row[0];
+      for (uint32_t q = 1; q < PXZ_FILTER_PAIRS; ++q) least = std::min(least, row[q]);
+      if (row[own] != least) {
+        pick = 0;
+        while (row[pick] != least) ++pick;
+      }
+    }
+    out->down[k] = (uint8_t)(pick / 5u);
+    out->up[k] = (uint8_t)(pick % 5u);
+  }
+  return PXZ_OK;
 }
 
 // host restatement of the plan kernel's scalar path (same threshold table)

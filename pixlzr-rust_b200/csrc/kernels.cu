@@ -10,6 +10,8 @@
 //                        (operations.rs:128-156)
 //   k_resample           per-block separable resample, image-crate order (block.rs:273-290):
 //                        image tiles -> packed payload (shrink) or payload -> image tiles (expand+paste)
+//   k_block_error        per-block squared error and largest difference of two images (integer, exact)
+//   k_bucket_sum         block errors summed per strategy bucket of the stored block value (strategy measure)
 //
 // Nothing here is a dense contraction, so no tensor cores: the kernels are HBM / FP32-pipe work with
 // 16-byte coalesced loads, shared-memory staging and warp-shuffle reductions (DESIGN.md).
@@ -2766,6 +2768,184 @@ __global__ void __launch_bounds__(kThreads) k_payload_convert(const pxz_block_de
     }
   }
   if (blockIdx.x == 0 && threadIdx.x == 0) *dtotal = *stotal / (unsigned)sc * (unsigned)dc;
+}
+
+// ------------------------------------------------------------------------------------------------
+// per-block error of two images of one geometry (pxz_image_error, pxz_strategy_measure).  Integer arithmetic only: per 4 bytes
+// one VABSDIFF4 (|a - b| per byte) and one IDP.4A (sum of the four squares), __vmaxu4 for the largest difference.  A work item is
+// a band of at most kErrRows rows inside one block row times kThreads consecutive units of a row; a thread keeps the same unit
+// in every row of its band, so its byte range maps to the same block column(s) and it sums in registers (u32: at most
+// 32 rows x 16 bytes x 255^2 < 2^32).  Units: 16 aligned bytes (kVec: both images' rows start 16-byte aligned and a block
+// row is >= 16 bytes, so a unit straddles at most one block-column edge) or one pixel (any pitch, any block width).  The
+// thread's sums go to shared per-column slots, then one 64-bit atomicAdd per block column and work item: integer sums, so the
+// result does not depend on the order.  sse[] / mx[] are zero on entry; trailing tiles count their real pixels only.
+// ------------------------------------------------------------------------------------------------
+constexpr int kErrRows = 32;
+constexpr int kErrCols = kThreads + 2;  // block columns one work item can touch (units of >= 16 bytes or one pixel)
+
+// the 16 bytes at p (only the first n when n < 16: the unit at the end of a row must not read past it), as 4 words
+__device__ __forceinline__ uint4 load_unit(const uint8_t* p, uint32_t n) {
+  if (n == 16) return ldg_nc_v4(p);
+  uint32_t w[4] = {0u, 0u, 0u, 0u};
+#pragma unroll
+  for (uint32_t i = 0; i < 16; ++i)  // unrolled: the words stay in registers
+    if (i < n) w[i >> 2] |= (uint32_t)__ldg(p + i) << (8 * (i & 3));
+  return make_uint4(w[0], w[1], w[2], w[3]);
+}
+// bytes [0, k) of a 16-byte unit as 4 word masks' word i
+__device__ __forceinline__ uint32_t lead_mask(uint32_t k, int i) {
+  const int n = (int)k - 4 * i;
+  return n <= 0 ? 0u : (n >= 4 ? 0xFFFFFFFFu : (1u << (8 * n)) - 1u);
+}
+
+template <bool kVec>
+__global__ void __launch_bounds__(kThreads) k_block_error(const uint8_t* __restrict__ a, size_t pa, const uint8_t* __restrict__ b, size_t pb,
+                                                          Geom g, uint32_t units, uint32_t ux, uint32_t bands_per_row,
+                                                          unsigned long long nwork, unsigned long long* __restrict__ sse,
+                                                          uint32_t* __restrict__ mx) {
+  __shared__ unsigned long long s_sse[kErrCols];
+  __shared__ uint32_t s_max[kErrCols];
+  const uint32_t tid = threadIdx.x;
+  const uint32_t rowb = g.W * g.C, bwc = g.bw * g.C;
+  for (unsigned long long w = blockIdx.x; w < nwork; w += gridDim.x) {
+    const uint32_t cx = (uint32_t)(w % ux);
+    const unsigned long long band = w / ux;
+    const uint32_t by = (uint32_t)(band / bands_per_row), k = (uint32_t)(band - (unsigned long long)by * bands_per_row);
+    const unsigned long long ytop = (unsigned long long)by * g.bh;
+    const unsigned long long y0 = ytop + (unsigned long long)k * kErrRows;
+    const unsigned long long y1 = min(min(y0 + kErrRows, ytop + g.bh), (unsigned long long)g.H);
+    if (y0 >= y1) continue;  // the last band of a trailing block row: uniform over the CTA
+    const uint32_t u0 = cx * kThreads;
+    const uint32_t bc_first = (kVec ? u0 * 16u : u0 * g.C) / bwc;
+    for (uint32_t i = tid; i < kErrCols; i += kThreads) {
+      s_sse[i] = 0ull;
+      s_max[i] = 0u;
+    }
+    __syncthreads();
+    const uint32_t u = u0 + tid;
+    if (u < units) {
+      const uint32_t xb = kVec ? u * 16u : u * g.C;
+      const uint32_t bc = xb / bwc;
+      const uint8_t* pa0 = a + (size_t)y0 * pa + xb;
+      const uint8_t* pb0 = b + (size_t)y0 * pb + xb;
+      const uint32_t nrows = (uint32_t)(y1 - y0);
+      uint32_t acc = 0u, m = 0u, acc2 = 0u, m2 = 0u;  // second column: the bytes of a 16-byte unit past a block-column edge
+      uint32_t split = 16u;
+      if (kVec) {
+        const uint32_t n = min(16u, rowb - xb);
+        split = min((bc + 1u) * bwc - xb, n);  // bytes of the unit in column bc
+        if (n == 16u && split == 16u) {
+#pragma unroll 4
+          for (uint32_t r = 0; r < nrows; ++r) {
+            const uint4 va = ldg_nc_v4(pa0 + (size_t)r * pa), vb = ldg_nc_v4(pb0 + (size_t)r * pb);
+            const uint32_t d0 = __vabsdiffu4(va.x, vb.x), d1 = __vabsdiffu4(va.y, vb.y);
+            const uint32_t d2 = __vabsdiffu4(va.z, vb.z), d3 = __vabsdiffu4(va.w, vb.w);
+            acc = __dp4a(d0, d0, acc);
+            acc = __dp4a(d1, d1, acc);
+            acc = __dp4a(d2, d2, acc);
+            acc = __dp4a(d3, d3, acc);
+            m = __vmaxu4(m, __vmaxu4(__vmaxu4(d0, d1), __vmaxu4(d2, d3)));
+          }
+        } else {  // the unit at the end of a row or across a block-column edge
+          uint32_t lo[4];
+#pragma unroll
+          for (int i = 0; i < 4; ++i) lo[i] = lead_mask(split, i);
+          for (uint32_t r = 0; r < nrows; ++r) {
+            const uint4 va = load_unit(pa0 + (size_t)r * pa, n), vb = load_unit(pb0 + (size_t)r * pb, n);
+            const uint32_t d[4] = {__vabsdiffu4(va.x, vb.x), __vabsdiffu4(va.y, vb.y), __vabsdiffu4(va.z, vb.z), __vabsdiffu4(va.w, vb.w)};
+#pragma unroll
+            for (int i = 0; i < 4; ++i) {
+              const uint32_t dl = d[i] & lo[i], dh = d[i] & ~lo[i];
+              acc = __dp4a(dl, dl, acc);
+              acc2 = __dp4a(dh, dh, acc2);
+              m = __vmaxu4(m, dl);
+              m2 = __vmaxu4(m2, dh);
+            }
+          }
+        }
+      } else {
+        const uint32_t C = g.C;
+        for (uint32_t r = 0; r < nrows; ++r) {
+          const uint8_t* qa = pa0 + (size_t)r * pa;
+          const uint8_t* qb = pb0 + (size_t)r * pb;
+          uint32_t wa = 0u, wb = 0u;
+          for (uint32_t c = 0; c < C; ++c) {
+            wa |= (uint32_t)__ldg(qa + c) << (8 * c);
+            wb |= (uint32_t)__ldg(qb + c) << (8 * c);
+          }
+          const uint32_t d = __vabsdiffu4(wa, wb);
+          acc = __dp4a(d, d, acc);
+          m = __vmaxu4(m, d);
+        }
+      }
+      auto bytes_max = [](uint32_t v) { return max(max(v & 0xFFu, (v >> 8) & 0xFFu), max((v >> 16) & 0xFFu, v >> 24)); };
+      if (acc) atomicAdd(&s_sse[bc - bc_first], (unsigned long long)acc);
+      if (m) atomicMax(&s_max[bc - bc_first], bytes_max(m));
+      if (acc2) atomicAdd(&s_sse[bc + 1u - bc_first], (unsigned long long)acc2);
+      if (m2) atomicMax(&s_max[bc + 1u - bc_first], bytes_max(m2));
+    }
+    __syncthreads();
+    const uint32_t u_end = min(u0 + (uint32_t)kThreads, units);
+    const uint32_t last_byte = (kVec ? min(u_end * 16u, rowb) : u_end * g.C) - 1u;
+    const uint32_t ncols = last_byte / bwc - bc_first + 1u;
+    for (uint32_t i = tid; i < ncols; i += kThreads) {
+      const size_t blk = (size_t)by * g.cols + bc_first + i;
+      if (s_sse[i]) atomicAdd(&sse[blk], s_sse[i]);
+      if (mx && s_max[i]) atomicMax(&mx[blk], s_max[i]);
+    }
+    __syncthreads();  // the slots are cleared for the next work item
+  }
+}
+
+// strategy measure: the block errors of one (down, up) pair added into sse[bucket * kFilterPairs + pair], the bucket taken from
+// the value the plan stored in the block's descriptor; count: also the block histogram.  A shared histogram per CTA, then one
+// global add per bucket.
+__global__ void __launch_bounds__(kThreads) k_bucket_sum(const pxz_block_desc* __restrict__ descs, const unsigned long long* __restrict__ block_sse,
+                                                         uint32_t nblocks, uint32_t pair, int count, unsigned long long* __restrict__ sse,
+                                                         uint32_t* __restrict__ blocks) {
+  __shared__ unsigned long long s_sse[kStrategyBuckets];
+  __shared__ uint32_t s_n[kStrategyBuckets];
+  for (int i = threadIdx.x; i < kStrategyBuckets; i += kThreads) {
+    s_sse[i] = 0ull;
+    s_n[i] = 0u;
+  }
+  __syncthreads();
+  for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < nblocks; i += gridDim.x * kThreads) {
+    const uint32_t k = strategy_bucket(descs[i].value);
+    const unsigned long long e = block_sse[i];
+    if (e) atomicAdd(&s_sse[k], e);
+    if (count) atomicAdd(&s_n[k], 1u);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < kStrategyBuckets; i += kThreads) {
+    if (s_sse[i]) atomicAdd(&sse[(size_t)i * kFilterPairs + pair], s_sse[i]);
+    if (count && s_n[i]) atomicAdd(&blocks[i], s_n[i]);
+  }
+}
+
+cudaError_t launch_block_error(const uint8_t* a, size_t pa, const uint8_t* b, size_t pb, const Geom& g, uint64_t* sse, uint32_t* mx,
+                               cudaStream_t s, int sm_count, uint64_t* launches) {
+  const bool vec = (((uintptr_t)a | (uintptr_t)b | pa | pb) & 15u) == 0 && g.bw * g.C >= 16u;
+  const uint32_t units = vec ? (g.W * g.C + 15u) / 16u : g.W;
+  const uint32_t ux = (units + kThreads - 1) / kThreads;
+  const uint32_t bands_per_row = (g.bh + kErrRows - 1) / kErrRows;
+  const unsigned long long nwork = (unsigned long long)g.rows * bands_per_row * ux;
+  const int grid = clamp_grid((long long)std::min<unsigned long long>(nwork, 1ull << 30), (long long)sm_count * 16);
+  ++*launches;
+  if (vec)
+    k_block_error<true><<<grid, kThreads, 0, s>>>(a, pa, b, pb, g, units, ux, bands_per_row, nwork, reinterpret_cast<unsigned long long*>(sse), mx);
+  else
+    k_block_error<false><<<grid, kThreads, 0, s>>>(a, pa, b, pb, g, units, ux, bands_per_row, nwork, reinterpret_cast<unsigned long long*>(sse), mx);
+  return cudaGetLastError();
+}
+
+cudaError_t launch_bucket_sum(const pxz_block_desc* descs, const uint64_t* block_sse, uint32_t nblocks, uint32_t pair, bool count,
+                              uint64_t* sse, uint32_t* blocks, cudaStream_t s, int sm_count, uint64_t* launches) {
+  ++*launches;
+  const int grid = clamp_grid(((long long)nblocks + kThreads - 1) / kThreads, (long long)sm_count * 2);
+  k_bucket_sum<<<grid, kThreads, 0, s>>>(descs, reinterpret_cast<const unsigned long long*>(block_sse), nblocks, pair, count ? 1 : 0,
+                                         reinterpret_cast<unsigned long long*>(sse), blocks);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_rgb_widen(const uint8_t* src, size_t spitch, uint8_t* dst, size_t dpitch, uint32_t w, uint32_t rows, int widen,

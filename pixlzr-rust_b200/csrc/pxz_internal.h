@@ -164,6 +164,16 @@ cudaError_t launch_qoi_encode(const pxz_block_desc* descs, const uint8_t* pixels
                               unsigned long long* total, cudaStream_t s, uint64_t* launches);
 cudaError_t launch_qoi_decode(const uint8_t* in, const unsigned long long* in_off, const uint32_t* qlen, const pxz_block_desc* descs,
                               const Geom& g, uint8_t* pixels, int* err, cudaStream_t s, uint64_t* launches);
+// per-block error of two images of geometry g (not a batch): sse[b] += sum of (a - b)^2 over the tile, mx[b] = max(mx[b], max |a - b|)
+// (mx may be NULL).  Both arrays are zero on entry.
+cudaError_t launch_block_error(const uint8_t* a, size_t pa, const uint8_t* b, size_t pb, const Geom& g, uint64_t* sse, uint32_t* mx,
+                               cudaStream_t s, int sm_count, uint64_t* launches);
+// strategy measure: sse[bucket * kFilterPairs + pair] += block_sse[i] with bucket = strategy_bucket(descs[i].value); count: also
+// blocks[bucket] += 1
+constexpr uint32_t kFilterPairs = 25;  // pair = down * 5 + up
+static_assert(kFilterPairs == PXZ_FILTER_PAIRS, "filter pair count");
+cudaError_t launch_bucket_sum(const pxz_block_desc* descs, const uint64_t* block_sse, uint32_t nblocks, uint32_t pair, bool count,
+                              uint64_t* sse, uint32_t* blocks, cudaStream_t s, int sm_count, uint64_t* launches);
 // direction 0: image tiles -> payload (shrink); 1: payload -> image tiles (expand)
 cudaError_t launch_resample(int direction, uint8_t* img, size_t pitch, const Geom& g, const pxz_block_desc* descs,
                             const uint32_t* tabidx, uint8_t* payload, const AxisTab* tabs, const uint32_t* pool,
