@@ -77,7 +77,8 @@ int pxz_abi_version(void);
 /* number of usable CUDA devices (0 if none / no driver) */
 int pxz_device_count(void);
 /* One context per host thread; it owns one CUDA stream and its scratch.  Environment read at creation (diagnostics only):
- *   PXZ_RESAMPLE_KERNELS=warp|cta  force one of the two resample kernel families (default: by tile count),
+ *   PXZ_RESAMPLE_KERNELS=warp|cta|tma  force a resample kernel family (default: by tile count): warp-per-tile with
+ *                                  the cp.async ring shrink kernel, CTA-per-tile, or warp-per-tile with the TMA shrink kernel,
  *   PXZ_GUARD_REL / PXZ_GUARD_ABS  guard band of the fast Oklab-MAD path (DESIGN.md section 3). */
 pxz_status pxz_ctx_create(int device, pxz_ctx** out);
 /* same, but work is ordered on an existing CUDA stream (cudaStream_t / CUstream passed as

@@ -13,7 +13,6 @@
 #include <string.h>
 
 #include <algorithm>
-#include <functional>
 #include <map>
 #include <memory>
 #include <new>
@@ -90,7 +89,7 @@ struct pxz_ctx {
   size_t values_cap = 0;
   float* d_minmax = nullptr;
   uint32_t* d_tile_counter = nullptr;  // work counter of the warp-per-tile resample kernels (they leave it at 0)
-  int resample_kernels = 0;            // 0 = by tile count, 1 = warp-per-tile (cp.async ring), 2 = CTA-per-tile, 3 = warp-per-tile with the TMA shrink kernel (PXZ_RESAMPLE_KERNELS=warp|cta|tma)
+  ResampleKernels resample_kernels = ResampleKernels::Auto;  // PXZ_RESAMPLE_KERNELS
   void* d_scan = nullptr;
   size_t scan_cap = 0;
   uint8_t* d_scratch = nullptr;
@@ -151,14 +150,16 @@ pxz_status fail(pxz_ctx* ctx, pxz_status st, const std::string& msg) {
   return st;
 }
 
+// A launch or an asynchronous call returned the error e: clear it and report "<what>: <error>" with status st
+pxz_status cuda_fail(pxz_ctx* ctx, cudaError_t e, const char* what, pxz_status st = PXZ_E_CUDA) {
+  cudaGetLastError();
+  return fail(ctx, st, std::string(what) + ": " + cudaGetErrorString(e));
+}
+
 #define PXZ_CUDA(ctx, expr)                                                                             \
   do {                                                                                                  \
     cudaError_t _e = (expr);                                                                            \
-    if (_e != cudaSuccess) {                                                                            \
-      cudaGetLastError();                                                                               \
-      return fail((ctx), _e == cudaErrorMemoryAllocation ? PXZ_E_OOM : PXZ_E_CUDA,                      \
-                  std::string(#expr) + ": " + cudaGetErrorString(_e));                                  \
-    }                                                                                                   \
+    if (_e != cudaSuccess) return cuda_fail((ctx), _e, #expr, _e == cudaErrorMemoryAllocation ? PXZ_E_OOM : PXZ_E_CUDA); \
   } while (0)
 
 // records an event pair around one kernel launch while profiling is on
@@ -189,6 +190,20 @@ struct ProfScope {
   }
 };
 
+// one launch (`launch()` returns its cudaError_t) timed under the profile id `prof`; a failure is reported as cuda_fail(what)
+template <class F>
+pxz_status profiled(pxz_ctx* ctx, int prof, const char* what, F&& launch) {
+  cudaError_t e;
+  {
+    ProfScope scope(ctx, prof);
+    e = launch();
+  }
+  return e == cudaSuccess ? PXZ_OK : cuda_fail(ctx, e, what);
+}
+
+// the filters of pxz_filter
+inline bool known_filter(pxz_filter f) { return (int)f >= 0 && (int)f <= 4; }
+
 inline uint32_t ceil_div_u32(uint32_t a, uint32_t b) { return (uint32_t)(((uint64_t)a + b - 1) / b); }
 
 pxz_status make_geom(pxz_ctx* ctx, uint32_t w, uint32_t h, uint32_t c, uint32_t bw, uint32_t bh, Geom* g, uint32_t nimg = 1) {
@@ -217,6 +232,29 @@ pxz_status dev_alloc(pxz_ctx* ctx, void** p, size_t bytes) {
 void dev_free(pxz_ctx* ctx, void* p) {
   if (p) cudaFreeAsync(p, ctx->stream);
 }
+
+// the dev_alloc blocks of one call (at most five), freed stream-ordered in allocation order when the owner goes out of scope
+struct DevBlocks {
+  pxz_ctx* ctx;
+  void* blocks[5] = {};
+  int n = 0;
+  explicit DevBlocks(pxz_ctx* c) : ctx(c) {}
+  DevBlocks(const DevBlocks&) = delete;
+  DevBlocks& operator=(const DevBlocks&) = delete;
+  ~DevBlocks() {
+    for (int i = 0; i < n; ++i) dev_free(ctx, blocks[i]);
+  }
+  template <class T>
+  pxz_status alloc(T** out, size_t bytes) {
+    void* q = nullptr;
+    const pxz_status st = dev_alloc(ctx, &q, bytes);
+    if (st != PXZ_OK) return st;
+    blocks[n++] = q;
+    *out = static_cast<T*>(q);
+    return PXZ_OK;
+  }
+  void keep() { n = 0; }  // the blocks have another owner now
+};
 
 // scan_bytes: the scan state the next plan / window launch needs (0: launch_plan's for nblocks)
 pxz_status ensure_scratch(pxz_ctx* ctx, uint32_t nblocks, size_t scan_bytes = 0) {
@@ -323,22 +361,16 @@ pxz_status get_tabset(pxz_ctx* ctx, const TabSpec& spec, int filter, int directi
     }
     ctx->tabs.clear();
   }
+  DevBlocks bufs(ctx);
   pxz_status st;
-  if ((st = dev_alloc(ctx, (void**)&ts.d_tabs, tabs.size() * sizeof(AxisTab))) != PXZ_OK) return st;
-  if ((st = dev_alloc(ctx, (void**)&ts.d_pool, pool.size() * 4)) != PXZ_OK) {
-    dev_free(ctx, ts.d_tabs);
-    return st;
-  }
+  if ((st = bufs.alloc(&ts.d_tabs, tabs.size() * sizeof(AxisTab))) != PXZ_OK) return st;
+  if ((st = bufs.alloc(&ts.d_pool, pool.size() * 4)) != PXZ_OK) return st;
   // pageable -> device copies are staged by the runtime before returning, so the vectors may die
   cudaError_t ce = cudaMemcpyAsync(ts.d_tabs, tabs.data(), tabs.size() * sizeof(AxisTab), cudaMemcpyHostToDevice, ctx->stream);
   if (ce == cudaSuccess) ce = cudaMemcpyAsync(ts.d_pool, pool.data(), pool.size() * 4, cudaMemcpyHostToDevice, ctx->stream);
   if (ce == cudaSuccess) ce = cudaStreamSynchronize(ctx->stream);
-  if (ce != cudaSuccess) {
-    cudaGetLastError();
-    dev_free(ctx, ts.d_tabs);
-    dev_free(ctx, ts.d_pool);
-    return fail(ctx, PXZ_E_CUDA, std::string("resample table upload: ") + cudaGetErrorString(ce));
-  }
+  if (ce != cudaSuccess) return cuda_fail(ctx, ce, "resample table upload");
+  bufs.keep();  // the cache owns them
   ctx->tabs[key] = ts;
   *out = ts;
   return PXZ_OK;
@@ -377,13 +409,34 @@ pxz_status run_resample(pxz_ctx* ctx, int direction, uint8_t* img, size_t pitch,
     }
     scratch = ctx->d_scratch;
   }
+  ResampleArgs a;
+  a.direction = direction;
+  a.img = img;
+  a.pitch = pitch;
+  a.g = g;
+  a.descs = p->d_descs;
+  a.tabidx = (direction == 1 && p->strategy == 1) ? p->d_up() : p->d_tabidx;
+  a.payload = p->d_pixels;
+  a.tabs = ts.d_tabs;
+  a.pool = ts.d_pool;
+  a.ntabs = ts.ntabs;
+  a.max_src_px = max_src_px;
+  a.max_src_dim = max_src_dim;
+  a.max_tmp_px = max_tmp_px;
+  a.max_tab_words = ts.max_words;
+  a.scratch = scratch;
+  a.scratch_per_cta = per_cta;
+  a.grid = grid;
+  a.fused = ctx->fast_resample;
+  a.opaque_flags = opaque_flags;
+  a.tile_counter = ctx->resample_kernels != ResampleKernels::Cta ? ctx->d_tile_counter : nullptr;
+  a.lists = p->d_order();
+  a.cap = (uint32_t)p->nblocks_cap;
+  a.warp_tables = ts.warp_ok;
+  a.kernels = ctx->resample_kernels;
+  a.has_noslide = ts.has_noslide;
   ProfScope prof(ctx, direction == 0 ? K_RESAMPLE_DOWN : K_RESAMPLE_UP);
-  const uint32_t* tabidx = (direction == 1 && p->strategy == 1) ? p->d_up() : p->d_tabidx;
-  PXZ_CUDA(ctx, launch_resample(direction, img, pitch, g, p->d_descs, tabidx, p->d_pixels, ts.d_tabs, ts.d_pool,
-                                ts.ntabs, max_src_px, max_src_dim, max_tmp_px, ts.max_words, scratch, per_cta, grid, ctx->fast_resample, opaque_flags,
-                                ctx->resample_kernels != 2 ? ctx->d_tile_counter : nullptr, p->d_order(), (uint32_t)p->nblocks_cap,
-                                ts.warp_ok, ctx->resample_kernels, ts.has_noslide, ctx->stream, ctx->sm_count,
-                                &ctx->launches));
+  PXZ_CUDA(ctx, launch_resample(a, ctx->stream, ctx->sm_count, &ctx->launches));
   return PXZ_OK;
 }
 
@@ -402,6 +455,50 @@ void payload_release(pxz_payload* p) {
     dev_free(ctx, p->d_total);
   }
   delete p;
+}
+
+// owners of a payload / an image on the internal paths: released when the owner goes out of scope
+struct PayloadRelease {
+  void operator()(pxz_payload* p) const { payload_release(p); }
+};
+using PayloadOwner = std::unique_ptr<pxz_payload, PayloadRelease>;
+struct ImageFree {
+  void operator()(pxz_image* im) const { pxz_image_free(im); }
+};
+using ImageOwner = std::unique_ptr<pxz_image, ImageFree>;
+
+pxz_status image_new(pxz_ctx* ctx, uint32_t w, uint32_t h, uint32_t c, uint32_t nimg, ImageOwner* out) {
+  pxz_image* im = nullptr;
+  const pxz_status st = pxz_image_alloc_batch(ctx, w, h, c, nimg, &im);
+  out->reset(im);
+  return st;
+}
+
+inline uint32_t pad8(uint32_t v) { return (v + 7u) & ~7u; }  // intermediate rows are padded to 8 columns
+
+// shared-memory bounds of the two resample directions for a payload planned on g (every block at most its tile);
+// coupled: both axes share the level (Oklab MAD)
+void set_plan_bounds(pxz_payload* p, const Geom& g, bool coupled) {
+  p->max_small_px = g.bw * g.bh;
+  p->max_small_dim = std::max(g.bw, g.bh);
+  if (coupled) {
+    p->max_tmp_down = ((g.bh + 1) / 2) * pad8(g.bw);  // dh <= ceil(th/2), sw = tw
+    p->max_tmp_up = g.bh * pad8((g.bw + 1) / 2);      // dh = th, sw <= ceil(tw/2)
+    // a 1-px-wide/-high trailing tile keeps that axis while the other shrinks: still within the bounds
+  } else {
+    p->max_tmp_down = g.bh * pad8(g.bw);
+    p->max_tmp_up = g.bh * pad8(g.bw);
+  }
+}
+
+// a payload over the same blocks as src (another channel count, a window): same tables, filters and bounds
+void copy_layout(pxz_payload* dst, const pxz_payload* src) {
+  dst->spec = src->spec;
+  dst->strategy = src->strategy;
+  dst->max_small_px = src->max_small_px;
+  dst->max_small_dim = src->max_small_dim;
+  dst->max_tmp_down = src->max_tmp_down;
+  dst->max_tmp_up = src->max_tmp_up;
 }
 
 pxz_status ctx_create_common(int device, cudaStream_t stream, bool own, pxz_ctx** out) {
@@ -446,7 +543,11 @@ pxz_status ctx_create_common(int device, cudaStream_t stream, bool own, pxz_ctx*
   if (const char* e = getenv("PXZ_GUARD_ABS")) ctx->band.abs_raw = (float)atof(e);
   if (const char* e = getenv("PXZ_RGB_VIA_RGBA")) ctx->rgb_via_rgba = atoi(e) != 0;
   if (const char* e = getenv("PXZ_RESIZE_SEMANTICS")) ctx->resize_semantics = !strcmp(e, "fir") ? PXZ_RESIZE_FIR : PXZ_RESIZE_IMAGE_RS;
-  if (const char* e = getenv("PXZ_RESAMPLE_KERNELS")) ctx->resample_kernels = !strcmp(e, "warp") ? 1 : !strcmp(e, "cta") ? 2 : !strcmp(e, "tma") ? 3 : 0;
+  if (const char* e = getenv("PXZ_RESAMPLE_KERNELS"))
+    ctx->resample_kernels = !strcmp(e, "warp") ? ResampleKernels::Warp
+                            : !strcmp(e, "cta") ? ResampleKernels::Cta
+                            : !strcmp(e, "tma") ? ResampleKernels::Tma
+                                                : ResampleKernels::Auto;
   if (cudaMalloc((void**)&ctx->d_minmax, 8 * sizeof(float)) != cudaSuccess ||
       cudaMalloc((void**)&ctx->d_tile_counter, 64) != cudaSuccess || cudaMemset(ctx->d_tile_counter, 0, 64) != cudaSuccess ||
       cudaMallocHost((void**)&ctx->h_total, 64) != cudaSuccess) {
@@ -667,7 +768,7 @@ pxz_status pxz_image_upload_batch(pxz_ctx* ctx, const uint8_t* host, uint32_t w,
   if (e != cudaSuccess) {
     pxz_image_free(*out);
     *out = nullptr;
-    return fail(ctx, PXZ_E_CUDA, std::string("cudaMemcpy2DAsync: ") + cudaGetErrorString(e));
+    return cuda_fail(ctx, e, "cudaMemcpy2DAsync");
   }
   return PXZ_OK;
 }
@@ -775,8 +876,8 @@ pxz_status pxz_analyze(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t
 }
 
 // ---- encode -------------------------------------------------------------------------------------------
-static pxz_status payload_new(pxz_ctx* ctx, const Geom& g, uint64_t capacity, pxz_payload** out) {
-  pxz_payload* p = new (std::nothrow) pxz_payload();
+static pxz_status payload_new(pxz_ctx* ctx, const Geom& g, uint64_t capacity, PayloadOwner* out) {
+  PayloadOwner p(new (std::nothrow) pxz_payload());
   if (!p) return fail(ctx, PXZ_E_OOM, "host allocation failed");
   p->ctx = ctx;
   p->g = g;
@@ -792,7 +893,7 @@ static pxz_status payload_new(pxz_ctx* ctx, const Geom& g, uint64_t capacity, px
     ctx->payload_cache.erase(ctx->payload_cache.begin() + best);
     p->d_descs = b.d_descs; p->d_tabidx = b.d_tabidx; p->d_pixels = b.d_pixels; p->d_total = b.d_total;
     p->nblocks_cap = b.nblocks; p->capacity = b.capacity;
-    *out = p;
+    *out = std::move(p);
     return PXZ_OK;
   }
   p->capacity = capacity;
@@ -801,14 +902,9 @@ static pxz_status payload_new(pxz_ctx* ctx, const Geom& g, uint64_t capacity, px
   if ((st = dev_alloc(ctx, (void**)&p->d_descs, nblocks * sizeof(pxz_block_desc))) != PXZ_OK ||
       (st = dev_alloc(ctx, (void**)&p->d_tabidx, (2 * nblocks + order_list_words(nblocks)) * 4)) != PXZ_OK ||  // table indices | work order lists | expand-side indices
       (st = dev_alloc(ctx, (void**)&p->d_pixels, capacity)) != PXZ_OK ||
-      (st = dev_alloc(ctx, (void**)&p->d_total, 8)) != PXZ_OK) {
-    // partial allocations must not enter the cache
-    dev_free(ctx, p->d_descs); dev_free(ctx, p->d_tabidx); dev_free(ctx, p->d_pixels); dev_free(ctx, p->d_total);
-    p->d_descs = nullptr; p->d_tabidx = nullptr; p->d_pixels = nullptr; p->d_total = nullptr;
-    delete p;
-    return st;
-  }
-  *out = p;
+      (st = dev_alloc(ctx, (void**)&p->d_total, 8)) != PXZ_OK)
+    return st;  // payload_release frees a partial set: only complete sets enter the cache
+  *out = std::move(p);
   return PXZ_OK;
 }
 
@@ -856,8 +952,7 @@ static bool rgb_on_rgba(const pxz_ctx* ctx, uint32_t w, uint32_t c, uint32_t bw,
 }
 
 // payload of the other channel count (3 <-> 4) with the same blocks, tables and work order
-static pxz_status payload_rechannel(pxz_ctx* ctx, const pxz_payload* src, uint32_t dc, pxz_payload** out) {
-  *out = nullptr;
+static pxz_status payload_rechannel(pxz_ctx* ctx, const pxz_payload* src, uint32_t dc, PayloadOwner* out) {
   Geom g = src->g;
   const uint32_t sc = g.C;
   g.C = dc;
@@ -865,53 +960,42 @@ static pxz_status payload_rechannel(pxz_ctx* ctx, const pxz_payload* src, uint32
   // k_payload_convert writes each block at offset / sc * dc.  Uploaded payloads may hold blocks larger than their tiles, so
   // W * H * dc does not bound that; every block lies inside src->capacity (payload_from_descs checks it).
   const uint64_t cap = std::max<uint64_t>((uint64_t)g.W * g.H * dc * g.nimg, (src->capacity + sc - 1) / sc * dc);
-  pxz_payload* p = nullptr;
+  PayloadOwner p;
   pxz_status st = payload_new(ctx, g, cap, &p);
   if (st != PXZ_OK) return st;
-  p->spec = src->spec;
-  p->strategy = src->strategy;
-  p->max_small_px = src->max_small_px; p->max_small_dim = src->max_small_dim;
-  p->max_tmp_down = src->max_tmp_down; p->max_tmp_up = src->max_tmp_up;
+  copy_layout(p.get(), src);
   if (src->bytes_known) { p->bytes = src->bytes / sc * dc; p->bytes_known = true; }
   cudaError_t e = launch_payload_convert(src->d_descs, src->d_pixels, src->d_tabidx, (uint32_t)src->nblocks_cap, src->d_total, p->d_descs,
                                          p->d_pixels, p->d_tabidx, (uint32_t)p->nblocks_cap, p->d_total, nblocks, (int)sc, (int)dc,
                                          ctx->stream, ctx->sm_count, &ctx->launches);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    payload_release(p);
-    return fail(ctx, PXZ_E_CUDA, std::string("payload convert: ") + cudaGetErrorString(e));
-  }
-  *out = p;
+  if (e != cudaSuccess) return cuda_fail(ctx, e, "payload convert");
+  *out = std::move(p);
   return PXZ_OK;
 }
 
 // An RGB image on the RGBA fast kernels: widen it to RGBA (alpha 255: its metric term is exactly +0 and the opaque resample
 // path never touches it), run `encode` on the 4-channel image, narrow the payload back
 extern "C++" {  // a template inside the extern "C" block
-static pxz_status rgb_widened(pxz_ctx* ctx, const pxz_image* img, pxz_image** wide) {
-  pxz_status st = pxz_image_alloc_batch(ctx, img->w, img->h, 4, img->nimg, wide);
+static pxz_status rgb_widened(pxz_ctx* ctx, const pxz_image* img, ImageOwner* wide) {
+  pxz_status st = image_new(ctx, img->w, img->h, 4, img->nimg, wide);
   if (st != PXZ_OK) return st;
   cudaError_t e = launch_rgb_widen(img->d, img->pitch, (*wide)->d, (*wide)->pitch, img->w, img->h * img->nimg, 1, ctx->stream, ctx->sm_count,
                                    &ctx->launches);
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    pxz_image_free(*wide);
-    *wide = nullptr;
-    return fail(ctx, PXZ_E_CUDA, std::string("rgb widen: ") + cudaGetErrorString(e));
-  }
-  return PXZ_OK;
+  return e == cudaSuccess ? PXZ_OK : cuda_fail(ctx, e, "rgb widen");
 }
 template <class F>
 static pxz_status encode_via_rgba(pxz_ctx* ctx, const pxz_image* img, F&& encode, pxz_payload** out) {
-  pxz_image* wide = nullptr;
+  ImageOwner wide;
   pxz_status st = rgb_widened(ctx, img, &wide);
   if (st != PXZ_OK) return st;
-  pxz_payload* p4 = nullptr;
-  st = encode(wide, &p4);
-  pxz_image_free(wide);  // stream-ordered: the kernels queued above keep it
+  pxz_payload* raw = nullptr;
+  st = encode(wide.get(), &raw);
+  wide.reset();  // stream-ordered: the kernels queued above keep it
+  const PayloadOwner p4(raw);
   if (st != PXZ_OK) return st;
-  st = payload_rechannel(ctx, p4, 3, out);
-  payload_release(p4);
+  PayloadOwner p3;
+  st = payload_rechannel(ctx, p4.get(), 3, &p3);
+  *out = p3.release();
   return st;
 }
 }  // extern "C++"
@@ -931,97 +1015,71 @@ static ValueMap shrink_value_map(const pxz_ctx* ctx, pxz_metric metric, uint32_t
 
 // min / max of the values in ctx->d_vx (and d_vy) into ctx->d_minmax
 static pxz_status run_minmax(pxz_ctx* ctx, pxz_metric metric, uint32_t nblocks) {
-  ProfScope prof(ctx, K_MINMAX);
-  cudaError_t me = launch_minmax(ctx->d_vx, metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr, nblocks, ctx->d_minmax, ctx->stream,
-                                 &ctx->launches);
-  if (me != cudaSuccess) {
-    cudaGetLastError();
-    return fail(ctx, PXZ_E_CUDA, std::string("minmax: ") + cudaGetErrorString(me));
-  }
-  return PXZ_OK;
+  return profiled(ctx, K_MINMAX, "minmax", [&] {
+    return launch_minmax(ctx->d_vx, metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr, nblocks, ctx->d_minmax, ctx->stream, &ctx->launches);
+  });
 }
 
 // Global normalisation on the fast Oklab path, first half: the exact extremes come from the few tiles that can hold them
 // (their reference-order values patched into ctx->d_vx), then a second min / max over the patched values
 static pxz_status run_exact_extremes(pxz_ctx* ctx, const pxz_image* img, const Geom& g, uint32_t nblocks) {
-  {
-    ProfScope prof(ctx, K_MAD_EXACT);
-    cudaError_t ee = launch_analyze_mad_exact(img->d, img->pitch, g, ctx->d_vx, ctx->d_vx, ctx->d_opaque, nullptr, &ctx->thr, &ctx->band,
-                                              ctx->d_minmax, ctx->d_list, ctx->d_list + nblocks, ctx->stream, ctx->sm_count,
-                                              &ctx->launches);
-    if (ee != cudaSuccess) {
-      cudaGetLastError();
-      return fail(ctx, PXZ_E_CUDA, std::string("extremes: ") + cudaGetErrorString(ee));
-    }
-  }
-  return run_minmax(ctx, PXZ_METRIC_OKLAB_MAD, nblocks);
+  const pxz_status st = profiled(ctx, K_MAD_EXACT, "extremes", [&] {
+    return launch_analyze_mad_exact(img->d, img->pitch, g, ctx->d_vx, ctx->d_vx, ctx->d_opaque, nullptr, &ctx->thr, &ctx->band, ctx->d_minmax,
+                                    ctx->d_list, ctx->d_list + nblocks, ctx->stream, ctx->sm_count, &ctx->launches);
+  });
+  return st != PXZ_OK ? st : run_minmax(ctx, PXZ_METRIC_OKLAB_MAD, nblocks);
 }
 
 // Guard band of the fast Oklab path for the factor of `vm`: the tiles listed from the fast values `vx_fast` get their
 // reference-order value in `vx` (in place when vx == vx_fast, as pxz_shrink does)
 static pxz_status run_guard_band(pxz_ctx* ctx, const pxz_image* img, const Geom& g, const ValueMap& vm, float* vx, const float* vx_fast) {
   const uint32_t nblocks = g.cols * g.rows;
-  ProfScope prof(ctx, K_MAD_EXACT);
-  cudaError_t ee = cudaMemsetAsync(ctx->d_list + nblocks, 0, sizeof(uint32_t), ctx->stream);  // the list counter
-  if (ee == cudaSuccess)
-    ee = launch_analyze_mad_exact(img->d, img->pitch, g, vx, vx_fast, ctx->d_opaque, &vm, &ctx->thr, &ctx->band, ctx->d_minmax, ctx->d_list,
-                                  ctx->d_list + nblocks, ctx->stream, ctx->sm_count, &ctx->launches);
-  if (ee != cudaSuccess) {
-    cudaGetLastError();
-    return fail(ctx, PXZ_E_CUDA, std::string("guard band: ") + cudaGetErrorString(ee));
-  }
-  return PXZ_OK;
+  return profiled(ctx, K_MAD_EXACT, "guard band", [&] {
+    const cudaError_t e = cudaMemsetAsync(ctx->d_list + nblocks, 0, sizeof(uint32_t), ctx->stream);  // the list counter
+    return e != cudaSuccess ? e
+                            : launch_analyze_mad_exact(img->d, img->pitch, g, vx, vx_fast, ctx->d_opaque, &vm, &ctx->thr, &ctx->band, ctx->d_minmax,
+                                                       ctx->d_list, ctx->d_list + nblocks, ctx->stream, ctx->sm_count, &ctx->launches);
+  });
+}
+
+// The analysis of pxz_shrink before the min / max exchange: the values into ctx->d_vx / d_vy, then with global normalisation
+// their min / max and, on the fast Oklab path, the exact extremes.  band_vm (may be NULL): the value map whose guard band the
+// fast Oklab path resolves in the same pass; with global normalisation the band waits for the exchanged range.
+static pxz_status run_shrink_analysis(pxz_ctx* ctx, const pxz_image* img, const Geom& g, pxz_metric metric, uint32_t flags,
+                                      const ValueMap* band_vm) {
+  const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
+  const bool exact_all = (flags & PXZ_FLAG_EXACT_VALUES) != 0;
+  const uint32_t nblocks = g.cols * g.rows;
+  pxz_status st = run_analysis(ctx, img, g, metric, exact_all, normalise ? nullptr : band_vm);
+  if (st != PXZ_OK || !normalise) return st;
+  if ((st = run_minmax(ctx, metric, nblocks)) != PXZ_OK) return st;
+  return metric == PXZ_METRIC_OKLAB_MAD && !exact_all ? run_exact_extremes(ctx, img, g, nblocks) : PXZ_OK;
 }
 
 // The part of pxz_shrink after the analysis: plan (value -> level -> dims -> offsets) from ctx->d_vx / d_vy, then the
 // resample into a new payload
 static pxz_status plan_and_resample(pxz_ctx* ctx, const pxz_image* img, const Geom& g, pxz_metric metric, const ValueMap& vm,
                                     pxz_filter filter_down, bool exact_all, pxz_payload** out) {
-  pxz_payload* p = nullptr;
+  PayloadOwner p;
   pxz_status st = payload_new(ctx, g, (uint64_t)g.W * g.H * g.C * g.nimg, &p);
   if (st != PXZ_OK) return st;
   p->spec = spec_for_geom(g);
-  {
-    // shared-memory bounds of the two resample directions for this geometry
-    const bool coupled = metric == PXZ_METRIC_OKLAB_MAD;  // both axes share the level
-    const uint32_t tw_max = g.bw, th_max = g.bh;
-    auto pad8 = [](uint32_t v) { return (v + 7u) & ~7u; };  // intermediate rows are padded to 8 columns
-    p->max_small_px = tw_max * th_max;
-    p->max_small_dim = std::max(tw_max, th_max);
-    if (coupled) {
-      p->max_tmp_down = ((th_max + 1) / 2) * pad8(tw_max);  // dh <= ceil(th/2), sw = tw
-      p->max_tmp_up = th_max * pad8((tw_max + 1) / 2);      // dh = th, sw <= ceil(tw/2)
-      // a 1-px-wide/-high trailing tile keeps that axis while the other shrinks: still within the bounds
-    } else {
-      p->max_tmp_down = th_max * pad8(tw_max);
-      p->max_tmp_up = th_max * pad8(tw_max);
-    }
-  }
-  cudaError_t e;
-  {
-    ProfScope prof(ctx, K_PLAN);
-    StrategyLut lut = ctx->strategy;
-    lut.stride = (uint32_t)p->spec->n_small.size();
-    p->strategy = lut.on ? 1 : 0;
-    e = launch_plan(ctx->d_vx, metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr, g, vm, ctx->d_minmax, ctx->thr, nullptr,
-                    p->d_descs, p->d_tabidx, p->d_total, ctx->d_scan, p->d_order(), (uint32_t)p->nblocks_cap, ctx->stream, &ctx->launches,
-                    &lut, p->d_up());
-  }
-  if (e != cudaSuccess) {
-    payload_release(p);
-    return fail(ctx, PXZ_E_CUDA, std::string("plan: ") + cudaGetErrorString(e));
-  }
+  set_plan_bounds(p.get(), g, metric == PXZ_METRIC_OKLAB_MAD);
+  StrategyLut lut = ctx->strategy;
+  lut.stride = (uint32_t)p->spec->n_small.size();
+  p->strategy = lut.on ? 1 : 0;
+  st = profiled(ctx, K_PLAN, "plan", [&] {
+    return launch_plan(ctx->d_vx, metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr, g, vm, ctx->d_minmax, ctx->thr, nullptr, p->d_descs,
+                       p->d_tabidx, p->d_total, ctx->d_scan, p->d_order(), (uint32_t)p->nblocks_cap, ctx->stream, &ctx->launches, &lut, p->d_up());
+  });
+  if (st != PXZ_OK) return st;
   TabSet ts;
-  st = get_tabset(ctx, *p->spec, p->strategy ? -1 : (int)filter_down, 0, &ts);
+  if ((st = get_tabset(ctx, *p->spec, p->strategy ? -1 : (int)filter_down, 0, &ts)) != PXZ_OK) return st;
   // the fast Oklab-MAD pass also told which tiles are fully opaque: their alpha channel needs no arithmetic
   const uint8_t* opaque_flags = (metric == PXZ_METRIC_OKLAB_MAD && !exact_all) ? ctx->d_opaque : nullptr;
-  if (st == PXZ_OK)
-    st = run_resample(ctx, 0, img->d, img->pitch, p, ts, g.bw * g.bh, std::max(g.bw, g.bh), p->max_tmp_down, opaque_flags);
-  if (st != PXZ_OK) {
-    payload_release(p);
+  if ((st = run_resample(ctx, 0, img->d, img->pitch, p.get(), ts, g.bw * g.bh, std::max(g.bw, g.bh), p->max_tmp_down, opaque_flags)) != PXZ_OK)
     return st;
-  }
-  *out = p;
+  *out = p.release();
   return PXZ_OK;
 }
 
@@ -1047,12 +1105,11 @@ pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t 
     }
     return why;
   };
-  if ((int)filter_down < 0 || (int)filter_down > 4) return bail(fail(ctx, PXZ_E_ARG, "unknown filter"));
+  if (!known_filter(filter_down)) return bail(fail(ctx, PXZ_E_ARG, "unknown filter"));
   Geom g;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g, img->nimg);
   if (st != PXZ_OK) return bail(st);
   if (normalise && img->nimg > 1) return bail(fail(ctx, PXZ_E_UNSUPPORTED, "global normalisation is per image: not available on a batch"));
-  const uint32_t nblocks = g.cols * g.rows;
 
   const ValueMap vm = shrink_value_map(ctx, metric, flags, factor);
 
@@ -1063,12 +1120,10 @@ pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t 
   // them, and the guard band (scaled by 1 / range) then decides as in the default mode which tiles need their
   // reference-order value; with PXZ_FLAG_EXACT_VALUES every tile is computed in reference order as before.
   const bool fast_norm = normalise && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
-  st = run_analysis(ctx, img, g, metric, exact_all, (metric == PXZ_METRIC_OKLAB_MAD && !exact_all && !normalise) ? &vm : nullptr);
+  st = run_shrink_analysis(ctx, img, g, metric, flags, &vm);
   if (st != PXZ_OK) return bail(st);
 
   if (normalise) {
-    if ((st = run_minmax(ctx, metric, nblocks)) != PXZ_OK) return bail(st);
-    if (fast_norm && (st = run_exact_extremes(ctx, img, g, nblocks)) != PXZ_OK) return bail(st);
     bool peers_ok = true;
     st = exchange_minmax(ctx, true, &peers_ok);
     if (st != PXZ_OK) return st;
@@ -1088,7 +1143,7 @@ static pxz_status shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw
           return shrink_to_size(ctx, wide, bw, bh, metric, max_bytes, filter_down, flags, 3, factor_out, p4);
         },
         out);
-  if ((int)filter_down < 0 || (int)filter_down > 4) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (!known_filter(filter_down)) return fail(ctx, PXZ_E_ARG, "unknown filter");
   if (metric != PXZ_METRIC_OKLAB_MAD && metric != PXZ_METRIC_SOBEL_DIR) return fail(ctx, PXZ_E_ARG, "unknown metric");
   if (flags & PXZ_FLAG_AFTER_IDENTITY) return fail(ctx, PXZ_E_ARG, "PXZ_FLAG_AFTER_IDENTITY ignores the factor: no size to choose");
   if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "a size budget is per image: not available on a batch");
@@ -1105,18 +1160,13 @@ static pxz_status shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw
   const bool fast = metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
 
   // analysis as pxz_shrink runs it, without the guard band (it depends on the factor)
-  st = run_analysis(ctx, img, g, metric, exact_all, nullptr);
-  if (st != PXZ_OK) return st;
-  if (normalise) {
-    if ((st = run_minmax(ctx, metric, nblocks)) != PXZ_OK) return st;
-    if (fast && (st = run_exact_extremes(ctx, img, g, nblocks)) != PXZ_OK) return st;
-  }
+  if ((st = run_shrink_analysis(ctx, img, g, metric, flags, nullptr)) != PXZ_OK) return st;
 
   // scratch: the sizes of one round, and on the fast path the copy of the values the search runs on
+  DevBlocks bufs(ctx);
   uint8_t* scratch = nullptr;
   const size_t sizes_bytes = (size_t)kMaxSizeCandidates * sizeof(uint64_t);
-  if ((st = dev_alloc(ctx, (void**)&scratch, sizes_bytes + (fast ? (size_t)nblocks * 4 : 0))) != PXZ_OK) return st;
-  std::unique_ptr<uint8_t, std::function<void(uint8_t*)>> scratch_guard(scratch, [ctx](uint8_t* q) { dev_free(ctx, q); });
+  if ((st = bufs.alloc(&scratch, sizes_bytes + (fast ? (size_t)nblocks * 4 : 0))) != PXZ_OK) return st;
   uint64_t* d_sizes = reinterpret_cast<uint64_t*>(scratch);
   float* d_search = fast ? reinterpret_cast<float*>(scratch + sizes_bytes) : ctx->d_vx;
   const float* d_search_y = metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr;
@@ -1228,9 +1278,9 @@ pxz_status pxz_image_error(pxz_ctx* ctx, const pxz_image* a, const pxz_image* b,
   pxz_status st = make_geom(ctx, a->w, a->h, a->c, bw, bh, &g);
   if (st != PXZ_OK) return st;
   const size_t nblocks = (size_t)g.cols * g.rows;
+  DevBlocks bufs(ctx);
   uint8_t* buf = nullptr;
-  if ((st = dev_alloc(ctx, (void**)&buf, nblocks * (sizeof(uint64_t) + sizeof(uint32_t)))) != PXZ_OK) return st;
-  std::unique_ptr<uint8_t, std::function<void(uint8_t*)>> buf_guard(buf, [ctx](uint8_t* q) { dev_free(ctx, q); });
+  if ((st = bufs.alloc(&buf, nblocks * (sizeof(uint64_t) + sizeof(uint32_t)))) != PXZ_OK) return st;
   uint64_t* d_sse = reinterpret_cast<uint64_t*>(buf);
   uint32_t* d_max = reinterpret_cast<uint32_t*>(buf + nblocks * sizeof(uint64_t));
   if ((st = run_block_error(ctx, a, b, g, d_sse, host_block_max ? d_max : nullptr)) != PXZ_OK) return st;
@@ -1257,12 +1307,10 @@ static pxz_status strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t 
   // payloads pxz_shrink narrows, and the decodes those pxz_expand_to_image narrows.  The alpha channel is 255 in the source and
   // in every decode, so it adds 0 to every sum and the report equals that of the 3-channel image.
   if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
-    pxz_image* wide = nullptr;
+    ImageOwner wide;
     pxz_status st = rgb_widened(ctx, img, &wide);
     if (st != PXZ_OK) return st;
-    st = strategy_measure(ctx, wide, bw, bh, metric, factor, flags, host_sse, host_blocks);
-    pxz_image_free(wide);
-    return st;
+    return strategy_measure(ctx, wide.get(), bw, bh, metric, factor, flags, host_sse, host_blocks);
   }
   Geom g;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g);
@@ -1272,51 +1320,38 @@ static pxz_status strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t 
   // (DESIGN.md §3); the dims are those of pxz_shrink in every mode
   ValueMap vm = shrink_value_map(ctx, metric, flags, factor);
   vm.bucket_edges = ~0ull;
-  const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
   const bool exact_all = (flags & PXZ_FLAG_EXACT_VALUES) != 0;
-  const bool fast_norm = normalise && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
-  st = run_analysis(ctx, img, g, metric, exact_all, (metric == PXZ_METRIC_OKLAB_MAD && !exact_all && !normalise) ? &vm : nullptr);
-  if (st != PXZ_OK) return st;
-  if (normalise) {
-    if ((st = run_minmax(ctx, metric, nblocks)) != PXZ_OK) return st;
-    if (fast_norm && (st = run_exact_extremes(ctx, img, g, nblocks)) != PXZ_OK) return st;
-    if (fast_norm && (st = run_guard_band(ctx, img, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
-  }
+  const bool fast_norm = (flags & PXZ_FLAG_NORMALISE_GLOBAL) && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
+  if ((st = run_shrink_analysis(ctx, img, g, metric, flags, &vm)) != PXZ_OK) return st;
+  if (fast_norm && (st = run_guard_band(ctx, img, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
   // device scratch: the report (65 x 25 sums, 65 counts), the block errors of one pair
   const size_t report_sse = (size_t)kStrategyBuckets * kFilterPairs * sizeof(uint64_t);
   const size_t report_bytes = report_sse + kStrategyBuckets * sizeof(uint32_t);
   const size_t block_sse_off = (report_bytes + 7) & ~(size_t)7;
+  DevBlocks bufs(ctx);
   uint8_t* buf = nullptr;
-  if ((st = dev_alloc(ctx, (void**)&buf, block_sse_off + (size_t)nblocks * sizeof(uint64_t))) != PXZ_OK) return st;
-  std::unique_ptr<uint8_t, std::function<void(uint8_t*)>> buf_guard(buf, [ctx](uint8_t* q) { dev_free(ctx, q); });
+  if ((st = bufs.alloc(&buf, block_sse_off + (size_t)nblocks * sizeof(uint64_t))) != PXZ_OK) return st;
   uint64_t* d_sse = reinterpret_cast<uint64_t*>(buf);
   uint32_t* d_blocks = reinterpret_cast<uint32_t*>(buf + report_sse);
   uint64_t* d_block_sse = reinterpret_cast<uint64_t*>(buf + block_sse_off);
   PXZ_CUDA(ctx, cudaMemsetAsync(buf, 0, report_bytes, ctx->stream));
-  pxz_image* dec = nullptr;
-  if ((st = pxz_image_alloc(ctx, img->w, img->h, img->c, &dec)) != PXZ_OK) return st;
-  std::unique_ptr<pxz_image, void (*)(pxz_image*)> dec_guard(dec, pxz_image_free);
+  ImageOwner dec;
+  if ((st = image_new(ctx, img->w, img->h, img->c, 1, &dec)) != PXZ_OK) return st;
   // down outer, up inner: one payload and one decode alive at a time.  The dims do not depend on the filter, so the five
   // payloads have the same descriptors and the bucket of a block is the same in all 25 passes.
   for (uint32_t down = 0; down < 5; ++down) {
-    pxz_payload* p = nullptr;
-    if ((st = plan_and_resample(ctx, img, g, metric, vm, (pxz_filter)down, exact_all, &p)) != PXZ_OK) return st;
-    for (uint32_t up = 0; up < 5 && st == PXZ_OK; ++up) {
+    pxz_payload* raw = nullptr;
+    if ((st = plan_and_resample(ctx, img, g, metric, vm, (pxz_filter)down, exact_all, &raw)) != PXZ_OK) return st;
+    const PayloadOwner p(raw);
+    for (uint32_t up = 0; up < 5; ++up) {
       const uint32_t pair = down * 5 + up;
-      st = pxz_expand_to_image(ctx, p, (pxz_filter)up, dec);
-      if (st == PXZ_OK) st = run_block_error(ctx, img, dec, g, d_block_sse, nullptr);
-      if (st == PXZ_OK) {
-        ProfScope prof(ctx, K_BUCKET_SUM);
-        const cudaError_t e = launch_bucket_sum(p->d_descs, d_block_sse, nblocks, pair, pair == 0, d_sse, d_blocks, ctx->stream, ctx->sm_count,
-                                                &ctx->launches);
-        if (e != cudaSuccess) {
-          cudaGetLastError();
-          st = fail(ctx, PXZ_E_CUDA, std::string("bucket sum: ") + cudaGetErrorString(e));
-        }
-      }
+      if ((st = pxz_expand_to_image(ctx, p.get(), (pxz_filter)up, dec.get())) != PXZ_OK) return st;
+      if ((st = run_block_error(ctx, img, dec.get(), g, d_block_sse, nullptr)) != PXZ_OK) return st;
+      st = profiled(ctx, K_BUCKET_SUM, "bucket sum", [&] {
+        return launch_bucket_sum(p->d_descs, d_block_sse, nblocks, pair, pair == 0, d_sse, d_blocks, ctx->stream, ctx->sm_count, &ctx->launches);
+      });
+      if (st != PXZ_OK) return st;
     }
-    payload_release(p);
-    if (st != PXZ_OK) return st;
   }
   PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, d_sse, report_sse, cudaMemcpyDeviceToHost, ctx->stream));
   PXZ_CUDA(ctx, cudaMemcpyAsync(host_blocks, d_blocks, kStrategyBuckets * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
@@ -1476,7 +1511,6 @@ static pxz_status payload_from_descs(pxz_ctx* ctx, uint32_t w, uint32_t h, uint3
   std::vector<uint32_t> tabidx(nblocks);
   std::vector<uint8_t> filt(ctx->strategy.on ? nblocks : 0);  // per-block expand filter (pxz_ctx_set_strategy)
   uint32_t max_small = 1, max_tmp_up = 1, max_tmp_down = 1, max_dim = 1;
-  auto pad8 = [](uint32_t v) { return (v + 7u) & ~7u; };
   auto idx_of = [&](uint32_t small, uint32_t tile) -> uint32_t {
     auto it = index.find({small, tile});
     if (it != index.end()) return it->second;
@@ -1505,16 +1539,13 @@ static pxz_status payload_from_descs(pxz_ctx* ctx, uint32_t w, uint32_t h, uint3
     max_tmp_up = std::max(max_tmp_up, th * pad8(d.w));
     max_tmp_down = std::max(max_tmp_down, (uint32_t)d.h * pad8(tw));
   }
-  pxz_payload* p = nullptr;
+  PayloadOwner p;
   st = payload_new(ctx, g, bytes, &p);
   if (st != PXZ_OK) return st;
   p->spec = spec;
   if (ctx->strategy.on) {
     const uint32_t per_filter = (uint32_t)spec->n_small.size();
-    if (per_filter * 5u > 0x10000u) {
-      payload_release(p);
-      return fail(ctx, PXZ_E_UNSUPPORTED, "too many distinct block sizes for per-block filters");
-    }
+    if (per_filter * 5u > 0x10000u) return fail(ctx, PXZ_E_UNSUPPORTED, "too many distinct block sizes for per-block filters");
     for (size_t b = 0; b < nblocks; ++b) tabidx[b] += (filt[b] * per_filter) * 0x10001u;
     p->strategy = 2;
   }
@@ -1533,11 +1564,8 @@ static pxz_status payload_from_descs(pxz_ctx* ctx, uint32_t w, uint32_t h, uint3
   if (e == cudaSuccess) e = launch_class_lists(p->d_descs, g, ctx->d_scan, p->d_order(), (uint32_t)p->nblocks_cap, ctx->stream, &ctx->launches);
   // tabidx is a pageable temporary and `pixels` may be reused by the caller right away
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-  if (e != cudaSuccess) {
-    payload_release(p);
-    return fail(ctx, PXZ_E_CUDA, std::string("payload upload: ") + cudaGetErrorString(e));
-  }
-  *out = p;
+  if (e != cudaSuccess) return cuda_fail(ctx, e, "payload upload");
+  *out = p.release();
   return PXZ_OK;
 }
 
@@ -1580,31 +1608,27 @@ pxz_status pxz_payload_to_container(pxz_ctx* ctx, const pxz_payload* p, uint32_t
   const uint32_t nblocks = g.cols * g.rows;
   const size_t arena_bytes = qoi_arena_bytes(nblocks, bytes, g.C);
   const size_t out_cap = 26 + (size_t)4 * g.rows + arena_bytes;
+  DevBlocks bufs(ctx);
   uint8_t *d_arena = nullptr, *d_out = nullptr;
   uint32_t* d_len = nullptr;
   unsigned long long *d_off = nullptr, *d_total = nullptr;
-  auto release = [&]() { dev_free(ctx, d_arena); dev_free(ctx, d_out); dev_free(ctx, d_len); dev_free(ctx, d_off); dev_free(ctx, d_total); };
-  if ((st = dev_alloc(ctx, (void**)&d_arena, arena_bytes)) != PXZ_OK || (st = dev_alloc(ctx, (void**)&d_out, out_cap)) != PXZ_OK ||
-      (st = dev_alloc(ctx, (void**)&d_len, (size_t)nblocks * 4)) != PXZ_OK || (st = dev_alloc(ctx, (void**)&d_off, (size_t)nblocks * 8)) != PXZ_OK ||
-      (st = dev_alloc(ctx, (void**)&d_total, 8)) != PXZ_OK) {
-    release();
+  if ((st = bufs.alloc(&d_arena, arena_bytes)) != PXZ_OK || (st = bufs.alloc(&d_out, out_cap)) != PXZ_OK ||
+      (st = bufs.alloc(&d_len, (size_t)nblocks * 4)) != PXZ_OK || (st = bufs.alloc(&d_off, (size_t)nblocks * 8)) != PXZ_OK ||
+      (st = bufs.alloc(&d_total, 8)) != PXZ_OK)
     return st;
-  }
-  cudaError_t e;
-  {
-    ProfScope prof(ctx, K_QOI_ENCODE);
-    e = launch_qoi_encode(p->d_descs, p->d_pixels, g, values_present, filter_byte, d_arena, d_len, d_off, d_out, d_total, ctx->stream,
-                          &ctx->launches);
-  }
+  st = profiled(ctx, K_QOI_ENCODE, "container encode", [&] {
+    return launch_qoi_encode(p->d_descs, p->d_pixels, g, values_present, filter_byte, d_arena, d_len, d_off, d_out, d_total, ctx->stream,
+                             &ctx->launches);
+  });
+  if (st != PXZ_OK) return st;
   unsigned long long total = 0;
-  if (e == cudaSuccess) e = cudaMemcpyAsync(&total, d_total, 8, cudaMemcpyDeviceToHost, ctx->stream);
+  cudaError_t e = cudaMemcpyAsync(&total, d_total, 8, cudaMemcpyDeviceToHost, ctx->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
   if (e == cudaSuccess && total <= cap) {
     e = cudaMemcpyAsync(host_out, d_out, total, cudaMemcpyDeviceToHost, ctx->stream);
     if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
   }
-  release();
-  if (e != cudaSuccess) return fail(ctx, PXZ_E_CUDA, std::string("container encode: ") + cudaGetErrorString(e));
+  if (e != cudaSuccess) return cuda_fail(ctx, e, "container encode");
   *bytes_out = total;
   if (total > cap) return fail(ctx, PXZ_E_ARG, "output buffer too small (size it with pxz_container_bound)");
   return PXZ_OK;
@@ -1641,20 +1665,18 @@ pxz_status pxz_payload_from_container(pxz_ctx* ctx, const uint8_t* data, size_t 
   }
   for (size_t b = 0; b < nblocks; ++b)
     if (ch == 4 && (descs[b].offset & 3u)) return fail(ctx, PXZ_E_UNSUPPORTED, "unaligned RGBA block");  // cannot happen: w*h*4
-  pxz_payload* p = nullptr;
-  st = payload_from_descs(ctx, w, h, bw, bh, ch, descs.data(), nullptr, false, bytes, &p);
+  pxz_payload* raw = nullptr;
+  st = payload_from_descs(ctx, w, h, bw, bh, ch, descs.data(), nullptr, false, bytes, &raw);
   if (st != PXZ_OK) return st;
+  PayloadOwner p(raw);
+  DevBlocks bufs(ctx);
   uint8_t* d_in = nullptr;
   unsigned long long* d_off = nullptr;
   uint32_t* d_len = nullptr;
   int* d_err = nullptr;
-  auto release = [&]() { dev_free(ctx, d_in); dev_free(ctx, d_off); dev_free(ctx, d_len); dev_free(ctx, d_err); };
-  if ((st = dev_alloc(ctx, (void**)&d_in, len)) != PXZ_OK || (st = dev_alloc(ctx, (void**)&d_off, nblocks * 8)) != PXZ_OK ||
-      (st = dev_alloc(ctx, (void**)&d_len, nblocks * 4)) != PXZ_OK || (st = dev_alloc(ctx, (void**)&d_err, 4)) != PXZ_OK) {
-    release();
-    payload_release(p);
+  if ((st = bufs.alloc(&d_in, len)) != PXZ_OK || (st = bufs.alloc(&d_off, nblocks * 8)) != PXZ_OK ||
+      (st = bufs.alloc(&d_len, nblocks * 4)) != PXZ_OK || (st = bufs.alloc(&d_err, 4)) != PXZ_OK)
     return st;
-  }
   int err = 0;
   cudaError_t e = cudaMemcpyAsync(d_in, data, len, cudaMemcpyHostToDevice, ctx->stream);
   if (e == cudaSuccess) e = cudaMemcpyAsync(d_off, in_off.data(), nblocks * 8, cudaMemcpyHostToDevice, ctx->stream);
@@ -1666,14 +1688,10 @@ pxz_status pxz_payload_from_container(pxz_ctx* ctx, const uint8_t* data, size_t 
   }
   if (e == cudaSuccess) e = cudaMemcpyAsync(&err, d_err, 4, cudaMemcpyDeviceToHost, ctx->stream);
   if (e == cudaSuccess) e = cudaStreamSynchronize(ctx->stream);
-  release();
-  if (e != cudaSuccess || err) {
-    payload_release(p);
-    return e != cudaSuccess ? fail(ctx, PXZ_E_CUDA, std::string("container decode: ") + cudaGetErrorString(e))
-                            : fail(ctx, PXZ_E_FORMAT, "truncated QOI stream");
-  }
+  if (e != cudaSuccess) return cuda_fail(ctx, e, "container decode");
+  if (err) return fail(ctx, PXZ_E_FORMAT, "truncated QOI stream");
   if (filter_byte) *filter_byte = filt;
-  *out = p;
+  *out = p.release();
   return PXZ_OK;
 }
 
@@ -1683,27 +1701,19 @@ void pxz_payload_free(pxz_payload* p) { payload_release(p); }
 pxz_status pxz_expand_to_image(pxz_ctx* ctx, const pxz_payload* p, pxz_filter filter_up, pxz_image* out) {
   if (!ctx || !p || !out) return PXZ_E_ARG;
   cudaSetDevice(ctx->device);
-  if ((int)filter_up < 0 || (int)filter_up > 4) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (!known_filter(filter_up)) return fail(ctx, PXZ_E_ARG, "unknown filter");
   if (out->w != p->g.W || out->h != p->g.H || out->c != p->g.C || out->nimg != p->g.nimg)
     return fail(ctx, PXZ_E_ARG, "output image geometry mismatch");
   if (rgb_on_rgba(ctx, p->g.W, p->g.C, p->g.bw, p->g.bh) && p->max_small_dim <= 64) {
-    pxz_payload* p4 = nullptr;
+    PayloadOwner p4;
     pxz_status st = payload_rechannel(ctx, p, 4, &p4);
     if (st != PXZ_OK) return st;
-    pxz_image* wide = nullptr;
-    st = pxz_image_alloc_batch(ctx, out->w, out->h, 4, out->nimg, &wide);
-    if (st == PXZ_OK) st = pxz_expand_to_image(ctx, p4, filter_up, wide);
-    if (st == PXZ_OK) {
-      cudaError_t e = launch_rgb_widen(wide->d, wide->pitch, out->d, out->pitch, out->w, out->h * out->nimg, 0, ctx->stream, ctx->sm_count,
-                                       &ctx->launches);
-      if (e != cudaSuccess) {
-        cudaGetLastError();
-        st = fail(ctx, PXZ_E_CUDA, std::string("rgb narrow: ") + cudaGetErrorString(e));
-      }
-    }
-    pxz_image_free(wide);
-    payload_release(p4);
-    return st;
+    ImageOwner wide;
+    if ((st = image_new(ctx, out->w, out->h, 4, out->nimg, &wide)) != PXZ_OK) return st;
+    if ((st = pxz_expand_to_image(ctx, p4.get(), filter_up, wide.get())) != PXZ_OK) return st;
+    cudaError_t e = launch_rgb_widen(wide->d, wide->pitch, out->d, out->pitch, out->w, out->h * out->nimg, 0, ctx->stream, ctx->sm_count,
+                                     &ctx->launches);
+    return e == cudaSuccess ? PXZ_OK : cuda_fail(ctx, e, "rgb narrow");
   }
   TabSet ts;
   pxz_status st = get_tabset(ctx, *p->spec, p->strategy ? -1 : (int)filter_up, 1, &ts);
@@ -1713,13 +1723,11 @@ pxz_status pxz_expand_to_image(pxz_ctx* ctx, const pxz_payload* p, pxz_filter fi
 
 pxz_status pxz_expand(pxz_ctx* ctx, const pxz_payload* p, pxz_filter filter_up, uint8_t* host_out, size_t host_pitch) {
   if (!ctx || !p || !host_out) return PXZ_E_ARG;
-  pxz_image* im = nullptr;
-  pxz_status st = pxz_image_alloc_batch(ctx, p->g.W, p->g.H, p->g.C, p->g.nimg, &im);
+  ImageOwner im;
+  pxz_status st = image_new(ctx, p->g.W, p->g.H, p->g.C, p->g.nimg, &im);
   if (st != PXZ_OK) return st;
-  st = pxz_expand_to_image(ctx, p, filter_up, im);
-  if (st == PXZ_OK) st = pxz_image_download(ctx, im, host_out, host_pitch);
-  pxz_image_free(im);
-  return st;
+  st = pxz_expand_to_image(ctx, p, filter_up, im.get());
+  return st != PXZ_OK ? st : pxz_image_download(ctx, im.get(), host_out, host_pitch);
 }
 
 // ---- random access (extension) ------------------------------------------------------------------------------------
@@ -1744,26 +1752,15 @@ pxz_status pxz_payload_window(pxz_ctx* ctx, const pxz_payload* p, uint32_t c0, u
   // max_small_px bounds every block of p, whatever made it (uploads may hold blocks larger than their tiles); the parent's
   // capacity alone could be the whole gigapixel frame
   const uint64_t capacity = std::min<uint64_t>(p->capacity, (uint64_t)nblocks * p->max_small_px * pg.C);
-  pxz_payload* wp = nullptr;
+  PayloadOwner wp;
   if ((st = payload_new(ctx, g, capacity, &wp)) != PXZ_OK) return st;
-  // the window's table indices are the parent's: same spec, same bounds, same kernel family
-  wp->spec = p->spec;
-  wp->strategy = p->strategy;
-  wp->max_small_px = p->max_small_px; wp->max_small_dim = p->max_small_dim;
-  wp->max_tmp_down = p->max_tmp_down; wp->max_tmp_up = p->max_tmp_up;
-  cudaError_t e;
-  {
-    ProfScope prof(ctx, K_PAYLOAD_WINDOW);
-    e = launch_payload_window(p->d_descs, p->d_tabidx, (uint32_t)p->nblocks_cap, p->d_pixels, pg.cols, c0, r0, g, p->strategy == 1,
-                              wp->d_descs, wp->d_tabidx, (uint32_t)wp->nblocks_cap, wp->d_pixels, wp->d_total, ctx->d_scan, ctx->stream,
-                              &ctx->launches);
-  }
-  if (e != cudaSuccess) {
-    cudaGetLastError();
-    payload_release(wp);
-    return fail(ctx, PXZ_E_CUDA, std::string("payload window: ") + cudaGetErrorString(e));
-  }
-  *out = wp;
+  copy_layout(wp.get(), p);  // the window's table indices are the parent's: same spec, same bounds, same kernel family
+  st = profiled(ctx, K_PAYLOAD_WINDOW, "payload window", [&] {
+    return launch_payload_window(p->d_descs, p->d_tabidx, (uint32_t)p->nblocks_cap, p->d_pixels, pg.cols, c0, r0, g, p->strategy == 1, wp->d_descs,
+                                 wp->d_tabidx, (uint32_t)wp->nblocks_cap, wp->d_pixels, wp->d_total, ctx->d_scan, ctx->stream, &ctx->launches);
+  });
+  if (st != PXZ_OK) return st;
+  *out = wp.release();
   return PXZ_OK;
 }
 
@@ -1773,36 +1770,26 @@ pxz_status pxz_expand_region(pxz_ctx* ctx, const pxz_payload* p, pxz_filter filt
   cudaSetDevice(ctx->device);
   const Geom& pg = p->g;
   if (pg.nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "regions of a batch payload are not supported");
-  if ((int)filter_up < 0 || (int)filter_up > 4) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (!known_filter(filter_up)) return fail(ctx, PXZ_E_ARG, "unknown filter");
   if (w == 0 || h == 0) return fail(ctx, PXZ_E_ARG, "empty rectangle");
   if (x >= pg.W || y >= pg.H || w > pg.W - x || h > pg.H - y) return fail(ctx, PXZ_E_ARG, "rectangle outside the image");
   if (out->w != w || out->h != h || out->c != pg.C || out->nimg != 1) return fail(ctx, PXZ_E_ARG, "output image geometry mismatch");
   if (x == 0 && y == 0 && w == pg.W && h == pg.H) return pxz_expand_to_image(ctx, p, filter_up, out);
   const uint32_t c0 = x / pg.bw, r0 = y / pg.bh;
   const uint32_t nc = (x + w - 1) / pg.bw - c0 + 1, nr = (y + h - 1) / pg.bh - r0 + 1;
-  pxz_payload* wp = nullptr;
-  pxz_status st = pxz_payload_window(ctx, p, c0, r0, nc, nr, &wp);
+  pxz_payload* raw = nullptr;
+  pxz_status st = pxz_payload_window(ctx, p, c0, r0, nc, nr, &raw);
   if (st != PXZ_OK) return st;
+  const PayloadOwner wp(raw);
   const uint32_t dx = x - c0 * pg.bw, dy = y - r0 * pg.bh;
-  if (dx == 0 && dy == 0 && w == wp->g.W && h == wp->g.H) {
-    st = pxz_expand_to_image(ctx, wp, filter_up, out);  // the rectangle is the window: no staging
-  } else {
-    pxz_image* stage = nullptr;
-    st = pxz_image_alloc(ctx, wp->g.W, wp->g.H, pg.C, &stage);
-    if (st == PXZ_OK) st = pxz_expand_to_image(ctx, wp, filter_up, stage);
-    if (st == PXZ_OK) {
-      ProfScope prof(ctx, K_REGION_COPY);
-      const cudaError_t e = cudaMemcpy2DAsync(out->d, out->pitch, stage->d + (size_t)dy * stage->pitch + (size_t)dx * pg.C, stage->pitch,
-                                              (size_t)w * pg.C, h, cudaMemcpyDeviceToDevice, ctx->stream);
-      if (e != cudaSuccess) {
-        cudaGetLastError();
-        st = fail(ctx, PXZ_E_CUDA, std::string("region copy: ") + cudaGetErrorString(e));
-      }
-    }
-    pxz_image_free(stage);  // stream-ordered: the copy queued above keeps it
-  }
-  payload_release(wp);
-  return st;
+  if (dx == 0 && dy == 0 && w == wp->g.W && h == wp->g.H) return pxz_expand_to_image(ctx, wp.get(), filter_up, out);  // no staging
+  ImageOwner stage;  // freed stream-ordered: the copy queued below keeps it
+  if ((st = image_new(ctx, wp->g.W, wp->g.H, pg.C, 1, &stage)) != PXZ_OK) return st;
+  if ((st = pxz_expand_to_image(ctx, wp.get(), filter_up, stage.get())) != PXZ_OK) return st;
+  return profiled(ctx, K_REGION_COPY, "region copy", [&] {
+    return cudaMemcpy2DAsync(out->d, out->pitch, stage->d + (size_t)dy * stage->pitch + (size_t)dx * pg.C, stage->pitch, (size_t)w * pg.C, h,
+                             cudaMemcpyDeviceToDevice, ctx->stream);
+  });
 }
 
 // ---- quadtree processing (process/tree.rs:23-109) ---------------------------------------------------------
@@ -1810,7 +1797,7 @@ pxz_status pxz_tree_process(pxz_ctx* ctx, const pxz_image* img, float threshold,
                             uint32_t min_bh, pxz_filter filter_down, pxz_filter filter_up, pxz_image* out) {
   if (!ctx || !img || !out) return PXZ_E_ARG;
   cudaSetDevice(ctx->device);
-  if ((int)filter_down < 0 || (int)filter_down > 4 || (int)filter_up < 0 || (int)filter_up > 4) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (!known_filter(filter_down) || !known_filter(filter_up)) return fail(ctx, PXZ_E_ARG, "unknown filter");
   if (out->w != img->w || out->h != img->h || out->c != img->c) return fail(ctx, PXZ_E_ARG, "output image geometry mismatch");
   if (img->nimg != 1 || out->nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "tree processing takes one image at a time");
   if (bw == 0 || bh == 0) return fail(ctx, PXZ_E_ARG, "block size must be >= 1");
@@ -1828,56 +1815,44 @@ pxz_status pxz_tree_process(pxz_ctx* ctx, const pxz_image* img, float threshold,
   const bool positive = threshold >= 0.0f;  // :38
   const float thr = fabsf(threshold);       // :39
 
+  DevBlocks bufs(ctx);
   uint8_t* d_leaf = nullptr;
   uint8_t* d_rec[2] = {nullptr, nullptr};
   Geom gl;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw >> (levels - 1), bh >> (levels - 1), &gl);
   if (st != PXZ_OK) return st;
   const size_t max_blocks = (size_t)gl.cols * gl.rows;
-  if ((st = dev_alloc(ctx, (void**)&d_leaf, max_blocks)) != PXZ_OK) return st;
-  if ((st = dev_alloc(ctx, (void**)&d_rec[0], max_blocks)) != PXZ_OK || (st = dev_alloc(ctx, (void**)&d_rec[1], max_blocks)) != PXZ_OK) {
-    dev_free(ctx, d_leaf); dev_free(ctx, d_rec[0]); dev_free(ctx, d_rec[1]);
+  if ((st = bufs.alloc(&d_leaf, max_blocks)) != PXZ_OK || (st = bufs.alloc(&d_rec[0], max_blocks)) != PXZ_OK ||
+      (st = bufs.alloc(&d_rec[1], max_blocks)) != PXZ_OK)
     return st;
-  }
   uint32_t parent_cols = 0;
-  for (int lv = 0; lv < levels && st == PXZ_OK; ++lv) {
+  for (int lv = 0; lv < levels; ++lv) {
     Geom g;
-    st = make_geom(ctx, img->w, img->h, img->c, bw >> lv, bh >> lv, &g);
-    if (st != PXZ_OK) break;
+    if ((st = make_geom(ctx, img->w, img->h, img->c, bw >> lv, bh >> lv, &g)) != PXZ_OK) return st;
     ValueMap vm;
     vm.factor = 1.0f; vm.mode = 1; vm.normalise = 0;  // after = identity (tree.rs:97)
     vm.extra_thr = thr;
-    st = run_analysis(ctx, img, g, PXZ_METRIC_OKLAB_MAD, false, &vm);
-    if (st != PXZ_OK) break;
+    if ((st = run_analysis(ctx, img, g, PXZ_METRIC_OKLAB_MAD, false, &vm)) != PXZ_OK) return st;
     cudaError_t e = launch_tree_mask(ctx->d_vx, g, lv == 0 ? nullptr : d_rec[(lv - 1) & 1], parent_cols, thr,
                                      (lv == 0 ? positive : true) ? 1 : 0,  // the recursion receives |threshold| (:70)
                                      d_leaf, d_rec[lv & 1], ctx->stream, &ctx->launches);
-    if (e != cudaSuccess) { st = fail(ctx, PXZ_E_CUDA, std::string("tree mask: ") + cudaGetErrorString(e)); break; }
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "tree mask");
     parent_cols = g.cols;
-    pxz_payload* p = nullptr;
-    st = payload_new(ctx, g, (uint64_t)g.W * g.H * g.C, &p);
-    if (st != PXZ_OK) break;
+    PayloadOwner p;
+    if ((st = payload_new(ctx, g, (uint64_t)g.W * g.H * g.C, &p)) != PXZ_OK) return st;
     p->spec = spec_for_geom(g);
-    auto pad8 = [](uint32_t v) { return (v + 7u) & ~7u; };
-    p->max_small_px = g.bw * g.bh;
-    p->max_small_dim = std::max(g.bw, g.bh);
-    p->max_tmp_down = ((g.bh + 1) / 2) * pad8(g.bw);
-    p->max_tmp_up = g.bh * pad8((g.bw + 1) / 2);
+    set_plan_bounds(p.get(), g, true);
     vm.extra_thr = NAN;
     e = launch_plan(ctx->d_vx, nullptr, g, vm, ctx->d_minmax, ctx->thr, d_leaf, p->d_descs, p->d_tabidx, p->d_total, ctx->d_scan, p->d_order(),
                     (uint32_t)p->nblocks_cap, ctx->stream, &ctx->launches);
-    if (e != cudaSuccess) st = fail(ctx, PXZ_E_CUDA, std::string("plan: ") + cudaGetErrorString(e));
+    if (e != cudaSuccess) return cuda_fail(ctx, e, "plan");
     TabSet ts;
-    if (st == PXZ_OK) st = get_tabset(ctx, *p->spec, (int)filter_down, 0, &ts);
-    if (st == PXZ_OK) st = run_resample(ctx, 0, img->d, img->pitch, p, ts, g.bw * g.bh, std::max(g.bw, g.bh), p->max_tmp_down);
-    if (st == PXZ_OK) st = get_tabset(ctx, *p->spec, (int)filter_up, 1, &ts);
-    if (st == PXZ_OK) st = run_resample(ctx, 1, out->d, out->pitch, p, ts, p->max_small_px, p->max_small_dim, p->max_tmp_up);
-    payload_release(p);
+    if ((st = get_tabset(ctx, *p->spec, (int)filter_down, 0, &ts)) != PXZ_OK) return st;
+    if ((st = run_resample(ctx, 0, img->d, img->pitch, p.get(), ts, g.bw * g.bh, std::max(g.bw, g.bh), p->max_tmp_down)) != PXZ_OK) return st;
+    if ((st = get_tabset(ctx, *p->spec, (int)filter_up, 1, &ts)) != PXZ_OK) return st;
+    if ((st = run_resample(ctx, 1, out->d, out->pitch, p.get(), ts, p->max_small_px, p->max_small_dim, p->max_tmp_up)) != PXZ_OK) return st;
   }
-  dev_free(ctx, d_leaf);
-  dev_free(ctx, d_rec[0]);
-  dev_free(ctx, d_rec[1]);
-  return st;
+  return PXZ_OK;
 }
 
 // ---- multi-GPU ----------------------------------------------------------------------------------------

@@ -2339,9 +2339,19 @@ __global__ void __launch_bounds__(kThreads) k_resample_fir(int direction, uint8_
 // ------------------------------------------------------------------------------------------------
 static inline int clamp_grid(long long want, long long cap) { return (int)(want < 1 ? 1 : (want > cap ? cap : want)); }
 
-// launch with programmatic stream serialization (see pdl_wait): the kernel may be scheduled while its predecessor drains
+template <typename K>
+static cudaError_t set_smem(K kernel, size_t bytes) {
+  if (bytes > 48 * 1024) return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+  return cudaSuccess;
+}
+
+// Both launchers raise the kernel's dynamic shared memory limit when `smem` is above the default 48 KB and return
+// cudaGetLastError() of the launch.
+// launch_pdl: programmatic stream serialization (see pdl_wait): the kernel may be scheduled while its predecessor drains
 template <typename... KArgs, typename... Args>
 static cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, size_t smem, cudaStream_t s, Args&&... args) {
+  cudaError_t e = set_smem(kernel, smem);
+  if (e != cudaSuccess) return e;
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = dim3((unsigned)grid);
   cfg.blockDim = dim3((unsigned)block);
@@ -2352,56 +2362,41 @@ static cudaError_t launch_pdl(void (*kernel)(KArgs...), int grid, int block, siz
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+  e = cudaLaunchKernelEx(&cfg, kernel, KArgs(args)...);
+  const cudaError_t last = cudaGetLastError();
+  return e != cudaSuccess ? e : last;
 }
-
-template <typename K>
-static cudaError_t set_smem(K kernel, size_t bytes) {
-  if (bytes > 48 * 1024) return cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
-  return cudaSuccess;
+// launch: an ordinary stream-ordered launch
+template <typename... KArgs, typename... Args>
+static cudaError_t launch(void (*kernel)(KArgs...), dim3 grid, int block, size_t smem, cudaStream_t s, Args&&... args) {
+  const cudaError_t e = set_smem(kernel, smem);
+  if (e != cudaSuccess) return e;
+  kernel<<<grid, block, smem, s>>>(KArgs(args)...);
+  return cudaGetLastError();
 }
 
 cudaError_t launch_analyze_mad_fast(const uint8_t* img, size_t pitch, const Geom& g, float* vx, uint8_t* opaque,
                                     uint32_t* zero_word, cudaStream_t s, int sm_count, uint64_t* launches) {
   const uint32_t ntiles = g.cols * g.rows;
-  const size_t smem_any = 256 * 32 * sizeof(float);
-  size_t smem = 256 * kMadLutStride * sizeof(float);  // k_analyze_mad_rgba
   const bool aligned = g.C == 4 && (g.bw % 4 == 0) && (g.W % 4 == 0) && (pitch % 16 == 0) &&
                        ((reinterpret_cast<uintptr_t>(img) & 15u) == 0);
   const uint32_t quads = (g.bw / 4) * g.bh;
-  cudaError_t e = cudaSuccess;
   ++*launches;
   if (aligned && quads <= 1024) {
-    // G threads per tile, <= 4 quads (16 px) per thread
-    if (quads > 512) {
-      e = set_smem(k_analyze_mad_rgba<256, 4>, smem);
-      if (e != cudaSuccess) return e;
-      e = launch_pdl(k_analyze_mad_rgba<256, 4>, clamp_grid(ntiles, sm_count * PXZ_MAD_MINBLOCKS), kThreads, smem, s, img, pitch, g, vx, opaque, zero_word);
-    } else if (quads > 256) {
-      e = set_smem(k_analyze_mad_rgba<128, 4>, smem);
-      if (e != cudaSuccess) return e;
-      e = launch_pdl(k_analyze_mad_rgba<128, 4>, clamp_grid((ntiles + 1) / 2, sm_count * PXZ_MAD_MINBLOCKS), kThreads, smem, s, img, pitch, g, vx, opaque, zero_word);
-    } else if (quads > 128) {
-      e = set_smem(k_analyze_mad_rgba<64, 4>, smem);
-      if (e != cudaSuccess) return e;
-      e = launch_pdl(k_analyze_mad_rgba<64, 4>, clamp_grid((ntiles + 3) / 4, sm_count * PXZ_MAD_MINBLOCKS), kThreads, smem, s, img, pitch, g, vx, opaque, zero_word);
-    } else {
-      e = set_smem(k_analyze_mad_rgba<32, 4>, smem);
-      if (e != cudaSuccess) return e;
-      e = launch_pdl(k_analyze_mad_rgba<32, 4>, clamp_grid((ntiles + 7) / 8, sm_count * PXZ_MAD_MINBLOCKS), kThreads, smem, s, img, pitch, g, vx, opaque, zero_word);
-    }
-  } else if (g.C == 4) {
-    smem = smem_any;
-    e = set_smem(k_analyze_mad_any<4>, smem);
-    if (e != cudaSuccess) return e;
-    e = launch_pdl(k_analyze_mad_any<4>, clamp_grid(ntiles, sm_count * 3), kThreads, smem, s, img, pitch, g, vx, opaque, zero_word);
-  } else {
-    smem = smem_any;
-    e = set_smem(k_analyze_mad_any<3>, smem);
-    if (e != cudaSuccess) return e;
-    e = launch_pdl(k_analyze_mad_any<3>, clamp_grid(ntiles, sm_count * 3), kThreads, smem, s, img, pitch, g, vx, opaque, zero_word);
+    // G threads per tile, <= 4 quads (16 px) per thread; 256 / G tiles per CTA
+    struct Variant {
+      void (*kernel)(const uint8_t*, size_t, Geom, float*, uint8_t*, uint32_t*);
+      uint32_t tiles_per_cta;
+    };
+    const Variant v = quads > 512   ? Variant{k_analyze_mad_rgba<256, 4>, 1}
+                      : quads > 256 ? Variant{k_analyze_mad_rgba<128, 4>, 2}
+                      : quads > 128 ? Variant{k_analyze_mad_rgba<64, 4>, 4}
+                                    : Variant{k_analyze_mad_rgba<32, 4>, 8};
+    return launch_pdl(v.kernel, clamp_grid((ntiles + v.tiles_per_cta - 1) / v.tiles_per_cta, sm_count * PXZ_MAD_MINBLOCKS), kThreads,
+                      256 * kMadLutStride * sizeof(float), s, img, pitch, g, vx, opaque, zero_word);
   }
-  return cudaGetLastError();
+  return launch_pdl(g.C == 4 ? k_analyze_mad_any<4> : k_analyze_mad_any<3>, clamp_grid(ntiles, sm_count * 3), kThreads,
+                    256 * 32 * sizeof(float), s, img, pitch, g, vx, opaque, zero_word);
 }
 
 cudaError_t launch_analyze_mad_exact(const uint8_t* img, size_t pitch, const Geom& g, float* vx, const float* vx_fast,
@@ -2409,19 +2404,16 @@ cudaError_t launch_analyze_mad_exact(const uint8_t* img, size_t pitch, const Geo
                                      const float* minmax, uint32_t* list, uint32_t* count, cudaStream_t s, int sm_count,
                                      uint64_t* launches) {
   const uint32_t ntiles = g.cols * g.rows;
-  const size_t smem = (size_t)4 * kExactStride * sizeof(float);
-  cudaError_t e;
   const bool banded = vx_fast != nullptr;
   if (banded) {
     // *count was zeroed by the fast analysis kernel that produced vx_fast (launch_analyze_mad_fast's zero_word), or by the
     // caller between two lists of one image
     ++*launches;
-    if (vm == nullptr)  // candidates for the image's extremes (global normalisation on the fast path)
-      e = launch_pdl(k_extreme_list, (ntiles + kThreads - 1) / kThreads, kThreads, 0, s, vx_fast, opaque, g, (int)g.C, *band, minmax, list, count);
-    else
-      e = launch_pdl(k_band_list, (ntiles + kThreads - 1) / kThreads, kThreads, 0, s, vx_fast, opaque, g, (int)g.C, *vm, *thr, *band, minmax,
-                     list, count);
-    e = cudaGetLastError();
+    const int lgrid = (ntiles + kThreads - 1) / kThreads;
+    const cudaError_t e =
+        vm == nullptr  // candidates for the image's extremes (global normalisation on the fast path)
+            ? launch_pdl(k_extreme_list, lgrid, kThreads, 0, s, vx_fast, opaque, g, (int)g.C, *band, minmax, list, count)
+            : launch_pdl(k_band_list, lgrid, kThreads, 0, s, vx_fast, opaque, g, (int)g.C, *vm, *thr, *band, minmax, list, count);
     if (e != cudaSuccess) return e;
   }
   ++*launches;
@@ -2429,16 +2421,8 @@ cudaError_t launch_analyze_mad_exact(const uint8_t* img, size_t pitch, const Geo
   // anything between a handful and all tiles (an image whose values all sit at the extremes): the grid covers both.
   const int threads = banded ? kExactThreads : kThreads;
   const int grid = clamp_grid(ntiles, (long long)sm_count * (banded ? 2 : 3));
-  if (g.C == 4) {
-    e = set_smem(k_mad_exact<4>, smem);
-    if (e != cudaSuccess) return e;
-    e = launch_pdl(k_mad_exact<4>, grid, threads, smem, s, img, pitch, g, vx, banded ? list : nullptr, count);
-  } else {
-    e = set_smem(k_mad_exact<3>, smem);
-    if (e != cudaSuccess) return e;
-    e = launch_pdl(k_mad_exact<3>, grid, threads, smem, s, img, pitch, g, vx, banded ? list : nullptr, count);
-  }
-  return cudaGetLastError();
+  return launch_pdl(g.C == 4 ? k_mad_exact<4> : k_mad_exact<3>, grid, threads, (size_t)4 * kExactStride * sizeof(float), s, img, pitch, g, vx,
+                    banded ? list : nullptr, count);
 }
 
 // cuTensorMapEncodeTiled through the runtime (the library links cudart statically and has no libcuda dependency)
@@ -2485,39 +2469,24 @@ cudaError_t launch_analyze_sobel(const uint8_t* img, size_t pitch, const Geom& g
   // RGBA, 64x64 tiles, rows a tensor copy can address: tiles streamed by TMA, dp4a row terms (analyze_sobel_tma.cuh)
   if (g.C == 4 && g.bw == 64 && g.bh == 64 && (pitch % 16 == 0) && ((reinterpret_cast<uintptr_t>(img) & 15u) == 0) && sobel_tma_enabled()) {
     CUtensorMap tm;
-    if (make_image_tmap(img, pitch, g.W, g.nimg > 1 ? (g.nimg - 1) * g.img_rows + g.H : g.H, &tm, 64)) {
-      cudaError_t e = set_smem(k_analyze_sobel_tma, (size_t)kSobSmemBytes);
-      if (e != cudaSuccess) return e;
-      k_analyze_sobel_tma<<<clamp_grid(ntiles, (long long)sm_count * PXZ_SOBEL_CTAS), 256, kSobSmemBytes, s>>>(tm, g, vx, vy);
-      return cudaGetLastError();
-    }
+    if (make_image_tmap(img, pitch, g.W, g.nimg > 1 ? (g.nimg - 1) * g.img_rows + g.H : g.H, &tm, 64))
+      return launch(k_analyze_sobel_tma, clamp_grid(ntiles, (long long)sm_count * PXZ_SOBEL_CTAS), 256, kSobSmemBytes, s, tm, g, vx, vy);
   }
   const bool small = g.bw <= 64 && g.bh <= 64 && (g.C == 3 || ((pitch & 3u) == 0 && (reinterpret_cast<uintptr_t>(img) & 3u) == 0));
-  if (small) {
-    if (g.C == 4)
-      k_analyze_sobel_tile64<4><<<clamp_grid(ntiles, sm_count * 8), kThreads, 0, s>>>(img, pitch, g, vx, vy);
-    else
-      k_analyze_sobel_tile64<3><<<clamp_grid(ntiles, sm_count * 8), kThreads, 0, s>>>(img, pitch, g, vx, vy);
-  } else if (g.C == 4) {
-    k_analyze_sobel<4><<<clamp_grid(ntiles, sm_count * 8), kThreads, 0, s>>>(img, pitch, g, vx, vy);
-  } else {
-    k_analyze_sobel<3><<<clamp_grid(ntiles, sm_count * 8), kThreads, 0, s>>>(img, pitch, g, vx, vy);
-  }
-  return cudaGetLastError();
+  const auto k = small ? (g.C == 4 ? k_analyze_sobel_tile64<4> : k_analyze_sobel_tile64<3>) : (g.C == 4 ? k_analyze_sobel<4> : k_analyze_sobel<3>);
+  return launch(k, clamp_grid(ntiles, sm_count * 8), kThreads, 0, s, img, pitch, g, vx, vy);
 }
 
 cudaError_t launch_tree_mask(const float* vx, const Geom& g, const uint8_t* parent_recurse, uint32_t parent_cols, float thr,
                              int positive, uint8_t* leaf, uint8_t* recurse, cudaStream_t s, uint64_t* launches) {
   const uint32_t n = g.cols * g.rows;
   ++*launches;
-  k_tree_mask<<<(n + kThreads - 1) / kThreads, kThreads, 0, s>>>(vx, g, parent_recurse, parent_cols, thr, positive, leaf, recurse);
-  return cudaGetLastError();
+  return launch(k_tree_mask, (n + kThreads - 1) / kThreads, kThreads, 0, s, vx, g, parent_recurse, parent_cols, thr, positive, leaf, recurse);
 }
 
 cudaError_t launch_minmax(const float* vx, const float* vy, uint32_t n, float* minmax4, cudaStream_t s, uint64_t* launches) {
   ++*launches;
-  k_minmax<<<1, 1024, 0, s>>>(vx, vy, n, minmax4);
-  return cudaGetLastError();
+  return launch(k_minmax, 1, 1024, 0, s, vx, vy, n, minmax4);
 }
 
 // layout: class_hist[16] | ScanState
@@ -2536,14 +2505,12 @@ cudaError_t launch_plan(const float* vx, const float* vy, const Geom& g, const V
   const bool adaptive = strategy != nullptr && strategy->on != 0 && tabidx_up != nullptr;
   StrategyLut lut = {};
   if (adaptive) lut = *strategy;
-  cudaError_t e = cudaSuccess;  // scan_state is zero on entry and on exit (ensure_scratch clears it once)
+  // scan_state is zero on entry and on exit (ensure_scratch clears it once)
   ++*launches;
   uint32_t* cursor = reinterpret_cast<uint32_t*>(scan_state);
   ScanState* st = reinterpret_cast<ScanState*>(reinterpret_cast<uint8_t*>(scan_state) + kClassHistBytes);
-  unsigned long long* total = reinterpret_cast<unsigned long long*>(total_bytes);
-  if (adaptive) e = launch_pdl(k_plan<true>, tiles, kThreads, 0, s, vx, vy, g, vm, minmax, thr, mask, descs, tabidx, total, st, cursor, lists, cap, lut, tabidx_up);
-  else e = launch_pdl(k_plan<false>, tiles, kThreads, 0, s, vx, vy, g, vm, minmax, thr, mask, descs, tabidx, total, st, cursor, lists, cap, lut, tabidx_up);
-  return e != cudaSuccess ? e : cudaGetLastError();
+  return launch_pdl(adaptive ? k_plan<true> : k_plan<false>, tiles, kThreads, 0, s, vx, vy, g, vm, minmax, thr, mask, descs, tabidx,
+                    reinterpret_cast<unsigned long long*>(total_bytes), st, cursor, lists, cap, lut, tabidx_up);
 }
 
 cudaError_t launch_size_curve(const float* vx, const float* vy, const Geom& g, const ValueMap& vm, const float* minmax,
@@ -2557,8 +2524,7 @@ cudaError_t launch_size_curve(const float* vx, const float* vy, const Geom& g, c
   // few blocks: split the candidates over more CTAs (at least 8 candidates per CTA) to fill the SMs
   const int gy = clamp_grid(std::min<long long>((long long)sm_count * 2 / gx, cand.n / 8), 32);
   ++*launches;
-  k_size_curve<<<dim3(gx, gy), kThreads, 0, s>>>(vx, vy, g, vm, minmax, thr, bpp, cand, reinterpret_cast<unsigned long long*>(bytes));
-  return cudaGetLastError();
+  return launch(k_size_curve, dim3(gx, gy), kThreads, 0, s, vx, vy, g, vm, minmax, thr, bpp, cand, reinterpret_cast<unsigned long long*>(bytes));
 }
 
 size_t window_scan_state_bytes(uint32_t nblocks) {
@@ -2573,10 +2539,8 @@ cudaError_t launch_payload_window(const pxz_block_desc* pdescs, const uint32_t* 
   uint32_t* cursor = reinterpret_cast<uint32_t*>(scan_state);  // zero on entry and on exit
   ScanState* st = reinterpret_cast<ScanState*>(reinterpret_cast<uint8_t*>(scan_state) + kClassHistBytes);
   ++*launches;
-  k_payload_window<<<(nblocks + kWindowTile - 1) / kWindowTile, kThreads, 0, s>>>(pdescs, pmeta, pcap, ppx, pcols, c0, r0, g, copy_up ? 1 : 0,
-                                                                            descs, meta, cap, px,
-                                                                            reinterpret_cast<unsigned long long*>(total_bytes), st, cursor);
-  return cudaGetLastError();
+  return launch(k_payload_window, (nblocks + kWindowTile - 1) / kWindowTile, kThreads, 0, s, pdescs, pmeta, pcap, ppx, pcols, c0, r0, g,
+                copy_up ? 1 : 0, descs, meta, cap, px, reinterpret_cast<unsigned long long*>(total_bytes), st, cursor);
 }
 
 cudaError_t launch_class_lists(const pxz_block_desc* descs, const Geom& g, void* scan_state, uint32_t* lists, uint32_t cap,
@@ -2584,8 +2548,7 @@ cudaError_t launch_class_lists(const pxz_block_desc* descs, const Geom& g, void*
   const uint32_t nblocks = g.cols * g.rows;
   uint32_t* cursor = reinterpret_cast<uint32_t*>(scan_state);  // zero on entry and on exit
   ++*launches;
-  k_class_lists<<<(nblocks + kThreads - 1) / kThreads, kThreads, 0, s>>>(descs, g, cursor, lists, cap);
-  return cudaGetLastError();
+  return launch(k_class_lists, (nblocks + kThreads - 1) / kThreads, kThreads, 0, s, descs, g, cursor, lists, cap);
 }
 
 size_t resample_smem_bytes(uint32_t max_src_px, uint32_t max_tmp_px, uint32_t C) {
@@ -2594,103 +2557,58 @@ size_t resample_smem_bytes(uint32_t max_src_px, uint32_t max_tmp_px, uint32_t C)
 
 int resample_grid(int sm_count, uint32_t nblocks) { return clamp_grid(nblocks, (long long)sm_count * 8); }
 
-cudaError_t launch_resample(int direction, uint8_t* img, size_t pitch, const Geom& g, const pxz_block_desc* descs,
-                            const uint32_t* tabidx, uint8_t* payload, const AxisTab* tabs, const uint32_t* pool,
-                            uint32_t ntabs, uint32_t max_src_px, uint32_t max_src_dim, uint32_t max_tmp_px, uint32_t max_tab_words,
-                            uint8_t* scratch, size_t scratch_per_cta, int grid, bool fused, const uint8_t* opaque_flags,
-                            uint32_t* tile_counter, const uint32_t* lists, uint32_t cap, bool warp_tables, int prefer, bool has_noslide,
-                            cudaStream_t s, int sm_count, uint64_t* launches) {
-  cudaError_t e;
+cudaError_t launch_resample(const ResampleArgs& a, cudaStream_t s, int sm_count, uint64_t* launches) {
+  const Geom& g = a.g;
   ++*launches;
   // RGBA fast paths: tiles <= 64x64 with 16-byte aligned rows
-  const bool fast = g.C == 4 && g.bw <= 64 && g.bh <= 64 && (g.bw % 4 == 0) && (g.W % 4 == 0) && (pitch % 16 == 0) &&
-                    ((reinterpret_cast<uintptr_t>(img) & 15u) == 0) && max_src_px <= (uint32_t)kFastMaxPx && max_src_dim <= 64u &&
-                    max_tmp_px <= (uint32_t)kFastMaxPx && max_tab_words <= (uint32_t)kFastMaxTabWords &&
-                    ntabs <= (uint32_t)kFastMaxTabs && scratch == nullptr;
+  const bool fast = g.C == 4 && g.bw <= 64 && g.bh <= 64 && (g.bw % 4 == 0) && (g.W % 4 == 0) && (a.pitch % 16 == 0) &&
+                    ((reinterpret_cast<uintptr_t>(a.img) & 15u) == 0) && a.max_src_px <= (uint32_t)kFastMaxPx && a.max_src_dim <= 64u &&
+                    a.max_tmp_px <= (uint32_t)kFastMaxPx && a.max_tab_words <= (uint32_t)kFastMaxTabWords &&
+                    a.ntabs <= (uint32_t)kFastMaxTabs && a.scratch == nullptr;
   // warp-per-tile kernels (resample_warp.cuh, resample_tma.cuh) once there are enough tiles to keep every warp slot of
   // the GPU busy for a few tiles; below that one tile's latency (15-40 us on one warp) decides and 8 warps per tile
-  // finish sooner.  prefer: 0 = by tile count, 1 = warp kernels (cp.async ring), 2 = CTA kernels, 3 = TMA shrink kernel
+  // finish sooner.  a.kernels forces a family (ResampleKernels).
   const long long ntiles = (long long)g.cols * g.rows;
-  const bool force_warp = prefer == 1 || prefer == 3;
-  if (fast && warp_tables && tile_counter != nullptr && prefer != 2 && (force_warp || ntiles >= (long long)sm_count * 16)) {
-    if (direction == 0) {
-      bool ring_kernel = prefer == 1;
-      if (!ring_kernel) {
-        CUtensorMap tm;
-        if (make_image_tmap(img, pitch, g.W, g.nimg > 1 ? (g.nimg - 1) * g.img_rows + g.H : g.H, &tm)) {
-          const size_t smem = (size_t)kTWarps * kTWarpBytes;
-          const int tgrid = clamp_grid((ntiles + kTWarps - 1) / kTWarps, (long long)sm_count * PXZ_SHRINK_TMA_CTAS);
-          if (fused) {
-            e = set_smem(k_shrink_tma<true>, smem);
-            if (e != cudaSuccess) return e;
-            e = launch_pdl(k_shrink_tma<true>, tgrid, kTWarps * 32, smem, s, tm, g, descs, tabidx, lists, cap, opaque_flags, payload, tabs, ntabs, pool, tile_counter, 1.0f, -0.0f);
-          } else {
-            e = set_smem(k_shrink_tma<false>, smem);
-            if (e != cudaSuccess) return e;
-            e = launch_pdl(k_shrink_tma<false>, tgrid, kTWarps * 32, smem, s, tm, g, descs, tabidx, lists, cap, opaque_flags, payload, tabs, ntabs, pool, tile_counter, 1.0f, -0.0f);
-          }
-          if (e != cudaSuccess) return e;
-          if (!has_noslide) return cudaGetLastError();
-          ++*launches;  // the tiles without a slide table go to the ring kernel
-        } else {
-          ring_kernel = true;
-        }
-      }
-      const uint32_t only_noslide = ring_kernel ? 0u : 1u;
-      const size_t smem = (size_t)kShrinkWarps * kShrinkWarpBytes;
-      const int wgrid = clamp_grid((ntiles + kShrinkWarps - 1) / kShrinkWarps, (long long)sm_count * PXZ_SHRINK_WARP_CTAS);
-      if (fused) {
-        e = set_smem(k_shrink_warp<true>, smem);
-        if (e != cudaSuccess) return e;
-        e = launch_pdl(k_shrink_warp<true>, wgrid, kShrinkCtaThreads, smem, s, img, pitch, g, descs, tabidx, lists, cap, opaque_flags, payload, tabs, pool, tile_counter, 1.0f, -0.0f, only_noslide);
-      } else {
-        e = set_smem(k_shrink_warp<false>, smem);
-        if (e != cudaSuccess) return e;
-        e = launch_pdl(k_shrink_warp<false>, wgrid, kShrinkCtaThreads, smem, s, img, pitch, g, descs, tabidx, lists, cap, opaque_flags, payload, tabs, pool, tile_counter, 1.0f, -0.0f, only_noslide);
-      }
-    } else {
-      const size_t smem = (size_t)kWarpsPerCta * kExpandWarpBytes;
+  const bool force_warp = a.kernels == ResampleKernels::Warp || a.kernels == ResampleKernels::Tma;
+  if (fast && a.warp_tables && a.tile_counter != nullptr && a.kernels != ResampleKernels::Cta &&
+      (force_warp || ntiles >= (long long)sm_count * 16)) {
+    if (a.direction == 1) {
       const int wgrid = clamp_grid((ntiles + kWarpsPerCta - 1) / kWarpsPerCta, (long long)sm_count * PXZ_EXPAND_WARP_CTAS);
-      if (fused) e = launch_pdl(k_expand_warp<true>, wgrid, kWarpCtaThreads, smem, s, img, pitch, g, descs, tabidx, lists, cap, payload, tabs, pool, tile_counter, 1.0f, -0.0f);
-      else e = launch_pdl(k_expand_warp<false>, wgrid, kWarpCtaThreads, smem, s, img, pitch, g, descs, tabidx, lists, cap, payload, tabs, pool, tile_counter, 1.0f, -0.0f);
+      return launch_pdl(a.fused ? k_expand_warp<true> : k_expand_warp<false>, wgrid, kWarpCtaThreads, (size_t)kWarpsPerCta * kExpandWarpBytes,
+                        s, a.img, a.pitch, g, a.descs, a.tabidx, a.lists, a.cap, a.payload, a.tabs, a.pool, a.tile_counter, 1.0f, -0.0f);
     }
-    return cudaGetLastError();
+    bool ring_kernel = a.kernels == ResampleKernels::Warp;
+    if (!ring_kernel) {
+      CUtensorMap tm;
+      if (make_image_tmap(a.img, a.pitch, g.W, g.nimg > 1 ? (g.nimg - 1) * g.img_rows + g.H : g.H, &tm)) {
+        const int tgrid = clamp_grid((ntiles + kTWarps - 1) / kTWarps, (long long)sm_count * PXZ_SHRINK_TMA_CTAS);
+        const cudaError_t e = launch_pdl(a.fused ? k_shrink_tma<true> : k_shrink_tma<false>, tgrid, kTWarps * 32, (size_t)kTWarps * kTWarpBytes, s, tm,
+                                         g, a.descs, a.tabidx, a.lists, a.cap, a.opaque_flags, a.payload, a.tabs, a.ntabs, a.pool, a.tile_counter,
+                                         1.0f, -0.0f);
+        if (e != cudaSuccess || !a.has_noslide) return e;
+        ++*launches;  // the tiles without a slide table go to the ring kernel
+      } else {
+        ring_kernel = true;
+      }
+    }
+    const uint32_t only_noslide = ring_kernel ? 0u : 1u;
+    const int wgrid = clamp_grid((ntiles + kShrinkWarps - 1) / kShrinkWarps, (long long)sm_count * PXZ_SHRINK_WARP_CTAS);
+    return launch_pdl(a.fused ? k_shrink_warp<true> : k_shrink_warp<false>, wgrid, kShrinkCtaThreads, (size_t)kShrinkWarps * kShrinkWarpBytes, s,
+                      a.img, a.pitch, g, a.descs, a.tabidx, a.lists, a.cap, a.opaque_flags, a.payload, a.tabs, a.pool, a.tile_counter, 1.0f, -0.0f,
+                      only_noslide);
   }
   if (fast) {
-    const size_t smem = fast_smem_bytes(max_tmp_px);
-    const int fgrid = clamp_grid((long long)g.cols * g.rows, (long long)sm_count * PXZ_RESAMPLE_MINBLOCKS);
-    if (direction == 0 && !fused) {
-      e = set_smem(k_shrink_rgba<false>, smem);
-      if (e != cudaSuccess) return e;
-      k_shrink_rgba<false><<<fgrid, kThreads, smem, s>>>(img, pitch, g, descs, tabidx, payload, tabs, ntabs, pool, max_tmp_px, 1.0f, -0.0f);
-    } else if (direction == 0) {
-      e = set_smem(k_shrink_rgba<true>, smem);
-      if (e != cudaSuccess) return e;
-      k_shrink_rgba<true><<<fgrid, kThreads, smem, s>>>(img, pitch, g, descs, tabidx, payload, tabs, ntabs, pool, max_tmp_px, 1.0f, -0.0f);
-    } else if (!fused) {
-      e = set_smem(k_expand_rgba<false>, smem);
-      if (e != cudaSuccess) return e;
-      k_expand_rgba<false><<<fgrid, kThreads, smem, s>>>(img, pitch, g, descs, tabidx, payload, tabs, ntabs, pool, max_tmp_px, 1.0f, -0.0f);
-    } else {
-      e = set_smem(k_expand_rgba<true>, smem);
-      if (e != cudaSuccess) return e;
-      k_expand_rgba<true><<<fgrid, kThreads, smem, s>>>(img, pitch, g, descs, tabidx, payload, tabs, ntabs, pool, max_tmp_px, 1.0f, -0.0f);
-    }
-    return cudaGetLastError();
+    const int fgrid = clamp_grid(ntiles, (long long)sm_count * PXZ_RESAMPLE_MINBLOCKS);
+    const size_t smem = fast_smem_bytes(a.max_tmp_px);
+    if (a.direction == 0)
+      return launch(a.fused ? k_shrink_rgba<true> : k_shrink_rgba<false>, fgrid, kThreads, smem, s, a.img, a.pitch, g, a.descs, a.tabidx, a.payload,
+                    a.tabs, a.ntabs, a.pool, a.max_tmp_px, 1.0f, -0.0f);
+    return launch(a.fused ? k_expand_rgba<true> : k_expand_rgba<false>, fgrid, kThreads, smem, s, a.img, a.pitch, g, a.descs, a.tabidx, a.payload,
+                  a.tabs, a.ntabs, a.pool, a.max_tmp_px, 1.0f, -0.0f);
   }
-  const size_t smem = scratch ? 0 : resample_smem_bytes(max_src_px, max_tmp_px, g.C);
-  if (g.C == 4) {
-    e = set_smem(k_resample<4>, smem);
-    if (e != cudaSuccess) return e;
-    k_resample<4><<<grid, kThreads, smem, s>>>(direction, img, pitch, g, descs, tabidx, payload, tabs, pool, max_src_px,
-                                              max_tmp_px, scratch, scratch_per_cta);
-  } else {
-    e = set_smem(k_resample<3>, smem);
-    if (e != cudaSuccess) return e;
-    k_resample<3><<<grid, kThreads, smem, s>>>(direction, img, pitch, g, descs, tabidx, payload, tabs, pool, max_src_px,
-                                              max_tmp_px, scratch, scratch_per_cta);
-  }
-  return cudaGetLastError();
+  const size_t smem = a.scratch ? 0 : resample_smem_bytes(a.max_src_px, a.max_tmp_px, g.C);
+  return launch(g.C == 4 ? k_resample<4> : k_resample<3>, a.grid, kThreads, smem, s, a.direction, a.img, a.pitch, g, a.descs, a.tabidx, a.payload,
+                a.tabs, a.pool, a.max_src_px, a.max_tmp_px, a.scratch, a.scratch_per_cta);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -2932,20 +2850,16 @@ cudaError_t launch_block_error(const uint8_t* a, size_t pa, const uint8_t* b, si
   const unsigned long long nwork = (unsigned long long)g.rows * bands_per_row * ux;
   const int grid = clamp_grid((long long)std::min<unsigned long long>(nwork, 1ull << 30), (long long)sm_count * 16);
   ++*launches;
-  if (vec)
-    k_block_error<true><<<grid, kThreads, 0, s>>>(a, pa, b, pb, g, units, ux, bands_per_row, nwork, reinterpret_cast<unsigned long long*>(sse), mx);
-  else
-    k_block_error<false><<<grid, kThreads, 0, s>>>(a, pa, b, pb, g, units, ux, bands_per_row, nwork, reinterpret_cast<unsigned long long*>(sse), mx);
-  return cudaGetLastError();
+  return launch(vec ? k_block_error<true> : k_block_error<false>, grid, kThreads, 0, s, a, pa, b, pb, g, units, ux, bands_per_row, nwork,
+                reinterpret_cast<unsigned long long*>(sse), mx);
 }
 
 cudaError_t launch_bucket_sum(const pxz_block_desc* descs, const uint64_t* block_sse, uint32_t nblocks, uint32_t pair, bool count,
                               uint64_t* sse, uint32_t* blocks, cudaStream_t s, int sm_count, uint64_t* launches) {
   ++*launches;
   const int grid = clamp_grid(((long long)nblocks + kThreads - 1) / kThreads, (long long)sm_count * 2);
-  k_bucket_sum<<<grid, kThreads, 0, s>>>(descs, reinterpret_cast<const unsigned long long*>(block_sse), nblocks, pair, count ? 1 : 0,
-                                         reinterpret_cast<unsigned long long*>(sse), blocks);
-  return cudaGetLastError();
+  return launch(k_bucket_sum, grid, kThreads, 0, s, descs, reinterpret_cast<const unsigned long long*>(block_sse), nblocks, pair, count ? 1 : 0,
+                reinterpret_cast<unsigned long long*>(sse), blocks);
 }
 
 cudaError_t launch_rgb_widen(const uint8_t* src, size_t spitch, uint8_t* dst, size_t dpitch, uint32_t w, uint32_t rows, int widen,
@@ -2953,9 +2867,7 @@ cudaError_t launch_rgb_widen(const uint8_t* src, size_t spitch, uint8_t* dst, si
   ++*launches;
   const long long quads = (long long)((w + 3) / 4) * rows;
   const int grid = clamp_grid((quads + kThreads - 1) / kThreads, (long long)sm_count * 8);
-  if (widen) k_rgb_to_rgba<<<grid, kThreads, 0, s>>>(src, spitch, dst, dpitch, w, rows);
-  else k_rgba_to_rgb<<<grid, kThreads, 0, s>>>(src, spitch, dst, dpitch, w, rows);
-  return cudaGetLastError();
+  return launch(widen ? k_rgb_to_rgba : k_rgba_to_rgb, grid, kThreads, 0, s, src, spitch, dst, dpitch, w, rows);
 }
 
 cudaError_t launch_payload_convert(const pxz_block_desc* sdescs, const uint8_t* spx, const uint32_t* smeta, uint32_t scap,
@@ -2963,9 +2875,8 @@ cudaError_t launch_payload_convert(const pxz_block_desc* sdescs, const uint8_t* 
                                    uint64_t* dtotal, uint32_t nblocks, int sc, int dc, cudaStream_t s, int sm_count, uint64_t* launches) {
   ++*launches;
   const int grid = clamp_grid(((long long)nblocks + 7) / 8, (long long)sm_count * 8);
-  k_payload_convert<<<grid, kThreads, 0, s>>>(sdescs, spx, smeta, scap, reinterpret_cast<const unsigned long long*>(stotal), ddescs, dpx, dmeta,
-                                              dcap, reinterpret_cast<unsigned long long*>(dtotal), nblocks, sc, dc);
-  return cudaGetLastError();
+  return launch(k_payload_convert, grid, kThreads, 0, s, sdescs, spx, smeta, scap, reinterpret_cast<const unsigned long long*>(stotal), ddescs, dpx,
+                dmeta, dcap, reinterpret_cast<unsigned long long*>(dtotal), nblocks, sc, dc);
 }
 
 size_t resample_fir_smem_bytes(uint32_t max_src_px, uint32_t max_tmp_px, uint32_t C) {
@@ -2977,23 +2888,8 @@ cudaError_t launch_resample_fir(int direction, uint8_t* img, size_t pitch, const
                                 uint32_t src_cap_bytes, cudaStream_t s, int sm_count, uint64_t* launches) {
   ++*launches;
   const int grid = clamp_grid((long long)g.cols * g.rows, (long long)sm_count * 8);
-  cudaError_t e;
-  if (g.C == 4) {
-    e = set_smem(k_resample_fir<4>, smem);
-    if (e != cudaSuccess) return e;
-    k_resample_fir<4><<<grid, kThreads, smem, s>>>(direction, img, pitch, g, descs, tabidx, payload, tabs, pool, src_cap_bytes);
-  } else {
-    e = set_smem(k_resample_fir<3>, smem);
-    if (e != cudaSuccess) return e;
-    k_resample_fir<3><<<grid, kThreads, smem, s>>>(direction, img, pitch, g, descs, tabidx, payload, tabs, pool, src_cap_bytes);
-  }
-  return cudaGetLastError();
+  return launch(g.C == 4 ? k_resample_fir<4> : k_resample_fir<3>, grid, kThreads, smem, s, direction, img, pitch, g, descs, tabidx, payload, tabs,
+                pool, src_cap_bytes);
 }
-
-#ifdef PXZ_WARP_STATS
-extern "C" int pxz_debug_warp_stats(unsigned long long* out, int n_words) {
-  return (int)cudaMemcpyFromSymbol(out, g_warp_stats, sizeof(unsigned long long) * (size_t)n_words);
-}
-#endif
 
 }  // namespace pxz

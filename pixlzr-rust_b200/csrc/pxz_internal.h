@@ -174,13 +174,35 @@ constexpr uint32_t kFilterPairs = 25;  // pair = down * 5 + up
 static_assert(kFilterPairs == PXZ_FILTER_PAIRS, "filter pair count");
 cudaError_t launch_bucket_sum(const pxz_block_desc* descs, const uint64_t* block_sse, uint32_t nblocks, uint32_t pair, bool count,
                               uint64_t* sse, uint32_t* blocks, cudaStream_t s, int sm_count, uint64_t* launches);
-// direction 0: image tiles -> payload (shrink); 1: payload -> image tiles (expand)
-cudaError_t launch_resample(int direction, uint8_t* img, size_t pitch, const Geom& g, const pxz_block_desc* descs,
-                            const uint32_t* tabidx, uint8_t* payload, const AxisTab* tabs, const uint32_t* pool,
-                            uint32_t ntabs, uint32_t max_src_px, uint32_t max_src_dim, uint32_t max_tmp_px, uint32_t max_tab_words,
-                            uint8_t* scratch, size_t scratch_per_cta, int grid_hint, bool fused, const uint8_t* opaque_flags,
-                            uint32_t* tile_counter, const uint32_t* lists, uint32_t cap, bool warp_tables, int prefer, bool has_noslide,
-                            cudaStream_t s, int sm_count, uint64_t* launches);
+// Which resample kernel family runs (PXZ_RESAMPLE_KERNELS=warp|cta|tma).  Auto: by tile count; Warp: warp-per-tile kernels
+// with the cp.async ring shrink kernel; Cta: CTA-per-tile kernels; Tma: warp-per-tile kernels with the TMA shrink kernel.
+// The forced warp families still need the RGBA fast geometry and tables that have the warp forms.
+enum class ResampleKernels { Auto, Warp, Cta, Tma };
+struct ResampleArgs {
+  int direction;  // 0: image tiles -> payload (shrink); 1: payload -> image tiles (expand)
+  uint8_t* img;
+  size_t pitch;
+  Geom g;
+  const pxz_block_desc* descs;
+  const uint32_t* tabidx;
+  uint8_t* payload;
+  const AxisTab* tabs;
+  const uint32_t* pool;
+  uint32_t ntabs;
+  uint32_t max_src_px, max_src_dim, max_tmp_px, max_tab_words;  // bounds of the source blocks, intermediate and tables
+  uint8_t* scratch;        // non-NULL: global scratch of scratch_per_cta bytes per CTA instead of shared memory (grid CTAs)
+  size_t scratch_per_cta;
+  int grid;                // CTA-per-tile kernel grid
+  bool fused;              // pxz_ctx_set_fast_resample
+  const uint8_t* opaque_flags;  // may be NULL: per tile, alpha is 255 everywhere
+  uint32_t* tile_counter;  // work counter of the warp-per-tile kernels; NULL: they are not used
+  const uint32_t* lists;   // work-order lists of capacity cap (launch_plan)
+  uint32_t cap;
+  bool warp_tables;        // every table has the forms the warp-per-tile kernels need
+  ResampleKernels kernels;
+  bool has_noslide;        // shrink: some table has no slide form (k_shrink_tma leaves those tiles to k_shrink_warp)
+};
+cudaError_t launch_resample(const ResampleArgs& a, cudaStream_t s, int sm_count, uint64_t* launches);
 size_t resample_smem_bytes(uint32_t max_src_px, uint32_t max_tmp_px, uint32_t C);
 // RGB images on the RGBA kernels: widen = 1: RGB rows -> RGBA rows (alpha 255); 0: RGBA rows -> RGB rows
 cudaError_t launch_rgb_widen(const uint8_t* src, size_t spitch, uint8_t* dst, size_t dpitch, uint32_t w, uint32_t rows, int widen,

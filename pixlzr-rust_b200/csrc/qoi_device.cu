@@ -272,8 +272,8 @@ cudaError_t launch_qoi_encode(const pxz_block_desc* descs, const uint8_t* pixels
   const uint32_t nblocks = g.cols * g.rows;
   const int grid = (int)((nblocks + kQoiThreads - 1) / kQoiThreads);
   *launches += 3;
-  if (g.C == 4) k_qoi_encode<4><<<grid, kQoiThreads, 0, s>>>(descs, pixels, nblocks, values_present, arena, enc_len);
-  else k_qoi_encode<3><<<grid, kQoiThreads, 0, s>>>(descs, pixels, nblocks, values_present, arena, enc_len);
+  const auto encode = g.C == 4 ? k_qoi_encode<4> : k_qoi_encode<3>;
+  encode<<<grid, kQoiThreads, 0, s>>>(descs, pixels, nblocks, values_present, arena, enc_len);
   k_qoi_layout<<<1, kScanThreads, 0, s>>>(enc_len, g, filter_byte, out_off, out, total);
   const int cgrid = (int)std::min<uint32_t>((nblocks + 7) / 8, 148u * 8u);
   k_qoi_compact<<<cgrid, 256, 0, s>>>(descs, arena, enc_len, out_off, nblocks, g.C, out);
@@ -285,8 +285,8 @@ cudaError_t launch_qoi_decode(const uint8_t* in, const unsigned long long* in_of
   const uint32_t nblocks = g.cols * g.rows;
   const int grid = (int)((nblocks + kQoiThreads - 1) / kQoiThreads);
   ++*launches;
-  if (g.C == 4) k_qoi_decode<4><<<grid, kQoiThreads, 0, s>>>(in, in_off, qlen, descs, nblocks, pixels, err);
-  else k_qoi_decode<3><<<grid, kQoiThreads, 0, s>>>(in, in_off, qlen, descs, nblocks, pixels, err);
+  const auto decode = g.C == 4 ? k_qoi_decode<4> : k_qoi_decode<3>;
+  decode<<<grid, kQoiThreads, 0, s>>>(in, in_off, qlen, descs, nblocks, pixels, err);
   return cudaGetLastError();
 }
 

@@ -96,7 +96,6 @@ struct TQueue {
   uint32_t* counter;
   uint32_t ntiles;
   TileOrder ord;
-  bool back;           // this warp draws from the back of the order list (draws_from_back)
   uint32_t raw;        // lane 0: the drawn position (atomic in flight)
   bool drawing;        // this warp has not yet drawn an index >= ntiles
   TDesc q;             // the tile being fetched
@@ -107,7 +106,7 @@ __device__ __forceinline__ void tq_start(TQueue& q) {
   q.raw = 0xFFFFFFFFu;
   if (q.drawing && (threadIdx.x & 31u) == 0) {
     uint32_t n;
-    q.raw = draw_position(q.counter, q.back, q.ntiles, n);
+    q.raw = draw_position(q.counter, q.ntiles, n);
   }
   q.step = 0; q.tick = 0; q.next_at = 4;
 }
@@ -375,17 +374,6 @@ __device__ __forceinline__ void tma_shrink_tile(TFeed& f, TQueue& q, const CUten
                                                 float4* strip, const HTab& ht, uint32_t* dst, const TapK& k) {
   constexpr int NC = (MODE & 1) ? 4 : 3;
   const uint32_t lane = threadIdx.x & 31u;
-#ifdef PXZ_TMA_STREAM_ONLY
-  {  // timing experiment: the tile's boxes are streamed and touched, nothing is computed
-    uint32_t x = 0;
-    for (uint32_t bx = 0; bx < (sh + kTBoxRows - 1) / kTBoxRows; ++bx) {
-      x ^= lds_u32(tfeed_wait(f) + lane * 4);
-      tfeed_release(f, tm, q);
-    }
-    if (x == 0x12345678u) dst[0] = x;
-    return;
-  }
-#endif
   u64 acc[A][NC];
 #pragma unroll
   for (int s = 0; s < A; ++s)
@@ -537,7 +525,6 @@ __global__ void __launch_bounds__(kTWarps * 32, PXZ_SHRINK_TMA_CTAS) k_shrink_tm
   q.descs = descs; q.tabidx = tabidx; q.opaque = opaque_flags; q.counter = counter; q.ntiles = ntiles;
   q.ord.init(lists, cap);
   q.drawing = true;
-  q.back = draws_from_back(PXZ_SHRINK_TMA_CTAS);
   tq_start(q);
   TDesc P0 = tq_finish(q);
   tq_start(q);

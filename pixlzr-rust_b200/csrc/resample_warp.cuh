@@ -64,53 +64,27 @@ struct TileOrder {
   }
 };
 
-// Two-ended draw (experiment, off: PXZ_TWO_ENDED=1 measured 117 / 96 us against 101 / 91 us for shrink / expand on the
-// bench frame).  The order list runs from the most expensive class to the cheapest; half of the warps of every
-// scheduler draw from its front and the other half from its back, so that a sub-partition holds arithmetic-bound tiles
-// next to tiles that only stream.  One 64-bit word holds both counts: low half = drawn from the front, high half = from
-// the back; with the experiment off every warp draws from the front.
-#ifndef PXZ_TWO_ENDED
-#define PXZ_TWO_ENDED 0
-#endif
-__device__ __forceinline__ bool draws_from_back(uint32_t ctas_per_sm) {
-#if PXZ_TWO_ENDED
-  // CTAs b, b + grid / ctas_per_sm, ... usually share an SM: alternate the roles over them as well as over the warps
-  const uint32_t per_wave = (gridDim.x + ctas_per_sm - 1) / ctas_per_sm;
-  return (((threadIdx.x >> 5) + blockIdx.x / per_wave) & 1u) != 0;
-#else
-  return false;
-#endif
-}
-// lane 0 only: position in the order list, or 0xFFFFFFFF when every tile has been handed out; `n_drawn` = draws before this one
-__device__ __forceinline__ uint32_t draw_position(uint32_t* counter, bool back, uint32_t ntiles, uint32_t& n_drawn) {
-  unsigned long long* c64 = reinterpret_cast<unsigned long long*>(counter);
-  const unsigned long long old = atomicAdd(c64, back ? (1ull << 32) : 1ull);
-  const uint32_t f = (uint32_t)old, bk = (uint32_t)(old >> 32);
-  n_drawn = f + bk;
-  return n_drawn < ntiles ? (back ? ntiles - 1u - bk : f) : 0xFFFFFFFFu;
+// lane 0 only: position in the order list, or 0xFFFFFFFF when every tile has been handed out; `n_drawn` = draws before this one.
+// The draw count is the 64-bit word at `counter`; n_drawn adds its two halves (the high half stays zero).  Reading the low
+// half alone would give the same values but changes the generated code of the three warp-per-tile kernels.
+__device__ __forceinline__ uint32_t draw_position(uint32_t* counter, uint32_t ntiles, uint32_t& n_drawn) {
+  const unsigned long long old = atomicAdd(reinterpret_cast<unsigned long long*>(counter), 1ull);
+  const uint32_t f = (uint32_t)old;
+  n_drawn = f + (uint32_t)(old >> 32);
+  return n_drawn < ntiles ? f : 0xFFFFFFFFu;
 }
 
 // next tile of this warp (lane 0 asks, everybody gets the answer).  Every warp draws exactly one position past the end;
 // the warp that draws the very last one puts the counter back to zero for the next launch on this stream.
-__device__ __forceinline__ uint32_t next_tile(uint32_t* counter, uint32_t ntiles, uint32_t total_warps, bool back) {
+__device__ __forceinline__ uint32_t next_tile(uint32_t* counter, uint32_t ntiles, uint32_t total_warps) {
   uint32_t v = 0;
   if ((threadIdx.x & 31u) == 0) {
     uint32_t n;
-    v = draw_position(counter, back, ntiles, n);
+    v = draw_position(counter, ntiles, n);
     if (n == ntiles + total_warps - 1) *reinterpret_cast<unsigned long long*>(counter) = 0ull;
   }
   return __shfl_sync(0xffffffffu, v, 0);
 }
-
-#ifdef PXZ_WARP_STATS
-// debug build only: per-warp start / end time (ns) and tile counts of the last warp-kernel launch
-__device__ unsigned long long g_warp_stats[8192 * 4];
-__device__ __forceinline__ unsigned long long globaltimer_ns() {
-  unsigned long long t;
-  asm volatile("mov.u64 %0, %globaltimer;" : "=l"(t));
-  return t;
-}
-#endif
 
 // ---- shrink ------------------------------------------------------------------------------------------------------
 constexpr uint32_t kBlockedFrom = 8;  // outputs per row from which the horizontal pass walks groups of 4 (else scalar chains)
@@ -538,37 +512,20 @@ __global__ void __launch_bounds__(kShrinkCtaThreads, PXZ_SHRINK_WARP_CTAS) k_shr
   // Tiles are drawn in the order of the `order` list (most expensive first, so the kernel does not end on a few warps
   // that drew a 20-microsecond tile last); the next tile's index, descriptor and table indices are requested while the
   // current tile is processed.
-#ifdef PXZ_WARP_STATS
-  const unsigned long long t_start = globaltimer_ns();
-  uint32_t drawn = 0;
-#endif
   TileOrder ord;
   ord.init(lists, cap);
-  const bool back = draws_from_back(PXZ_SHRINK_WARP_CTAS);
-  uint32_t v = next_tile(counter, ntiles, total_warps, back);
+  uint32_t v = next_tile(counter, ntiles, total_warps);
   uint32_t b = 0, ti = 0;
   pxz_block_desc d{};
   if (v < ntiles) { b = ord.at(v); d = descs[b]; ti = tabidx[b]; }
   while (v < ntiles) {
-    const uint32_t vn = next_tile(counter, ntiles, total_warps, back);
+    const uint32_t vn = next_tile(counter, ntiles, total_warps);
     uint32_t bn = 0, tin = 0;
     pxz_block_desc dn{};
     if (vn < ntiles) { bn = ord.at(vn); dn = descs[bn]; tin = tabidx[bn]; }
-#ifdef PXZ_WARP_STATS
-    ++drawn;
-#endif
     process(b, d, ti);
     v = vn; b = bn; d = dn; ti = tin;
   }
-#ifdef PXZ_WARP_STATS
-  if (lane == 0) {
-    const uint32_t w = blockIdx.x * kShrinkWarps + (threadIdx.x >> 5);
-    g_warp_stats[4 * w + 0] = t_start;
-    g_warp_stats[4 * w + 1] = globaltimer_ns();
-    g_warp_stats[4 * w + 2] = 0;
-    g_warp_stats[4 * w + 3] = drawn;
-  }
-#endif
 }
 
 // ---- expand ------------------------------------------------------------------------------------------------------
@@ -878,13 +835,12 @@ __global__ void __launch_bounds__(kWarpCtaThreads, PXZ_EXPAND_WARP_CTAS) k_expan
   // current tile is processed.
   TileOrder ord;
   ord.init(lists, cap);
-  const bool back = draws_from_back(PXZ_EXPAND_WARP_CTAS);
-  uint32_t v = next_tile(counter, ntiles, total_warps, back);
+  uint32_t v = next_tile(counter, ntiles, total_warps);
   uint32_t b = 0, ti = 0;
   pxz_block_desc d{};
   if (v < ntiles) { b = ord.at(v); d = descs[b]; ti = tabidx[b]; }
   while (v < ntiles) {
-    const uint32_t vn = next_tile(counter, ntiles, total_warps, back);
+    const uint32_t vn = next_tile(counter, ntiles, total_warps);
     uint32_t bn = 0, tin = 0;
     pxz_block_desc dn{};
     if (vn < ntiles) { bn = ord.at(vn); dn = descs[bn]; tin = tabidx[bn]; }
