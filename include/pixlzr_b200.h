@@ -78,8 +78,7 @@ int pxz_abi_version(void);
 int pxz_device_count(void);
 /* One context per host thread; it owns one CUDA stream and its scratch.  Environment read at creation (diagnostics only):
  *   PXZ_RESAMPLE_KERNELS=warp|cta|tma  force a resample kernel family (default: by tile count): warp-per-tile with
- *                                  the cp.async ring shrink kernel, CTA-per-tile, or warp-per-tile with the TMA shrink kernel,
- *   PXZ_GUARD_REL / PXZ_GUARD_ABS  guard band of the fast Oklab-MAD path (DESIGN.md section 3). */
+ *                                  the cp.async ring shrink kernel, CTA-per-tile, or warp-per-tile with the TMA shrink kernel. */
 pxz_status pxz_ctx_create(int device, pxz_ctx** out);
 /* same, but work is ordered on an existing CUDA stream (cudaStream_t / CUstream passed as
  * void*), e.g. torch.cuda.current_stream().cuda_stream.  The stream must outlive the ctx. */
@@ -98,8 +97,7 @@ uint64_t pxz_launch_count(const pxz_ctx* ctx);
  *   PXZ_RESIZE_FIR: the `fast_image_resize` branch (block.rs:292-333 with FilterType::to_fir_resizing_algorithm,
  *       data_types/mod.rs:65-107), the crate's default cargo feature — 16-bit fixed-point convolution, horizontal pass
  *       first into a u8 image, Triangle = Hamming when shrinking / Bilinear when growing, pre-multiplied alpha for RGBA.
- *       Restated from the crate's published algorithm: PARITY UNPINNED (no artefact of the reference was made with it).
- * Also selectable with PXZ_RESIZE_SEMANTICS=fir in the environment when the context is created. */
+ *       Restated from the crate's published algorithm: PARITY UNPINNED (no artefact of the reference was made with it). */
 typedef enum { PXZ_RESIZE_IMAGE_RS = 0, PXZ_RESIZE_FIR = 1 } pxz_resize_semantics;
 pxz_status pxz_ctx_set_resize_semantics(pxz_ctx* ctx, pxz_resize_semantics semantics);
 pxz_status pxz_ctx_set_fast_resample(pxz_ctx* ctx, int on);

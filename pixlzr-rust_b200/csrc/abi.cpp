@@ -98,7 +98,6 @@ struct pxz_ctx {
   std::map<TabKey, TabSet> tabs;
   void* comm = nullptr;
   bool fast_resample = false;
-  bool rgb_via_rgba = true;            // RGB images run on the RGBA fast kernels (PXZ_RGB_VIA_RGBA=0: the 3-channel kernels)
   int resize_semantics = PXZ_RESIZE_IMAGE_RS;  // which branch of PixlzrBlock::resize (pxz_ctx_set_resize_semantics)
   std::vector<PayloadBufs> payload_cache;  // at most kPayloadCacheMax entries
   // per-kernel timing
@@ -429,7 +428,7 @@ pxz_status run_resample(pxz_ctx* ctx, int direction, uint8_t* img, size_t pitch,
   a.grid = grid;
   a.fused = ctx->fast_resample;
   a.opaque_flags = opaque_flags;
-  a.tile_counter = ctx->resample_kernels != ResampleKernels::Cta ? ctx->d_tile_counter : nullptr;
+  a.tile_counter = ctx->d_tile_counter;
   a.lists = p->d_order();
   a.cap = (uint32_t)p->nblocks_cap;
   a.warp_tables = ts.warp_ok;
@@ -539,10 +538,6 @@ pxz_status ctx_create_common(int device, cudaStream_t stream, bool own, pxz_ctx*
   build_level_thresholds(&ctx->thr);
   ctx->band.rel = 2.0e-5f;     // fast arithmetic, relative
   ctx->band.abs_raw = 8.0e-6f; // fast arithmetic, absolute (SFU cube roots; measured <= 4e-6)
-  if (const char* e = getenv("PXZ_GUARD_REL")) ctx->band.rel = (float)atof(e);
-  if (const char* e = getenv("PXZ_GUARD_ABS")) ctx->band.abs_raw = (float)atof(e);
-  if (const char* e = getenv("PXZ_RGB_VIA_RGBA")) ctx->rgb_via_rgba = atoi(e) != 0;
-  if (const char* e = getenv("PXZ_RESIZE_SEMANTICS")) ctx->resize_semantics = !strcmp(e, "fir") ? PXZ_RESIZE_FIR : PXZ_RESIZE_IMAGE_RS;
   if (const char* e = getenv("PXZ_RESAMPLE_KERNELS"))
     ctx->resample_kernels = !strcmp(e, "warp") ? ResampleKernels::Warp
                             : !strcmp(e, "cta") ? ResampleKernels::Cta
@@ -948,7 +943,7 @@ pxz_status pxz_comm_join_empty(pxz_ctx* ctx) {
 
 // RGB images whose geometry suits the RGBA fast kernels run on them (kernels.cu "RGB images on the RGBA fast kernels")
 static bool rgb_on_rgba(const pxz_ctx* ctx, uint32_t w, uint32_t c, uint32_t bw, uint32_t bh) {
-  return c == 3 && ctx->rgb_via_rgba && ctx->resize_semantics == PXZ_RESIZE_IMAGE_RS && bw <= 64 && bh <= 64 && bw % 4 == 0 && w % 4 == 0;
+  return c == 3 && ctx->resize_semantics == PXZ_RESIZE_IMAGE_RS && bw <= 64 && bh <= 64 && bw % 4 == 0 && w % 4 == 0;
 }
 
 // payload of the other channel count (3 <-> 4) with the same blocks, tables and work order

@@ -2453,21 +2453,12 @@ static bool make_image_tmap(const uint8_t* img, size_t pitch, uint32_t W, uint32
             CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// PXZ_SOBEL_KERNEL=tile64 keeps the shared-memory kernel (A/B timing and a fallback that needs no tensor map)
-static bool sobel_tma_enabled() {
-  static const bool on = [] {
-    const char* e = getenv("PXZ_SOBEL_KERNEL");
-    return !(e && strcmp(e, "tile64") == 0);
-  }();
-  return on;
-}
-
 cudaError_t launch_analyze_sobel(const uint8_t* img, size_t pitch, const Geom& g, float* vx, float* vy, cudaStream_t s,
                                  int sm_count, uint64_t* launches) {
   const uint32_t ntiles = g.cols * g.rows;
   ++*launches;
   // RGBA, 64x64 tiles, rows a tensor copy can address: tiles streamed by TMA, dp4a row terms (analyze_sobel_tma.cuh)
-  if (g.C == 4 && g.bw == 64 && g.bh == 64 && (pitch % 16 == 0) && ((reinterpret_cast<uintptr_t>(img) & 15u) == 0) && sobel_tma_enabled()) {
+  if (g.C == 4 && g.bw == 64 && g.bh == 64 && (pitch % 16 == 0) && ((reinterpret_cast<uintptr_t>(img) & 15u) == 0)) {
     CUtensorMap tm;
     if (make_image_tmap(img, pitch, g.W, g.nimg > 1 ? (g.nimg - 1) * g.img_rows + g.H : g.H, &tm, 64))
       return launch(k_analyze_sobel_tma, clamp_grid(ntiles, (long long)sm_count * PXZ_SOBEL_CTAS), 256, kSobSmemBytes, s, tm, g, vx, vy);
@@ -2570,7 +2561,7 @@ cudaError_t launch_resample(const ResampleArgs& a, cudaStream_t s, int sm_count,
   // finish sooner.  a.kernels forces a family (ResampleKernels).
   const long long ntiles = (long long)g.cols * g.rows;
   const bool force_warp = a.kernels == ResampleKernels::Warp || a.kernels == ResampleKernels::Tma;
-  if (fast && a.warp_tables && a.tile_counter != nullptr && a.kernels != ResampleKernels::Cta &&
+  if (fast && a.warp_tables && a.kernels != ResampleKernels::Cta &&
       (force_warp || ntiles >= (long long)sm_count * 16)) {
     if (a.direction == 1) {
       const int wgrid = clamp_grid((ntiles + kWarpsPerCta - 1) / kWarpsPerCta, (long long)sm_count * PXZ_EXPAND_WARP_CTAS);

@@ -195,7 +195,7 @@ struct ResampleArgs {
   int grid;                // CTA-per-tile kernel grid
   bool fused;              // pxz_ctx_set_fast_resample
   const uint8_t* opaque_flags;  // may be NULL: per tile, alpha is 255 everywhere
-  uint32_t* tile_counter;  // work counter of the warp-per-tile kernels; NULL: they are not used
+  uint32_t* tile_counter;  // work counter of the warp-per-tile kernels
   const uint32_t* lists;   // work-order lists of capacity cap (launch_plan)
   uint32_t cap;
   bool warp_tables;        // every table has the forms the warp-per-tile kernels need

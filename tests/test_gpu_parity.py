@@ -126,9 +126,10 @@ def test_sobel_values_bit_exact(ctx, w, h, c, bw, bh):
 
 
 def test_sobel_tensor_copy_kernel_matches_shared_memory_kernel(ctx):
-    """RGBA + 64x64 tiles take k_analyze_sobel_tma (tiles streamed by tensor copies); PXZ_SOBEL_KERNEL=tile64 keeps the
-    round-1 kernel.  Both against the oracle, on a stacked batch too (a tile's box then runs into the next image)."""
-    import subprocess, sys, textwrap
+    """RGBA + 64x64 tiles take k_analyze_sobel_tma (tiles streamed by tensor copies) when a tensor map can address the rows
+    (16-byte aligned base and pitch), and the shared-memory kernel k_analyze_sobel_tile64<4> when they are only 4-byte
+    aligned.  Both against the oracle, on a stacked batch too (a tile's box then runs into the next image)."""
+    torch = pytest.importorskip("torch")
     imgs = np.stack([synth(323, 150, 4, seed=70 + i) for i in range(3)])
     want = [O.analyze(im, 64, 64, O.METRIC_SOBEL_DIR, nthreads=8) for im in imgs]
     b = ctx.image_upload_batch(imgs)
@@ -138,25 +139,21 @@ def test_sobel_tensor_copy_kernel_matches_shared_memory_kernel(ctx):
     for i, (hz, vr) in enumerate(want):
         assert np.array_equal(ghz.reshape(-1)[i * per:(i + 1) * per].view("<u4"), hz.reshape(-1).view("<u4")), i
         assert np.array_equal(gvr.reshape(-1)[i * per:(i + 1) * per].view("<u4"), vr.reshape(-1).view("<u4")), i
-    # the other kernel needs a fresh process (the switch is read once)
-    code = textwrap.dedent("""
-        import sys, numpy as np
-        sys.path.insert(0, %r)
-        import pixlzr_b200 as P
-        N = P.native
-        img = np.load(sys.argv[1])
-        c = N.Context(0)
-        d = c.image_upload(img)
-        hz, vr = d.analyze(64, 64, N.METRIC_SOBEL_DIR)
-        np.save(sys.argv[2], np.stack([hz, vr]))
-    """ % os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
-    import tempfile
-    with tempfile.TemporaryDirectory() as td:
-        np.save(os.path.join(td, "in.npy"), imgs[0])
-        env = dict(os.environ, PXZ_SOBEL_KERNEL="tile64")
-        subprocess.run([sys.executable, "-c", code, os.path.join(td, "in.npy"), os.path.join(td, "out.npy")], check=True, env=env)
-        other = np.load(os.path.join(td, "out.npy"))
-    assert np.array_equal(other[0].view("<u4"), want[0][0].view("<u4")) and np.array_equal(other[1].view("<u4"), want[0][1].view("<u4"))
+    # the first image once more on each kernel: uploaded (128-byte rows: tensor copies), and wrapped with a base and a pitch
+    # that are multiples of 4 but not of 16 (shared memory)
+    h, w = imgs[0].shape[:2]
+    pitch = w * 4 + 8
+    assert pitch % 16 != 0
+    host = np.zeros(4 + h * pitch, np.uint8)
+    host[4:].reshape(h, pitch)[:, : w * 4] = imgs[0].reshape(h, w * 4)
+    buf = torch.from_numpy(host).cuda()
+    torch.cuda.synchronize()
+    got = []
+    for d in (ctx.image_upload(imgs[0]), ctx.image_wrap(buf.data_ptr() + 4, w, h, 4, pitch)):
+        got.append(np.stack(d.analyze(64, 64, N.METRIC_SOBEL_DIR)).view("<u4"))
+        d.free()
+    assert np.array_equal(got[0], got[1])
+    assert np.array_equal(got[1], np.stack(want[0]).view("<u4"))
 
 
 def test_sobel_rejects_blocks_thinner_than_two(ctx):
@@ -575,28 +572,22 @@ def test_resample_kernel_families_match_oracle(forced_ctx, kind, shape, bs, metr
 
 
 # ---------------------------------------------------------------------------------------------
-# RGB images run on the RGBA fast kernels by default (widened with alpha 255, payload narrowed back); PXZ_RGB_VIA_RGBA=0
-# keeps them on the 3-channel kernels.  Both must give the oracle's 3-channel result bit for bit, values included.
+# RGB images: the input chooses the kernels.  A width that is a multiple of 4, with tiles of at most 64 px on a side and a
+# multiple of 4 wide, runs on the RGBA fast kernels (widened with alpha 255, payload narrowed back); any other width runs on
+# the 3-channel kernels.  Both must give the oracle's 3-channel result bit for bit, values included.
 # ---------------------------------------------------------------------------------------------
-@pytest.mark.parametrize("via_rgba", ["1", "0"])
 @pytest.mark.parametrize("shape,bs,metric,factor,fd,fu", [
-    ((200, 264), 64, 0, 1.0, O.LANCZOS3, O.LANCZOS3),
+    ((200, 264), 64, 0, 1.0, O.LANCZOS3, O.LANCZOS3),  # RGBA kernels
     ((136, 192), 32, 1, 6.0, O.CATMULLROM, O.TRIANGLE),
     ((130, 172), 16, 0, 0.25, O.GAUSSIAN, O.NEAREST),
+    ((200, 263), 64, 0, 1.0, O.LANCZOS3, O.LANCZOS3),  # 3-channel kernels
+    ((136, 190), 32, 1, 6.0, O.CATMULLROM, O.TRIANGLE),
+    ((130, 171), 16, 0, 0.25, O.GAUSSIAN, O.NEAREST),
 ])
-def test_rgb_paths_match_oracle(via_rgba, shape, bs, metric, factor, fd, fu):
-    old = os.environ.get("PXZ_RGB_VIA_RGBA")
-    os.environ["PXZ_RGB_VIA_RGBA"] = via_rgba
-    try:
-        c = N.Context(0)
-    finally:
-        if old is None:
-            del os.environ["PXZ_RGB_VIA_RGBA"]
-        else:
-            os.environ["PXZ_RGB_VIA_RGBA"] = old
+def test_rgb_paths_match_oracle(ctx, shape, bs, metric, factor, fd, fu):
     img = synth(shape[1], shape[0], 3, seed=41)
     ref = O.shrink(img, bs, bs, metric, factor, fd)
-    d = c.image_upload(img)
+    d = ctx.image_upload(img)
     pl = d.shrink(bs, bs, metric, factor, fd, N.FLAG_EXACT_VALUES)
     descs, px = pl.download()
     assert np.array_equal(descs["w"], ref.descs["w"]) and np.array_equal(descs["h"], ref.descs["h"])
@@ -604,7 +595,7 @@ def test_rgb_paths_match_oracle(via_rgba, shape, bs, metric, factor, fd, fu):
     assert np.array_equal(descs["value"].view(np.uint32), ref.descs["value"].view(np.uint32))
     assert np.array_equal(px, ref.payload)
     assert np.array_equal(pl.expand(fu), O.expand(ref, fu))
-    pl2 = c.payload_upload(shape[1], shape[0], bs, bs, 3, descs, px)
+    pl2 = ctx.payload_upload(shape[1], shape[0], bs, bs, 3, descs, px)
     assert np.array_equal(pl2.expand(fu), O.expand(ref, fu))
     pl2.free(); pl.free(); d.free()
 
