@@ -224,6 +224,35 @@ pxz_status pxz_strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw,
  * PXZ_E_ARG: a NULL sse / blocks / out, an unknown filter in base. */
 pxz_status pxz_strategy_choose(const uint64_t* sse, const uint32_t* blocks, const pxz_strategy* base, pxz_strategy* out);
 
+/* EXTENSION (rate-distortion).  For one (filter_down, filter_up) pair: every distinct payload pxz_shrink(img, bw, bh, metric, k,
+ * filter_down, flags) produces over the finite factors k > 0, in increasing k.  Point i: factor[i] = the SMALLEST f32 k giving that
+ * payload geometry (factor[0] = the smallest positive f32), bytes[i] = its payload bytes (pxz_payload_info; an RGB image counts 3
+ * per pixel), sse[i] = the total squared error of pxz_expand_to_image(that payload, filter_up) against img (pxz_image_error).
+ * bytes is strictly increasing.  n <= 1 + cols*rows*(ceil(log2 bw) + ceil(log2 bh)) (Oklab-MAD: ceil(log2 max(bw, bh))).
+ * *n_out is always set; cap < n -> PXZ_E_ARG (message names n), nothing written.  sse is exact in the default resample
+ * arithmetic (both resize semantics); with pxz_ctx_set_fast_resample(1) it is not claimed.
+ * One reference-order analysis, then one plan + resample + expand + error pass per level pair (Oklab-MAD: 1 + ceil(log2
+ * max(bw, bh)) passes, 7 at 64x64; Sobel: (1 + ceil(log2 bw)) * (1 + ceil(log2 bh)), 49 at 64x64), then per block the factors
+ * at which its dims change, one sort and one scan (DESIGN.md §3).  Device scratch: passes x blocks x 8 bytes for the error table
+ * (about 100 MB for Sobel on a 32768 x 32768 image at 64x64) plus about 100 bytes per possible point.  The host arrays may be
+ * NULL when cap = 0.  Synchronises the stream.
+ * PXZ_E_ARG and PXZ_E_UNSUPPORTED: as pxz_shrink_to_size, an unknown filter_up; PXZ_E_UNSUPPORTED: a strategy installed on the
+ * context (the filter pair would follow the stored value, which moves with k). */
+pxz_status pxz_rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, pxz_filter filter_down,
+                        pxz_filter filter_up, uint32_t flags, float* host_factor, uint64_t* host_bytes, uint64_t* host_sse,
+                        size_t cap, size_t* n_out);
+
+/* EXTENSION (rate control by error).  k = the smallest finite f32 > 0 whose decode (filter_up) has total SSE <= max_sse: the first
+ * point of pxz_rd_curve within the budget.  Payload size is monotone in k, so this is the smallest payload any factor gives
+ * within the budget.  *out = pxz_shrink(k, filter_down, flags) byte for byte (descriptors incl. stored values, pixels);
+ * *factor_out = k, *sse_out = its SSE (each may be NULL).  Synchronises the stream.
+ * PXZ_E_ARG: no factor reaches max_sse (the message names the least SSE reachable), PXZ_FLAG_AFTER_IDENTITY, unknown filter /
+ *            metric.
+ * PXZ_E_UNSUPPORTED: a batch image, a strategy installed on the context, PXZ_FLAG_NORMALISE_GLOBAL with a communicator. */
+pxz_status pxz_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_sse,
+                               pxz_filter filter_down, pxz_filter filter_up, uint32_t flags, float* factor_out, uint64_t* sse_out,
+                               pxz_payload** out);
+
 /* Scalar part of reduce_image_section (operations.rs:128-156) on the host: (v0, v1) after `after`
  * -> parse_value -> level -> reduced size of a w x h block and the stored block value.  Uses the
  * same threshold table as the device plan kernel. */

@@ -12,6 +12,7 @@ from .api import (  # noqa: F401
     FilterType,
     Pixlzr,
     PixlzrBlock,
+    RateDistortion,
     Strategy,
     StrategyReport,
     get_block_variance,
@@ -23,7 +24,9 @@ from .api import (  # noqa: F401
     process_by_strategy,
     process_custom,
     psnr_of,
+    rd_curve,
     reduce_image_section,
+    sse_budget,
     tree_process,
     tree_process_custom,
 )

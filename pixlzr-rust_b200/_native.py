@@ -90,6 +90,8 @@ SYMBOLS = {
     "pxz_image_error": (_i, [_vp, _vp, _vp, _u32, _u32, _vp, _vp, _P(_u64)]),
     "pxz_strategy_measure": (_i, [_vp, _vp, _u32, _u32, _i, C.c_float, _u32, _vp, _vp]),
     "pxz_strategy_choose": (_i, [_vp, _vp, _vp, _vp]),
+    "pxz_rd_curve": (_i, [_vp, _vp, _u32, _u32, _i, _i, _i, _u32, _vp, _vp, _vp, _sz, _P(_sz)]),
+    "pxz_shrink_to_error": (_i, [_vp, _vp, _u32, _u32, _i, _u64, _i, _i, _u32, _P(C.c_float), _P(_u64), _P(_vp)]),
 }
 
 
@@ -404,6 +406,27 @@ class Image:
         self.ctx.check(lib().pxz_strategy_measure(self.ctx.handle, self._h, bw, bh, metric, factor, flags, ptr(sse), ptr(blocks)))
         return sse, blocks
 
+    def rd_curve(self, bw: int, bh: int, metric: int, filter_down: int, filter_up: int, flags: int = 0):
+        """(factor float32 [n], bytes uint64 [n], sse uint64 [n]): every distinct payload shrink(bw, bh, metric, k, filter_down,
+        flags) gives over the finite k > 0, at the smallest k giving it, with the squared error of its decode with filter_up
+        against this image (pxz_rd_curve)."""
+        cap = rd_curve_bound(self.w, self.h, bw, bh, metric)
+        factor = np.empty(cap, np.float32)
+        nbytes = np.empty(cap, np.uint64)
+        sse = np.empty(cap, np.uint64)
+        n = C.c_size_t()
+        self.ctx.check(lib().pxz_rd_curve(self.ctx.handle, self._h, bw, bh, metric, int(filter_down), int(filter_up), flags, ptr(factor),
+                                          ptr(nbytes), ptr(sse), cap, C.byref(n)))
+        return factor[:n.value].copy(), nbytes[:n.value].copy(), sse[:n.value].copy()
+
+    def shrink_to_error(self, bw: int, bh: int, metric: int, max_sse: int, filter_down: int, filter_up: int, flags: int = 0):
+        """(Payload, k, sse): the payload of shrink(..., k, ...) for the smallest factor k whose decode with filter_up has a
+        squared error of at most `max_sse` against this image, and that error (pxz_shrink_to_error)."""
+        h, k, sse = C.c_void_p(), C.c_float(), C.c_uint64()
+        self.ctx.check(lib().pxz_shrink_to_error(self.ctx.handle, self._h, bw, bh, metric, int(max_sse), int(filter_down), int(filter_up),
+                                                 flags, C.byref(k), C.byref(sse), C.byref(h)))
+        return Payload(self.ctx, h), float(k.value), int(sse.value)
+
     def tree_process(self, threshold: float, bw: int, bh: int, min_bw: int, min_bh: int, filter_down: int, filter_up: int,
                      out: "Image"):
         self.ctx.check(lib().pxz_tree_process(self.ctx.handle, self._h, threshold, bw, bh, min_bw, min_bh, int(filter_down),
@@ -533,6 +556,16 @@ def grid(w, h, bw, bh):
     if st != OK:
         raise PixlzrError(st, "pxz_grid")
     return c.value, r.value
+
+
+def rd_curve_bound(w: int, h: int, bw: int, bh: int, metric: int) -> int:
+    """Most points pxz_rd_curve can return: 1 + blocks * (ceil(log2 bw) + ceil(log2 bh)), Oklab-MAD ceil(log2 max(bw, bh)) (a
+    block's dims change at most once per level it can step through)."""
+    if w <= 0 or h <= 0 or bw <= 0 or bh <= 0:
+        raise ValueError("image and block sizes must be positive")
+    lx, ly = (bw - 1).bit_length(), (bh - 1).bit_length()
+    steps = lx + ly if metric == METRIC_SOBEL_DIR else max(lx, ly)
+    return 1 + -(-w // bw) * -(-h // bh) * steps
 
 
 def reduce_dims(v0: float, v1: float, w: int, h: int):

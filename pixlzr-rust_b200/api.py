@@ -189,6 +189,59 @@ def psnr_of(total_sse: int, samples: int) -> float:
     return 10.0 * float(np.log10(255.0 * 255.0 * samples / float(total_sse)))
 
 
+def sse_budget(psnr: float, samples: int) -> int:
+    """The largest squared error whose psnr_of(..., samples) is >= `psnr` dB: the formula's value, then corrected by single
+    steps against psnr_of itself, so that the two never disagree (0 for a target of inf: only an exact decode reaches it)."""
+    psnr = float(psnr)
+    if psnr != psnr or samples <= 0:
+        raise ValueError("a PSNR target needs a number of dB and a positive sample count")
+    top = 2 ** 64 - 1  # the budget is a u64
+    with np.errstate(over="ignore", divide="ignore"):
+        bound = np.float64(255.0 * 255.0 * samples) / np.power(np.float64(10.0), psnr / 10.0)
+    budget = top if not bound < top else int(np.floor(bound))
+    while budget < top and psnr_of(budget + 1, samples) >= psnr:
+        budget += 1
+    while budget > 0 and psnr_of(budget, samples) < psnr:
+        budget -= 1
+    return budget
+
+
+@dataclass
+class RateDistortion:
+    """EXTENSION (pxz_rd_curve): every distinct payload a factor gives, in increasing factor.  factor[i] is the smallest f32
+    factor giving payload i, bytes[i] its payload bytes (strictly increasing), sse[i] the squared error of its decode against
+    the source; a factor between factor[i] and factor[i + 1] gives payload i."""
+    factor: np.ndarray  # float32 [n]
+    bytes: np.ndarray   # uint64 [n]
+    sse: np.ndarray     # uint64 [n]
+    samples: int        # width * height * channels of the source
+
+    @property
+    def psnr(self) -> np.ndarray:
+        return np.array([psnr_of(int(e), self.samples) for e in self.sse], np.float64)
+
+    def smallest_within(self, max_sse: int) -> Optional[int]:
+        """Index of the smallest payload whose error is at most `max_sse` (the point pxz_shrink_to_error picks), None if no
+        factor reaches it."""
+        ok = np.nonzero(self.sse <= np.uint64(max_sse))[0]
+        return int(ok[0]) if ok.size else None
+
+
+def rd_curve(image, block_width: int, block_height: int, filter_down: FilterType, filter_up: FilterType, directionally: bool = False,
+             ctx: Optional[N.Context] = None) -> RateDistortion:
+    """EXTENSION: the exact (bytes, squared error) curve of shrink_by (or shrink_directionally) with `filter_down` and a decode
+    with `filter_up`, over every finite factor, computed on the device (numpy or device image)."""
+    ctx = ctx or (image.ctx if isinstance(image, N.Image) else default_context())
+    img = image if isinstance(image, N.Image) else ctx.image_upload(_check_image(image))
+    try:
+        metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
+        factor, nbytes, sse = img.rd_curve(block_width, block_height, metric, int(filter_down), int(filter_up), 0)
+        return RateDistortion(factor, nbytes, sse, img.w * img.h * img.c)
+    finally:
+        if img is not image:
+            img.free()
+
+
 @dataclass
 class ErrorReport:
     """EXTENSION: the error of one image against another, per block of a grid (pxz_image_error)."""
@@ -418,6 +471,30 @@ class Pixlzr:
             metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
             pl, k = img.shrink_to_size(self.block_width, self.block_height, metric, max_bytes, int(filter_downscale),
                                        N.FLAG_EXACT_VALUES if exact_values else 0)
+            try:
+                self._descs, self._pixels = pl.download()
+            finally:
+                pl.free()
+        finally:
+            img.free()
+        self._values_present = True
+        self._image = None
+        return k
+
+    def shrink_to_psnr(self, filter_downscale: FilterType, filter_upscale: FilterType, psnr: float, directionally: bool = False,
+                       exact_values: bool = False) -> float:
+        """EXTENSION (rate control by error): shrink_by (or shrink_directionally) with the smallest factor whose decode with
+        `filter_upscale` reaches `psnr` dB against the source (sse_budget; pxz_shrink_to_error); returns that factor, which is
+        also the smallest payload reaching the target.  shrink_by / shrink_directionally with the returned factor give the same
+        blocks.  Needs the source image: refused on a decoded or already shrunk Pixlzr."""
+        if self._image is None:
+            raise ValueError("shrink_to_psnr needs the source image (Pixlzr.from_image), not a decoded or already shrunk one")
+        ctx = self._ctx()
+        img = ctx.image_upload(self._image)
+        try:
+            metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
+            pl, k, _ = img.shrink_to_error(self.block_width, self.block_height, metric, sse_budget(psnr, img.w * img.h * img.c),
+                                           int(filter_downscale), int(filter_upscale), N.FLAG_EXACT_VALUES if exact_values else 0)
             try:
                 self._descs, self._pixels = pl.download()
             finally:

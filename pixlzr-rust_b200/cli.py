@@ -43,6 +43,10 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--payload-bytes", type=parse_payload_bytes, default=None, metavar="N",
                    help="Shrink with the largest factor whose block payload has at most N bytes, and print that factor "
                         "(image input, with --force; replaces -k)")
+    # extension (rate control by error): not a flag of the reference
+    p.add_argument("--target-psnr", type=parse_target_psnr, default=None, metavar="DB",
+                   help="Shrink with the smallest factor whose decode (with -f) reaches DB dB PSNR against the input, and print "
+                        "that factor, the payload bytes and the PSNR reached (image input, with --force; replaces -k)")
     # extension (decode error): not a flag of the reference
     p.add_argument("--psnr", action="store_true",
                    help="Decode what was written (with -f), compare it with the input image on the device and print the PSNR "
@@ -58,6 +62,16 @@ def parse_payload_bytes(s: str) -> int:
     if n < 0:
         raise argparse.ArgumentTypeError(f"expected a byte count >= 0, got {s!r}")
     return n
+
+
+def parse_target_psnr(s: str) -> float:
+    try:
+        db = float(s)
+    except ValueError:
+        raise argparse.ArgumentTypeError(f"expected a PSNR in dB, got {s!r}") from None
+    if db != db:
+        raise argparse.ArgumentTypeError(f"expected a PSNR in dB, got {s!r}")
+    return db
 
 
 def parse_region(s: str) -> Tuple[int, int, int, int]:
@@ -91,6 +105,23 @@ def payload_bytes_error(args) -> Optional[str]:
         return "--payload-bytes chooses the shrinking factor: it cannot be combined with -k"
     if args.region is not None:
         return "--payload-bytes does not apply to a region decode"
+    return None
+
+
+def target_psnr_error(args) -> Optional[str]:
+    """Why --target-psnr does not apply to these arguments, or None."""
+    if getattr(args, "target_psnr", None) is None:
+        return None
+    if operation(args.input, args.output)[0] != "image":
+        return "--target-psnr chooses the factor of an encode: the input must be an image, not a container"
+    if not args.force:
+        return "--target-psnr shrinks the blocks: it needs --force"
+    if getattr(args, "factor_given", False):
+        return "--target-psnr chooses the shrinking factor: it cannot be combined with -k"
+    if args.payload_bytes is not None:
+        return "--target-psnr and --payload-bytes each choose the factor: give one of them"
+    if args.region is not None:
+        return "--target-psnr does not apply to a region decode"
     return None
 
 
@@ -159,9 +190,12 @@ def run(args) -> None:
     filt = FILTERS[args.filter]
     shrink_by = api.parse_shrinking_factor(args.shrinking_factor)
     src, dst = operation(args.input, args.output)
-    err = region_error(args) or payload_bytes_error(args) or psnr_error(args)
+    err = region_error(args) or payload_bytes_error(args) or target_psnr_error(args) or psnr_error(args)
     if err:
         raise ValueError(err)
+    if args.target_psnr is not None:
+        _run_psnr_target(args, bw, bh, filt, dst)
+        return
     if args.payload_bytes is not None:
         _run_sized(args, bw, bh, filt, src, dst)
         return
@@ -210,6 +244,32 @@ def _run_sized(args, bw: int, bh: int, filt, src: str, dst: str) -> None:
     print(f"shrinking factor: {api.format_shrinking_factor(k)}")
 
 
+def _run_psnr_target(args, bw: int, bh: int, filt, dst: str) -> None:
+    """image -> container / image with the smallest factor whose decode with -f (the filter a decoder of the written file uses)
+    reaches --target-psnr; prints the factor in a form -k reads back, the payload bytes and the PSNR reached."""
+    image = _open_image(args.input)
+    ctx = api.default_context()
+    img = ctx.image_upload(image)
+    try:
+        samples = img.w * img.h * img.c
+        metric = api.N.METRIC_SOBEL_DIR if args.direction_wise else api.N.METRIC_OKLAB_MAD
+        pl, k, sse = img.shrink_to_error(bw, bh, metric, api.sse_budget(args.target_psnr, samples), int(filt), int(filt), 0)
+    finally:
+        img.free()
+    try:
+        nbytes = pl.info()["bytes"]
+        if dst == "pix":
+            with open(args.output, "wb") as f:
+                f.write(pl.to_container(0, True))
+        else:
+            _save_image(args.output, pl.expand(int(filt)))
+    finally:
+        pl.free()
+    print(f"shrinking factor: {api.format_shrinking_factor(k)}")
+    print(f"payload bytes: {nbytes}")
+    print(f"psnr: {format_psnr(api.psnr_of(sse, samples))} dB")
+
+
 def format_psnr(psnr: float) -> str:
     return "inf" if psnr == float("inf") else f"{psnr:.6f}"
 
@@ -234,7 +294,7 @@ def report_psnr(args) -> None:
 
 def main(argv: Optional[List[str]] = None) -> int:
     args = parse_args(argv)
-    err = region_error(args) or payload_bytes_error(args) or psnr_error(args)
+    err = region_error(args) or payload_bytes_error(args) or target_psnr_error(args) or psnr_error(args)
     if err:
         print(f"pixlzr: {err}", file=sys.stderr)
         return 2

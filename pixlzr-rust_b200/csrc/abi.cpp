@@ -47,11 +47,12 @@ using TabKey = std::tuple<std::vector<uint32_t>, std::vector<uint32_t>, int, int
 
 // K_REGION_COPY times the device-to-device copy of pxz_expand_region out of its staging image (not a kernel)
 enum KernelId { K_MAD_FAST = 0, K_MAD_EXACT, K_SOBEL, K_MINMAX, K_PLAN, K_RESAMPLE_DOWN, K_RESAMPLE_UP, K_QOI_ENCODE, K_QOI_DECODE,
-                K_PAYLOAD_WINDOW, K_REGION_COPY, K_SIZE_CURVE, K_BLOCK_ERROR, K_BUCKET_SUM, K_COUNT };
+                K_PAYLOAD_WINDOW, K_REGION_COPY, K_SIZE_CURVE, K_BLOCK_ERROR, K_BUCKET_SUM, K_RD_LEVELS, K_RD_EVENTS, K_RD_CURVE, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"analyze_mad_fast", "mad_exact",      "analyze_sobel", "minmax",
                                            "plan",             "resample_down",  "resample_up",   "qoi_encode",
                                            "qoi_decode",       "payload_window", "region_copy",   "size_curve",
-                                           "block_error",      "bucket_sum"};
+                                           "block_error",      "bucket_sum",     "rd_levels",     "rd_events",
+                                           "rd_curve"};
 struct ProfRec {
   int id;
   cudaEvent_t a, b;
@@ -1369,6 +1370,184 @@ pxz_status pxz_strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw,
     ~StrategyOff() { c->strategy = saved; }
   } off(ctx);
   return strategy_measure(ctx, img, bw, bh, metric, factor, flags, host_sse, host_blocks);
+}
+
+// ---- rate-distortion curve (extension) ---------------------------------------------------------------------------
+// What pxz_rd_curve and pxz_shrink_to_error refuse: pxz_shrink_to_size's refusals, plus an installed strategy (its filter pair
+// follows the stored value, which moves with the factor) and an unknown up filter
+static pxz_status rd_refusal(pxz_ctx* ctx, const pxz_image* img, pxz_metric metric, pxz_filter filter_down, pxz_filter filter_up, uint32_t flags) {
+  if (!known_filter(filter_down) || !known_filter(filter_up)) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (metric != PXZ_METRIC_OKLAB_MAD && metric != PXZ_METRIC_SOBEL_DIR) return fail(ctx, PXZ_E_ARG, "unknown metric");
+  if (flags & PXZ_FLAG_AFTER_IDENTITY) return fail(ctx, PXZ_E_ARG, "PXZ_FLAG_AFTER_IDENTITY ignores the factor: no curve over it");
+  if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "a rate-distortion curve is per image: not available on a batch");
+  if ((flags & PXZ_FLAG_NORMALISE_GLOBAL) && ctx->comm)
+    return fail(ctx, PXZ_E_UNSUPPORTED, "a rate-distortion curve with global normalisation over a communicator is not available");
+  if (ctx->strategy.on)
+    return fail(ctx, PXZ_E_UNSUPPORTED, "a rate-distortion curve with a strategy installed is not available (the filter pair moves with the factor)");
+  return PXZ_OK;
+}
+
+// What one curve computation returns to the host besides the points
+struct RdSummary {
+  uint32_t n = 0;                  // curve points
+  uint32_t first = 0xFFFFFFFFu;    // first point with sse <= max_sse (0xFFFFFFFF: none)
+  uint32_t first_bits = 0;         // its factor's bit pattern
+  uint64_t first_sse = 0;
+  uint64_t least_sse = 0;          // least sse of any point
+};
+
+static uint32_t ceil_log2(uint32_t n) { return n <= 1 ? 0u : 32u - (uint32_t)__builtin_clz(n - 1); }
+
+// The curve of pxz_rd_curve after the checks (DESIGN.md §3).  bpp: bytes per pixel counted (3 for an RGB image on the RGBA
+// kernels).  The points are copied to the host arrays when cap >= n.
+static pxz_status rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, pxz_filter filter_down,
+                           pxz_filter filter_up, uint32_t flags, uint32_t bpp, uint64_t max_sse, float* host_factor, uint64_t* host_bytes,
+                           uint64_t* host_sse, size_t cap, RdSummary* sum) {
+  // An RGB image that pxz_shrink runs on the RGBA kernels is measured as its RGBA widening, as in strategy_measure: alpha is 255
+  // in the source and in every decode and adds 0
+  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
+    ImageOwner wide;
+    pxz_status st = rgb_widened(ctx, img, &wide);
+    if (st != PXZ_OK) return st;
+    return rd_curve(ctx, wide.get(), bw, bh, metric, filter_down, filter_up, flags, 3, max_sse, host_factor, host_bytes, host_sse, cap, sum);
+  }
+  Geom g;
+  pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g);
+  if (st != PXZ_OK) return st;
+  const size_t nblocks = (size_t)g.cols * g.rows;
+  const bool sobel = metric == PXZ_METRIC_SOBEL_DIR;
+  // Error passes: Oklab-MAD has one level for both axes (the diagonal), Sobel every (lx, ly) pair.  A level above Lx (Ly) gives
+  // the dims of Lx (Ly), so those passes cover every level a block can reach.
+  const uint32_t lx_max = ceil_log2(bw), ly_max = ceil_log2(bh), l_max = std::max(lx_max, ly_max);
+  const RdPasses ps = sobel ? RdPasses{lx_max, ly_max, ly_max + 1, 1} : RdPasses{l_max, l_max, 1, 0};
+  const uint32_t npass = sobel ? (lx_max + 1) * (ly_max + 1) : l_max + 1;
+  const uint32_t maxev = sobel ? lx_max + ly_max : l_max;  // dims changes per block
+  const uint64_t nev64 = (uint64_t)nblocks * maxev;
+  if (nev64 > 0x7FFFFFFFull) return fail(ctx, PXZ_E_UNSUPPORTED, "more than 2^31 curve events (blocks x levels)");
+  const uint32_t nev = (uint32_t)nev64;
+
+  // 1. reference-order values (their dims are pxz_shrink's in every mode), the min / max as pxz_shrink takes it, and a copy
+  if ((st = run_shrink_analysis(ctx, img, g, metric, flags | PXZ_FLAG_EXACT_VALUES, nullptr)) != PXZ_OK) return st;
+  DevBlocks bufs(ctx);
+  float* vals = nullptr;
+  uint64_t* table = nullptr;  // [npass][nblocks] block errors
+  uint8_t* ev = nullptr;      // events: keys | ids | dbytes | dsse | base[2] | points: key | bytes | sse | RdOut
+  void* scratch = nullptr;
+  const size_t scratch_bytes = rd_curve_scratch_bytes(nev);
+  const size_t npt = (size_t)nev + 1;
+  const size_t ev_bytes = (size_t)nev * 24 + 16 + npt * 20 + sizeof(RdOut) + 64;
+  if ((st = bufs.alloc(&vals, nblocks * 4 * (sobel ? 2 : 1))) != PXZ_OK || (st = bufs.alloc(&table, (size_t)npass * nblocks * 8)) != PXZ_OK ||
+      (st = bufs.alloc(&ev, ev_bytes)) != PXZ_OK || (st = bufs.alloc(&scratch, scratch_bytes)) != PXZ_OK)
+    return st;
+  // 8-byte words first
+  uint64_t* dbytes = reinterpret_cast<uint64_t*>(ev);
+  uint64_t* dsse = dbytes + nev;
+  uint64_t* base = dsse + nev;
+  uint64_t* pt_bytes = base + 2;
+  uint64_t* pt_sse = pt_bytes + npt;
+  RdOut* d_out = reinterpret_cast<RdOut*>(pt_sse + npt);
+  uint32_t* keys = reinterpret_cast<uint32_t*>(d_out + 1);
+  uint32_t* ids = keys + nev;
+  uint32_t* pt_key = ids + nev;
+  PXZ_CUDA(ctx, cudaMemcpyAsync(vals, ctx->d_vx, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+  if (sobel) PXZ_CUDA(ctx, cudaMemcpyAsync(vals + nblocks, ctx->d_vy, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+
+  // 2. error table: per pass the plan + resample of pxz_shrink with every block forced to (lx, ly) — values 2^-lx / 2^-ly under
+  // the directional map at factor 1, no normalisation — then the decode and its per-block error
+  ImageOwner dec;
+  if ((st = image_new(ctx, img->w, img->h, img->c, 1, &dec)) != PXZ_OK) return st;
+  const ValueMap forced = shrink_value_map(ctx, PXZ_METRIC_SOBEL_DIR, 0, 1.0f);
+  for (uint32_t lx = 0; lx <= (sobel ? lx_max : l_max); ++lx) {
+    for (uint32_t ly = sobel ? 0 : lx; ly <= (sobel ? ly_max : lx); ++ly) {
+      const float fx = ldexpf(1.0f, -(int)lx), fy = ldexpf(1.0f, -(int)ly);
+      uint32_t w = 0, h = 0;  // level_k(2^-l) = l: the plan sees exactly these levels
+      pxz_reduce_dims(fx, fy, bw, bh, &w, &h, nullptr);
+      if (w != std::max(1u, ceil_div_u32(bw, 1u << lx)) || h != std::max(1u, ceil_div_u32(bh, 1u << ly)))
+        return fail(ctx, PXZ_E_CUDA, "level table does not map 2^-l to level l");
+      st = profiled(ctx, K_RD_LEVELS, "rd levels", [&] {
+        return launch_rd_levels(ctx->d_vx, ctx->d_vy, (uint32_t)nblocks, fx, fy, ctx->stream, ctx->sm_count, &ctx->launches);
+      });
+      if (st != PXZ_OK) return st;
+      pxz_payload* raw = nullptr;
+      if ((st = plan_and_resample(ctx, img, g, PXZ_METRIC_SOBEL_DIR, forced, filter_down, true, &raw)) != PXZ_OK) return st;
+      const PayloadOwner p(raw);
+      if ((st = pxz_expand_to_image(ctx, p.get(), filter_up, dec.get())) != PXZ_OK) return st;
+      const uint32_t pass = lx * ps.stride_x + ly * ps.stride_y;
+      if ((st = run_block_error(ctx, img, dec.get(), g, table + (size_t)pass * nblocks, nullptr)) != PXZ_OK) return st;
+    }
+  }
+
+  // 3. events of every block, 4. the curve
+  const ValueMap vm = shrink_value_map(ctx, metric, flags & PXZ_FLAG_NORMALISE_GLOBAL, 1.0f);
+  PXZ_CUDA(ctx, cudaMemsetAsync(base, 0, 2 * sizeof(uint64_t), ctx->stream));
+  st = profiled(ctx, K_RD_EVENTS, "rd events", [&] {
+    return launch_rd_events(vals, sobel ? vals + nblocks : nullptr, g, vm, ctx->d_minmax, ctx->thr, bpp, table, ps, maxev, keys, ids, dbytes, dsse,
+                            base, ctx->stream, &ctx->launches);
+  });
+  if (st != PXZ_OK) return st;
+  st = profiled(ctx, K_RD_CURVE, "rd curve", [&] {
+    return launch_rd_curve(keys, ids, dbytes, dsse, nev, base, max_sse, scratch, scratch_bytes, pt_key, pt_bytes, pt_sse, d_out, ctx->stream,
+                           ctx->sm_count, &ctx->launches);
+  });
+  if (st != PXZ_OK) return st;
+
+  // 5. to the host: the summary, the first point within max_sse, and the points when they fit
+  RdOut o;
+  PXZ_CUDA(ctx, cudaMemcpyAsync(&o, d_out, sizeof(o), cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  sum->n = o.count;
+  sum->first = o.first_within;
+  sum->least_sse = o.least_sse;
+  if (o.first_within < o.count) {
+    PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->first_bits, pt_key + o.first_within, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->first_sse, pt_sse + o.first_within, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  if (cap >= o.count && host_factor && host_bytes && host_sse) {
+    PXZ_CUDA(ctx, cudaMemcpyAsync(host_factor, pt_key, (size_t)o.count * 4, cudaMemcpyDeviceToHost, ctx->stream));  // f32 bits
+    PXZ_CUDA(ctx, cudaMemcpyAsync(host_bytes, pt_bytes, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, pt_sse, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
+  }
+  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return PXZ_OK;
+}
+
+pxz_status pxz_rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, pxz_filter filter_down,
+                        pxz_filter filter_up, uint32_t flags, float* host_factor, uint64_t* host_bytes, uint64_t* host_sse, size_t cap,
+                        size_t* n_out) {
+  if (n_out) *n_out = 0;
+  if (!ctx || !img || !n_out || (cap > 0 && (!host_factor || !host_bytes || !host_sse))) return PXZ_E_ARG;
+  cudaSetDevice(ctx->device);
+  pxz_status st = rd_refusal(ctx, img, metric, filter_down, filter_up, flags);
+  if (st != PXZ_OK) return st;
+  RdSummary sum;
+  st = rd_curve(ctx, img, bw, bh, metric, filter_down, filter_up, flags, img->c, 0, host_factor, host_bytes, host_sse, cap, &sum);
+  if (st != PXZ_OK) return st;
+  *n_out = sum.n;
+  if (cap < sum.n) return fail(ctx, PXZ_E_ARG, "cap " + std::to_string(cap) + " is below the curve's " + std::to_string(sum.n) + " points");
+  return PXZ_OK;
+}
+
+pxz_status pxz_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_sse,
+                               pxz_filter filter_down, pxz_filter filter_up, uint32_t flags, float* factor_out, uint64_t* sse_out,
+                               pxz_payload** out) {
+  if (!ctx || !img || !out) return PXZ_E_ARG;
+  *out = nullptr;
+  cudaSetDevice(ctx->device);
+  pxz_status st = rd_refusal(ctx, img, metric, filter_down, filter_up, flags);
+  if (st != PXZ_OK) return st;
+  RdSummary sum;
+  st = rd_curve(ctx, img, bw, bh, metric, filter_down, filter_up, flags, img->c, max_sse, nullptr, nullptr, nullptr, 0, &sum);
+  if (st != PXZ_OK) return st;
+  if (sum.first >= sum.n)
+    return fail(ctx, PXZ_E_ARG, "max_sse " + std::to_string(max_sse) + " is below the least squared error any factor reaches (" +
+                                    std::to_string(sum.least_sse) + ")");
+  float k;
+  memcpy(&k, &sum.first_bits, 4);
+  // the curve's point is the payload of pxz_shrink(k): encode it exactly so
+  if ((st = pxz_shrink(ctx, img, bw, bh, metric, k, filter_down, flags, out)) != PXZ_OK) return st;
+  if (factor_out) *factor_out = k;
+  if (sse_out) *sse_out = sum.first_sse;
+  return PXZ_OK;
 }
 
 pxz_status pxz_strategy_choose(const uint64_t* sse, const uint32_t* blocks, const pxz_strategy* base, pxz_strategy* out) {

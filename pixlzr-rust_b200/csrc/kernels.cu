@@ -12,6 +12,9 @@
 //                        image tiles -> packed payload (shrink) or payload -> image tiles (expand+paste)
 //   k_block_error        per-block squared error and largest difference of two images (integer, exact)
 //   k_bucket_sum         block errors summed per strategy bucket of the stored block value (strategy measure)
+//   k_rd_levels          forced levels of one error pass of the rate-distortion curve
+//   k_rd_events          per block, the factors at which its dims change and what that changes (rate-distortion curve)
+//   k_rd_gather / k_rd_compact   sorted events -> scan input -> curve points (around CUB's radix sort and scan)
 //
 // Nothing here is a dense contraction, so no tensor cores: the kernels are HBM / FP32-pipe work with
 // 16-byte coalesced loads, shared-memory staging and warp-shuffle reductions (DESIGN.md).
@@ -20,6 +23,9 @@
 #include <stdint.h>
 #include <stdlib.h>
 #include <string.h>
+
+#include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include "pxz_internal.h"
 
@@ -1317,6 +1323,152 @@ __global__ void __launch_bounds__(kThreads) k_size_curve(const float* __restrict
 #pragma unroll
     for (int w = 0; w < kThreads / 32; ++w) s += s_part[w][c - c0];
     if (s != 0ull) atomicAdd(&bytes[c], s * bpp);
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// rate-distortion curve (pxz_rd_curve, pxz_shrink_to_error; DESIGN.md §3).  A block's dims at factor k follow from its raw
+// values through the helpers k_plan uses, and they grow monotonically with k (raw values are >= +0 or NaN), so each block
+// steps through its few distinct dims at exact f32 bit patterns.  k_rd_events finds them by bisection over the patterns and
+// prices each step with the block's error at the new dims, read from the per-pass error table.
+// ------------------------------------------------------------------------------------------------
+constexpr uint32_t kMaxPattern = 0x7F7FFFFFu;  // FLT_MAX; patterns 1 .. kMaxPattern are the finite factors > 0
+
+__global__ void __launch_bounds__(kThreads) k_rd_levels(float* __restrict__ vx, float* __restrict__ vy, uint32_t n, float fx, float fy) {
+  for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < n; i += gridDim.x * kThreads) {
+    vx[i] = fx;
+    vy[i] = fy;
+  }
+}
+
+// dims and error pass of a block with raw values (rx, ry) and tile (tw, th) at the factor with bit pattern `bits`
+struct RdAt {
+  uint32_t dw, dh, pass;
+};
+__device__ __forceinline__ RdAt rd_at(const ValueMap& vm, const float* minmax, const LevelThresholds& thr, const RdPasses& ps, float rx, float ry,
+                                      uint32_t tw, uint32_t th, uint32_t bits) {
+  ValueMap v = vm;
+  v.factor = __uint_as_float(bits);
+  float v0, v1;
+  map_values(v, minmax, rx, ry, v0, v1);
+  const uint32_t kx = level_k(parse_value_dev(v0), thr), ky = level_k(parse_value_dev(v1), thr);
+  return RdAt{scaled_dim(tw, kx), scaled_dim(th, ky), min(kx, ps.cap_x) * ps.stride_x + min(ky, ps.cap_y) * ps.stride_y};
+}
+
+__global__ void __launch_bounds__(kThreads) k_rd_events(const float* __restrict__ vx, const float* __restrict__ vy, Geom g, ValueMap vm,
+                                                        const float* __restrict__ minmax, LevelThresholds thr, uint32_t bpp,
+                                                        const unsigned long long* __restrict__ sse_table, RdPasses ps, uint32_t maxev,
+                                                        uint32_t* __restrict__ keys, uint32_t* __restrict__ ids,
+                                                        unsigned long long* __restrict__ dbytes, unsigned long long* __restrict__ dsse,
+                                                        unsigned long long* __restrict__ base) {
+  const uint32_t nblocks = g.cols * g.rows;
+  const uint32_t b = blockIdx.x * kThreads + threadIdx.x;
+  unsigned long long bytes0 = 0, sse0 = 0;
+  if (b < nblocks) {
+    const Tile t = tile_of(g, b);
+    // the global normalisation does not depend on the factor: applied once here (the directional map at factor 1 returns the
+    // normalised values exactly), then every pattern maps the normalised values
+    float rx, ry;
+    {
+      ValueMap n = vm;
+      n.mode = 2;
+      n.factor = 1.0f;
+      map_values(n, minmax, vx[b], vy ? vy[b] : vx[b], rx, ry);
+      vm.normalise = 0;
+    }
+    RdAt cur = rd_at(vm, minmax, thr, ps, rx, ry, t.tw, t.th, 1u);
+    const RdAt end = rd_at(vm, minmax, thr, ps, rx, ry, t.tw, t.th, kMaxPattern);
+    unsigned long long sse = sse_table[(size_t)cur.pass * nblocks + b];
+    bytes0 = (unsigned long long)cur.dw * cur.dh * bpp;
+    sse0 = sse;
+    uint32_t p = 1u, n = 0;
+    for (; n < maxev && (cur.dw != end.dw || cur.dh != end.dh); ++n) {
+      // the smallest pattern above p whose dims differ from cur's: dims(lo) == cur, dims(hi) != cur
+      uint32_t lo = p, hi = kMaxPattern;
+      while (hi - lo > 1u) {
+        const uint32_t mid = lo + (hi - lo) / 2u;
+        const RdAt m = rd_at(vm, minmax, thr, ps, rx, ry, t.tw, t.th, mid);
+        if (m.dw == cur.dw && m.dh == cur.dh) lo = mid; else hi = mid;
+      }
+      const RdAt next = rd_at(vm, minmax, thr, ps, rx, ry, t.tw, t.th, hi);
+      const unsigned long long nsse = sse_table[(size_t)next.pass * nblocks + b];
+      const size_t slot = (size_t)b * maxev + n;
+      keys[slot] = hi;
+      ids[slot] = (uint32_t)slot;
+      dbytes[slot] = ((unsigned long long)next.dw * next.dh - (unsigned long long)cur.dw * cur.dh) * bpp;
+      dsse[slot] = nsse - sse;  // mod 2^64: the scan's sums are exact
+      cur = next;
+      sse = nsse;
+      p = hi;
+    }
+    for (; n < maxev; ++n) {
+      const size_t slot = (size_t)b * maxev + n;
+      keys[slot] = kRdNoEvent;
+      ids[slot] = (uint32_t)slot;
+      dbytes[slot] = 0ull;
+      dsse[slot] = 0ull;
+    }
+  }
+  bytes0 = warp_sum_u64(bytes0);
+  sse0 = warp_sum_u64(sse0);
+  if ((threadIdx.x & 31) == 0) {
+    if (bytes0) atomicAdd(&base[0], bytes0);
+    if (sse0) atomicAdd(&base[1], sse0);
+  }
+}
+
+// running sums of the sorted events: payload bytes and squared error (mod 2^64); the curve points (last event of each key) are
+// counted by a second scan over u32 flags, which keeps the 16-byte scan free of spills
+struct RdAcc {
+  unsigned long long bytes, sse;
+};
+struct RdAccSum {
+  __host__ __device__ RdAcc operator()(const RdAcc& a, const RdAcc& b) const { return {a.bytes + b.bytes, a.sse + b.sse}; }
+};
+
+__device__ __forceinline__ bool rd_last_of_key(const uint32_t* keys, uint32_t i, uint32_t nev) {
+  const uint32_t k = keys[i];
+  return k != kRdNoEvent && (i + 1 == nev || keys[i + 1] != k);
+}
+
+__global__ void __launch_bounds__(kThreads) k_rd_gather(const uint32_t* __restrict__ keys, const uint32_t* __restrict__ ids,
+                                                        const unsigned long long* __restrict__ dbytes,
+                                                        const unsigned long long* __restrict__ dsse, uint32_t nev, RdAcc* __restrict__ acc,
+                                                        uint32_t* __restrict__ last) {
+  for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < nev; i += gridDim.x * kThreads) {
+    const uint32_t id = ids[i];
+    acc[i] = RdAcc{dbytes[id], dsse[id]};
+    last[i] = rd_last_of_key(keys, i, nev) ? 1u : 0u;
+  }
+}
+
+__device__ __forceinline__ void rd_point(uint32_t j, uint32_t key, unsigned long long bytes, unsigned long long sse, unsigned long long max_sse,
+                                         uint32_t* pt_key, unsigned long long* pt_bytes, unsigned long long* pt_sse, RdOut* out) {
+  pt_key[j] = key;
+  pt_bytes[j] = bytes;
+  pt_sse[j] = sse;
+  atomicMin(&out->least_sse, sse);
+  if (sse <= max_sse) atomicMin(&out->first_within, j);
+}
+
+// out is all ones on entry (least = first = max)
+__global__ void __launch_bounds__(kThreads) k_rd_compact(const uint32_t* __restrict__ keys, const RdAcc* __restrict__ acc,
+                                                         const uint32_t* __restrict__ points, uint32_t nev,
+                                                         const unsigned long long* __restrict__ base, unsigned long long max_sse,
+                                                         uint32_t* __restrict__ pt_key, unsigned long long* __restrict__ pt_bytes,
+                                                         unsigned long long* __restrict__ pt_sse, RdOut* __restrict__ out) {
+  const uint32_t first = blockIdx.x * kThreads + threadIdx.x;
+  if (first == 0) {
+    rd_point(0, 1u, base[0], base[1], max_sse, pt_key, pt_bytes, pt_sse, out);
+    if (nev == 0) out->count = 1;
+  }
+  for (uint32_t i = first; i < nev; i += gridDim.x * kThreads) {
+    const uint32_t j = points[i];
+    if (rd_last_of_key(keys, i, nev)) {
+      const RdAcc a = acc[i];
+      rd_point(j, keys[i], base[0] + a.bytes, base[1] + a.sse, max_sse, pt_key, pt_bytes, pt_sse, out);
+    }
+    if (i + 1 == nev) out->count = j + 1;
   }
 }
 
@@ -2868,6 +3020,80 @@ cudaError_t launch_payload_convert(const pxz_block_desc* sdescs, const uint8_t* 
   const int grid = clamp_grid(((long long)nblocks + 7) / 8, (long long)sm_count * 8);
   return launch(k_payload_convert, grid, kThreads, 0, s, sdescs, spx, smeta, scap, reinterpret_cast<const unsigned long long*>(stotal), ddescs, dpx,
                 dmeta, dcap, reinterpret_cast<unsigned long long*>(dtotal), nblocks, sc, dc);
+}
+
+cudaError_t launch_rd_levels(float* vx, float* vy, uint32_t n, float fx, float fy, cudaStream_t s, int sm_count, uint64_t* launches) {
+  ++*launches;
+  const int grid = clamp_grid(((long long)n + kThreads - 1) / kThreads, (long long)sm_count * 8);
+  return launch(k_rd_levels, grid, kThreads, 0, s, vx, vy, n, fx, fy);
+}
+
+cudaError_t launch_rd_events(const float* vx, const float* vy, const Geom& g, const ValueMap& vm, const float* minmax,
+                             const LevelThresholds& thr, uint32_t bpp, const uint64_t* sse_table, const RdPasses& ps, uint32_t maxev,
+                             uint32_t* keys, uint32_t* ids, uint64_t* dbytes, uint64_t* dsse, uint64_t* base, cudaStream_t s,
+                             uint64_t* launches) {
+  const uint32_t nblocks = g.cols * g.rows;
+  ++*launches;
+  return launch(k_rd_events, (nblocks + kThreads - 1) / kThreads, kThreads, 0, s, vx, vy, g, vm, minmax, thr, bpp,
+                reinterpret_cast<const unsigned long long*>(sse_table), ps, maxev, keys, ids, reinterpret_cast<unsigned long long*>(dbytes),
+                reinterpret_cast<unsigned long long*>(dsse), reinterpret_cast<unsigned long long*>(base));
+}
+
+// scratch of launch_rd_curve: sorted keys | sorted ids | last-of-key flags | point indices | scan input | scan output | CUB's
+// temporary storage
+static size_t rd_align(size_t n) { return (n + 255) & ~(size_t)255; }
+static size_t rd_cub_bytes(uint32_t nev) {
+  size_t sort = 0, scan = 0, count = 0;
+  cub::DeviceRadixSort::SortPairs(nullptr, sort, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const uint32_t*)nullptr, (uint32_t*)nullptr,
+                                  (int)nev, 0, 32);
+  cub::DeviceScan::InclusiveScan(nullptr, scan, (const RdAcc*)nullptr, (RdAcc*)nullptr, RdAccSum(), (int)nev);
+  cub::DeviceScan::InclusiveSum(nullptr, count, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)nev);
+  return std::max(sort, std::max(scan, count));
+}
+size_t rd_curve_scratch_bytes(uint32_t nev) {
+  return 4 * rd_align((size_t)nev * 4) + 2 * rd_align((size_t)nev * sizeof(RdAcc)) + rd_align(rd_cub_bytes(nev));
+}
+
+cudaError_t launch_rd_curve(const uint32_t* keys, const uint32_t* ids, const uint64_t* dbytes, const uint64_t* dsse, uint32_t nev,
+                            const uint64_t* base, uint64_t max_sse, void* scratch, size_t scratch_bytes, uint32_t* pt_key, uint64_t* pt_bytes,
+                            uint64_t* pt_sse, RdOut* out, cudaStream_t s, int sm_count, uint64_t* launches) {
+  if (scratch_bytes < rd_curve_scratch_bytes(nev) || nev > 0x7FFFFFFFu) return cudaErrorInvalidValue;
+  uint8_t* p = static_cast<uint8_t*>(scratch);
+  uint32_t* skeys = reinterpret_cast<uint32_t*>(p);
+  p += rd_align((size_t)nev * 4);
+  uint32_t* sids = reinterpret_cast<uint32_t*>(p);
+  p += rd_align((size_t)nev * 4);
+  uint32_t* last = reinterpret_cast<uint32_t*>(p);
+  p += rd_align((size_t)nev * 4);
+  uint32_t* points = reinterpret_cast<uint32_t*>(p);
+  p += rd_align((size_t)nev * 4);
+  RdAcc* acc = reinterpret_cast<RdAcc*>(p);
+  p += rd_align((size_t)nev * sizeof(RdAcc));
+  RdAcc* sums = reinterpret_cast<RdAcc*>(p);
+  p += rd_align((size_t)nev * sizeof(RdAcc));
+  size_t cub_bytes = rd_cub_bytes(nev);
+  cudaError_t e = cudaMemsetAsync(out, 0xFF, sizeof(RdOut), s);
+  const int grid = clamp_grid(((long long)nev + kThreads - 1) / kThreads, (long long)sm_count * 8);
+  if (e == cudaSuccess && nev > 0) {
+    // sort, gather, two scans: CUB's sort and scans launch several kernels each and count as one launch here
+    *launches += 4;
+    e = cub::DeviceRadixSort::SortPairs(p, cub_bytes, keys, skeys, ids, sids, (int)nev, 0, 32, s);
+    if (e == cudaSuccess) e = launch(k_rd_gather, grid, kThreads, 0, s, skeys, sids, reinterpret_cast<const unsigned long long*>(dbytes),
+                                     reinterpret_cast<const unsigned long long*>(dsse), nev, acc, last);
+    if (e == cudaSuccess) {
+      cub_bytes = rd_cub_bytes(nev);
+      e = cub::DeviceScan::InclusiveScan(p, cub_bytes, acc, sums, RdAccSum(), (int)nev, s);
+    }
+    if (e == cudaSuccess) {
+      cub_bytes = rd_cub_bytes(nev);
+      e = cub::DeviceScan::InclusiveSum(p, cub_bytes, last, points, (int)nev, s);
+    }
+  }
+  if (e != cudaSuccess) return e;
+  ++*launches;
+  return launch(k_rd_compact, grid, kThreads, 0, s, skeys, sums, points, nev, reinterpret_cast<const unsigned long long*>(base),
+                (unsigned long long)max_sse, pt_key, reinterpret_cast<unsigned long long*>(pt_bytes), reinterpret_cast<unsigned long long*>(pt_sse),
+                out);
 }
 
 size_t resample_fir_smem_bytes(uint32_t max_src_px, uint32_t max_tmp_px, uint32_t C) {

@@ -174,6 +174,35 @@ constexpr uint32_t kFilterPairs = 25;  // pair = down * 5 + up
 static_assert(kFilterPairs == PXZ_FILTER_PAIRS, "filter pair count");
 cudaError_t launch_bucket_sum(const pxz_block_desc* descs, const uint64_t* block_sse, uint32_t nblocks, uint32_t pair, bool count,
                               uint64_t* sse, uint32_t* blocks, cudaStream_t s, int sm_count, uint64_t* launches);
+// Rate-distortion curve (pxz_rd_curve / pxz_shrink_to_error).
+// launch_rd_levels: vx[b] = fx, vy[b] = fy for b < n (the forced levels of one error pass).
+cudaError_t launch_rd_levels(float* vx, float* vy, uint32_t n, float fx, float fy, cudaStream_t s, int sm_count, uint64_t* launches);
+// The error pass of a block at levels (kx, ky): min(kx, cap_x) * stride_x + min(ky, cap_y) * stride_y; block b's error in that
+// pass is sse_table[pass * nblocks + b].
+struct RdPasses {
+  uint32_t cap_x, cap_y, stride_x, stride_y;
+};
+constexpr uint32_t kRdNoEvent = 0xFFFFFFFFu;  // key of an unused event slot (above every finite factor's bit pattern)
+// launch_rd_events: per block, from its raw values (vm.factor ignored) the factors at which its dims change: slot
+// b * maxev + i < b * maxev + maxev holds key = the smallest f32 bit pattern with the new dims, dbytes / dsse = the change of
+// the block's payload bytes / squared error there (dsse two's complement: it may fall), id = the slot; unused slots have key
+// kRdNoEvent and zero changes.  base[0] / base[1] += the bytes / errors of all blocks at pattern 1 (zero on entry).
+cudaError_t launch_rd_events(const float* vx, const float* vy, const Geom& g, const ValueMap& vm, const float* minmax,
+                             const LevelThresholds& thr, uint32_t bpp, const uint64_t* sse_table, const RdPasses& ps, uint32_t maxev,
+                             uint32_t* keys, uint32_t* ids, uint64_t* dbytes, uint64_t* dsse, uint64_t* base, cudaStream_t s,
+                             uint64_t* launches);
+// launch_rd_curve: the events sorted by key, prefix sums of their changes, one point per distinct key.  Point 0 = pattern 1
+// with the base totals; point j = the j-th distinct key with base + the changes up to it.  out: least sse of any point, the
+// point count, the first point with sse <= max_sse (0xFFFFFFFF: none).  scratch: rd_curve_scratch_bytes(nev).
+struct RdOut {
+  unsigned long long least_sse;
+  uint32_t count;
+  uint32_t first_within;
+};
+size_t rd_curve_scratch_bytes(uint32_t nev);
+cudaError_t launch_rd_curve(const uint32_t* keys, const uint32_t* ids, const uint64_t* dbytes, const uint64_t* dsse, uint32_t nev,
+                            const uint64_t* base, uint64_t max_sse, void* scratch, size_t scratch_bytes, uint32_t* pt_key, uint64_t* pt_bytes,
+                            uint64_t* pt_sse, RdOut* out, cudaStream_t s, int sm_count, uint64_t* launches);
 // Which resample kernel family runs (PXZ_RESAMPLE_KERNELS=warp|cta|tma).  Auto: by tile count; Warp: warp-per-tile kernels
 // with the cp.async ring shrink kernel; Cta: CTA-per-tile kernels; Tma: warp-per-tile kernels with the TMA shrink kernel.
 // The forced warp families still need the RGBA fast geometry and tables that have the warp forms.
