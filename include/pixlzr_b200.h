@@ -253,6 +253,40 @@ pxz_status pxz_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, 
                                pxz_filter filter_down, pxz_filter filter_up, uint32_t flags, float* factor_out, uint64_t* sse_out,
                                pxz_payload** out);
 
+/* EXTENSION (rate-distortion optimised encode).  A decoder takes each block's dims from its QOI header, so an encoder may give
+ * every block any size.  A block's candidates are the dims scaled_dim(tw, lx) x scaled_dim(th, ly) of every level pair
+ * 0 <= lx <= ceil(log2 bw), 0 <= ly <= ceil(log2 bh), priced at bytes = w' * h' * (channels; 3 for RGB) and sse = the error of
+ * that block's decode (filter_down, then filter_up).  Every payload pxz_shrink gives (any metric, factor, flags) is one choice
+ * among them.  The curve: point 0 has every block at 1 x 1; each next point takes the next segment, by falling rate
+ * (error removed per byte added, compared exactly), of the blocks' lower convex hulls.  bytes strictly increases, sse strictly
+ * decreases, the last point has sse 0, and no choice of sizes has at most a point's bytes and less error than it.
+ * n <= 1 + blocks * ((1 + ceil(log2 bw)) * (1 + ceil(log2 bh)) - 1).  *n_out is always set; cap < n -> PXZ_E_ARG (message names
+ * n), nothing written.  sse is exact in the default resample arithmetic (both resize semantics); with
+ * pxz_ctx_set_fast_resample(1) it is not claimed.  One plan + resample + expand + error pass per level pair (49 at 64x64), then
+ * per block its hull, one merge sort and one scan (DESIGN.md §3 "Per-block sizes").  Device scratch: passes x blocks x 8 bytes
+ * for the error table plus about 100 bytes per possible event.  The host arrays may be NULL when cap = 0.  Synchronises the
+ * stream.
+ * PXZ_E_ARG: an unknown filter, a block size of 0.
+ * PXZ_E_UNSUPPORTED: a batch image, a strategy installed on the context (its filter pair follows the stored value), more than
+ *                    2^31 events. */
+pxz_status pxz_rdo_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_filter filter_down, pxz_filter filter_up,
+                         uint64_t* host_bytes, uint64_t* host_sse, size_t cap, size_t* n_out);
+
+/* EXTENSION (rate-distortion optimised encode).  The payload of one point of pxz_rdo_curve: to size, the last point with
+ * bytes <= max_bytes (the least error within the budget); to error, the first point with sse <= max_sse (the fewest bytes
+ * within the budget).  Each block is encoded at its vertex's smallest level pair (lx, ly) with the stored value
+ * hypot(2^-lx, 2^-ly) (= pxz_reduce_dims(2^-lx, 2^-ly, tw, th)), so every reader of the format decodes it.  *bytes_out /
+ * *sse_out (each may be NULL) = the point's bytes and sse, which the payload's pxz_payload_info bytes and its decode with
+ * filter_up (pxz_image_error) equal in the default resample arithmetic.  Against pxz_shrink_to_error with the same filter pair
+ * (payload B_A bytes): the first curve point with bytes >= B_A is within max_sse, so pxz_rdo_shrink_to_error's payload is at most
+ * one hull segment larger than B_A.  Synchronises the stream.
+ * PXZ_E_ARG: as pxz_rdo_curve; max_bytes below the payload with every block at 1 x 1 (the message names that size).
+ * PXZ_E_UNSUPPORTED: as pxz_rdo_curve. */
+pxz_status pxz_rdo_shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, uint64_t max_bytes, pxz_filter filter_down,
+                                  pxz_filter filter_up, uint64_t* bytes_out, uint64_t* sse_out, pxz_payload** out);
+pxz_status pxz_rdo_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, uint64_t max_sse, pxz_filter filter_down,
+                                   pxz_filter filter_up, uint64_t* bytes_out, uint64_t* sse_out, pxz_payload** out);
+
 /* Scalar part of reduce_image_section (operations.rs:128-156) on the host: (v0, v1) after `after`
  * -> parse_value -> level -> reduced size of a w x h block and the stored block value.  Uses the
  * same threshold table as the device plan kernel. */

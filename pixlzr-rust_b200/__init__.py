@@ -10,6 +10,7 @@ Layout
 from .api import (  # noqa: F401
     ErrorReport,
     FilterType,
+    OptimalCurve,
     Pixlzr,
     PixlzrBlock,
     RateDistortion,
@@ -25,6 +26,7 @@ from .api import (  # noqa: F401
     process_custom,
     psnr_of,
     rd_curve,
+    rdo_curve,
     reduce_image_section,
     sse_budget,
     tree_process,

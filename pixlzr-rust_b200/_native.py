@@ -92,6 +92,9 @@ SYMBOLS = {
     "pxz_strategy_choose": (_i, [_vp, _vp, _vp, _vp]),
     "pxz_rd_curve": (_i, [_vp, _vp, _u32, _u32, _i, _i, _i, _u32, _vp, _vp, _vp, _sz, _P(_sz)]),
     "pxz_shrink_to_error": (_i, [_vp, _vp, _u32, _u32, _i, _u64, _i, _i, _u32, _P(C.c_float), _P(_u64), _P(_vp)]),
+    "pxz_rdo_curve": (_i, [_vp, _vp, _u32, _u32, _i, _i, _vp, _vp, _sz, _P(_sz)]),
+    "pxz_rdo_shrink_to_size": (_i, [_vp, _vp, _u32, _u32, _u64, _i, _i, _P(_u64), _P(_u64), _P(_vp)]),
+    "pxz_rdo_shrink_to_error": (_i, [_vp, _vp, _u32, _u32, _u64, _i, _i, _P(_u64), _P(_u64), _P(_vp)]),
 }
 
 
@@ -427,6 +430,33 @@ class Image:
                                                  flags, C.byref(k), C.byref(sse), C.byref(h)))
         return Payload(self.ctx, h), float(k.value), int(sse.value)
 
+    def rdo_curve(self, bw: int, bh: int, filter_down: int, filter_up: int):
+        """(bytes uint64 [n], sse uint64 [n]): the rate-distortion optimised curve of this image, every block free to take the
+        dims of any level pair, decoded with filter_up (pxz_rdo_curve)."""
+        cap = rdo_curve_bound(self.w, self.h, bw, bh)
+        nbytes = np.empty(cap, np.uint64)
+        sse = np.empty(cap, np.uint64)
+        n = C.c_size_t()
+        self.ctx.check(lib().pxz_rdo_curve(self.ctx.handle, self._h, bw, bh, int(filter_down), int(filter_up), ptr(nbytes), ptr(sse), cap,
+                                           C.byref(n)))
+        return nbytes[:n.value].copy(), sse[:n.value].copy()
+
+    def rdo_shrink_to_size(self, bw: int, bh: int, max_bytes: int, filter_down: int, filter_up: int):
+        """(Payload, bytes, sse): the payload of the last optimised curve point with at most `max_bytes` payload bytes, its bytes
+        and the squared error of its decode with filter_up (pxz_rdo_shrink_to_size)."""
+        h, nbytes, sse = C.c_void_p(), C.c_uint64(), C.c_uint64()
+        self.ctx.check(lib().pxz_rdo_shrink_to_size(self.ctx.handle, self._h, bw, bh, int(max_bytes), int(filter_down), int(filter_up),
+                                                    C.byref(nbytes), C.byref(sse), C.byref(h)))
+        return Payload(self.ctx, h), int(nbytes.value), int(sse.value)
+
+    def rdo_shrink_to_error(self, bw: int, bh: int, max_sse: int, filter_down: int, filter_up: int):
+        """(Payload, bytes, sse): the payload of the first optimised curve point whose decode with filter_up has a squared
+        error of at most `max_sse`, its bytes and that error (pxz_rdo_shrink_to_error)."""
+        h, nbytes, sse = C.c_void_p(), C.c_uint64(), C.c_uint64()
+        self.ctx.check(lib().pxz_rdo_shrink_to_error(self.ctx.handle, self._h, bw, bh, int(max_sse), int(filter_down), int(filter_up),
+                                                     C.byref(nbytes), C.byref(sse), C.byref(h)))
+        return Payload(self.ctx, h), int(nbytes.value), int(sse.value)
+
     def tree_process(self, threshold: float, bw: int, bh: int, min_bw: int, min_bh: int, filter_down: int, filter_up: int,
                      out: "Image"):
         self.ctx.check(lib().pxz_tree_process(self.ctx.handle, self._h, threshold, bw, bh, min_bw, min_bh, int(filter_down),
@@ -566,6 +596,15 @@ def rd_curve_bound(w: int, h: int, bw: int, bh: int, metric: int) -> int:
     lx, ly = (bw - 1).bit_length(), (bh - 1).bit_length()
     steps = lx + ly if metric == METRIC_SOBEL_DIR else max(lx, ly)
     return 1 + -(-w // bw) * -(-h // bh) * steps
+
+
+def rdo_curve_bound(w: int, h: int, bw: int, bh: int) -> int:
+    """Most points pxz_rdo_curve can return: 1 + blocks * ((1 + ceil(log2 bw)) * (1 + ceil(log2 bh)) - 1) (a block has at most
+    one hull segment per candidate size after its first)."""
+    if w <= 0 or h <= 0 or bw <= 0 or bh <= 0:
+        raise ValueError("image and block sizes must be positive")
+    lx, ly = (bw - 1).bit_length(), (bh - 1).bit_length()
+    return 1 + -(-w // bw) * -(-h // bh) * ((1 + lx) * (1 + ly) - 1)
 
 
 def reduce_dims(v0: float, v1: float, w: int, h: int):

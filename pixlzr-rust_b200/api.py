@@ -243,6 +243,45 @@ def rd_curve(image, block_width: int, block_height: int, filter_down: FilterType
 
 
 @dataclass
+class OptimalCurve:
+    """EXTENSION (pxz_rdo_curve): the rate-distortion optimised curve, every block free to take the dims of any level pair.
+    Point 0 has every block at 1 x 1; bytes strictly increases, sse strictly decreases and the last point has sse 0.  No choice of
+    block sizes has at most bytes[i] payload bytes and less error than sse[i]."""
+    bytes: np.ndarray   # uint64 [n]
+    sse: np.ndarray     # uint64 [n]
+    samples: int        # width * height * channels of the source
+
+    @property
+    def psnr(self) -> np.ndarray:
+        return np.array([psnr_of(int(e), self.samples) for e in self.sse], np.float64)
+
+    def best_within(self, max_bytes: int) -> Optional[int]:
+        """Index of the least error within `max_bytes` payload bytes (the point pxz_rdo_shrink_to_size picks), None if even
+        point 0 is larger."""
+        ok = np.nonzero(self.bytes <= np.uint64(max_bytes))[0]
+        return int(ok[-1]) if ok.size else None
+
+    def smallest_within(self, max_sse: int) -> Optional[int]:
+        """Index of the fewest bytes whose error is at most `max_sse` (the point pxz_rdo_shrink_to_error picks)."""
+        ok = np.nonzero(self.sse <= np.uint64(max_sse))[0]
+        return int(ok[0]) if ok.size else None
+
+
+def rdo_curve(image, block_width: int, block_height: int, filter_down: FilterType, filter_up: FilterType,
+              ctx: Optional[N.Context] = None) -> OptimalCurve:
+    """EXTENSION: the rate-distortion optimised (bytes, squared error) curve of an image when each block's size is chosen on its
+    own, shrunk with `filter_down` and decoded with `filter_up`, computed on the device (numpy or device image)."""
+    ctx = ctx or (image.ctx if isinstance(image, N.Image) else default_context())
+    img = image if isinstance(image, N.Image) else ctx.image_upload(_check_image(image))
+    try:
+        nbytes, sse = img.rdo_curve(block_width, block_height, int(filter_down), int(filter_up))
+        return OptimalCurve(nbytes, sse, img.w * img.h * img.c)
+    finally:
+        if img is not image:
+            img.free()
+
+
+@dataclass
 class ErrorReport:
     """EXTENSION: the error of one image against another, per block of a grid (pxz_image_error)."""
     block_sse: np.ndarray  # uint64 [rows, cols]: sum of (a - b)^2 over the tile's pixels and channels
@@ -504,6 +543,37 @@ class Pixlzr:
         self._values_present = True
         self._image = None
         return k
+
+    def shrink_optimally_to_size(self, filter_downscale: FilterType, filter_upscale: FilterType, max_bytes: int) -> Tuple[int, int]:
+        """EXTENSION (optimised encode): each block at its own size, the least error of a decode with `filter_upscale` within
+        `max_bytes` payload bytes (pxz_rdo_shrink_to_size); returns (payload bytes, squared error).  Needs the source image:
+        refused on a decoded or already shrunk Pixlzr."""
+        return self._shrink_optimally("shrink_optimally_to_size", "rdo_shrink_to_size", filter_downscale, filter_upscale,
+                                      lambda img: max_bytes)
+
+    def shrink_optimally_to_psnr(self, filter_downscale: FilterType, filter_upscale: FilterType, psnr: float) -> Tuple[int, int]:
+        """EXTENSION (optimised encode): each block at its own size, the fewest payload bytes whose decode with `filter_upscale`
+        reaches `psnr` dB against the source (sse_budget; pxz_rdo_shrink_to_error); returns (payload bytes, squared error).
+        Needs the source image: refused on a decoded or already shrunk Pixlzr."""
+        return self._shrink_optimally("shrink_optimally_to_psnr", "rdo_shrink_to_error", filter_downscale, filter_upscale,
+                                      lambda img: sse_budget(psnr, img.w * img.h * img.c))
+
+    def _shrink_optimally(self, name: str, call: str, filter_downscale: FilterType, filter_upscale: FilterType, budget) -> Tuple[int, int]:
+        if self._image is None:
+            raise ValueError(f"{name} needs the source image (Pixlzr.from_image), not a decoded or already shrunk one")
+        ctx = self._ctx()
+        img = ctx.image_upload(self._image)
+        try:
+            pl, nbytes, sse = getattr(img, call)(self.block_width, self.block_height, budget(img), int(filter_downscale), int(filter_upscale))
+            try:
+                self._descs, self._pixels = pl.download()
+            finally:
+                pl.free()
+        finally:
+            img.free()
+        self._values_present = True
+        self._image = None
+        return nbytes, sse
 
     def shrink_directionally(self, filter_downscale: FilterType, factor: float):
         """Pixlzr::shrink_directionally (pixlzr.rs:187-205)."""

@@ -47,6 +47,11 @@ def build_parser() -> argparse.ArgumentParser:
     p.add_argument("--target-psnr", type=parse_target_psnr, default=None, metavar="DB",
                    help="Shrink with the smallest factor whose decode (with -f) reaches DB dB PSNR against the input, and print "
                         "that factor, the payload bytes and the PSNR reached (image input, with --force; replaces -k)")
+    # extension (optimised encode): not a flag of the reference
+    p.add_argument("--optimal", action="store_true",
+                   help="With --payload-bytes N or --target-psnr DB: choose every block's size on its own rather than one factor "
+                        "for all (the least error within N bytes, or the fewest bytes reaching DB dB, decoded with -f), and print "
+                        "the payload bytes and the PSNR reached (no -d: no metric is used)")
     # extension (decode error): not a flag of the reference
     p.add_argument("--psnr", action="store_true",
                    help="Decode what was written (with -f), compare it with the input image on the device and print the PSNR "
@@ -125,6 +130,17 @@ def target_psnr_error(args) -> Optional[str]:
     return None
 
 
+def optimal_error(args) -> Optional[str]:
+    """Why --optimal does not apply to these arguments, or None."""
+    if not getattr(args, "optimal", False):
+        return None
+    if args.payload_bytes is None and args.target_psnr is None:
+        return "--optimal chooses every block's size for a budget: it needs --payload-bytes or --target-psnr"
+    if args.direction_wise is not None:
+        return "--optimal uses no metric: it cannot be combined with -d"
+    return None
+
+
 def psnr_error(args) -> Optional[str]:
     """Why --psnr does not apply to these arguments, or None."""
     if getattr(args, "psnr", False) and operation(args.input, args.output)[0] != "image":
@@ -190,9 +206,12 @@ def run(args) -> None:
     filt = FILTERS[args.filter]
     shrink_by = api.parse_shrinking_factor(args.shrinking_factor)
     src, dst = operation(args.input, args.output)
-    err = region_error(args) or payload_bytes_error(args) or target_psnr_error(args) or psnr_error(args)
+    err = region_error(args) or payload_bytes_error(args) or target_psnr_error(args) or optimal_error(args) or psnr_error(args)
     if err:
         raise ValueError(err)
+    if args.optimal:
+        _run_optimal(args, bw, bh, filt, dst)
+        return
     if args.target_psnr is not None:
         _run_psnr_target(args, bw, bh, filt, dst)
         return
@@ -270,6 +289,32 @@ def _run_psnr_target(args, bw: int, bh: int, filt, dst: str) -> None:
     print(f"psnr: {format_psnr(api.psnr_of(sse, samples))} dB")
 
 
+def _run_optimal(args, bw: int, bh: int, filt, dst: str) -> None:
+    """image -> container / image with every block's size chosen for --payload-bytes (the least error of a decode with -f
+    within N bytes) or --target-psnr (the fewest bytes reaching it); prints the payload bytes and the PSNR reached."""
+    image = _open_image(args.input)
+    ctx = api.default_context()
+    img = ctx.image_upload(image)
+    try:
+        samples = img.w * img.h * img.c
+        if args.payload_bytes is not None:
+            pl, nbytes, sse = img.rdo_shrink_to_size(bw, bh, args.payload_bytes, int(filt), int(filt))
+        else:
+            pl, nbytes, sse = img.rdo_shrink_to_error(bw, bh, api.sse_budget(args.target_psnr, samples), int(filt), int(filt))
+    finally:
+        img.free()
+    try:
+        if dst == "pix":
+            with open(args.output, "wb") as f:
+                f.write(pl.to_container(0, True))
+        else:
+            _save_image(args.output, pl.expand(int(filt)))
+    finally:
+        pl.free()
+    print(f"payload bytes: {nbytes}")
+    print(f"psnr: {format_psnr(api.psnr_of(sse, samples))} dB")
+
+
 def format_psnr(psnr: float) -> str:
     return "inf" if psnr == float("inf") else f"{psnr:.6f}"
 
@@ -294,7 +339,7 @@ def report_psnr(args) -> None:
 
 def main(argv: Optional[List[str]] = None) -> int:
     args = parse_args(argv)
-    err = region_error(args) or payload_bytes_error(args) or target_psnr_error(args) or psnr_error(args)
+    err = region_error(args) or payload_bytes_error(args) or target_psnr_error(args) or optimal_error(args) or psnr_error(args)
     if err:
         print(f"pixlzr: {err}", file=sys.stderr)
         return 2

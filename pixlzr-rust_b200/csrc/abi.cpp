@@ -47,12 +47,13 @@ using TabKey = std::tuple<std::vector<uint32_t>, std::vector<uint32_t>, int, int
 
 // K_REGION_COPY times the device-to-device copy of pxz_expand_region out of its staging image (not a kernel)
 enum KernelId { K_MAD_FAST = 0, K_MAD_EXACT, K_SOBEL, K_MINMAX, K_PLAN, K_RESAMPLE_DOWN, K_RESAMPLE_UP, K_QOI_ENCODE, K_QOI_DECODE,
-                K_PAYLOAD_WINDOW, K_REGION_COPY, K_SIZE_CURVE, K_BLOCK_ERROR, K_BUCKET_SUM, K_RD_LEVELS, K_RD_EVENTS, K_RD_CURVE, K_COUNT };
+                K_PAYLOAD_WINDOW, K_REGION_COPY, K_SIZE_CURVE, K_BLOCK_ERROR, K_BUCKET_SUM, K_RD_LEVELS, K_RD_EVENTS, K_RD_CURVE,
+                K_RDO_HULL, K_RDO_CURVE, K_RDO_LEVELS, K_COUNT };
 const char* const kKernelNames[K_COUNT] = {"analyze_mad_fast", "mad_exact",      "analyze_sobel", "minmax",
                                            "plan",             "resample_down",  "resample_up",   "qoi_encode",
                                            "qoi_decode",       "payload_window", "region_copy",   "size_curve",
                                            "block_error",      "bucket_sum",     "rd_levels",     "rd_events",
-                                           "rd_curve"};
+                                           "rd_curve",         "rdo_hull",       "rdo_curve",     "rdo_levels"};
 struct ProfRec {
   int id;
   cudaEvent_t a, b;
@@ -1398,6 +1399,39 @@ struct RdSummary {
 
 static uint32_t ceil_log2(uint32_t n) { return n <= 1 ? 0u : 32u - (uint32_t)__builtin_clz(n - 1); }
 
+// The error table of the rate-distortion curves: per level pair (lx, ly) the plan + resample of pxz_shrink with every block
+// forced to it — values 2^-lx / 2^-ly under the directional map at factor 1, no normalisation — then the decode with filter_up
+// and its per-block error into table + pass * nblocks, pass = lx * ps.stride_x + ly * ps.stride_y.  diagonal: the pairs (l, l)
+// for l <= lx_max, else every pair up to (lx_max, ly_max).  Overwrites ctx->d_vx / d_vy.
+static pxz_status rd_error_table(pxz_ctx* ctx, const pxz_image* img, const Geom& g, pxz_filter filter_down, pxz_filter filter_up, bool diagonal,
+                                 uint32_t lx_max, uint32_t ly_max, const RdPasses& ps, uint64_t* table) {
+  const size_t nblocks = (size_t)g.cols * g.rows;
+  ImageOwner dec;
+  pxz_status st = image_new(ctx, img->w, img->h, img->c, 1, &dec);
+  if (st != PXZ_OK) return st;
+  const ValueMap forced = shrink_value_map(ctx, PXZ_METRIC_SOBEL_DIR, 0, 1.0f);
+  for (uint32_t lx = 0; lx <= lx_max; ++lx) {
+    for (uint32_t ly = diagonal ? lx : 0; ly <= (diagonal ? lx : ly_max); ++ly) {
+      const float fx = ldexpf(1.0f, -(int)lx), fy = ldexpf(1.0f, -(int)ly);
+      uint32_t w = 0, h = 0;  // level_k(2^-l) = l: the plan sees exactly these levels
+      pxz_reduce_dims(fx, fy, g.bw, g.bh, &w, &h, nullptr);
+      if (w != std::max(1u, ceil_div_u32(g.bw, 1u << lx)) || h != std::max(1u, ceil_div_u32(g.bh, 1u << ly)))
+        return fail(ctx, PXZ_E_CUDA, "level table does not map 2^-l to level l");
+      st = profiled(ctx, K_RD_LEVELS, "rd levels", [&] {
+        return launch_rd_levels(ctx->d_vx, ctx->d_vy, (uint32_t)nblocks, fx, fy, ctx->stream, ctx->sm_count, &ctx->launches);
+      });
+      if (st != PXZ_OK) return st;
+      pxz_payload* raw = nullptr;
+      if ((st = plan_and_resample(ctx, img, g, PXZ_METRIC_SOBEL_DIR, forced, filter_down, true, &raw)) != PXZ_OK) return st;
+      const PayloadOwner p(raw);
+      if ((st = pxz_expand_to_image(ctx, p.get(), filter_up, dec.get())) != PXZ_OK) return st;
+      const uint32_t pass = lx * ps.stride_x + ly * ps.stride_y;
+      if ((st = run_block_error(ctx, img, dec.get(), g, table + (size_t)pass * nblocks, nullptr)) != PXZ_OK) return st;
+    }
+  }
+  return PXZ_OK;
+}
+
 // The curve of pxz_rd_curve after the checks (DESIGN.md §3).  bpp: bytes per pixel counted (3 for an RGB image on the RGBA
 // kernels).  The points are copied to the host arrays when cap >= n.
 static pxz_status rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, pxz_filter filter_down,
@@ -1452,30 +1486,9 @@ static pxz_status rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint
   PXZ_CUDA(ctx, cudaMemcpyAsync(vals, ctx->d_vx, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
   if (sobel) PXZ_CUDA(ctx, cudaMemcpyAsync(vals + nblocks, ctx->d_vy, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
 
-  // 2. error table: per pass the plan + resample of pxz_shrink with every block forced to (lx, ly) — values 2^-lx / 2^-ly under
-  // the directional map at factor 1, no normalisation — then the decode and its per-block error
-  ImageOwner dec;
-  if ((st = image_new(ctx, img->w, img->h, img->c, 1, &dec)) != PXZ_OK) return st;
-  const ValueMap forced = shrink_value_map(ctx, PXZ_METRIC_SOBEL_DIR, 0, 1.0f);
-  for (uint32_t lx = 0; lx <= (sobel ? lx_max : l_max); ++lx) {
-    for (uint32_t ly = sobel ? 0 : lx; ly <= (sobel ? ly_max : lx); ++ly) {
-      const float fx = ldexpf(1.0f, -(int)lx), fy = ldexpf(1.0f, -(int)ly);
-      uint32_t w = 0, h = 0;  // level_k(2^-l) = l: the plan sees exactly these levels
-      pxz_reduce_dims(fx, fy, bw, bh, &w, &h, nullptr);
-      if (w != std::max(1u, ceil_div_u32(bw, 1u << lx)) || h != std::max(1u, ceil_div_u32(bh, 1u << ly)))
-        return fail(ctx, PXZ_E_CUDA, "level table does not map 2^-l to level l");
-      st = profiled(ctx, K_RD_LEVELS, "rd levels", [&] {
-        return launch_rd_levels(ctx->d_vx, ctx->d_vy, (uint32_t)nblocks, fx, fy, ctx->stream, ctx->sm_count, &ctx->launches);
-      });
-      if (st != PXZ_OK) return st;
-      pxz_payload* raw = nullptr;
-      if ((st = plan_and_resample(ctx, img, g, PXZ_METRIC_SOBEL_DIR, forced, filter_down, true, &raw)) != PXZ_OK) return st;
-      const PayloadOwner p(raw);
-      if ((st = pxz_expand_to_image(ctx, p.get(), filter_up, dec.get())) != PXZ_OK) return st;
-      const uint32_t pass = lx * ps.stride_x + ly * ps.stride_y;
-      if ((st = run_block_error(ctx, img, dec.get(), g, table + (size_t)pass * nblocks, nullptr)) != PXZ_OK) return st;
-    }
-  }
+  // 2. error table
+  if ((st = rd_error_table(ctx, img, g, filter_down, filter_up, !sobel, sobel ? lx_max : l_max, sobel ? ly_max : l_max, ps, table)) != PXZ_OK)
+    return st;
 
   // 3. events of every block, 4. the curve
   const ValueMap vm = shrink_value_map(ctx, metric, flags & PXZ_FLAG_NORMALISE_GLOBAL, 1.0f);
@@ -1548,6 +1561,182 @@ pxz_status pxz_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, 
   if (factor_out) *factor_out = k;
   if (sse_out) *sse_out = sum.first_sse;
   return PXZ_OK;
+}
+
+// ---- rate-distortion optimised encode (extension) ----------------------------------------------------------------
+// No metric, flags or factor: every block takes the dims of any level pair (DESIGN.md §3 "Per-block sizes")
+static pxz_status rdo_refusal(pxz_ctx* ctx, const pxz_image* img, pxz_filter filter_down, pxz_filter filter_up) {
+  if (!known_filter(filter_down) || !known_filter(filter_up)) return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "an optimised encode is per image: not available on a batch");
+  if (ctx->strategy.on)
+    return fail(ctx, PXZ_E_UNSUPPORTED, "an optimised encode with a strategy installed is not available (its filter pair follows the stored value)");
+  return PXZ_OK;
+}
+
+// Most events a block can have: its distinct byte counts over every level pair, less one, over the (up to four) tile shapes
+static uint32_t rdo_max_events(const Geom& g) {
+  const uint32_t lx_max = ceil_log2(g.bw), ly_max = ceil_log2(g.bh);
+  uint32_t most = 0;
+  for (uint32_t tw : {g.bw, g.trail_w ? g.trail_w : g.bw}) {
+    for (uint32_t th : {g.bh, g.trail_h ? g.trail_h : g.bh}) {
+      std::vector<uint64_t> sizes;
+      for (uint32_t lx = 0; lx <= lx_max; ++lx)
+        for (uint32_t ly = 0; ly <= ly_max; ++ly)
+          sizes.push_back((uint64_t)std::max(1u, ceil_div_u32(tw, 1u << lx)) * std::max(1u, ceil_div_u32(th, 1u << ly)));
+      std::sort(sizes.begin(), sizes.end());
+      most = std::max(most, (uint32_t)(std::unique(sizes.begin(), sizes.end()) - sizes.begin()) - 1);
+    }
+  }
+  return most;
+}
+
+enum class RdoPick { None, Size, Error };
+
+// What one optimised curve returns to the host besides the points
+struct RdoSummary {
+  uint32_t n = 0;       // curve points
+  uint64_t bytes0 = 0;  // payload bytes with every block at 1 x 1 (point 0)
+  uint64_t bytes = 0;   // the chosen point's bytes and sse
+  uint64_t sse = 0;
+};
+
+// The optimised curve after the checks, and with pick != None the payload of the point a budget picks (to size: the last with
+// bytes <= budget; to error: the first with sse <= budget) into *out.  bpp: bytes per pixel counted (3 for an RGB image on the
+// RGBA kernels).  The points are copied to the host arrays when cap >= n.
+static pxz_status rdo(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_filter filter_down, pxz_filter filter_up, uint32_t bpp,
+                      RdoPick pick, uint64_t budget, uint64_t* host_bytes, uint64_t* host_sse, size_t cap, RdoSummary* sum, pxz_payload** out) {
+  // An RGB image that pxz_shrink runs on the RGBA kernels is measured and encoded as its RGBA widening (alpha is 255 in the
+  // source and every decode and adds 0); the payload is narrowed back as pxz_shrink narrows it
+  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
+    auto wide_rdo = [&](const pxz_image* wide, pxz_payload** p4) {
+      return rdo(ctx, wide, bw, bh, filter_down, filter_up, 3, pick, budget, host_bytes, host_sse, cap, sum, p4);
+    };
+    if (pick != RdoPick::None) return encode_via_rgba(ctx, img, wide_rdo, out);
+    ImageOwner wide;
+    pxz_status st = rgb_widened(ctx, img, &wide);
+    return st != PXZ_OK ? st : wide_rdo(wide.get(), nullptr);
+  }
+  Geom g;
+  pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g);
+  if (st != PXZ_OK) return st;
+  const uint32_t nblocks = g.cols * g.rows;
+  const uint32_t lx_max = ceil_log2(bw), ly_max = ceil_log2(bh);
+  const uint32_t npass = (lx_max + 1) * (ly_max + 1);
+  const uint32_t maxev = rdo_max_events(g);
+  const uint64_t nev64 = (uint64_t)nblocks * maxev;
+  if (nev64 > 0x7FFFFFFFull) return fail(ctx, PXZ_E_UNSUPPORTED, "more than 2^31 optimised curve events (blocks x sizes)");
+  const uint32_t nev = (uint32_t)nev64;
+  if ((st = ensure_scratch(ctx, nblocks)) != PXZ_OK) return st;
+
+  DevBlocks bufs(ctx);
+  uint64_t* table = nullptr;  // [npass][nblocks] block errors
+  uint8_t* ev = nullptr;      // events | base[3] | points: bytes | sse | ids | ev_pass | rank | pass0 | RdoOut
+  void* scratch = nullptr;
+  const size_t scratch_bytes = rdo_curve_scratch_bytes(nev);
+  const size_t npt = (size_t)nev + 1;
+  const size_t ev_bytes = (size_t)nev * (sizeof(RdoEvent) + 12) + 24 + npt * 16 + (size_t)nblocks * 4 + sizeof(RdoOut);
+  if ((st = bufs.alloc(&table, (size_t)npass * nblocks * 8)) != PXZ_OK || (st = bufs.alloc(&ev, ev_bytes)) != PXZ_OK ||
+      (st = bufs.alloc(&scratch, scratch_bytes)) != PXZ_OK)
+    return st;
+  RdoEvent* events = reinterpret_cast<RdoEvent*>(ev);
+  uint64_t* base = reinterpret_cast<uint64_t*>(events + nev);
+  uint64_t* pt_bytes = base + 3;
+  uint64_t* pt_sse = pt_bytes + npt;
+  uint32_t* ids = reinterpret_cast<uint32_t*>(pt_sse + npt);
+  uint32_t* ev_pass = ids + nev;
+  uint32_t* rank = ev_pass + nev;
+  uint32_t* pass0 = rank + nev;
+  RdoOut* d_out = reinterpret_cast<RdoOut*>(pass0 + nblocks);
+
+  // 1. error table over every level pair, 2. per-block hulls, 3. the curve
+  const RdPasses ps{lx_max, ly_max, ly_max + 1, 1};
+  if ((st = rd_error_table(ctx, img, g, filter_down, filter_up, false, lx_max, ly_max, ps, table)) != PXZ_OK) return st;
+  PXZ_CUDA(ctx, cudaMemsetAsync(base, 0, 3 * sizeof(uint64_t), ctx->stream));
+  st = profiled(ctx, K_RDO_HULL, "rdo hull", [&] {
+    return launch_rdo_hull(table, g, bpp, lx_max, ly_max, maxev, events, ids, ev_pass, pass0, base, ctx->stream, &ctx->launches);
+  });
+  if (st != PXZ_OK) return st;
+  st = profiled(ctx, K_RDO_CURVE, "rdo curve", [&] {
+    return launch_rdo_curve(events, ids, nev, base, pick == RdoPick::Size ? budget : 0, pick == RdoPick::Error ? budget : 0, scratch, scratch_bytes,
+                            rank, pt_bytes, pt_sse, d_out, ctx->stream, ctx->sm_count, &ctx->launches);
+  });
+  if (st != PXZ_OK) return st;
+
+  // 4. to the host: the summary, the chosen point, and the points when they fit
+  RdoOut o;
+  PXZ_CUDA(ctx, cudaMemcpyAsync(&o, d_out, sizeof(o), cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->bytes0, pt_bytes, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  sum->n = o.count;
+  if (cap >= o.count && host_bytes && host_sse) {
+    PXZ_CUDA(ctx, cudaMemcpyAsync(host_bytes, pt_bytes, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, pt_sse, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  }
+  if (pick == RdoPick::None) return PXZ_OK;
+  const uint32_t j = pick == RdoPick::Size ? o.best_within - 1 : o.first_within;
+  if (pick == RdoPick::Size && o.best_within == 0)
+    return fail(ctx, PXZ_E_ARG, "max_bytes " + std::to_string(budget) + " is below the payload with every block at 1 x 1 (" +
+                                    std::to_string(sum->bytes0) + " bytes)");
+  if (j >= o.count) {  // the last point has sse 0 in the default resample arithmetic; with the fused one it may not
+    uint64_t least = 0;
+    PXZ_CUDA(ctx, cudaMemcpyAsync(&least, pt_sse + o.count - 1, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+    return fail(ctx, PXZ_E_ARG, "max_sse " + std::to_string(budget) + " is below the least squared error of any point (" + std::to_string(least) + ")");
+  }
+
+  // 5. the payload: every block forced to its vertex at point j, planned and resampled as the error table's passes are
+  st = profiled(ctx, K_RDO_LEVELS, "rdo levels", [&] {
+    return launch_rdo_levels(pass0, ev_pass, rank, maxev, nblocks, ly_max, j, ctx->d_vx, ctx->d_vy, ctx->stream, ctx->sm_count, &ctx->launches);
+  });
+  if (st != PXZ_OK) return st;
+  if ((st = plan_and_resample(ctx, img, g, PXZ_METRIC_SOBEL_DIR, shrink_value_map(ctx, PXZ_METRIC_SOBEL_DIR, 0, 1.0f), filter_down, true, out)) !=
+      PXZ_OK)
+    return st;
+  PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->bytes, pt_bytes + j, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->sse, pt_sse + j, 8, cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return PXZ_OK;
+}
+
+pxz_status pxz_rdo_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_filter filter_down, pxz_filter filter_up,
+                         uint64_t* host_bytes, uint64_t* host_sse, size_t cap, size_t* n_out) {
+  if (n_out) *n_out = 0;
+  if (!ctx || !img || !n_out || (cap > 0 && (!host_bytes || !host_sse))) return PXZ_E_ARG;
+  cudaSetDevice(ctx->device);
+  pxz_status st = rdo_refusal(ctx, img, filter_down, filter_up);
+  if (st != PXZ_OK) return st;
+  RdoSummary sum;
+  st = rdo(ctx, img, bw, bh, filter_down, filter_up, img->c, RdoPick::None, 0, host_bytes, host_sse, cap, &sum, nullptr);
+  if (st != PXZ_OK) return st;
+  *n_out = sum.n;
+  if (cap < sum.n) return fail(ctx, PXZ_E_ARG, "cap " + std::to_string(cap) + " is below the curve's " + std::to_string(sum.n) + " points");
+  return PXZ_OK;
+}
+
+static pxz_status rdo_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, RdoPick pick, uint64_t budget, pxz_filter filter_down,
+                             pxz_filter filter_up, uint64_t* bytes_out, uint64_t* sse_out, pxz_payload** out) {
+  if (!ctx || !img || !out) return PXZ_E_ARG;
+  *out = nullptr;
+  cudaSetDevice(ctx->device);
+  pxz_status st = rdo_refusal(ctx, img, filter_down, filter_up);
+  if (st != PXZ_OK) return st;
+  RdoSummary sum;
+  st = rdo(ctx, img, bw, bh, filter_down, filter_up, img->c, pick, budget, nullptr, nullptr, 0, &sum, out);
+  if (st != PXZ_OK) return st;
+  if (bytes_out) *bytes_out = sum.bytes;
+  if (sse_out) *sse_out = sum.sse;
+  return PXZ_OK;
+}
+
+pxz_status pxz_rdo_shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, uint64_t max_bytes, pxz_filter filter_down,
+                                  pxz_filter filter_up, uint64_t* bytes_out, uint64_t* sse_out, pxz_payload** out) {
+  return rdo_shrink(ctx, img, bw, bh, RdoPick::Size, max_bytes, filter_down, filter_up, bytes_out, sse_out, out);
+}
+
+pxz_status pxz_rdo_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, uint64_t max_sse, pxz_filter filter_down,
+                                   pxz_filter filter_up, uint64_t* bytes_out, uint64_t* sse_out, pxz_payload** out) {
+  return rdo_shrink(ctx, img, bw, bh, RdoPick::Error, max_sse, filter_down, filter_up, bytes_out, sse_out, out);
 }
 
 pxz_status pxz_strategy_choose(const uint64_t* sse, const uint32_t* blocks, const pxz_strategy* base, pxz_strategy* out) {

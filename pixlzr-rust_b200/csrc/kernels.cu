@@ -15,6 +15,9 @@
 //   k_rd_levels          forced levels of one error pass of the rate-distortion curve
 //   k_rd_events          per block, the factors at which its dims change and what that changes (rate-distortion curve)
 //   k_rd_gather / k_rd_compact   sorted events -> scan input -> curve points (around CUB's radix sort and scan)
+//   k_rdo_hull           per block, the lower convex hull of its (bytes, error) over every level pair (optimised encode)
+//   k_rdo_gather / k_rdo_points  events sorted by rate -> scan input -> curve points (around CUB's merge sort and scan)
+//   k_rdo_levels         per block, the levels of one point of the optimised curve
 //
 // Nothing here is a dense contraction, so no tensor cores: the kernels are HBM / FP32-pipe work with
 // 16-byte coalesced loads, shared-memory staging and warp-shuffle reductions (DESIGN.md).
@@ -24,6 +27,7 @@
 #include <stdlib.h>
 #include <string.h>
 
+#include <cub/device/device_merge_sort.cuh>
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_scan.cuh>
 
@@ -1469,6 +1473,166 @@ __global__ void __launch_bounds__(kThreads) k_rd_compact(const uint32_t* __restr
       rd_point(j, keys[i], base[0] + a.bytes, base[1] + a.sse, max_sse, pt_key, pt_bytes, pt_sse, out);
     }
     if (i + 1 == nev) out->count = j + 1;
+  }
+}
+
+// ------------------------------------------------------------------------------------------------
+// rate-distortion optimised encode (pxz_rdo_curve, pxz_rdo_shrink_to_size / _to_error; DESIGN.md §3 "Per-block sizes").  Each
+// block may take the dims of any level pair; the error table holds its decode error at every pair.  k_rdo_hull turns a
+// block's candidates into the segments of their lower convex hull (the events), the events sorted by rate gain / cost and
+// summed in that order give the curve, and k_rdo_levels forces the levels of one curve point for the encode.
+// ------------------------------------------------------------------------------------------------
+constexpr int kRdoHullThreads = 128;
+
+// gain_a / cost_a > gain_b / cost_b, exactly (costs > 0): the 128-bit products gain_a * cost_b and gain_b * cost_a.  Errors and
+// bytes of u16 blocks reach 2^50 and 2^34, so 64-bit products overflow and an f64 rate cannot tell close rates apart.
+__device__ __forceinline__ bool rdo_rate_above(unsigned long long ga, unsigned long long ca, unsigned long long gb, unsigned long long cb) {
+  const unsigned long long ha = __umul64hi(ga, cb), hb = __umul64hi(gb, ca);
+  return ha != hb ? ha > hb : ga * cb > gb * ca;
+}
+
+// the merge sort's order: rate descending (padding, gain 0 and cost 1, has rate 0 and sorts after every event)
+struct RdoRateDesc {
+  __device__ bool operator()(const RdoEvent& a, const RdoEvent& b) const { return rdo_rate_above(a.gain, a.cost, b.gain, b.cost); }
+};
+
+// One thread per block; its candidates live in shared memory, column `threadIdx.x` of ncand rows (ncand * 20 bytes per thread).
+// The shared memory, not registers, bounds the CTAs per SM: the minimum of one block keeps ptxas from spilling to reach more.
+// Candidates, sorted by bytes: one per distinct byte count, the least error, on a tie the lower pass (a block's decode at equal
+// dims is the same, so this also keeps the smallest level pair of each dims).  Then from the fewest bytes (1 x 1) the points
+// whose error strictly falls, reduced to their lower convex hull in place (a point strictly above the chord of its neighbours
+// goes; collinear points stay).
+__global__ void __launch_bounds__(kRdoHullThreads, 1) k_rdo_hull(const unsigned long long* __restrict__ sse_table, Geom g, uint32_t bpp,
+                                                                 uint32_t lx_max, uint32_t ly_max, uint32_t maxev, RdoEvent* __restrict__ ev,
+                                                                 uint32_t* __restrict__ ids, uint32_t* __restrict__ ev_pass,
+                                                                 uint32_t* __restrict__ pass0, unsigned long long* __restrict__ base) {
+  extern __shared__ __align__(16) uint8_t smem_rdo[];
+  const uint32_t ncand = maxev + 1, T = blockDim.x;
+  unsigned long long* cb = reinterpret_cast<unsigned long long*>(smem_rdo) + threadIdx.x;  // bytes, row stride T
+  unsigned long long* cs = cb + (size_t)ncand * T;                                         // error
+  uint32_t* cp = reinterpret_cast<uint32_t*>(smem_rdo + (size_t)ncand * T * 16) + threadIdx.x;  // pass
+  const uint32_t nblocks = g.cols * g.rows;
+  const uint32_t b = blockIdx.x * T + threadIdx.x;
+  unsigned long long bytes0 = 0, sse0 = 0, events = 0;
+  if (b < nblocks) {
+    const Tile t = tile_of(g, b);
+    uint32_t n = 0;
+    for (uint32_t lx = 0; lx <= lx_max; ++lx) {
+      const unsigned long long w = scaled_dim(t.tw, lx);
+      for (uint32_t ly = 0; ly <= ly_max; ++ly) {
+        const uint32_t pass = lx * (ly_max + 1) + ly;
+        const unsigned long long bytes = w * scaled_dim(t.th, ly) * bpp;
+        const unsigned long long sse = sse_table[(size_t)pass * nblocks + b];
+        uint32_t i = n;
+        while (i > 0 && cb[(i - 1) * T] > bytes) --i;
+        if (i > 0 && cb[(i - 1) * T] == bytes) {
+          if (sse < cs[(i - 1) * T]) {
+            cs[(i - 1) * T] = sse;
+            cp[(i - 1) * T] = pass;
+          }
+          continue;
+        }
+        if (n == ncand) continue;  // not reached: ncand bounds the distinct byte counts of every tile
+        for (uint32_t j = n; j > i; --j) {
+          cb[j * T] = cb[(j - 1) * T];
+          cs[j * T] = cs[(j - 1) * T];
+          cp[j * T] = cp[(j - 1) * T];
+        }
+        cb[i * T] = bytes;
+        cs[i * T] = sse;
+        cp[i * T] = pass;
+        ++n;
+      }
+    }
+    uint32_t top = 0;  // the hull is rows 0 .. top
+    for (uint32_t i = 1; i < n; ++i) {
+      const unsigned long long pb = cb[i * T], ps = cs[i * T];
+      if (ps >= cs[top * T]) continue;  // no less error than a point with fewer bytes
+      while (top > 0) {
+        const unsigned long long ob = cb[(top - 1) * T], os = cs[(top - 1) * T];
+        // the middle point goes when the chord from the point before it falls faster than the step to it
+        if (!rdo_rate_above(os - ps, pb - ob, os - cs[top * T], cb[top * T] - ob)) break;
+        --top;
+      }
+      ++top;
+      cb[top * T] = pb;
+      cs[top * T] = ps;
+      cp[top * T] = cp[i * T];
+    }
+    bytes0 = cb[0];
+    sse0 = cs[0];
+    events = top;
+    pass0[b] = cp[0];
+    for (uint32_t k = 0; k < maxev; ++k) {
+      const size_t slot = (size_t)b * maxev + k;
+      ids[slot] = (uint32_t)slot;
+      if (k < top) {
+        ev[slot] = RdoEvent{cs[k * T] - cs[(k + 1) * T], cb[(k + 1) * T] - cb[k * T]};
+        ev_pass[slot] = cp[(k + 1) * T];
+      } else {
+        ev[slot] = RdoEvent{0ull, 1ull};
+        ev_pass[slot] = kRdNoEvent;
+      }
+    }
+  }
+  bytes0 = warp_sum_u64(bytes0);
+  sse0 = warp_sum_u64(sse0);
+  events = warp_sum_u64(events);
+  if ((threadIdx.x & 31) == 0) {
+    if (bytes0) atomicAdd(&base[0], bytes0);
+    if (sse0) atomicAdd(&base[1], sse0);
+    if (events) atomicAdd(&base[2], events);
+  }
+}
+
+// after the sort: the scan input (bytes up, error down, mod 2^64; padding adds nothing) and each slot's rank in rate order
+__global__ void __launch_bounds__(kThreads) k_rdo_gather(const RdoEvent* __restrict__ ev, const uint32_t* __restrict__ ids, uint32_t nev,
+                                                         RdAcc* __restrict__ acc, uint32_t* __restrict__ rank) {
+  for (uint32_t i = blockIdx.x * kThreads + threadIdx.x; i < nev; i += gridDim.x * kThreads) {
+    const RdoEvent e = ev[i];
+    acc[i] = e.gain ? RdAcc{e.cost, 0ull - e.gain} : RdAcc{0ull, 0ull};
+    rank[ids[i]] = i;
+  }
+}
+
+// point 0 = the base totals, point i + 1 = base + the first i + 1 sorted events.  out: count, the last point with bytes <=
+// max_bytes plus one (0 on entry: none) and the first with sse <= max_sse (all ones on entry: none)
+__global__ void __launch_bounds__(kThreads) k_rdo_points(const RdoEvent* __restrict__ ev, const RdAcc* __restrict__ sums, uint32_t nev,
+                                                         const unsigned long long* __restrict__ base, unsigned long long max_bytes,
+                                                         unsigned long long max_sse, unsigned long long* __restrict__ pt_bytes,
+                                                         unsigned long long* __restrict__ pt_sse, RdoOut* __restrict__ out) {
+  const uint32_t first = blockIdx.x * kThreads + threadIdx.x;
+  for (uint32_t j = first; j <= nev; j += gridDim.x * kThreads) {
+    if (j > 0 && ev[j - 1].gain == 0) break;  // padding: sorted after every event
+    unsigned long long bytes = base[0], sse = base[1];
+    if (j > 0) {
+      const RdAcc a = sums[j - 1];
+      bytes += a.bytes;
+      sse += a.sse;
+    }
+    pt_bytes[j] = bytes;
+    pt_sse[j] = sse;
+    if (bytes <= max_bytes) atomicMax(&out->best_within, j + 1);
+    if (sse <= max_sse) atomicMin(&out->first_within, j);
+  }
+  if (first == 0) out->count = (uint32_t)base[2] + 1;
+}
+
+// levels of curve point j: per block the vertex after its events of rank < j (a block's events are ranked in hull order)
+__global__ void __launch_bounds__(kThreads) k_rdo_levels(const uint32_t* __restrict__ pass0, const uint32_t* __restrict__ ev_pass,
+                                                         const uint32_t* __restrict__ rank, uint32_t maxev, uint32_t nblocks, uint32_t ly_max,
+                                                         uint32_t j, float* __restrict__ vx, float* __restrict__ vy) {
+  for (uint32_t b = blockIdx.x * kThreads + threadIdx.x; b < nblocks; b += gridDim.x * kThreads) {
+    uint32_t pass = pass0[b];
+    for (uint32_t k = 0; k < maxev; ++k) {
+      const size_t slot = (size_t)b * maxev + k;
+      const uint32_t p = ev_pass[slot];
+      if (p == kRdNoEvent || rank[slot] >= j) break;
+      pass = p;
+    }
+    const uint32_t lx = pass / (ly_max + 1), ly = pass - lx * (ly_max + 1);
+    vx[b] = __uint_as_float((127u - lx) << 23);  // 2^-lx
+    vy[b] = __uint_as_float((127u - ly) << 23);
   }
 }
 
@@ -3094,6 +3258,66 @@ cudaError_t launch_rd_curve(const uint32_t* keys, const uint32_t* ids, const uin
   return launch(k_rd_compact, grid, kThreads, 0, s, skeys, sums, points, nev, reinterpret_cast<const unsigned long long*>(base),
                 (unsigned long long)max_sse, pt_key, reinterpret_cast<unsigned long long*>(pt_bytes), reinterpret_cast<unsigned long long*>(pt_sse),
                 out);
+}
+
+cudaError_t launch_rdo_hull(const uint64_t* sse_table, const Geom& g, uint32_t bpp, uint32_t lx_max, uint32_t ly_max, uint32_t maxev, RdoEvent* ev,
+                            uint32_t* ids, uint32_t* ev_pass, uint32_t* pass0, uint64_t* base, cudaStream_t s, uint64_t* launches) {
+  const uint32_t nblocks = g.cols * g.rows;
+  // 20 bytes per candidate and thread: 128 threads while that fits 96 KB (13 candidates at 64 x 64), fewer for very large blocks
+  const size_t per_thread = (size_t)(maxev + 1) * 20;
+  int threads = kRdoHullThreads;
+  while (threads > 32 && per_thread * threads > 96 * 1024) threads /= 2;
+  if (per_thread * threads > 200 * 1024) return cudaErrorInvalidValue;
+  ++*launches;
+  return launch(k_rdo_hull, (nblocks + threads - 1) / threads, threads, per_thread * threads, s,
+                reinterpret_cast<const unsigned long long*>(sse_table), g, bpp, lx_max, ly_max, maxev, ev, ids, ev_pass, pass0,
+                reinterpret_cast<unsigned long long*>(base));
+}
+
+// scratch of launch_rdo_curve: scan input | scan output | CUB's temporary storage (merge sort or scan)
+static size_t rdo_cub_bytes(uint32_t nev) {
+  size_t sort = 0, scan = 0;
+  cub::DeviceMergeSort::StableSortPairs(nullptr, sort, (RdoEvent*)nullptr, (uint32_t*)nullptr, (int)nev, RdoRateDesc());
+  cub::DeviceScan::InclusiveScan(nullptr, scan, (const RdAcc*)nullptr, (RdAcc*)nullptr, RdAccSum(), (int)nev);
+  return std::max(sort, scan);
+}
+size_t rdo_curve_scratch_bytes(uint32_t nev) { return 2 * rd_align((size_t)nev * sizeof(RdAcc)) + rd_align(rdo_cub_bytes(nev)); }
+
+cudaError_t launch_rdo_curve(RdoEvent* ev, uint32_t* ids, uint32_t nev, const uint64_t* base, uint64_t max_bytes, uint64_t max_sse, void* scratch,
+                             size_t scratch_bytes, uint32_t* rank, uint64_t* pt_bytes, uint64_t* pt_sse, RdoOut* out, cudaStream_t s, int sm_count,
+                             uint64_t* launches) {
+  if (scratch_bytes < rdo_curve_scratch_bytes(nev) || nev > 0x7FFFFFFFu) return cudaErrorInvalidValue;
+  uint8_t* p = static_cast<uint8_t*>(scratch);
+  RdAcc* acc = reinterpret_cast<RdAcc*>(p);
+  p += rd_align((size_t)nev * sizeof(RdAcc));
+  RdAcc* sums = reinterpret_cast<RdAcc*>(p);
+  p += rd_align((size_t)nev * sizeof(RdAcc));
+  size_t cub_bytes = rdo_cub_bytes(nev);
+  // best_within = 0 (none), first_within = all ones (none)
+  cudaError_t e = cudaMemsetAsync(out, 0, sizeof(RdoOut), s);
+  if (e == cudaSuccess) e = cudaMemsetAsync(&out->first_within, 0xFF, sizeof(uint32_t), s);
+  const int grid = clamp_grid(((long long)nev + kThreads) / kThreads, (long long)sm_count * 8);
+  if (e == cudaSuccess && nev > 0) {
+    // sort, gather, scan: CUB's sort and scan launch several kernels each and count as one launch here
+    *launches += 3;
+    e = cub::DeviceMergeSort::StableSortPairs(p, cub_bytes, ev, ids, (int)nev, RdoRateDesc(), s);
+    if (e == cudaSuccess) e = launch(k_rdo_gather, grid, kThreads, 0, s, ev, ids, nev, acc, rank);
+    if (e == cudaSuccess) {
+      cub_bytes = rdo_cub_bytes(nev);
+      e = cub::DeviceScan::InclusiveScan(p, cub_bytes, acc, sums, RdAccSum(), (int)nev, s);
+    }
+  }
+  if (e != cudaSuccess) return e;
+  ++*launches;
+  return launch(k_rdo_points, grid, kThreads, 0, s, ev, sums, nev, reinterpret_cast<const unsigned long long*>(base), (unsigned long long)max_bytes,
+                (unsigned long long)max_sse, reinterpret_cast<unsigned long long*>(pt_bytes), reinterpret_cast<unsigned long long*>(pt_sse), out);
+}
+
+cudaError_t launch_rdo_levels(const uint32_t* pass0, const uint32_t* ev_pass, const uint32_t* rank, uint32_t maxev, uint32_t nblocks,
+                              uint32_t ly_max, uint32_t j, float* vx, float* vy, cudaStream_t s, int sm_count, uint64_t* launches) {
+  ++*launches;
+  const int grid = clamp_grid(((long long)nblocks + kThreads - 1) / kThreads, (long long)sm_count * 8);
+  return launch(k_rdo_levels, grid, kThreads, 0, s, pass0, ev_pass, rank, maxev, nblocks, ly_max, j, vx, vy);
 }
 
 size_t resample_fir_smem_bytes(uint32_t max_src_px, uint32_t max_tmp_px, uint32_t C) {

@@ -203,6 +203,35 @@ size_t rd_curve_scratch_bytes(uint32_t nev);
 cudaError_t launch_rd_curve(const uint32_t* keys, const uint32_t* ids, const uint64_t* dbytes, const uint64_t* dsse, uint32_t nev,
                             const uint64_t* base, uint64_t max_sse, void* scratch, size_t scratch_bytes, uint32_t* pt_key, uint64_t* pt_bytes,
                             uint64_t* pt_sse, RdOut* out, cudaStream_t s, int sm_count, uint64_t* launches);
+// Rate-distortion optimised encode (pxz_rdo_*).  The error table has every level pair: block b's error at (lx, ly) is
+// sse_table[(lx * (ly_max + 1) + ly) * nblocks + b].  An event is one segment of a block's hull: gain = the error it removes,
+// cost = the bytes it adds (both > 0); padding has gain 0, cost 1.
+struct RdoEvent {
+  unsigned long long gain, cost;
+};
+// launch_rdo_hull: per block its candidates (one per distinct byte count, from dims scaled_dim(tw, lx) x scaled_dim(th, ly)), the
+// lower convex hull of those whose error strictly falls from the 1 x 1 one, and its segments in slots b * maxev + i: ev, the
+// pass of the vertex the segment ends at (ev_pass; kRdNoEvent: padding), id = the slot.  pass0[b] = the pass of the first vertex.
+// base[0] / base[1] / base[2] += the bytes / errors of all blocks at that vertex / the event count (zero on entry).  maxev + 1
+// must bound every tile's distinct byte counts.
+cudaError_t launch_rdo_hull(const uint64_t* sse_table, const Geom& g, uint32_t bpp, uint32_t lx_max, uint32_t ly_max, uint32_t maxev, RdoEvent* ev,
+                            uint32_t* ids, uint32_t* ev_pass, uint32_t* pass0, uint64_t* base, cudaStream_t s, uint64_t* launches);
+// launch_rdo_curve: the events stable-sorted in place by rate gain / cost (descending, exact), rank[slot] = its place in that
+// order, and the curve: point 0 = base, point j = base + the first j events (pt_bytes / pt_sse: nev + 1 words).  out: point
+// count, the last point with bytes <= max_bytes plus one (0: none), the first with sse <= max_sse (0xFFFFFFFF: none).
+// scratch: rdo_curve_scratch_bytes(nev).
+struct RdoOut {
+  uint32_t count;
+  uint32_t best_within;
+  uint32_t first_within;
+};
+size_t rdo_curve_scratch_bytes(uint32_t nev);
+cudaError_t launch_rdo_curve(RdoEvent* ev, uint32_t* ids, uint32_t nev, const uint64_t* base, uint64_t max_bytes, uint64_t max_sse, void* scratch,
+                             size_t scratch_bytes, uint32_t* rank, uint64_t* pt_bytes, uint64_t* pt_sse, RdoOut* out, cudaStream_t s, int sm_count,
+                             uint64_t* launches);
+// launch_rdo_levels: vx[b] = 2^-lx, vy[b] = 2^-ly of block b's vertex at curve point j (after its events of rank < j).
+cudaError_t launch_rdo_levels(const uint32_t* pass0, const uint32_t* ev_pass, const uint32_t* rank, uint32_t maxev, uint32_t nblocks,
+                              uint32_t ly_max, uint32_t j, float* vx, float* vy, cudaStream_t s, int sm_count, uint64_t* launches);
 // Which resample kernel family runs (PXZ_RESAMPLE_KERNELS=warp|cta|tma).  Auto: by tile count; Warp: warp-per-tile kernels
 // with the cp.async ring shrink kernel; Cta: CTA-per-tile kernels; Tma: warp-per-tile kernels with the TMA shrink kernel.
 // The forced warp families still need the RGBA fast geometry and tables that have the warp forms.
