@@ -77,8 +77,8 @@ int pxz_abi_version(void);
 /* number of usable CUDA devices (0 if none / no driver) */
 int pxz_device_count(void);
 /* One context per host thread; it owns one CUDA stream and its scratch.  Environment read at creation (diagnostics only):
- *   PXZ_RESAMPLE_KERNELS=warp|cta|tma  force a resample kernel family (default: by tile count): warp-per-tile with
- *                                  the cp.async ring shrink kernel, CTA-per-tile, or warp-per-tile with the TMA shrink kernel. */
+ *   PXZ_RESAMPLE_KERNELS=warp|cta  force a resample kernel family (default: by tile count): warp-per-tile (the
+ *                                  TMA-fed shrink kernel) or CTA-per-tile. */
 pxz_status pxz_ctx_create(int device, pxz_ctx** out);
 /* same, but work is ordered on an existing CUDA stream (cudaStream_t / CUstream passed as
  * void*), e.g. torch.cuda.current_stream().cuda_stream.  The stream must outlive the ctx. */

@@ -40,7 +40,7 @@ struct TabSet {  // device copy of the axis tables of one (spec, filter, directi
   uint32_t max_words = 0;  // largest single table (left | count | weights), in 32-bit words
   uint32_t ntabs = 0;
   bool warp_ok = false;    // every table has the form the warp-per-tile kernels need
-  bool has_noslide = false;  // direction 0: some table has no slide form (k_shrink_tma leaves those tiles to k_shrink_warp)
+  bool has_noslide = false;  // direction 0: some table has no slide2 form (k_shrink_tma leaves those tiles to k_shrink_warp)
 };
 
 using TabKey = std::tuple<std::vector<uint32_t>, std::vector<uint32_t>, int, int>;
@@ -543,7 +543,6 @@ pxz_status ctx_create_common(int device, cudaStream_t stream, bool own, pxz_ctx*
   if (const char* e = getenv("PXZ_RESAMPLE_KERNELS"))
     ctx->resample_kernels = !strcmp(e, "warp") ? ResampleKernels::Warp
                             : !strcmp(e, "cta") ? ResampleKernels::Cta
-                            : !strcmp(e, "tma") ? ResampleKernels::Tma
                                                 : ResampleKernels::Auto;
   if (cudaMalloc((void**)&ctx->d_minmax, 8 * sizeof(float)) != cudaSuccess ||
       cudaMalloc((void**)&ctx->d_tile_counter, 64) != cudaSuccess || cudaMemset(ctx->d_tile_counter, 0, 64) != cudaSuccess ||

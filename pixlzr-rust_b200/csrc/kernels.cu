@@ -2876,33 +2876,27 @@ cudaError_t launch_resample(const ResampleArgs& a, cudaStream_t s, int sm_count,
   // the GPU busy for a few tiles; below that one tile's latency (15-40 us on one warp) decides and 8 warps per tile
   // finish sooner.  a.kernels forces a family (ResampleKernels).
   const long long ntiles = (long long)g.cols * g.rows;
-  const bool force_warp = a.kernels == ResampleKernels::Warp || a.kernels == ResampleKernels::Tma;
   if (fast && a.warp_tables && a.kernels != ResampleKernels::Cta &&
-      (force_warp || ntiles >= (long long)sm_count * 16)) {
+      (a.kernels == ResampleKernels::Warp || ntiles >= (long long)sm_count * 16)) {
     if (a.direction == 1) {
       const int wgrid = clamp_grid((ntiles + kWarpsPerCta - 1) / kWarpsPerCta, (long long)sm_count * PXZ_EXPAND_WARP_CTAS);
       return launch_pdl(a.fused ? k_expand_warp<true> : k_expand_warp<false>, wgrid, kWarpCtaThreads, (size_t)kWarpsPerCta * kExpandWarpBytes,
                         s, a.img, a.pitch, g, a.descs, a.tabidx, a.lists, a.cap, a.payload, a.tabs, a.pool, a.tile_counter, 1.0f, -0.0f);
     }
-    bool ring_kernel = a.kernels == ResampleKernels::Warp;
-    if (!ring_kernel) {
-      CUtensorMap tm;
-      if (make_image_tmap(a.img, a.pitch, g.W, g.nimg > 1 ? (g.nimg - 1) * g.img_rows + g.H : g.H, &tm)) {
-        const int tgrid = clamp_grid((ntiles + kTWarps - 1) / kTWarps, (long long)sm_count * PXZ_SHRINK_TMA_CTAS);
-        const cudaError_t e = launch_pdl(a.fused ? k_shrink_tma<true> : k_shrink_tma<false>, tgrid, kTWarps * 32, (size_t)kTWarps * kTWarpBytes, s, tm,
-                                         g, a.descs, a.tabidx, a.lists, a.cap, a.opaque_flags, a.payload, a.tabs, a.ntabs, a.pool, a.tile_counter,
-                                         1.0f, -0.0f);
-        if (e != cudaSuccess || !a.has_noslide) return e;
-        ++*launches;  // the tiles without a slide table go to the ring kernel
-      } else {
-        ring_kernel = true;
-      }
+    // an image no tensor map can address (driver entry point missing, beyond the tensor-map limits) takes the
+    // CTA-per-tile kernel below
+    CUtensorMap tm;
+    if (make_image_tmap(a.img, a.pitch, g.W, g.nimg > 1 ? (g.nimg - 1) * g.img_rows + g.H : g.H, &tm)) {
+      const int tgrid = clamp_grid((ntiles + kTWarps - 1) / kTWarps, (long long)sm_count * PXZ_SHRINK_TMA_CTAS);
+      const cudaError_t e = launch_pdl(a.fused ? k_shrink_tma<true> : k_shrink_tma<false>, tgrid, kTWarps * 32, (size_t)kTWarps * kTWarpBytes, s, tm,
+                                       g, a.descs, a.tabidx, a.lists, a.cap, a.opaque_flags, a.payload, a.tabs, a.ntabs, a.pool, a.tile_counter,
+                                       1.0f, -0.0f);
+      if (e != cudaSuccess || !a.has_noslide) return e;
+      ++*launches;  // the tiles whose vertical table has no slide2 form
+      const int wgrid = clamp_grid((ntiles + kShrinkWarps - 1) / kShrinkWarps, (long long)sm_count * PXZ_SHRINK_WARP_CTAS);
+      return launch_pdl(a.fused ? k_shrink_warp<true> : k_shrink_warp<false>, wgrid, kShrinkCtaThreads, (size_t)kShrinkWarps * kShrinkWarpBytes, s,
+                        a.img, a.pitch, g, a.descs, a.tabidx, a.lists, a.cap, a.opaque_flags, a.payload, a.tabs, a.pool, a.tile_counter, 1.0f, -0.0f);
     }
-    const uint32_t only_noslide = ring_kernel ? 0u : 1u;
-    const int wgrid = clamp_grid((ntiles + kShrinkWarps - 1) / kShrinkWarps, (long long)sm_count * PXZ_SHRINK_WARP_CTAS);
-    return launch_pdl(a.fused ? k_shrink_warp<true> : k_shrink_warp<false>, wgrid, kShrinkCtaThreads, (size_t)kShrinkWarps * kShrinkWarpBytes, s,
-                      a.img, a.pitch, g, a.descs, a.tabidx, a.lists, a.cap, a.opaque_flags, a.payload, a.tabs, a.pool, a.tile_counter, 1.0f, -0.0f,
-                      only_noslide);
   }
   if (fast) {
     const int fgrid = clamp_grid(ntiles, (long long)sm_count * PXZ_RESAMPLE_MINBLOCKS);

@@ -23,13 +23,14 @@ constexpr uint32_t kLevelOnePixel = 0xFFu; // "level 0" / below every threshold:
 // A kernel walks source samples lo .. lo+rows once per group and feeds 4 accumulators, so each accumulator still
 // receives its taps in ascending order (adding p * 0 is exact).
 //
-// Two more forms serve the warp-per-tile kernels (k_shrink_warp / k_expand_warp):
-//  * slide form at `soff` (downscale, n_in >= n_out; pool offset is a multiple of 4 words): n_in rows of 8 floats —
-//    row r holds, for every accumulator slot s < slots, the weight of the output o with o % slots == s whose
-//    (zero-trimmed) window contains source sample r, else +0 — followed by done[n_in]: how many outputs (in ascending
-//    order) receive their last tap at sample r.  One walk over the source samples feeds all live outputs, so every
-//    sample is loaded and converted once and no multiply is wasted; each accumulator still sees its taps in
-//    ascending order.  slots in {2, 4, 6}; 0 = the table has no slide form (more than 6 outputs live at once).
+// Two more forms serve the warp-per-tile kernels (k_shrink_tma / k_expand_warp):
+//  * slide2 form at `s2off` (downscale, n_in >= n_out; pool offset and s2words are multiples of 4 words, so one bulk copy
+//    stages it): n_in rows of `slots` f32 pairs — pair s of row r holds (w, w), w = the weight of the output o with
+//    o % slots == s whose (zero-trimmed) window contains source sample r, else +0; one f32x2 operand whose lanes are two
+//    image columns — followed by end[n_out]: the source sample that holds output o's last tap.  One walk over the source
+//    samples feeds all live outputs, so every sample is loaded and converted once and no multiply is wasted; each
+//    accumulator still sees its taps in ascending order.  slots in {2, 4, 6}; slots = s2words = 0: the table has no
+//    slide2 form (more than 6 outputs live at once; k_shrink_warp shrinks those tiles from the blocked form).
 //  * gather8 form at `goff` (upscale, every output has <= 7 taps): n_out rows of 8 floats (weights, +0 padded),
 //    then left[n_out]; at `gpoff` (multiple of 4 words) ceil(n_out / 2) rows of 8 float pairs
 //    (w[2p][i], w[2p+1][i]): two output rows with the same first tap run as the two lanes of one f32x2 operation.
@@ -38,7 +39,7 @@ constexpr uint32_t kLevelOnePixel = 0xFFu; // "level 0" / below every threshold:
 struct AxisTab {
   uint32_t n_in, n_out, stride, off;
   uint32_t boff, nb, brows_total, bwords;
-  uint32_t soff, slots, goff, gpoff;
+  uint32_t pad1_, slots, goff, gpoff;
   uint32_t bpad, s2off, s2words, pad2_;  // s2off / s2words: slide2 form (tables.cpp), 0 words = none
 };
 
@@ -232,10 +233,11 @@ cudaError_t launch_rdo_curve(RdoEvent* ev, uint32_t* ids, uint32_t nev, const ui
 // launch_rdo_levels: vx[b] = 2^-lx, vy[b] = 2^-ly of block b's vertex at curve point j (after its events of rank < j).
 cudaError_t launch_rdo_levels(const uint32_t* pass0, const uint32_t* ev_pass, const uint32_t* rank, uint32_t maxev, uint32_t nblocks,
                               uint32_t ly_max, uint32_t j, float* vx, float* vy, cudaStream_t s, int sm_count, uint64_t* launches);
-// Which resample kernel family runs (PXZ_RESAMPLE_KERNELS=warp|cta|tma).  Auto: by tile count; Warp: warp-per-tile kernels
-// with the cp.async ring shrink kernel; Cta: CTA-per-tile kernels; Tma: warp-per-tile kernels with the TMA shrink kernel.
-// The forced warp families still need the RGBA fast geometry and tables that have the warp forms.
-enum class ResampleKernels { Auto, Warp, Cta, Tma };
+// Which resample kernel family runs (PXZ_RESAMPLE_KERNELS=warp|cta).  Auto: by tile count; Warp: warp-per-tile kernels
+// (shrink: k_shrink_tma, then k_shrink_warp for the tiles without a slide2 table; expand: k_expand_warp); Cta: CTA-per-tile
+// kernels.  The forced warp family still needs the RGBA fast geometry, tables that have the warp forms and, to shrink, an
+// image a tensor map can address; otherwise the CTA-per-tile kernels run.
+enum class ResampleKernels { Auto, Warp, Cta };
 struct ResampleArgs {
   int direction;  // 0: image tiles -> payload (shrink); 1: payload -> image tiles (expand)
   uint8_t* img;
@@ -258,7 +260,7 @@ struct ResampleArgs {
   uint32_t cap;
   bool warp_tables;        // every table has the forms the warp-per-tile kernels need
   ResampleKernels kernels;
-  bool has_noslide;        // shrink: some table has no slide form (k_shrink_tma leaves those tiles to k_shrink_warp)
+  bool has_noslide;        // shrink: some table has no slide2 form (k_shrink_tma leaves those tiles to k_shrink_warp)
 };
 cudaError_t launch_resample(const ResampleArgs& a, cudaStream_t s, int sm_count, uint64_t* launches);
 size_t resample_smem_bytes(uint32_t max_src_px, uint32_t max_tmp_px, uint32_t C);

@@ -368,7 +368,7 @@ __device__ __forceinline__ void tma_shrink_tile_simple(TFeed& f, TQueue& q, cons
 }
 
 // ---- vertical pass + horizontal batches of one tile -----------------------------------------------------------------
-// A = accumulator slots of the tile's slide table (2, 4, 6); the stream has this tile's boxes next.
+// A = accumulator slots of the tile's slide2 table (2, 4, 6); the stream has this tile's boxes next.
 template <int MODE, int A>
 __device__ __forceinline__ void tma_shrink_tile(TFeed& f, TQueue& q, const CUtensorMap* tm, uint32_t sh, uint32_t dw, uint32_t dh, uint32_t vtab,
                                                 float4* strip, const HTab& ht, uint32_t* dst, const TapK& k) {
@@ -514,7 +514,7 @@ __global__ void __launch_bounds__(kTWarps * 32, PXZ_SHRINK_TMA_CTAS) k_shrink_tm
   AxisTab ty{};
   HTab ht{};
   // does a block stream its source tile?  masked-out blocks (quadtree levels) and tiles whose vertical table has no
-  // slide form (left to k_shrink_warp by the launcher) do not
+  // slide2 form (left to k_shrink_warp by the launcher) do not
   auto boxes_of = [&](const Tile& t, const pxz_block_desc& d, uint32_t ti) -> uint32_t {
     if (d.w == 0 || d.h == 0) return 0u;
     if (!(d.w == t.tw && d.h == t.th) && s_noslide[ti >> 16]) return 0u;

@@ -2,10 +2,11 @@
 //
 // Every warp owns one tile at a time (tiles are handed out through an atomic counter), so there is no CTA barrier
 // anywhere and a light tile never idles the threads of a heavy one:
-//   * shrink: the source tile is streamed from global memory exactly once through a 16-row cp.async ring in shared
-//     memory (lane = columns 2x and 2x + 1); the vertical pass keeps all live output rows in registers ("slide" table
-//     form, pxz_internal.h) and emits one finished row of f32 intermediates at a time into an 8-row strip; whenever
-//     the strip is full the warp runs the horizontal pass over it and writes the packed payload pixels.
+//   * shrink (k_shrink_warp): the tiles k_shrink_tma (resample_tma.cuh) leaves, those whose vertical table has no slide2
+//     form (more than 6 outputs live at once).  Lane = columns 2x and 2x + 1; every group of 4 output rows walks its
+//     source rows straight from global memory / L1 (blocked table form) into an 8-row strip of f32 intermediates in
+//     shared memory; whenever the strip is full the warp runs the horizontal pass over it and writes the packed payload
+//     pixels.
 //   * expand: the (small) source block is streamed once through a 7-row register window of converted samples; two
 //     rows of intermediates at a time go through shared memory to the horizontal pass, which writes the image tile
 //     (the paste is fused: 16-byte stores into the pitched image).
@@ -16,29 +17,17 @@
 #ifndef PXZ_SHRINK_WARPS
 #define PXZ_SHRINK_WARPS 4
 #endif
-#ifndef PXZ_RING_ROWS
-#define PXZ_RING_ROWS 16
-#endif
 constexpr int kWarpCtaThreads = 128;  // expand: 4 warps per CTA
 constexpr int kWarpsPerCta = kWarpCtaThreads / 32;
 constexpr int kShrinkWarps = PXZ_SHRINK_WARPS;
 constexpr int kShrinkCtaThreads = kShrinkWarps * 32;
 constexpr int kStripRows = 8;         // shrink: rows of intermediates per horizontal batch
 constexpr int kStripStride = 65;      // float4 per strip row: 64 + 1, so 8 rows of one column sit in 8 different banks
-constexpr int kRingRows = PXZ_RING_ROWS;  // shrink: source rows in flight per warp (x 256 B)
 constexpr int kHTabWords = 512;       // shrink: per-warp copy of the tile's horizontal table (2 KB), else read via L1
-constexpr int kShrinkWarpBytes = kStripRows * kStripStride * 16 + kRingRows * 64 * 4 + kHTabWords * 4;
+constexpr int kShrinkWarpBytes = kStripRows * kStripStride * 16 + kHTabWords * 4;
 constexpr int kExpandRow1 = 68;       // expand: second strip row starts at 64 + pad (pad chosen per tile, <= 4)
 constexpr int kExpandPairPx = kExpandRow1 + 64 + 8;  // one pair of strip rows (second row at 64 + pad), + the walk's overrun
 constexpr int kExpandWarpBytes = 2 * kExpandPairPx * 16;  // two pairs: blocks at most 16 wide run two row pairs per vertical pass
-
-__device__ __forceinline__ void cp_async_16(void* smem_dst, const void* gmem_src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"((uint32_t)__cvta_generic_to_shared(smem_dst)), "l"(gmem_src));
-}
-template <int N>
-__device__ __forceinline__ void cp_async_wait() {
-  asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory");
-}
 
 // v-th block in cost order (lists: see launch_plan); nullptr = natural order
 struct TileOrder {
@@ -178,273 +167,43 @@ __device__ __forceinline__ void shrink_horizontal(const float4* strip, uint32_t 
   }
 }
 
-// Everything the vertical pass of one tile keeps between two horizontal batches (all in registers).
+// Vertical pass from the blocked table (two groups of 4 output rows per strip, each walking its source rows straight from
+// global memory / L1), then the horizontal pass over the strip.
 template <int MODE>
-struct ShrinkRun {
-  static constexpr int NC = (MODE & 1) ? 4 : 3;
-  u64 acc[2][NC][3];  // [column][channel][slot pair]; tables with fewer slots use the first pairs
-  const ulonglong2* wp;          // slide table row of source row r
-  const uint32_t* dp;            // done[r]
-  ulonglong2 wa_n;               // table row of source row r, requested one row ahead
-  u64 wb_n;
-  uint32_t nd_n;
-  uint32_t r;                    // next source row
-  uint32_t pend;                 // outputs finished by row r - 1 that still have to be emitted
-  uint32_t o_next, slot, batch0; // next output row, its accumulator slot, first output row of the strip
-  uint32_t ob;                   // blocked fallback: next group of 4 output rows
-};
-
-template <int MODE, int NPMAX, int S>
-__device__ __forceinline__ void take_slot3(u64 (&acc)[2][(MODE & 1) ? 4 : 3][NPMAX], float4& v0, float4& v1) {
-  constexpr int NC = (MODE & 1) ? 4 : 3;
-  constexpr int jp = S / 2;
-  constexpr bool high = (S & 1) != 0;
-  float a[4] = {0.f, 0.f, 0.f, 0.f}, b[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-  for (int c = 0; c < NC; ++c) {
-    float l, h;
-    unpk2(acc[0][c][jp], l, h);
-    a[c] = high ? h : l;
-    acc[0][c][jp] = high ? pk2(l, 0.f) : pk2(0.f, h);
-    unpk2(acc[1][c][jp], l, h);
-    b[c] = high ? h : l;
-    acc[1][c][jp] = high ? pk2(l, 0.f) : pk2(0.f, h);
-  }
-  v0 = make_float4(a[0], a[1], a[2], a[3]);
-  v1 = make_float4(b[0], b[1], b[2], b[3]);
-}
-
-// vertical pass with the slide table, A accumulator slots (A / 2 register pairs) per column and channel: consumes
-// source rows until the strip holds kStripRows finished rows or the last output row is out
-template <int MODE, int A>
-__device__ __forceinline__ void shrink_vrun(ShrinkRun<MODE>& st, const uint8_t* tile0, size_t pitch, uint32_t sw, uint32_t sh,
-                                            uint32_t dh, float4* strip, uint32_t* ring, const TapK& k) {
-  constexpr int NC = (MODE & 1) ? 4 : 3;
-  constexpr int NP = A / 2;
+__device__ __forceinline__ void shrink_tile_warp(const uint8_t* __restrict__ img, size_t pitch, const Tile& t,
+                                                 const pxz_block_desc& d, const HTab& ht, const AxisTab& ty,
+                                                 const uint32_t* __restrict__ pool, float4* strip,
+                                                 uint8_t* __restrict__ payload, const TapK& k) {
   const uint32_t lane = threadIdx.x & 31u;
-  const uint32_t crow = lane >> 4, cchunk = lane & 15u;
-  const bool ccol = cchunk * 4 < sw;
-  for (;;) {
-    while (st.pend > 0 && st.o_next - st.batch0 < (uint32_t)kStripRows) {
-      float4 v0, v1;
-      switch (st.slot) {
-        case 0: take_slot3<MODE, 3, 0>(st.acc, v0, v1); break;
-        case 1: take_slot3<MODE, 3, 1>(st.acc, v0, v1); break;
-        case 2: if (A > 2) take_slot3<MODE, 3, (A > 2 ? 2 : 0)>(st.acc, v0, v1); break;
-        case 3: if (A > 2) take_slot3<MODE, 3, (A > 2 ? 3 : 0)>(st.acc, v0, v1); break;
-        case 4: if (A > 4) take_slot3<MODE, 3, (A > 4 ? 4 : 0)>(st.acc, v0, v1); break;
-        default: if (A > 4) take_slot3<MODE, 3, (A > 4 ? 5 : 0)>(st.acc, v0, v1); break;
-      }
-      float4* srow = strip + (st.o_next - st.batch0) * kStripStride + 2 * lane;
-      srow[0] = v0;
-      srow[1] = v1;
-      ++st.o_next;
-      st.slot = (st.slot + 1 == (uint32_t)A) ? 0u : st.slot + 1;
-      --st.pend;
-    }
-    if (st.o_next - st.batch0 == (uint32_t)kStripRows || st.o_next == dh) return;
-    const uint32_t r = st.r;
-    if ((r & 1u) == 0) {
-      cp_async_wait<kRingRows / 2 - 1>();  // the pair of rows (r, r + 1) has landed
-      __syncwarp();
-    }
-    const uint2 px = *reinterpret_cast<const uint2*>(ring + (r & (kRingRows - 1)) * 64 + 2 * lane);
-    u64 w[NP];
-    w[0] = st.wa_n.x;
-    if (NP > 1) w[NP > 1 ? 1 : 0] = st.wa_n.y;
-    if (NP > 2) w[NP > 2 ? 2 : 0] = st.wb_n;
-    st.pend = st.nd_n;
-    st.wp += 2;
-    ++st.dp;
-    // the table row of the next source row is requested before this row's arithmetic — unconditionally (a predicated
-    // load makes ptxas copy the registers out and back): after the last row it reads the words behind the table, which
-    // the pool always has (build_axis_table pads it) and nobody uses
-    st.wa_n = __ldg(st.wp);
-    if (NP > 2) st.wb_n = __ldg(reinterpret_cast<const u64*>(st.wp + 1));
-    st.nd_n = __ldg(st.dp);
-    const float4 pa = px_to_f4<MODE>(px.x), pb = px_to_f4<MODE>(px.y);
-    const float ca[4] = {pa.x, pa.y, pa.z, pa.w}, cb[4] = {pb.x, pb.y, pb.z, pb.w};
-#pragma unroll
-    for (int c = 0; c < NC; ++c) {
-      const u64 ppa = pk2(ca[c], ca[c]), ppb = pk2(cb[c], cb[c]);
-#pragma unroll
-      for (int jp = 0; jp < NP; ++jp) {
-        mac2_acc<MODE>(st.acc[0][c][jp], ppa, w[jp], k);
-        mac2_acc<MODE>(st.acc[1][c][jp], ppb, w[jp], k);
-      }
-    }
-    st.r = r + 1;
-    if ((st.r & 1u) == 0 || st.r == sh) {
-      // both rows of the pair are consumed: refill their ring slots with the pair 8 ahead
-      __syncwarp();
-      const uint32_t rn = ((st.r + 1) & ~1u) - 2 + kRingRows + crow;
-      if (rn < sh && ccol) cp_async_16(ring + (rn & (kRingRows - 1)) * 64 + cchunk * 4, tile0 + (size_t)rn * pitch + cchunk * 16);
-      cp_async_commit();
-    }
-  }
-}
-
-// Tiles whose output rows all fit the accumulator slots (n_out <= A: every output keeps its own slot for the whole walk,
-// nothing is emitted on the way): one plain loop over the source rows, then all rows go to the strip at once.  This is
-// every tile reduced to at most 4 rows — the state machine of shrink_vrun costs them twice the instructions.
-template <int MODE, int A>
-__device__ __forceinline__ void shrink_vsimple(const uint8_t* tile0, size_t pitch, uint32_t sw, uint32_t sh, uint32_t dh,
-                                               const AxisTab& ty, const uint32_t* __restrict__ pool, float4* strip, uint32_t* ring,
-                                               const TapK& k) {
-  constexpr int NC = (MODE & 1) ? 4 : 3;
-  constexpr int NP = A / 2;
-  constexpr int RING = kRingRows;
-  const uint32_t lane = threadIdx.x & 31u;
-  const uint32_t crow = lane >> 4, cchunk = lane & 15u;
-  const bool ccol = cchunk * 4 < sw;
-  u64 acc[2][NC][NP];
-#pragma unroll
-  for (int c = 0; c < NC; ++c)
-#pragma unroll
-    for (int j = 0; j < NP; ++j) acc[0][c][j] = acc[1][c][j] = 0ull;
-  auto issue = [&](uint32_t g) {
-    const uint32_t r = 2 * g + crow;
-    if (r < sh && ccol) cp_async_16(ring + (r & (RING - 1)) * 64 + cchunk * 4, tile0 + (size_t)r * pitch + cchunk * 16);
-    cp_async_commit();
-  };
-#pragma unroll
-  for (int g = 0; g < RING / 2; ++g) issue((uint32_t)g);
-  const ulonglong2* wp = reinterpret_cast<const ulonglong2*>(pool + ty.soff);
-  ulonglong2 wn = __ldg(wp);  // slots 0..3 of source row 0 (A <= 4 here); the next row's are requested one row ahead
-  const uint32_t npairs = (sh + 1) >> 1;
-#pragma unroll 1
-  for (uint32_t g = 0; g < npairs; ++g) {
-    cp_async_wait<RING / 2 - 1>();
-    __syncwarp();
-#pragma unroll
-    for (int h = 0; h < 2; ++h) {
-      const uint32_t r = 2 * g + h;
-      if (r < sh) {
-        const uint2 px = *reinterpret_cast<const uint2*>(ring + (r & (RING - 1)) * 64 + 2 * lane);
-        u64 w[NP];
-        w[0] = wn.x;
-        if (NP > 1) w[NP > 1 ? 1 : 0] = wn.y;
-        wp += 2;
-        wn = __ldg(wp);  // unconditional, see shrink_vrun
-        const float4 pa = px_to_f4<MODE>(px.x), pb = px_to_f4<MODE>(px.y);
-        const float ca[4] = {pa.x, pa.y, pa.z, pa.w}, cb[4] = {pb.x, pb.y, pb.z, pb.w};
-#pragma unroll
-        for (int c = 0; c < NC; ++c) {
-          const u64 ppa = pk2(ca[c], ca[c]), ppb = pk2(cb[c], cb[c]);
-#pragma unroll
-          for (int jp = 0; jp < NP; ++jp) {
-            mac2_acc<MODE>(acc[0][c][jp], ppa, w[jp], k);
-            mac2_acc<MODE>(acc[1][c][jp], ppb, w[jp], k);
-          }
-        }
-      }
-    }
-    __syncwarp();
-    issue(g + RING / 2);
-  }
-  cp_async_wait<0>();
-#pragma unroll
-  for (int o = 0; o < A; ++o) {
-    if ((uint32_t)o < dh) {
-      float a[4] = {0.f, 0.f, 0.f, 0.f}, b[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-      for (int c = 0; c < NC; ++c) {
-        a[c] = (o & 1) ? hi2(acc[0][c][o / 2]) : lo2(acc[0][c][o / 2]);
-        b[c] = (o & 1) ? hi2(acc[1][c][o / 2]) : lo2(acc[1][c][o / 2]);
-      }
-      float4* srow = strip + o * kStripStride + 2 * lane;
-      srow[0] = make_float4(a[0], a[1], a[2], a[3]);
-      srow[1] = make_float4(b[0], b[1], b[2], b[3]);
-    }
-  }
-}
-
-// vertical pass for tables without a slide form (more than 6 outputs live at once): two groups of 4 output rows per
-// call walk their source rows straight from global memory / L1
-template <int MODE>
-__device__ __forceinline__ void shrink_vrun_blocked(ShrinkRun<MODE>& st, const uint8_t* tile0, size_t pitch, uint32_t sw, uint32_t dh,
-                                                    const AxisTab& ty, const uint32_t* __restrict__ pool, float4* strip,
-                                                    const TapK& k) {
-  const uint32_t lane = threadIdx.x & 31u;
-  const bool has = 2 * lane < sw;  // tile widths are multiples of 4 here
-  const uint8_t* col0 = tile0 + (size_t)lane * 8;
+  const uint32_t dw = d.w, dh = d.h;
+  const bool has = 2 * lane < t.tw;  // tile widths are multiples of 4 here
+  const uint8_t* col0 = img + (size_t)t.y0 * pitch + (size_t)t.x0 * 4 + (size_t)lane * 8;
+  uint32_t* dst = reinterpret_cast<uint32_t*>(payload + d.offset);
   const ulonglong2* w4 = reinterpret_cast<const ulonglong2*>(pool + ty.boff);
   const uint32_t* lo = pool + ty.boff + 4 * ty.brows_total;
   const uint32_t* rows = lo + ty.nb;
   const uint32_t* first = rows + ty.nb;
-  for (uint32_t j = 0; j < 2 && st.ob < ty.nb; ++j, ++st.ob) {
-    const uint32_t n = __ldg(rows + st.ob), r0 = __ldg(lo + st.ob);
-    const ulonglong2* wp = w4 + __ldg(first + st.ob);
-    Acc4<MODE> a0, a1;
-    for (uint32_t r = 0; r < n; ++r) {
-      const uint2 px = has ? __ldg(reinterpret_cast<const uint2*>(col0 + (size_t)(r0 + r) * pitch)) : make_uint2(0u, 0u);
-      const ulonglong2 w = __ldg(wp + r);
-      a0.step(px_to_f4<MODE>(px.x), w, k);
-      a1.step(px_to_f4<MODE>(px.y), w, k);
-    }
-    float4* srow = strip + (j * 4) * kStripStride + 2 * lane;
-    srow[0] = a0.out(0); srow[1] = a1.out(0);
-    srow[kStripStride] = a0.out(1); srow[kStripStride + 1] = a1.out(1);
-    srow[2 * kStripStride] = a0.out(2); srow[2 * kStripStride + 1] = a1.out(2);
-    srow[3 * kStripStride] = a0.out(3); srow[3 * kStripStride + 1] = a1.out(3);
-    st.o_next = min(dh, st.o_next + 4);
-  }
-}
-
-template <int MODE>
-__device__ __forceinline__ void shrink_tile_warp(const uint8_t* __restrict__ img, size_t pitch, const Tile& t,
-                                                 const pxz_block_desc& d, const HTab& ht, const AxisTab& ty,
-                                                 const uint32_t* __restrict__ pool, float4* strip, uint32_t* ring,
-                                                 uint8_t* __restrict__ payload, const TapK& k) {
-  constexpr int NC = (MODE & 1) ? 4 : 3;
-  const uint32_t lane = threadIdx.x & 31u;
-  const uint32_t sw = t.tw, sh = t.th, dw = d.w, dh = d.h;
-  const uint8_t* tile0 = img + (size_t)t.y0 * pitch + (size_t)t.x0 * 4;
-  uint32_t* dst = reinterpret_cast<uint32_t*>(payload + d.offset);
-  ShrinkRun<MODE> st;
-#pragma unroll
-  for (int c = 0; c < NC; ++c)
-#pragma unroll
-    for (int j = 0; j < 3; ++j) st.acc[0][c][j] = st.acc[1][c][j] = 0ull;
-  st.wp = reinterpret_cast<const ulonglong2*>(pool + ty.soff);
-  st.dp = pool + ty.soff + 8 * ty.n_in;
-  st.r = 0; st.pend = 0; st.o_next = 0; st.slot = 0; st.batch0 = 0; st.ob = 0;
-  st.wa_n = make_ulonglong2(0ull, 0ull); st.wb_n = 0ull; st.nd_n = 0;
-  const uint32_t slots = ty.slots;
-  // every output row keeps its own slot for the whole walk: plain loop, all rows to the strip at the end
-  const bool simple = (slots == 2 && dh <= 2) || (slots == 4 && dh <= 4);
-  if (simple) {
-    if (slots == 2) shrink_vsimple<MODE, 2>(tile0, pitch, sw, sh, dh, ty, pool, strip, ring, k);
-    else shrink_vsimple<MODE, 4>(tile0, pitch, sw, sh, dh, ty, pool, strip, ring, k);
-    st.o_next = dh;
-  } else if (slots) {
-    // cp.async ring: pair g = source rows 2g, 2g+1 (lanes 0-15 / 16-31 copy 16 bytes each); 8 pairs in flight
-    const uint32_t crow = lane >> 4, cchunk = lane & 15u;
-#pragma unroll
-    for (int g = 0; g < kRingRows / 2; ++g) {
-      const uint32_t r = 2 * g + crow;
-      if (r < sh && cchunk * 4 < sw) cp_async_16(ring + r * 64 + cchunk * 4, tile0 + (size_t)r * pitch + cchunk * 16);
-      cp_async_commit();
-    }
-    st.wa_n = __ldg(st.wp);
-    st.wb_n = slots > 4 ? __ldg(reinterpret_cast<const u64*>(st.wp + 1)) : 0ull;
-    st.nd_n = __ldg(st.dp);
-  }
-  do {
-    if (!simple) {
-      switch (slots) {
-        case 2: shrink_vrun<MODE, 2>(st, tile0, pitch, sw, sh, dh, strip, ring, k); break;
-        case 4: shrink_vrun<MODE, 4>(st, tile0, pitch, sw, sh, dh, strip, ring, k); break;
-        case 6: shrink_vrun<MODE, 6>(st, tile0, pitch, sw, sh, dh, strip, ring, k); break;
-        default: shrink_vrun_blocked<MODE>(st, tile0, pitch, sw, dh, ty, pool, strip, k); break;
+  for (uint32_t batch0 = 0, ob = 0; batch0 < dh; batch0 += kStripRows) {
+    for (uint32_t j = 0; j < 2 && ob < ty.nb; ++j, ++ob) {
+      const uint32_t n = __ldg(rows + ob), r0 = __ldg(lo + ob);
+      const ulonglong2* wp = w4 + __ldg(first + ob);
+      Acc4<MODE> a0, a1;
+      for (uint32_t r = 0; r < n; ++r) {
+        const uint2 px = has ? __ldg(reinterpret_cast<const uint2*>(col0 + (size_t)(r0 + r) * pitch)) : make_uint2(0u, 0u);
+        const ulonglong2 w = __ldg(wp + r);
+        a0.step(px_to_f4<MODE>(px.x), w, k);
+        a1.step(px_to_f4<MODE>(px.y), w, k);
       }
+      float4* srow = strip + (j * 4) * kStripStride + 2 * lane;
+      srow[0] = a0.out(0); srow[1] = a1.out(0);
+      srow[kStripStride] = a0.out(1); srow[kStripStride + 1] = a1.out(1);
+      srow[2 * kStripStride] = a0.out(2); srow[2 * kStripStride + 1] = a1.out(2);
+      srow[3 * kStripStride] = a0.out(3); srow[3 * kStripStride + 1] = a1.out(3);
     }
     __syncwarp();
-    shrink_horizontal<MODE>(strip, st.batch0, st.o_next - st.batch0, dw, ht, dst, k);
+    shrink_horizontal<MODE>(strip, batch0, min((uint32_t)kStripRows, dh - batch0), dw, ht, dst, k);
     __syncwarp();
-    st.batch0 = st.o_next;
-  } while (st.o_next < dh);
-  if (slots && !simple) cp_async_wait<0>();
+  }
 }
 
 template <bool FUSED>
@@ -452,16 +211,13 @@ __global__ void __launch_bounds__(kShrinkCtaThreads, PXZ_SHRINK_WARP_CTAS) k_shr
     const uint8_t* __restrict__ img, size_t pitch, Geom g, const pxz_block_desc* __restrict__ descs,
     const uint32_t* __restrict__ tabidx, const uint32_t* __restrict__ lists, uint32_t cap, const uint8_t* __restrict__ opaque_flags,
     uint8_t* __restrict__ payload,
-    const AxisTab* __restrict__ tabs, const uint32_t* __restrict__ pool, uint32_t* counter, float rt_one, float rt_negzero,
-    uint32_t only_noslide) {
+    const AxisTab* __restrict__ tabs, const uint32_t* __restrict__ pool, uint32_t* counter, float rt_one, float rt_negzero) {
   extern __shared__ float4 s_warp[];
   float4* strip = s_warp + (threadIdx.x >> 5) * (kShrinkWarpBytes / 16);
-  uint32_t* ring = reinterpret_cast<uint32_t*>(strip + kStripRows * kStripStride);
-  uint32_t* htab_smem = ring + kRingRows * 64;
+  uint32_t* htab_smem = reinterpret_cast<uint32_t*>(strip + kStripRows * kStripStride);
   const TapK k = make_tapk(rt_one, rt_negzero);
   pdl_wait();
   pdl_trigger();
-  const uint32_t lane = threadIdx.x & 31u;
   const uint32_t ntiles = g.cols * g.rows, total_warps = gridDim.x * kShrinkWarps;
   constexpr int F = FUSED ? 2 : 0;
   uint32_t last_tx = 0xFFFFFFFFu, last_ty = 0xFFFFFFFFu;
@@ -470,30 +226,9 @@ __global__ void __launch_bounds__(kShrinkCtaThreads, PXZ_SHRINK_WARP_CTAS) k_shr
   auto process = [&](uint32_t b, const pxz_block_desc& d, uint32_t ti) {
     const Tile t = tile_of(g, b);
     if (d.w == 0 || d.h == 0) return;  // masked out (quadtree levels)
-    // second launch behind k_shrink_tma: only the tiles whose vertical table has no slide form are left
-    if (only_noslide && ((d.w == t.tw && d.h == t.th) || tabs[ti >> 16].s2words != 0)) return;
-    if (d.w == t.tw && d.h == t.th) {
-      // block.rs:279-281: clone.  The block is contiguous in the payload (4-byte aligned only).  Two rows per
-      // instruction, 16 bytes per lane, 16 rows in flight.
-      const uint32_t rr = lane >> 4, ch = lane & 15u;
-      const bool has = ch * 4 < t.tw;
-      const uint8_t* src = img + (size_t)(t.y0 + rr) * pitch + (size_t)t.x0 * 4 + ch * 16;
-      uint32_t* dst = reinterpret_cast<uint32_t*>(payload + d.offset) + ch * 4;
-      for (uint32_t r0 = 0; r0 < t.th; r0 += 16) {
-        uint4 v[8];
-#pragma unroll
-        for (int j = 0; j < 8; ++j)
-          v[j] = (r0 + 2 * j + rr < t.th && has) ? ldg_nc_v4(src + (size_t)(r0 + 2 * j) * pitch) : make_uint4(0u, 0u, 0u, 0u);
-#pragma unroll
-        for (int j = 0; j < 8; ++j) {
-          if (r0 + 2 * j + rr < t.th && has) {
-            uint32_t* o = dst + (size_t)(r0 + 2 * j + rr) * t.tw;
-            o[0] = v[j].x; o[1] = v[j].y; o[2] = v[j].z; o[3] = v[j].w;
-          }
-        }
-      }
-      return;
-    }
+    // launched behind k_shrink_tma, which copies the full-size blocks and shrinks every tile whose vertical table has a
+    // slide2 form
+    if ((d.w == t.tw && d.h == t.th) || tabs[ti >> 16].s2words != 0) return;
     // tiles come in cost order, so a warp's consecutive tiles mostly share their tables: keep them
     if ((ti >> 16) != last_ty) {
       ty = tabs[ti >> 16];
@@ -506,8 +241,8 @@ __global__ void __launch_bounds__(kShrinkCtaThreads, PXZ_SHRINK_WARP_CTAS) k_shr
       last_tx = ti & 0xFFFFu;
     }
     const bool opaque = opaque_flags != nullptr && opaque_flags[b] != 0;
-    if (opaque) shrink_tile_warp<F>(img, pitch, t, d, ht, ty, pool, strip, ring, payload, k);
-    else shrink_tile_warp<F | 1>(img, pitch, t, d, ht, ty, pool, strip, ring, payload, k);
+    if (opaque) shrink_tile_warp<F>(img, pitch, t, d, ht, ty, pool, strip, payload, k);
+    else shrink_tile_warp<F | 1>(img, pitch, t, d, ht, ty, pool, strip, payload, k);
   };
   // Tiles are drawn in the order of the `order` list (most expensive first, so the kernel does not end on a few warps
   // that drew a 20-microsecond tile last); the next tile's index, descriptor and table indices are requested while the

@@ -167,8 +167,8 @@ bool build_axis_table(uint32_t n_in, uint32_t n_out, int filter, std::vector<uin
   pool->insert(pool->end(), first.begin(), first.end());
   tab->bwords = (uint32_t)(pool->size() - w4base);
 
-  // ---- slide form (see pxz_internal.h) ----
-  tab->soff = 0;
+  // ---- slide2 form (see pxz_internal.h) ----
+  tab->pad1_ = 0;
   tab->slots = 0;
   tab->goff = 0xFFFFFFFFu;
   tab->gpoff = 0;
@@ -205,30 +205,16 @@ bool build_axis_table(uint32_t n_in, uint32_t n_out, int filter, std::vector<uin
     if (ok && slots) {
       // with windows ordered on both ends the live outputs at any sample are consecutive, so o % slots never collides
       while (pool->size() % 4) pool->push_back(0u);
-      const size_t sbase = pool->size();
-      pool->resize(sbase + (size_t)n_in * 8 + n_in, 0u);
-      for (uint32_t o = 0; o < n_out; ++o) {
-        for (uint32_t r = tl[o]; r < tr[o]; ++r)
-          (*pool)[sbase + (size_t)r * 8 + (o % slots)] = (*pool)[wbase + (size_t)o * stride + (r - lefts[o])];
-        (*pool)[sbase + (size_t)n_in * 8 + (tr[o] - 1)] += 1u;
-      }
-      pool->resize(pool->size() + 12, 0u);  // the kernels prefetch one table row (and one count) past the end
-      tab->soff = (uint32_t)sbase;
-      tab->slots = slots;
-      // ---- slide2 form (k_shrink_tma): the same rows with every weight stored twice, (w, w) = one f32x2 operand
-      // whose lanes are two image columns, `slots` pairs per row, then end[n_out] = the source sample that holds
-      // output o's last tap.  Staged into shared memory per warp with one bulk copy (16-byte multiple).
-      while (pool->size() % 4) pool->push_back(0u);
       const size_t s2 = pool->size();
       pool->resize(s2 + (size_t)n_in * slots * 2, 0u);
-      for (uint32_t r = 0; r < n_in; ++r)
-        for (uint32_t s = 0; s < slots; ++s) {
-          const uint32_t wbits = (*pool)[sbase + (size_t)r * 8 + s];
-          (*pool)[s2 + ((size_t)r * slots + s) * 2] = wbits;
-          (*pool)[s2 + ((size_t)r * slots + s) * 2 + 1] = wbits;
+      for (uint32_t o = 0; o < n_out; ++o)
+        for (uint32_t r = tl[o]; r < tr[o]; ++r) {
+          const size_t at = s2 + ((size_t)r * slots + o % slots) * 2;
+          (*pool)[at] = (*pool)[at + 1] = (*pool)[wbase + (size_t)o * stride + (r - lefts[o])];
         }
       for (uint32_t o = 0; o < n_out; ++o) pool->push_back(tr[o] - 1);
       while (pool->size() % 4) pool->push_back(0u);
+      tab->slots = slots;
       tab->s2off = (uint32_t)s2;
       tab->s2words = (uint32_t)(pool->size() - s2);
     }

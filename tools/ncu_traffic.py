@@ -7,7 +7,7 @@ import subprocess
 import sys
 
 NAMES = {"k_analyze_mad_rgba": "analyze_mad_fast", "k_band_list": "band_list", "k_mad_exact": "mad_exact", "k_plan": "plan",
-         "k_shrink_tma": "resample_down", "k_shrink_warp": "resample_down_ring", "k_expand_warp": "resample_up",
+         "k_shrink_tma": "resample_down", "k_shrink_warp": "resample_down_noslide", "k_expand_warp": "resample_up",
          "k_analyze_sobel_tma": "analyze_sobel"}
 out = subprocess.run(["ncu", "-i", sys.argv[1], "--page", "raw", "--csv"], capture_output=True, text=True).stdout
 rows = list(csv.reader(io.StringIO(out)))
