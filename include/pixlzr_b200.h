@@ -138,7 +138,12 @@ void pxz_host_free(void* p);
 pxz_status pxz_image_upload(pxz_ctx* ctx, const uint8_t* host, uint32_t w, uint32_t h, uint32_t channels /* 3|4 */,
                             size_t host_pitch, pxz_image** out);
 pxz_status pxz_image_alloc(pxz_ctx* ctx, uint32_t w, uint32_t h, uint32_t channels, pxz_image** out);
-/* non-owning view of device memory the caller keeps alive (e.g. a torch uint8 tensor) */
+/* non-owning view of device memory the caller keeps alive (e.g. a torch uint8 tensor).  Layout: any base address and any
+ * pitch >= w * channels work for pxz_analyze and pxz_image_error, and for every call on an RGB view.  An RGBA view that is
+ * shrunk (pxz_shrink*, pxz_rd_curve, pxz_rdo_*, pxz_strategy_measure, pxz_tree_process) or expanded into
+ * (pxz_expand_to_image, pxz_expand_batch, pxz_expand_region, pxz_tree_process's output) needs a base address and a pitch
+ * that are multiples of 4; otherwise those calls return PXZ_E_UNSUPPORTED and leave the view unwritten.  Base and pitch
+ * multiples of 16 select the fastest kernels. */
 pxz_status pxz_image_wrap(pxz_ctx* ctx, void* device_ptr, uint32_t w, uint32_t h, uint32_t channels, size_t pitch,
                           pxz_image** out);
 pxz_status pxz_image_info(const pxz_image* img, uint32_t* w, uint32_t* h, uint32_t* channels, size_t* pitch,

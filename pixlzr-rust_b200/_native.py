@@ -464,7 +464,8 @@ class Image:
 
     def free(self):
         if self._h:
-            lib().pxz_image_free(self._h)
+            if self.ctx.handle:  # see Payload.free
+                lib().pxz_image_free(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):
@@ -570,7 +571,11 @@ class Payload:
 
     def free(self):
         if self._h:
-            lib().pxz_payload_free(self._h)
+            # pxz_payload_free returns the buffers to the context (its cache, its stream).  Once the context is closed — or
+            # finalised first, as the garbage collector may do with a cycle holding both — the handle is only dropped: its
+            # device memory stays allocated until the process ends.
+            if self.ctx.handle:
+                lib().pxz_payload_free(self._h)
             self._h = C.c_void_p()
 
     def __del__(self):

@@ -377,9 +377,19 @@ pxz_status get_tabset(pxz_ctx* ctx, const TabSpec& spec, int filter, int directi
   return PXZ_OK;
 }
 
+// The 4-channel resample kernels move pixels as 32-bit words, so an RGBA image that is shrunk or expanded needs a 4-byte
+// aligned base and pitch.  One rule for both resize semantics; analysis and pxz_image_error read bytes and take any layout.
+static pxz_status check_resample_layout(pxz_ctx* ctx, uint32_t channels, const uint8_t* d, size_t pitch) {
+  if (channels == 4 && ((reinterpret_cast<uintptr_t>(d) | pitch) & 3u) != 0)
+    return fail(ctx, PXZ_E_UNSUPPORTED, "an RGBA image that is shrunk or expanded needs a base address and a pitch that are multiples of 4");
+  return PXZ_OK;
+}
+
 pxz_status run_resample(pxz_ctx* ctx, int direction, uint8_t* img, size_t pitch, const pxz_payload* p, const TabSet& ts,
                         uint32_t max_src_px, uint32_t max_src_dim, uint32_t max_tmp_px, const uint8_t* opaque_flags = nullptr) {
   const Geom& g = p->g;
+  const pxz_status layout = check_resample_layout(ctx, g.C, img, pitch);
+  if (layout != PXZ_OK) return layout;
   const uint32_t nblocks = g.cols * g.rows;
   if (ctx->resize_semantics == PXZ_RESIZE_FIR) {
     // integer convolution, horizontal pass first: its own kernel (one CTA per block, source + u8 intermediate in smem)
@@ -2136,6 +2146,9 @@ pxz_status pxz_expand_region(pxz_ctx* ctx, const pxz_payload* p, pxz_filter filt
   if (w == 0 || h == 0) return fail(ctx, PXZ_E_ARG, "empty rectangle");
   if (x >= pg.W || y >= pg.H || w > pg.W - x || h > pg.H - y) return fail(ctx, PXZ_E_ARG, "rectangle outside the image");
   if (out->w != w || out->h != h || out->c != pg.C || out->nimg != 1) return fail(ctx, PXZ_E_ARG, "output image geometry mismatch");
+  // refused on every path, the staged copy below included
+  const pxz_status layout = check_resample_layout(ctx, out->c, out->d, out->pitch);
+  if (layout != PXZ_OK) return layout;
   if (x == 0 && y == 0 && w == pg.W && h == pg.H) return pxz_expand_to_image(ctx, p, filter_up, out);
   const uint32_t c0 = x / pg.bw, r0 = y / pg.bh;
   const uint32_t nc = (x + w - 1) / pg.bw - c0 + 1, nr = (y + h - 1) / pg.bh - r0 + 1;
@@ -2163,6 +2176,10 @@ pxz_status pxz_tree_process(pxz_ctx* ctx, const pxz_image* img, float threshold,
   if (out->w != img->w || out->h != img->h || out->c != img->c) return fail(ctx, PXZ_E_ARG, "output image geometry mismatch");
   if (img->nimg != 1 || out->nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "tree processing takes one image at a time");
   if (bw == 0 || bh == 0) return fail(ctx, PXZ_E_ARG, "block size must be >= 1");
+  // before the copy below, so that a refused call leaves `out` untouched
+  pxz_status st = check_resample_layout(ctx, img->c, img->d, img->pitch);
+  if (st == PXZ_OK) st = check_resample_layout(ctx, out->c, out->d, out->pitch);
+  if (st != PXZ_OK) return st;
   // unchanged pixels (blocks that reach the minimum size, tree.rs:35-37) come straight from the source
   PXZ_CUDA(ctx, cudaMemcpy2DAsync(out->d, out->pitch, img->d, img->pitch, (size_t)img->w * img->c, img->h, cudaMemcpyDeviceToDevice,
                                   ctx->stream));
@@ -2181,7 +2198,7 @@ pxz_status pxz_tree_process(pxz_ctx* ctx, const pxz_image* img, float threshold,
   uint8_t* d_leaf = nullptr;
   uint8_t* d_rec[2] = {nullptr, nullptr};
   Geom gl;
-  pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw >> (levels - 1), bh >> (levels - 1), &gl);
+  st = make_geom(ctx, img->w, img->h, img->c, bw >> (levels - 1), bh >> (levels - 1), &gl);
   if (st != PXZ_OK) return st;
   const size_t max_blocks = (size_t)gl.cols * gl.rows;
   if ((st = bufs.alloc(&d_leaf, max_blocks)) != PXZ_OK || (st = bufs.alloc(&d_rec[0], max_blocks)) != PXZ_OK ||

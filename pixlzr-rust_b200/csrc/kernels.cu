@@ -273,7 +273,7 @@ __global__ void __launch_bounds__(kThreads, PXZ_MAD_MINBLOCKS) k_analyze_mad_rgb
   const uint32_t qpr = g.bw >> 2;  // quads (4 px = 16 B) per full tile row
   // this thread's quads: the (row, column) mapping does not depend on the tile
   uint32_t qrc[QPT];   // row << 16 | first column
-  uint32_t qoff[QPT];  // byte offset inside the tile (tile rows * pitch < 2^32, checked by the launcher)
+  uint32_t qoff[QPT];  // byte offset inside the tile ((bh - 1) * pitch + bw * 4 < 2^32, checked by the launcher)
   bool all_in = true;  // every quad of this thread lies inside a FULL tile
 #pragma unroll
   for (int j = 0; j < QPT; ++j) {
@@ -2697,8 +2697,11 @@ cudaError_t launch_analyze_mad_fast(const uint8_t* img, size_t pitch, const Geom
   const bool aligned = g.C == 4 && (g.bw % 4 == 0) && (g.W % 4 == 0) && (pitch % 16 == 0) &&
                        ((reinterpret_cast<uintptr_t>(img) & 15u) == 0);
   const uint32_t quads = (g.bw / 4) * g.bh;
+  // k_analyze_mad_rgba keeps in-tile byte offsets in 32 bits; a wider tile (a view into a very wide tensor) takes
+  // k_analyze_mad_any, which addresses with size_t
+  const bool offsets32 = (size_t)(g.bh - 1) * pitch + (size_t)g.bw * 4 <= 0xFFFFFFFFull;
   ++*launches;
-  if (aligned && quads <= 1024) {
+  if (aligned && offsets32 && quads <= 1024) {
     // G threads per tile, <= 4 quads (16 px) per thread; 256 / G tiles per CTA
     struct Variant {
       void (*kernel)(const uint8_t*, size_t, Geom, float*, uint8_t*, uint32_t*);
