@@ -21,6 +21,7 @@ from __future__ import annotations
 
 import enum
 import os
+from contextlib import contextmanager
 from dataclasses import dataclass
 from typing import List, Optional, Tuple
 
@@ -107,6 +108,19 @@ def _check_image(image: np.ndarray) -> np.ndarray:
     if image.shape[0] == 0 or image.shape[1] == 0:
         raise ValueError("empty image")
     return np.ascontiguousarray(image)
+
+
+@contextmanager
+def _on_device(image, ctx: N.Context):
+    """`image` as a device image: a device image as it is, a numpy image uploaded for the block and freed after it."""
+    if isinstance(image, N.Image):
+        yield image
+        return
+    img = ctx.image_upload(_check_image(image))
+    try:
+        yield img
+    finally:
+        img.free()
 
 
 def _check_rect(width: int, height: int, x: int, y: int, w: int, h: int) -> None:
@@ -232,14 +246,10 @@ def rd_curve(image, block_width: int, block_height: int, filter_down: FilterType
     """EXTENSION: the exact (bytes, squared error) curve of shrink_by (or shrink_directionally) with `filter_down` and a decode
     with `filter_up`, over every finite factor, computed on the device (numpy or device image)."""
     ctx = ctx or (image.ctx if isinstance(image, N.Image) else default_context())
-    img = image if isinstance(image, N.Image) else ctx.image_upload(_check_image(image))
-    try:
+    with _on_device(image, ctx) as img:
         metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
         factor, nbytes, sse = img.rd_curve(block_width, block_height, metric, int(filter_down), int(filter_up), 0)
         return RateDistortion(factor, nbytes, sse, img.w * img.h * img.c)
-    finally:
-        if img is not image:
-            img.free()
 
 
 @dataclass
@@ -272,13 +282,9 @@ def rdo_curve(image, block_width: int, block_height: int, filter_down: FilterTyp
     """EXTENSION: the rate-distortion optimised (bytes, squared error) curve of an image when each block's size is chosen on its
     own, shrunk with `filter_down` and decoded with `filter_up`, computed on the device (numpy or device image)."""
     ctx = ctx or (image.ctx if isinstance(image, N.Image) else default_context())
-    img = image if isinstance(image, N.Image) else ctx.image_upload(_check_image(image))
-    try:
+    with _on_device(image, ctx) as img:
         nbytes, sse = img.rdo_curve(block_width, block_height, int(filter_down), int(filter_up))
         return OptimalCurve(nbytes, sse, img.w * img.h * img.c)
-    finally:
-        if img is not image:
-            img.free()
 
 
 @dataclass
@@ -306,34 +312,17 @@ def image_error(a, b, block_width: int, block_height: int, ctx: Optional[N.Conte
     """EXTENSION: per-block squared error and largest difference of `a` against `b` (numpy images or device images of one
     geometry), computed on the device in one streaming pass; only the per-block figures come back."""
     ctx = ctx or (a.ctx if isinstance(a, N.Image) else default_context())
-    owned = []
-
-    def on_device(x):
-        if isinstance(x, N.Image):
-            return x
-        owned.append(ctx.image_upload(_check_image(x)))
-        return owned[-1]
-
-    try:
-        da, db = on_device(a), on_device(b)
+    with _on_device(a, ctx) as da, _on_device(b, ctx) as db:
         sse, mx, total = da.error(db, block_width, block_height)
         return ErrorReport(sse, mx, total, da.w * da.h * da.c)
-    finally:
-        for x in owned:
-            x.free()
 
 
 def payload_error(payload: N.Payload, source, filter_up: FilterType) -> ErrorReport:
     """EXTENSION: the error of a payload's decode with `filter_up` against its source image (numpy or device image), on the
     payload's block grid (Payload.error): the decode stays on the device."""
-    ctx = payload.ctx
-    src = source if isinstance(source, N.Image) else ctx.image_upload(_check_image(source))
-    try:
+    with _on_device(source, payload.ctx) as src:
         sse, mx, total = payload.error(src, int(filter_up))
         return ErrorReport(sse, mx, total, src.w * src.h * src.c)
-    finally:
-        if src is not source:
-            src.free()
 
 
 class Pixlzr:
@@ -426,18 +415,23 @@ class Pixlzr:
     def _shrink(self, metric: int, filter_downscale: FilterType, factor: float, flags: int):
         if self._image is None:
             return self._reshrink_blocks(metric, filter_downscale, factor, flags)
-        ctx = self._ctx()
-        img = ctx.image_upload(self._image)
-        try:
-            pl = img.shrink(self.block_width, self.block_height, metric, factor, int(filter_downscale), flags)
+        self._encode_source("shrink", lambda img: (img.shrink(self.block_width, self.block_height, metric, factor, int(filter_downscale),
+                                                              flags),))
+
+    def _encode_source(self, name: str, encode) -> tuple:
+        """Uploads the source image, runs `encode(img)`, which returns a tuple whose first item is a payload, and adopts that
+        payload as this Pixlzr's blocks; returns the tuple's other items.  Refused on a decoded or already shrunk Pixlzr."""
+        if self._image is None:
+            raise ValueError(f"{name} needs the source image (Pixlzr.from_image), not a decoded or already shrunk one")
+        with _on_device(self._image, self._ctx()) as img:
+            out = encode(img)
             try:
-                self._descs, self._pixels = pl.download()
+                self._descs, self._pixels = out[0].download()
             finally:
-                pl.free()
-        finally:
-            img.free()
+                out[0].free()
         self._values_present = True
         self._image = None
+        return out[1:]
 
     def _reshrink_blocks(self, metric: int, filter_downscale: FilterType, factor: float, flags: int):
         """Shrinks blocks that are no longer windows of the source image (an already shrunk or decoded Pixlzr): the
@@ -502,22 +496,10 @@ class Pixlzr:
         """EXTENSION (rate control): shrink_by (or shrink_directionally) with the largest factor whose payload has at most
         `max_bytes` bytes; returns that factor (pxz_shrink_to_size).  shrink_by / shrink_directionally with the returned
         factor give the same blocks.  Needs the source image: refused on a decoded or already shrunk Pixlzr."""
-        if self._image is None:
-            raise ValueError("shrink_to_size needs the source image (Pixlzr.from_image), not a decoded or already shrunk one")
-        ctx = self._ctx()
-        img = ctx.image_upload(self._image)
-        try:
-            metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
-            pl, k = img.shrink_to_size(self.block_width, self.block_height, metric, max_bytes, int(filter_downscale),
-                                       N.FLAG_EXACT_VALUES if exact_values else 0)
-            try:
-                self._descs, self._pixels = pl.download()
-            finally:
-                pl.free()
-        finally:
-            img.free()
-        self._values_present = True
-        self._image = None
+        metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
+        flags = N.FLAG_EXACT_VALUES if exact_values else 0
+        k, = self._encode_source("shrink_to_size", lambda img: img.shrink_to_size(self.block_width, self.block_height, metric, max_bytes,
+                                                                                  int(filter_downscale), flags))
         return k
 
     def shrink_to_psnr(self, filter_downscale: FilterType, filter_upscale: FilterType, psnr: float, directionally: bool = False,
@@ -526,54 +508,26 @@ class Pixlzr:
         `filter_upscale` reaches `psnr` dB against the source (sse_budget; pxz_shrink_to_error); returns that factor, which is
         also the smallest payload reaching the target.  shrink_by / shrink_directionally with the returned factor give the same
         blocks.  Needs the source image: refused on a decoded or already shrunk Pixlzr."""
-        if self._image is None:
-            raise ValueError("shrink_to_psnr needs the source image (Pixlzr.from_image), not a decoded or already shrunk one")
-        ctx = self._ctx()
-        img = ctx.image_upload(self._image)
-        try:
-            metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
-            pl, k, _ = img.shrink_to_error(self.block_width, self.block_height, metric, sse_budget(psnr, img.w * img.h * img.c),
-                                           int(filter_downscale), int(filter_upscale), N.FLAG_EXACT_VALUES if exact_values else 0)
-            try:
-                self._descs, self._pixels = pl.download()
-            finally:
-                pl.free()
-        finally:
-            img.free()
-        self._values_present = True
-        self._image = None
+        metric = N.METRIC_SOBEL_DIR if directionally else N.METRIC_OKLAB_MAD
+        flags = N.FLAG_EXACT_VALUES if exact_values else 0
+        k, _ = self._encode_source("shrink_to_psnr", lambda img: img.shrink_to_error(
+            self.block_width, self.block_height, metric, sse_budget(psnr, img.w * img.h * img.c), int(filter_downscale),
+            int(filter_upscale), flags))
         return k
 
     def shrink_optimally_to_size(self, filter_downscale: FilterType, filter_upscale: FilterType, max_bytes: int) -> Tuple[int, int]:
         """EXTENSION (optimised encode): each block at its own size, the least error of a decode with `filter_upscale` within
         `max_bytes` payload bytes (pxz_rdo_shrink_to_size); returns (payload bytes, squared error).  Needs the source image:
         refused on a decoded or already shrunk Pixlzr."""
-        return self._shrink_optimally("shrink_optimally_to_size", "rdo_shrink_to_size", filter_downscale, filter_upscale,
-                                      lambda img: max_bytes)
+        return self._encode_source("shrink_optimally_to_size", lambda img: img.rdo_shrink_to_size(
+            self.block_width, self.block_height, max_bytes, int(filter_downscale), int(filter_upscale)))
 
     def shrink_optimally_to_psnr(self, filter_downscale: FilterType, filter_upscale: FilterType, psnr: float) -> Tuple[int, int]:
         """EXTENSION (optimised encode): each block at its own size, the fewest payload bytes whose decode with `filter_upscale`
         reaches `psnr` dB against the source (sse_budget; pxz_rdo_shrink_to_error); returns (payload bytes, squared error).
         Needs the source image: refused on a decoded or already shrunk Pixlzr."""
-        return self._shrink_optimally("shrink_optimally_to_psnr", "rdo_shrink_to_error", filter_downscale, filter_upscale,
-                                      lambda img: sse_budget(psnr, img.w * img.h * img.c))
-
-    def _shrink_optimally(self, name: str, call: str, filter_downscale: FilterType, filter_upscale: FilterType, budget) -> Tuple[int, int]:
-        if self._image is None:
-            raise ValueError(f"{name} needs the source image (Pixlzr.from_image), not a decoded or already shrunk one")
-        ctx = self._ctx()
-        img = ctx.image_upload(self._image)
-        try:
-            pl, nbytes, sse = getattr(img, call)(self.block_width, self.block_height, budget(img), int(filter_downscale), int(filter_upscale))
-            try:
-                self._descs, self._pixels = pl.download()
-            finally:
-                pl.free()
-        finally:
-            img.free()
-        self._values_present = True
-        self._image = None
-        return nbytes, sse
+        return self._encode_source("shrink_optimally_to_psnr", lambda img: img.rdo_shrink_to_error(
+            self.block_width, self.block_height, sse_budget(psnr, img.w * img.h * img.c), int(filter_downscale), int(filter_upscale)))
 
     def shrink_directionally(self, filter_downscale: FilterType, factor: float):
         """Pixlzr::shrink_directionally (pixlzr.rs:187-205)."""

@@ -209,11 +209,8 @@ def run(args) -> None:
     err = region_error(args) or payload_bytes_error(args) or target_psnr_error(args) or optimal_error(args) or psnr_error(args)
     if err:
         raise ValueError(err)
-    if args.optimal:
-        _run_optimal(args, bw, bh, filt, dst)
-        return
-    if args.target_psnr is not None:
-        _run_psnr_target(args, bw, bh, filt, dst)
+    if args.optimal or args.target_psnr is not None:
+        _run_budgeted(args, bw, bh, filt, dst)
         return
     if args.payload_bytes is not None:
         _run_sized(args, bw, bh, filt, src, dst)
@@ -263,47 +260,29 @@ def _run_sized(args, bw: int, bh: int, filt, src: str, dst: str) -> None:
     print(f"shrinking factor: {api.format_shrinking_factor(k)}")
 
 
-def _run_psnr_target(args, bw: int, bh: int, filt, dst: str) -> None:
-    """image -> container / image with the smallest factor whose decode with -f (the filter a decoder of the written file uses)
-    reaches --target-psnr; prints the factor in a form -k reads back, the payload bytes and the PSNR reached."""
+def _run_budgeted(args, bw: int, bh: int, filt, dst: str) -> None:
+    """image -> container / image for a budget on the decode with -f (the filter a decoder of the written file uses).  Without
+    --optimal: the smallest factor whose decode reaches --target-psnr; prints the factor in a form -k reads back.  With
+    --optimal: every block's size chosen for --payload-bytes (the least error within N bytes) or --target-psnr (the fewest
+    bytes reaching it).  Then prints the payload bytes and the PSNR reached."""
     image = _open_image(args.input)
     ctx = api.default_context()
     img = ctx.image_upload(image)
+    k = nbytes = None
     try:
         samples = img.w * img.h * img.c
-        metric = api.N.METRIC_SOBEL_DIR if args.direction_wise else api.N.METRIC_OKLAB_MAD
-        pl, k, sse = img.shrink_to_error(bw, bh, metric, api.sse_budget(args.target_psnr, samples), int(filt), int(filt), 0)
-    finally:
-        img.free()
-    try:
-        nbytes = pl.info()["bytes"]
-        if dst == "pix":
-            with open(args.output, "wb") as f:
-                f.write(pl.to_container(0, True))
-        else:
-            _save_image(args.output, pl.expand(int(filt)))
-    finally:
-        pl.free()
-    print(f"shrinking factor: {api.format_shrinking_factor(k)}")
-    print(f"payload bytes: {nbytes}")
-    print(f"psnr: {format_psnr(api.psnr_of(sse, samples))} dB")
-
-
-def _run_optimal(args, bw: int, bh: int, filt, dst: str) -> None:
-    """image -> container / image with every block's size chosen for --payload-bytes (the least error of a decode with -f
-    within N bytes) or --target-psnr (the fewest bytes reaching it); prints the payload bytes and the PSNR reached."""
-    image = _open_image(args.input)
-    ctx = api.default_context()
-    img = ctx.image_upload(image)
-    try:
-        samples = img.w * img.h * img.c
-        if args.payload_bytes is not None:
+        if not args.optimal:
+            metric = api.N.METRIC_SOBEL_DIR if args.direction_wise else api.N.METRIC_OKLAB_MAD
+            pl, k, sse = img.shrink_to_error(bw, bh, metric, api.sse_budget(args.target_psnr, samples), int(filt), int(filt), 0)
+        elif args.payload_bytes is not None:
             pl, nbytes, sse = img.rdo_shrink_to_size(bw, bh, args.payload_bytes, int(filt), int(filt))
         else:
             pl, nbytes, sse = img.rdo_shrink_to_error(bw, bh, api.sse_budget(args.target_psnr, samples), int(filt), int(filt))
     finally:
         img.free()
     try:
+        if nbytes is None:
+            nbytes = pl.info()["bytes"]
         if dst == "pix":
             with open(args.output, "wb") as f:
                 f.write(pl.to_container(0, True))
@@ -311,6 +290,8 @@ def _run_optimal(args, bw: int, bh: int, filt, dst: str) -> None:
             _save_image(args.output, pl.expand(int(filt)))
     finally:
         pl.free()
+    if k is not None:
+        print(f"shrinking factor: {api.format_shrinking_factor(k)}")
     print(f"payload bytes: {nbytes}")
     print(f"psnr: {format_psnr(api.psnr_of(sse, samples))} dB")
 

@@ -254,6 +254,14 @@ struct DevBlocks {
     *out = static_cast<T*>(q);
     return PXZ_OK;
   }
+  // one block holding the arrays of `layout`, their pointers set
+  template <class... T>
+  pxz_status alloc(const Layout<T...>& layout) {
+    uint8_t* q = nullptr;
+    const pxz_status st = alloc(&q, layout.bytes());
+    if (st == PXZ_OK) layout.place(q);
+    return st;
+  }
   void keep() { n = 0; }  // the blocks have another owner now
 };
 
@@ -979,23 +987,23 @@ static pxz_status payload_rechannel(pxz_ctx* ctx, const pxz_payload* src, uint32
   return PXZ_OK;
 }
 
-// An RGB image on the RGBA fast kernels: widen it to RGBA (alpha 255: its metric term is exactly +0 and the opaque resample
-// path never touches it), run `encode` on the 4-channel image, narrow the payload back
+// Runs `body(image, bpp, out)` on the image the kernels take for blocks of bw x bh.  An RGB image that rgb_on_rgba selects is
+// widened to RGBA: alpha 255 adds exactly +0 to the metric and to every error sum, and the opaque resample path never touches
+// it.  bpp is the source's channel count, the bytes per pixel that byte counts use.  A payload `body` returns is narrowed
+// back to the source's channels; out may be NULL when the call returns no payload.
 extern "C++" {  // a template inside the extern "C" block
-static pxz_status rgb_widened(pxz_ctx* ctx, const pxz_image* img, ImageOwner* wide) {
-  pxz_status st = image_new(ctx, img->w, img->h, 4, img->nimg, wide);
-  if (st != PXZ_OK) return st;
-  cudaError_t e = launch_rgb_widen(img->d, img->pitch, (*wide)->d, (*wide)->pitch, img->w, img->h * img->nimg, 1, ctx->stream, ctx->sm_count,
-                                   &ctx->launches);
-  return e == cudaSuccess ? PXZ_OK : cuda_fail(ctx, e, "rgb widen");
-}
 template <class F>
-static pxz_status encode_via_rgba(pxz_ctx* ctx, const pxz_image* img, F&& encode, pxz_payload** out) {
+static pxz_status on_kernel_image(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_payload** out, F&& body) {
+  if (!rgb_on_rgba(ctx, img->w, img->c, bw, bh)) return body(img, img->c, out);
   ImageOwner wide;
-  pxz_status st = rgb_widened(ctx, img, &wide);
+  pxz_status st = image_new(ctx, img->w, img->h, 4, img->nimg, &wide);
   if (st != PXZ_OK) return st;
+  const cudaError_t e = launch_rgb_widen(img->d, img->pitch, wide->d, wide->pitch, img->w, img->h * img->nimg, 1, ctx->stream, ctx->sm_count,
+                                         &ctx->launches);
+  if (e != cudaSuccess) return cuda_fail(ctx, e, "rgb widen");
+  if (!out) return body(wide.get(), img->c, nullptr);
   pxz_payload* raw = nullptr;
-  st = encode(wide.get(), &raw);
+  st = body(wide.get(), img->c, &raw);
   wide.reset();  // stream-ordered: the kernels queued above keep it
   const PayloadOwner p4(raw);
   if (st != PXZ_OK) return st;
@@ -1005,6 +1013,25 @@ static pxz_status encode_via_rgba(pxz_ctx* ctx, const pxz_image* img, F&& encode
   return st;
 }
 }  // extern "C++"
+
+// The shared refusals of the rate-control calls, in this order, before anything is allocated or launched.  `what` names the
+// call in the messages ("a size budget"); `checks` adds the checks that only some calls make.
+enum RateChecks : uint32_t { kCheckDown = 1, kCheckUp = 2, kCheckMetric = 4, kCheckAfterIdentity = 8, kCheckStrategy = 16 };
+static pxz_status rate_refusal(pxz_ctx* ctx, const pxz_image* img, const char* what, uint32_t checks, pxz_filter filter_down,
+                               pxz_filter filter_up, pxz_metric metric, uint32_t flags) {
+  const std::string call(what);
+  if (((checks & kCheckDown) && !known_filter(filter_down)) || ((checks & kCheckUp) && !known_filter(filter_up)))
+    return fail(ctx, PXZ_E_ARG, "unknown filter");
+  if ((checks & kCheckMetric) && metric != PXZ_METRIC_OKLAB_MAD && metric != PXZ_METRIC_SOBEL_DIR) return fail(ctx, PXZ_E_ARG, "unknown metric");
+  if ((checks & kCheckAfterIdentity) && (flags & PXZ_FLAG_AFTER_IDENTITY))
+    return fail(ctx, PXZ_E_ARG, call + " needs the factor, which PXZ_FLAG_AFTER_IDENTITY ignores");
+  if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, call + " is per image: not available on a batch");
+  if ((flags & PXZ_FLAG_NORMALISE_GLOBAL) && ctx->comm)
+    return fail(ctx, PXZ_E_UNSUPPORTED, call + " with global normalisation over a communicator is not available");
+  if ((checks & kCheckStrategy) && ctx->strategy.on)
+    return fail(ctx, PXZ_E_UNSUPPORTED, call + " with a strategy installed is not available (its filter pair follows the stored value)");
+  return PXZ_OK;
+}
 
 static ValueMap shrink_value_map(const pxz_ctx* ctx, pxz_metric metric, uint32_t flags, float factor) {
   ValueMap vm;
@@ -1089,33 +1116,15 @@ static pxz_status plan_and_resample(pxz_ctx* ctx, const pxz_image* img, const Ge
   return PXZ_OK;
 }
 
-pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
-                      pxz_filter filter_down, uint32_t flags, pxz_payload** out) {
-  if (!ctx || !img || !out) return PXZ_E_ARG;
-  *out = nullptr;
-  cudaSetDevice(ctx->device);
-  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh))
-    return encode_via_rgba(
-        ctx, img, [&](const pxz_image* wide, pxz_payload** p4) { return pxz_shrink(ctx, wide, bw, bh, metric, factor, filter_down, flags, p4); },
-        out);
+// pxz_shrink up to its result; *exchanged: this rank reached the min/max exchange
+static pxz_status shrink_image(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor, pxz_filter filter_down,
+                               uint32_t flags, bool* exchanged, pxz_payload** out) {
   const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
-  // Every rank of a communicator must reach the min/max exchange, whatever happens to it before: a rank-local failure
-  // (an unknown filter, a trailing block the Sobel metric cannot take, no memory) joins with neutral values and an
-  // error flag instead of leaving its peers in the collective.
-  auto bail = [&](pxz_status why) -> pxz_status {
-    if (normalise && ctx->comm) {
-      const std::string msg = ctx->err;
-      bool peers_ok = true;
-      exchange_minmax(ctx, false, &peers_ok);
-      ctx->err = msg;
-    }
-    return why;
-  };
-  if (!known_filter(filter_down)) return bail(fail(ctx, PXZ_E_ARG, "unknown filter"));
+  if (!known_filter(filter_down)) return fail(ctx, PXZ_E_ARG, "unknown filter");
   Geom g;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g, img->nimg);
-  if (st != PXZ_OK) return bail(st);
-  if (normalise && img->nimg > 1) return bail(fail(ctx, PXZ_E_UNSUPPORTED, "global normalisation is per image: not available on a batch"));
+  if (st != PXZ_OK) return st;
+  if (normalise && img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "global normalisation is per image: not available on a batch");
 
   const ValueMap vm = shrink_value_map(ctx, metric, flags, factor);
 
@@ -1126,36 +1135,44 @@ pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t 
   // them, and the guard band (scaled by 1 / range) then decides as in the default mode which tiles need their
   // reference-order value; with PXZ_FLAG_EXACT_VALUES every tile is computed in reference order as before.
   const bool fast_norm = normalise && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
-  st = run_shrink_analysis(ctx, img, g, metric, flags, &vm);
-  if (st != PXZ_OK) return bail(st);
-
-  if (normalise) {
-    bool peers_ok = true;
-    st = exchange_minmax(ctx, true, &peers_ok);
+  return on_kernel_image(ctx, img, bw, bh, out, [&](const pxz_image* im, uint32_t, pxz_payload** p) {
+    g.C = im->c;
+    pxz_status st = run_shrink_analysis(ctx, im, g, metric, flags, &vm);
     if (st != PXZ_OK) return st;
-    if (!peers_ok) return fail(ctx, PXZ_E_NCCL, "another rank failed before the min/max exchange");
-    if (fast_norm && (st = run_guard_band(ctx, img, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
-  }
-  return plan_and_resample(ctx, img, g, metric, vm, filter_down, exact_all, out);
+    if (normalise) {
+      *exchanged = true;
+      bool peers_ok = true;
+      st = exchange_minmax(ctx, true, &peers_ok);
+      if (st != PXZ_OK) return st;
+      if (!peers_ok) return fail(ctx, PXZ_E_NCCL, "another rank failed before the min/max exchange");
+      if (fast_norm && (st = run_guard_band(ctx, im, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
+    }
+    return plan_and_resample(ctx, im, g, metric, vm, filter_down, exact_all, p);
+  });
 }
 
-// Rate control (pxz_shrink_to_size).  bpp: bytes per pixel the budget counts (3 for an RGB image on the RGBA kernels).
+pxz_status pxz_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
+                      pxz_filter filter_down, uint32_t flags, pxz_payload** out) {
+  if (!ctx || !img || !out) return PXZ_E_ARG;
+  *out = nullptr;
+  cudaSetDevice(ctx->device);
+  // Every rank of a communicator must reach the min/max exchange, whatever happens to it before: a rank-local failure
+  // (an unknown filter, a trailing block the Sobel metric cannot take, no memory for the RGB widening or the analysis) joins
+  // with neutral values and an error flag instead of leaving its peers in the collective.
+  bool exchanged = false;
+  const pxz_status st = shrink_image(ctx, img, bw, bh, metric, factor, filter_down, flags, &exchanged, out);
+  if (st != PXZ_OK && !exchanged && (flags & PXZ_FLAG_NORMALISE_GLOBAL) && ctx->comm) {
+    const std::string msg = ctx->err;
+    bool peers_ok = true;
+    exchange_minmax(ctx, false, &peers_ok);
+    ctx->err = msg;
+  }
+  return st;
+}
+
+// Rate control (pxz_shrink_to_size) after the checks.  bpp: bytes per pixel the budget counts.
 static pxz_status shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_bytes,
                                  pxz_filter filter_down, uint32_t flags, uint32_t bpp, float* factor_out, pxz_payload** out) {
-  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh))
-    return encode_via_rgba(
-        ctx, img,
-        [&](const pxz_image* wide, pxz_payload** p4) {
-          return shrink_to_size(ctx, wide, bw, bh, metric, max_bytes, filter_down, flags, 3, factor_out, p4);
-        },
-        out);
-  if (!known_filter(filter_down)) return fail(ctx, PXZ_E_ARG, "unknown filter");
-  if (metric != PXZ_METRIC_OKLAB_MAD && metric != PXZ_METRIC_SOBEL_DIR) return fail(ctx, PXZ_E_ARG, "unknown metric");
-  if (flags & PXZ_FLAG_AFTER_IDENTITY) return fail(ctx, PXZ_E_ARG, "PXZ_FLAG_AFTER_IDENTITY ignores the factor: no size to choose");
-  if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "a size budget is per image: not available on a batch");
-  const bool normalise = (flags & PXZ_FLAG_NORMALISE_GLOBAL) != 0;
-  if (normalise && ctx->comm)
-    return fail(ctx, PXZ_E_UNSUPPORTED, "a size budget with global normalisation over a communicator is not available");
   Geom g;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g, img->nimg);
   if (st != PXZ_OK) return st;
@@ -1170,11 +1187,10 @@ static pxz_status shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw
 
   // scratch: the sizes of one round, and on the fast path the copy of the values the search runs on
   DevBlocks bufs(ctx);
-  uint8_t* scratch = nullptr;
-  const size_t sizes_bytes = (size_t)kMaxSizeCandidates * sizeof(uint64_t);
-  if ((st = bufs.alloc(&scratch, sizes_bytes + (fast ? (size_t)nblocks * 4 : 0))) != PXZ_OK) return st;
-  uint64_t* d_sizes = reinterpret_cast<uint64_t*>(scratch);
-  float* d_search = fast ? reinterpret_cast<float*>(scratch + sizes_bytes) : ctx->d_vx;
+  uint64_t* d_sizes = nullptr;
+  float* d_copy = nullptr;
+  if ((st = bufs.alloc(layout_of(part(d_sizes, kMaxSizeCandidates), part(d_copy, fast ? nblocks : 0)))) != PXZ_OK) return st;
+  float* d_search = fast ? d_copy : ctx->d_vx;
   const float* d_search_y = metric == PXZ_METRIC_SOBEL_DIR ? ctx->d_vy : nullptr;
   if (fast) PXZ_CUDA(ctx, cudaMemcpyAsync(d_search, ctx->d_vx, (size_t)nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
 
@@ -1260,7 +1276,12 @@ pxz_status pxz_shrink_to_size(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, u
   if (!ctx || !img || !out || !factor_out) return PXZ_E_ARG;
   *out = nullptr;
   cudaSetDevice(ctx->device);
-  return shrink_to_size(ctx, img, bw, bh, metric, max_bytes, filter_down, flags, img->c, factor_out, out);
+  const pxz_status st =
+      rate_refusal(ctx, img, "a size budget", kCheckDown | kCheckMetric | kCheckAfterIdentity, filter_down, filter_down, metric, flags);
+  if (st != PXZ_OK) return st;
+  return on_kernel_image(ctx, img, bw, bh, out, [&](const pxz_image* im, uint32_t bpp, pxz_payload** p) {
+    return shrink_to_size(ctx, im, bw, bh, metric, max_bytes, filter_down, flags, bpp, factor_out, p);
+  });
 }
 
 // ---- decode error and strategy fit (extension) -------------------------------------------------------------------
@@ -1285,10 +1306,9 @@ pxz_status pxz_image_error(pxz_ctx* ctx, const pxz_image* a, const pxz_image* b,
   if (st != PXZ_OK) return st;
   const size_t nblocks = (size_t)g.cols * g.rows;
   DevBlocks bufs(ctx);
-  uint8_t* buf = nullptr;
-  if ((st = bufs.alloc(&buf, nblocks * (sizeof(uint64_t) + sizeof(uint32_t)))) != PXZ_OK) return st;
-  uint64_t* d_sse = reinterpret_cast<uint64_t*>(buf);
-  uint32_t* d_max = reinterpret_cast<uint32_t*>(buf + nblocks * sizeof(uint64_t));
+  uint64_t* d_sse = nullptr;
+  uint32_t* d_max = nullptr;
+  if ((st = bufs.alloc(layout_of(part(d_sse, nblocks), part(d_max, nblocks)))) != PXZ_OK) return st;
   if ((st = run_block_error(ctx, a, b, g, d_sse, host_block_max ? d_max : nullptr)) != PXZ_OK) return st;
   // the total is summed on the host from the block sums (cols * rows words; the grid is what the caller asked for)
   std::vector<uint64_t> sse(nblocks);
@@ -1306,18 +1326,11 @@ pxz_status pxz_image_error(pxz_ctx* ctx, const pxz_image* a, const pxz_image* b,
 }
 
 // pxz_strategy_measure after the checks, with the context's strategy cleared: one analysis, then for each down filter the plan
-// + resample of pxz_shrink and for each up filter an expand into one scratch image and the error / bucket passes
+// + resample of pxz_shrink and for each up filter an expand into one scratch image and the error / bucket passes.  An RGB image
+// that pxz_shrink runs on the RGBA kernels is measured as its RGBA widening: the payloads are then the 4-channel payloads
+// pxz_shrink narrows, and the decodes those pxz_expand_to_image narrows, so the report equals that of the 3-channel image.
 static pxz_status strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, float factor,
                                    uint32_t flags, uint64_t* host_sse, uint32_t* host_blocks) {
-  // An RGB image that pxz_shrink runs on the RGBA kernels is measured as its RGBA widening: the payloads are then the 4-channel
-  // payloads pxz_shrink narrows, and the decodes those pxz_expand_to_image narrows.  The alpha channel is 255 in the source and
-  // in every decode, so it adds 0 to every sum and the report equals that of the 3-channel image.
-  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
-    ImageOwner wide;
-    pxz_status st = rgb_widened(ctx, img, &wide);
-    if (st != PXZ_OK) return st;
-    return strategy_measure(ctx, wide.get(), bw, bh, metric, factor, flags, host_sse, host_blocks);
-  }
   Geom g;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g);
   if (st != PXZ_OK) return st;
@@ -1330,17 +1343,16 @@ static pxz_status strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t 
   const bool fast_norm = (flags & PXZ_FLAG_NORMALISE_GLOBAL) && metric == PXZ_METRIC_OKLAB_MAD && !exact_all;
   if ((st = run_shrink_analysis(ctx, img, g, metric, flags, &vm)) != PXZ_OK) return st;
   if (fast_norm && (st = run_guard_band(ctx, img, g, vm, ctx->d_vx, ctx->d_vx)) != PXZ_OK) return st;
-  // device scratch: the report (65 x 25 sums, 65 counts), the block errors of one pair
-  const size_t report_sse = (size_t)kStrategyBuckets * kFilterPairs * sizeof(uint64_t);
-  const size_t report_bytes = report_sse + kStrategyBuckets * sizeof(uint32_t);
-  const size_t block_sse_off = (report_bytes + 7) & ~(size_t)7;
+  // device scratch: the report, the block errors of one pair
+  struct Report {
+    uint64_t sse[kStrategyBuckets * kFilterPairs];
+    uint32_t blocks[kStrategyBuckets];
+  };
   DevBlocks bufs(ctx);
-  uint8_t* buf = nullptr;
-  if ((st = bufs.alloc(&buf, block_sse_off + (size_t)nblocks * sizeof(uint64_t))) != PXZ_OK) return st;
-  uint64_t* d_sse = reinterpret_cast<uint64_t*>(buf);
-  uint32_t* d_blocks = reinterpret_cast<uint32_t*>(buf + report_sse);
-  uint64_t* d_block_sse = reinterpret_cast<uint64_t*>(buf + block_sse_off);
-  PXZ_CUDA(ctx, cudaMemsetAsync(buf, 0, report_bytes, ctx->stream));
+  Report* d_report = nullptr;
+  uint64_t* d_block_sse = nullptr;
+  if ((st = bufs.alloc(layout_of(part(d_report, 1), part(d_block_sse, nblocks)))) != PXZ_OK) return st;
+  PXZ_CUDA(ctx, cudaMemsetAsync(d_report, 0, sizeof(Report), ctx->stream));
   ImageOwner dec;
   if ((st = image_new(ctx, img->w, img->h, img->c, 1, &dec)) != PXZ_OK) return st;
   // down outer, up inner: one payload and one decode alive at a time.  The dims do not depend on the filter, so the five
@@ -1354,13 +1366,14 @@ static pxz_status strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t 
       if ((st = pxz_expand_to_image(ctx, p.get(), (pxz_filter)up, dec.get())) != PXZ_OK) return st;
       if ((st = run_block_error(ctx, img, dec.get(), g, d_block_sse, nullptr)) != PXZ_OK) return st;
       st = profiled(ctx, K_BUCKET_SUM, "bucket sum", [&] {
-        return launch_bucket_sum(p->d_descs, d_block_sse, nblocks, pair, pair == 0, d_sse, d_blocks, ctx->stream, ctx->sm_count, &ctx->launches);
+        return launch_bucket_sum(p->d_descs, d_block_sse, nblocks, pair, pair == 0, d_report->sse, d_report->blocks, ctx->stream, ctx->sm_count,
+                                 &ctx->launches);
       });
       if (st != PXZ_OK) return st;
     }
   }
-  PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, d_sse, report_sse, cudaMemcpyDeviceToHost, ctx->stream));
-  PXZ_CUDA(ctx, cudaMemcpyAsync(host_blocks, d_blocks, kStrategyBuckets * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, d_report->sse, sizeof(Report::sse), cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaMemcpyAsync(host_blocks, d_report->blocks, sizeof(Report::blocks), cudaMemcpyDeviceToHost, ctx->stream));
   PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return PXZ_OK;
 }
@@ -1369,9 +1382,8 @@ pxz_status pxz_strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw,
                                 uint32_t flags, uint64_t* host_sse, uint32_t* host_blocks) {
   if (!ctx || !img || !host_sse || !host_blocks) return PXZ_E_ARG;
   cudaSetDevice(ctx->device);
-  if (img->nimg != 1) return fail(ctx, PXZ_E_UNSUPPORTED, "a strategy measure is per image: not available on a batch");
-  if ((flags & PXZ_FLAG_NORMALISE_GLOBAL) && ctx->comm)
-    return fail(ctx, PXZ_E_UNSUPPORTED, "a strategy measure with global normalisation over a communicator is not available");
+  const pxz_status st = rate_refusal(ctx, img, "a strategy measure", 0, PXZ_NEAREST, PXZ_NEAREST, metric, flags);
+  if (st != PXZ_OK) return st;
   // the installed strategy would pick one pair per block: cleared for the call, restored on every return path
   struct StrategyOff {
     pxz_ctx* c;
@@ -1379,24 +1391,12 @@ pxz_status pxz_strategy_measure(pxz_ctx* ctx, const pxz_image* img, uint32_t bw,
     explicit StrategyOff(pxz_ctx* cc) : c(cc), saved(cc->strategy) { c->strategy.on = 0; }
     ~StrategyOff() { c->strategy = saved; }
   } off(ctx);
-  return strategy_measure(ctx, img, bw, bh, metric, factor, flags, host_sse, host_blocks);
+  return on_kernel_image(ctx, img, bw, bh, nullptr, [&](const pxz_image* im, uint32_t, pxz_payload**) {
+    return strategy_measure(ctx, im, bw, bh, metric, factor, flags, host_sse, host_blocks);
+  });
 }
 
 // ---- rate-distortion curve (extension) ---------------------------------------------------------------------------
-// What pxz_rd_curve and pxz_shrink_to_error refuse: pxz_shrink_to_size's refusals, plus an installed strategy (its filter pair
-// follows the stored value, which moves with the factor) and an unknown up filter
-static pxz_status rd_refusal(pxz_ctx* ctx, const pxz_image* img, pxz_metric metric, pxz_filter filter_down, pxz_filter filter_up, uint32_t flags) {
-  if (!known_filter(filter_down) || !known_filter(filter_up)) return fail(ctx, PXZ_E_ARG, "unknown filter");
-  if (metric != PXZ_METRIC_OKLAB_MAD && metric != PXZ_METRIC_SOBEL_DIR) return fail(ctx, PXZ_E_ARG, "unknown metric");
-  if (flags & PXZ_FLAG_AFTER_IDENTITY) return fail(ctx, PXZ_E_ARG, "PXZ_FLAG_AFTER_IDENTITY ignores the factor: no curve over it");
-  if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "a rate-distortion curve is per image: not available on a batch");
-  if ((flags & PXZ_FLAG_NORMALISE_GLOBAL) && ctx->comm)
-    return fail(ctx, PXZ_E_UNSUPPORTED, "a rate-distortion curve with global normalisation over a communicator is not available");
-  if (ctx->strategy.on)
-    return fail(ctx, PXZ_E_UNSUPPORTED, "a rate-distortion curve with a strategy installed is not available (the filter pair moves with the factor)");
-  return PXZ_OK;
-}
-
 // What one curve computation returns to the host besides the points
 struct RdSummary {
   uint32_t n = 0;                  // curve points
@@ -1407,6 +1407,22 @@ struct RdSummary {
 };
 
 static uint32_t ceil_log2(uint32_t n) { return n <= 1 ? 0u : 32u - (uint32_t)__builtin_clz(n - 1); }
+
+// The end of pxz_rd_curve and pxz_rdo_curve: *n_out = the curve's n points, copied from each device array to its host array
+// when cap >= n, else refused
+struct PointArray {
+  void* host;
+  const void* dev;
+  size_t bytes;  // per point
+};
+static pxz_status curve_points(pxz_ctx* ctx, uint32_t n, size_t cap, size_t* n_out, std::initializer_list<PointArray> arrays) {
+  *n_out = n;
+  if (cap < n) return fail(ctx, PXZ_E_ARG, "cap " + std::to_string(cap) + " is below the curve's " + std::to_string(n) + " points");
+  if (n == 0) return PXZ_OK;
+  for (const PointArray& a : arrays) PXZ_CUDA(ctx, cudaMemcpyAsync(a.host, a.dev, (size_t)n * a.bytes, cudaMemcpyDeviceToHost, ctx->stream));
+  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  return PXZ_OK;
+}
 
 // The error table of the rate-distortion curves: per level pair (lx, ly) the plan + resample of pxz_shrink with every block
 // forced to it — values 2^-lx / 2^-ly under the directional map at factor 1, no normalisation — then the decode with filter_up
@@ -1441,19 +1457,15 @@ static pxz_status rd_error_table(pxz_ctx* ctx, const pxz_image* img, const Geom&
   return PXZ_OK;
 }
 
-// The curve of pxz_rd_curve after the checks (DESIGN.md §3).  bpp: bytes per pixel counted (3 for an RGB image on the RGBA
-// kernels).  The points are copied to the host arrays when cap >= n.
+// The checks of pxz_rd_curve and pxz_shrink_to_error.  An installed strategy is refused: its filter pair follows the stored value,
+// which moves with the factor.
+constexpr uint32_t kRdChecks = kCheckDown | kCheckUp | kCheckMetric | kCheckAfterIdentity | kCheckStrategy;
+
+// The curve of pxz_rd_curve after the checks (DESIGN.md §3).  bpp: bytes per pixel counted.  With n_out the points go to the
+// host arrays (curve_points); without, *sum is filled for the first point within max_sse.
 static pxz_status rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, pxz_filter filter_down,
                            pxz_filter filter_up, uint32_t flags, uint32_t bpp, uint64_t max_sse, float* host_factor, uint64_t* host_bytes,
-                           uint64_t* host_sse, size_t cap, RdSummary* sum) {
-  // An RGB image that pxz_shrink runs on the RGBA kernels is measured as its RGBA widening, as in strategy_measure: alpha is 255
-  // in the source and in every decode and adds 0
-  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
-    ImageOwner wide;
-    pxz_status st = rgb_widened(ctx, img, &wide);
-    if (st != PXZ_OK) return st;
-    return rd_curve(ctx, wide.get(), bw, bh, metric, filter_down, filter_up, flags, 3, max_sse, host_factor, host_bytes, host_sse, cap, sum);
-  }
+                           uint64_t* host_sse, size_t cap, size_t* n_out, RdSummary* sum) {
   Geom g;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g);
   if (st != PXZ_OK) return st;
@@ -1471,29 +1483,21 @@ static pxz_status rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint
 
   // 1. reference-order values (their dims are pxz_shrink's in every mode), the min / max as pxz_shrink takes it, and a copy
   if ((st = run_shrink_analysis(ctx, img, g, metric, flags | PXZ_FLAG_EXACT_VALUES, nullptr)) != PXZ_OK) return st;
+  // the values' copy, the error table [npass][nblocks], the events, the points, CUB's scratch
   DevBlocks bufs(ctx);
-  float* vals = nullptr;
-  uint64_t* table = nullptr;  // [npass][nblocks] block errors
-  uint8_t* ev = nullptr;      // events: keys | ids | dbytes | dsse | base[2] | points: key | bytes | sse | RdOut
-  void* scratch = nullptr;
+  float *vx = nullptr, *vy = nullptr;
+  uint64_t *table = nullptr, *dbytes = nullptr, *dsse = nullptr, *base = nullptr, *pt_bytes = nullptr, *pt_sse = nullptr;
+  uint32_t *keys = nullptr, *ids = nullptr, *pt_key = nullptr;
+  RdOut* d_out = nullptr;
+  uint8_t* scratch = nullptr;
   const size_t scratch_bytes = rd_curve_scratch_bytes(nev);
   const size_t npt = (size_t)nev + 1;
-  const size_t ev_bytes = (size_t)nev * 24 + 16 + npt * 20 + sizeof(RdOut) + 64;
-  if ((st = bufs.alloc(&vals, nblocks * 4 * (sobel ? 2 : 1))) != PXZ_OK || (st = bufs.alloc(&table, (size_t)npass * nblocks * 8)) != PXZ_OK ||
-      (st = bufs.alloc(&ev, ev_bytes)) != PXZ_OK || (st = bufs.alloc(&scratch, scratch_bytes)) != PXZ_OK)
+  if ((st = bufs.alloc(layout_of(part(vx, nblocks), part(vy, sobel ? nblocks : 0), part(table, (size_t)npass * nblocks), part(keys, nev),
+                                 part(ids, nev), part(dbytes, nev), part(dsse, nev), part(base, 2), part(pt_key, npt), part(pt_bytes, npt),
+                                 part(pt_sse, npt), part(d_out, 1), part(scratch, scratch_bytes)))) != PXZ_OK)
     return st;
-  // 8-byte words first
-  uint64_t* dbytes = reinterpret_cast<uint64_t*>(ev);
-  uint64_t* dsse = dbytes + nev;
-  uint64_t* base = dsse + nev;
-  uint64_t* pt_bytes = base + 2;
-  uint64_t* pt_sse = pt_bytes + npt;
-  RdOut* d_out = reinterpret_cast<RdOut*>(pt_sse + npt);
-  uint32_t* keys = reinterpret_cast<uint32_t*>(d_out + 1);
-  uint32_t* ids = keys + nev;
-  uint32_t* pt_key = ids + nev;
-  PXZ_CUDA(ctx, cudaMemcpyAsync(vals, ctx->d_vx, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-  if (sobel) PXZ_CUDA(ctx, cudaMemcpyAsync(vals + nblocks, ctx->d_vy, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+  PXZ_CUDA(ctx, cudaMemcpyAsync(vx, ctx->d_vx, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
+  if (sobel) PXZ_CUDA(ctx, cudaMemcpyAsync(vy, ctx->d_vy, nblocks * 4, cudaMemcpyDeviceToDevice, ctx->stream));
 
   // 2. error table
   if ((st = rd_error_table(ctx, img, g, filter_down, filter_up, !sobel, sobel ? lx_max : l_max, sobel ? ly_max : l_max, ps, table)) != PXZ_OK)
@@ -1503,7 +1507,7 @@ static pxz_status rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint
   const ValueMap vm = shrink_value_map(ctx, metric, flags & PXZ_FLAG_NORMALISE_GLOBAL, 1.0f);
   PXZ_CUDA(ctx, cudaMemsetAsync(base, 0, 2 * sizeof(uint64_t), ctx->stream));
   st = profiled(ctx, K_RD_EVENTS, "rd events", [&] {
-    return launch_rd_events(vals, sobel ? vals + nblocks : nullptr, g, vm, ctx->d_minmax, ctx->thr, bpp, table, ps, maxev, keys, ids, dbytes, dsse,
+    return launch_rd_events(vx, sobel ? vy : nullptr, g, vm, ctx->d_minmax, ctx->thr, bpp, table, ps, maxev, keys, ids, dbytes, dsse,
                             base, ctx->stream, &ctx->launches);
   });
   if (st != PXZ_OK) return st;
@@ -1513,23 +1517,20 @@ static pxz_status rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint
   });
   if (st != PXZ_OK) return st;
 
-  // 5. to the host: the summary, the first point within max_sse, and the points when they fit
+  // 5. to the host: the points, or the summary and the first point within max_sse
   RdOut o;
   PXZ_CUDA(ctx, cudaMemcpyAsync(&o, d_out, sizeof(o), cudaMemcpyDeviceToHost, ctx->stream));
   PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
+  if (n_out)  // the factors as their f32 bits
+    return curve_points(ctx, o.count, cap, n_out, {{host_factor, pt_key, 4}, {host_bytes, pt_bytes, 8}, {host_sse, pt_sse, 8}});
   sum->n = o.count;
   sum->first = o.first_within;
   sum->least_sse = o.least_sse;
   if (o.first_within < o.count) {
     PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->first_bits, pt_key + o.first_within, 4, cudaMemcpyDeviceToHost, ctx->stream));
     PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->first_sse, pt_sse + o.first_within, 8, cudaMemcpyDeviceToHost, ctx->stream));
+    PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   }
-  if (cap >= o.count && host_factor && host_bytes && host_sse) {
-    PXZ_CUDA(ctx, cudaMemcpyAsync(host_factor, pt_key, (size_t)o.count * 4, cudaMemcpyDeviceToHost, ctx->stream));  // f32 bits
-    PXZ_CUDA(ctx, cudaMemcpyAsync(host_bytes, pt_bytes, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, pt_sse, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
-  }
-  PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
   return PXZ_OK;
 }
 
@@ -1539,14 +1540,11 @@ pxz_status pxz_rd_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_
   if (n_out) *n_out = 0;
   if (!ctx || !img || !n_out || (cap > 0 && (!host_factor || !host_bytes || !host_sse))) return PXZ_E_ARG;
   cudaSetDevice(ctx->device);
-  pxz_status st = rd_refusal(ctx, img, metric, filter_down, filter_up, flags);
+  const pxz_status st = rate_refusal(ctx, img, "a rate-distortion curve", kRdChecks, filter_down, filter_up, metric, flags);
   if (st != PXZ_OK) return st;
-  RdSummary sum;
-  st = rd_curve(ctx, img, bw, bh, metric, filter_down, filter_up, flags, img->c, 0, host_factor, host_bytes, host_sse, cap, &sum);
-  if (st != PXZ_OK) return st;
-  *n_out = sum.n;
-  if (cap < sum.n) return fail(ctx, PXZ_E_ARG, "cap " + std::to_string(cap) + " is below the curve's " + std::to_string(sum.n) + " points");
-  return PXZ_OK;
+  return on_kernel_image(ctx, img, bw, bh, nullptr, [&](const pxz_image* im, uint32_t bpp, pxz_payload**) {
+    return rd_curve(ctx, im, bw, bh, metric, filter_down, filter_up, flags, bpp, 0, host_factor, host_bytes, host_sse, cap, n_out, nullptr);
+  });
 }
 
 pxz_status pxz_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_metric metric, uint64_t max_sse,
@@ -1555,10 +1553,12 @@ pxz_status pxz_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, 
   if (!ctx || !img || !out) return PXZ_E_ARG;
   *out = nullptr;
   cudaSetDevice(ctx->device);
-  pxz_status st = rd_refusal(ctx, img, metric, filter_down, filter_up, flags);
+  pxz_status st = rate_refusal(ctx, img, "a rate-distortion curve", kRdChecks, filter_down, filter_up, metric, flags);
   if (st != PXZ_OK) return st;
   RdSummary sum;
-  st = rd_curve(ctx, img, bw, bh, metric, filter_down, filter_up, flags, img->c, max_sse, nullptr, nullptr, nullptr, 0, &sum);
+  st = on_kernel_image(ctx, img, bw, bh, nullptr, [&](const pxz_image* im, uint32_t bpp, pxz_payload**) {
+    return rd_curve(ctx, im, bw, bh, metric, filter_down, filter_up, flags, bpp, max_sse, nullptr, nullptr, nullptr, 0, nullptr, &sum);
+  });
   if (st != PXZ_OK) return st;
   if (sum.first >= sum.n)
     return fail(ctx, PXZ_E_ARG, "max_sse " + std::to_string(max_sse) + " is below the least squared error any factor reaches (" +
@@ -1573,14 +1573,9 @@ pxz_status pxz_shrink_to_error(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, 
 }
 
 // ---- rate-distortion optimised encode (extension) ----------------------------------------------------------------
-// No metric, flags or factor: every block takes the dims of any level pair (DESIGN.md §3 "Per-block sizes")
-static pxz_status rdo_refusal(pxz_ctx* ctx, const pxz_image* img, pxz_filter filter_down, pxz_filter filter_up) {
-  if (!known_filter(filter_down) || !known_filter(filter_up)) return fail(ctx, PXZ_E_ARG, "unknown filter");
-  if (img->nimg > 1) return fail(ctx, PXZ_E_UNSUPPORTED, "an optimised encode is per image: not available on a batch");
-  if (ctx->strategy.on)
-    return fail(ctx, PXZ_E_UNSUPPORTED, "an optimised encode with a strategy installed is not available (its filter pair follows the stored value)");
-  return PXZ_OK;
-}
+// No metric, flags or factor: every block takes the dims of any level pair (DESIGN.md §3 "Per-block sizes").  An installed
+// strategy is refused: its filter pair follows the stored value.
+constexpr uint32_t kRdoChecks = kCheckDown | kCheckUp | kCheckStrategy;
 
 // Most events a block can have: its distinct byte counts over every level pair, less one, over the (up to four) tile shapes
 static uint32_t rdo_max_events(const Geom& g) {
@@ -1601,30 +1596,19 @@ static uint32_t rdo_max_events(const Geom& g) {
 
 enum class RdoPick { None, Size, Error };
 
-// What one optimised curve returns to the host besides the points
+// What one optimised encode returns to the host
 struct RdoSummary {
-  uint32_t n = 0;       // curve points
   uint64_t bytes0 = 0;  // payload bytes with every block at 1 x 1 (point 0)
   uint64_t bytes = 0;   // the chosen point's bytes and sse
   uint64_t sse = 0;
 };
 
-// The optimised curve after the checks, and with pick != None the payload of the point a budget picks (to size: the last with
-// bytes <= budget; to error: the first with sse <= budget) into *out.  bpp: bytes per pixel counted (3 for an RGB image on the
-// RGBA kernels).  The points are copied to the host arrays when cap >= n.
+// The optimised curve after the checks.  pick == None: the points go to the host arrays (curve_points).  Otherwise the payload
+// of the point a budget picks (to size: the last with bytes <= budget; to error: the first with sse <= budget) into *out.
+// bpp: bytes per pixel counted.
 static pxz_status rdo(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, pxz_filter filter_down, pxz_filter filter_up, uint32_t bpp,
-                      RdoPick pick, uint64_t budget, uint64_t* host_bytes, uint64_t* host_sse, size_t cap, RdoSummary* sum, pxz_payload** out) {
-  // An RGB image that pxz_shrink runs on the RGBA kernels is measured and encoded as its RGBA widening (alpha is 255 in the
-  // source and every decode and adds 0); the payload is narrowed back as pxz_shrink narrows it
-  if (rgb_on_rgba(ctx, img->w, img->c, bw, bh)) {
-    auto wide_rdo = [&](const pxz_image* wide, pxz_payload** p4) {
-      return rdo(ctx, wide, bw, bh, filter_down, filter_up, 3, pick, budget, host_bytes, host_sse, cap, sum, p4);
-    };
-    if (pick != RdoPick::None) return encode_via_rgba(ctx, img, wide_rdo, out);
-    ImageOwner wide;
-    pxz_status st = rgb_widened(ctx, img, &wide);
-    return st != PXZ_OK ? st : wide_rdo(wide.get(), nullptr);
-  }
+                      RdoPick pick, uint64_t budget, uint64_t* host_bytes, uint64_t* host_sse, size_t cap, size_t* n_out, RdoSummary* sum,
+                      pxz_payload** out) {
   Geom g;
   pxz_status st = make_geom(ctx, img->w, img->h, img->c, bw, bh, &g);
   if (st != PXZ_OK) return st;
@@ -1637,25 +1621,19 @@ static pxz_status rdo(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t 
   const uint32_t nev = (uint32_t)nev64;
   if ((st = ensure_scratch(ctx, nblocks)) != PXZ_OK) return st;
 
+  // the error table [npass][nblocks], the events, the points, CUB's scratch
   DevBlocks bufs(ctx);
-  uint64_t* table = nullptr;  // [npass][nblocks] block errors
-  uint8_t* ev = nullptr;      // events | base[3] | points: bytes | sse | ids | ev_pass | rank | pass0 | RdoOut
-  void* scratch = nullptr;
+  uint64_t *table = nullptr, *base = nullptr, *pt_bytes = nullptr, *pt_sse = nullptr;
+  RdoEvent* events = nullptr;
+  uint32_t *ids = nullptr, *ev_pass = nullptr, *rank = nullptr, *pass0 = nullptr;
+  RdoOut* d_out = nullptr;
+  uint8_t* scratch = nullptr;
   const size_t scratch_bytes = rdo_curve_scratch_bytes(nev);
   const size_t npt = (size_t)nev + 1;
-  const size_t ev_bytes = (size_t)nev * (sizeof(RdoEvent) + 12) + 24 + npt * 16 + (size_t)nblocks * 4 + sizeof(RdoOut);
-  if ((st = bufs.alloc(&table, (size_t)npass * nblocks * 8)) != PXZ_OK || (st = bufs.alloc(&ev, ev_bytes)) != PXZ_OK ||
-      (st = bufs.alloc(&scratch, scratch_bytes)) != PXZ_OK)
+  if ((st = bufs.alloc(layout_of(part(table, (size_t)npass * nblocks), part(events, nev), part(base, 3), part(pt_bytes, npt), part(pt_sse, npt),
+                                 part(ids, nev), part(ev_pass, nev), part(rank, nev), part(pass0, nblocks), part(d_out, 1),
+                                 part(scratch, scratch_bytes)))) != PXZ_OK)
     return st;
-  RdoEvent* events = reinterpret_cast<RdoEvent*>(ev);
-  uint64_t* base = reinterpret_cast<uint64_t*>(events + nev);
-  uint64_t* pt_bytes = base + 3;
-  uint64_t* pt_sse = pt_bytes + npt;
-  uint32_t* ids = reinterpret_cast<uint32_t*>(pt_sse + npt);
-  uint32_t* ev_pass = ids + nev;
-  uint32_t* rank = ev_pass + nev;
-  uint32_t* pass0 = rank + nev;
-  RdoOut* d_out = reinterpret_cast<RdoOut*>(pass0 + nblocks);
 
   // 1. error table over every level pair, 2. per-block hulls, 3. the curve
   const RdPasses ps{lx_max, ly_max, ly_max + 1, 1};
@@ -1671,18 +1649,12 @@ static pxz_status rdo(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t 
   });
   if (st != PXZ_OK) return st;
 
-  // 4. to the host: the summary, the chosen point, and the points when they fit
+  // 4. to the host: the points, or the summary and the chosen point
   RdoOut o;
   PXZ_CUDA(ctx, cudaMemcpyAsync(&o, d_out, sizeof(o), cudaMemcpyDeviceToHost, ctx->stream));
   PXZ_CUDA(ctx, cudaMemcpyAsync(&sum->bytes0, pt_bytes, 8, cudaMemcpyDeviceToHost, ctx->stream));
   PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  sum->n = o.count;
-  if (cap >= o.count && host_bytes && host_sse) {
-    PXZ_CUDA(ctx, cudaMemcpyAsync(host_bytes, pt_bytes, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    PXZ_CUDA(ctx, cudaMemcpyAsync(host_sse, pt_sse, (size_t)o.count * 8, cudaMemcpyDeviceToHost, ctx->stream));
-    PXZ_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  }
-  if (pick == RdoPick::None) return PXZ_OK;
+  if (pick == RdoPick::None) return curve_points(ctx, o.count, cap, n_out, {{host_bytes, pt_bytes, 8}, {host_sse, pt_sse, 8}});
   const uint32_t j = pick == RdoPick::Size ? o.best_within - 1 : o.first_within;
   if (pick == RdoPick::Size && o.best_within == 0)
     return fail(ctx, PXZ_E_ARG, "max_bytes " + std::to_string(budget) + " is below the payload with every block at 1 x 1 (" +
@@ -1713,14 +1685,12 @@ pxz_status pxz_rdo_curve(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32
   if (n_out) *n_out = 0;
   if (!ctx || !img || !n_out || (cap > 0 && (!host_bytes || !host_sse))) return PXZ_E_ARG;
   cudaSetDevice(ctx->device);
-  pxz_status st = rdo_refusal(ctx, img, filter_down, filter_up);
+  const pxz_status st = rate_refusal(ctx, img, "an optimised encode", kRdoChecks, filter_down, filter_up, PXZ_METRIC_OKLAB_MAD, 0);
   if (st != PXZ_OK) return st;
   RdoSummary sum;
-  st = rdo(ctx, img, bw, bh, filter_down, filter_up, img->c, RdoPick::None, 0, host_bytes, host_sse, cap, &sum, nullptr);
-  if (st != PXZ_OK) return st;
-  *n_out = sum.n;
-  if (cap < sum.n) return fail(ctx, PXZ_E_ARG, "cap " + std::to_string(cap) + " is below the curve's " + std::to_string(sum.n) + " points");
-  return PXZ_OK;
+  return on_kernel_image(ctx, img, bw, bh, nullptr, [&](const pxz_image* im, uint32_t bpp, pxz_payload**) {
+    return rdo(ctx, im, bw, bh, filter_down, filter_up, bpp, RdoPick::None, 0, host_bytes, host_sse, cap, n_out, &sum, nullptr);
+  });
 }
 
 static pxz_status rdo_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, uint32_t bh, RdoPick pick, uint64_t budget, pxz_filter filter_down,
@@ -1728,10 +1698,12 @@ static pxz_status rdo_shrink(pxz_ctx* ctx, const pxz_image* img, uint32_t bw, ui
   if (!ctx || !img || !out) return PXZ_E_ARG;
   *out = nullptr;
   cudaSetDevice(ctx->device);
-  pxz_status st = rdo_refusal(ctx, img, filter_down, filter_up);
+  pxz_status st = rate_refusal(ctx, img, "an optimised encode", kRdoChecks, filter_down, filter_up, PXZ_METRIC_OKLAB_MAD, 0);
   if (st != PXZ_OK) return st;
   RdoSummary sum;
-  st = rdo(ctx, img, bw, bh, filter_down, filter_up, img->c, pick, budget, nullptr, nullptr, 0, &sum, out);
+  st = on_kernel_image(ctx, img, bw, bh, out, [&](const pxz_image* im, uint32_t bpp, pxz_payload** p) {
+    return rdo(ctx, im, bw, bh, filter_down, filter_up, bpp, pick, budget, nullptr, nullptr, 0, nullptr, &sum, p);
+  });
   if (st != PXZ_OK) return st;
   if (bytes_out) *bytes_out = sum.bytes;
   if (sse_out) *sse_out = sum.sse;

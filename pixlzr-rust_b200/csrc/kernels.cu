@@ -3202,7 +3202,6 @@ cudaError_t launch_rd_events(const float* vx, const float* vy, const Geom& g, co
 
 // scratch of launch_rd_curve: sorted keys | sorted ids | last-of-key flags | point indices | scan input | scan output | CUB's
 // temporary storage
-static size_t rd_align(size_t n) { return (n + 255) & ~(size_t)255; }
 static size_t rd_cub_bytes(uint32_t nev) {
   size_t sort = 0, scan = 0, count = 0;
   cub::DeviceRadixSort::SortPairs(nullptr, sort, (const uint32_t*)nullptr, (uint32_t*)nullptr, (const uint32_t*)nullptr, (uint32_t*)nullptr,
@@ -3211,48 +3210,50 @@ static size_t rd_cub_bytes(uint32_t nev) {
   cub::DeviceScan::InclusiveSum(nullptr, count, (const uint32_t*)nullptr, (uint32_t*)nullptr, (int)nev);
   return std::max(sort, std::max(scan, count));
 }
+struct RdCurveScratch {
+  uint32_t *skeys = nullptr, *sids = nullptr, *last = nullptr, *points = nullptr;
+  RdAcc *acc = nullptr, *sums = nullptr;
+  uint8_t* cub = nullptr;
+  size_t cub_bytes = 0;
+};
+static auto rd_curve_layout(uint32_t nev, RdCurveScratch& sc) {
+  sc.cub_bytes = rd_cub_bytes(nev);
+  return layout_of(part(sc.skeys, nev), part(sc.sids, nev), part(sc.last, nev), part(sc.points, nev), part(sc.acc, nev), part(sc.sums, nev),
+                   part(sc.cub, sc.cub_bytes));
+}
 size_t rd_curve_scratch_bytes(uint32_t nev) {
-  return 4 * rd_align((size_t)nev * 4) + 2 * rd_align((size_t)nev * sizeof(RdAcc)) + rd_align(rd_cub_bytes(nev));
+  RdCurveScratch sc;
+  return rd_curve_layout(nev, sc).bytes();
 }
 
 cudaError_t launch_rd_curve(const uint32_t* keys, const uint32_t* ids, const uint64_t* dbytes, const uint64_t* dsse, uint32_t nev,
                             const uint64_t* base, uint64_t max_sse, void* scratch, size_t scratch_bytes, uint32_t* pt_key, uint64_t* pt_bytes,
                             uint64_t* pt_sse, RdOut* out, cudaStream_t s, int sm_count, uint64_t* launches) {
-  if (scratch_bytes < rd_curve_scratch_bytes(nev) || nev > 0x7FFFFFFFu) return cudaErrorInvalidValue;
-  uint8_t* p = static_cast<uint8_t*>(scratch);
-  uint32_t* skeys = reinterpret_cast<uint32_t*>(p);
-  p += rd_align((size_t)nev * 4);
-  uint32_t* sids = reinterpret_cast<uint32_t*>(p);
-  p += rd_align((size_t)nev * 4);
-  uint32_t* last = reinterpret_cast<uint32_t*>(p);
-  p += rd_align((size_t)nev * 4);
-  uint32_t* points = reinterpret_cast<uint32_t*>(p);
-  p += rd_align((size_t)nev * 4);
-  RdAcc* acc = reinterpret_cast<RdAcc*>(p);
-  p += rd_align((size_t)nev * sizeof(RdAcc));
-  RdAcc* sums = reinterpret_cast<RdAcc*>(p);
-  p += rd_align((size_t)nev * sizeof(RdAcc));
-  size_t cub_bytes = rd_cub_bytes(nev);
+  RdCurveScratch sc;
+  const auto lay = rd_curve_layout(nev, sc);
+  if (scratch_bytes < lay.bytes() || nev > 0x7FFFFFFFu) return cudaErrorInvalidValue;
+  lay.place(scratch);
+  size_t cub_bytes = sc.cub_bytes;
   cudaError_t e = cudaMemsetAsync(out, 0xFF, sizeof(RdOut), s);
   const int grid = clamp_grid(((long long)nev + kThreads - 1) / kThreads, (long long)sm_count * 8);
   if (e == cudaSuccess && nev > 0) {
     // sort, gather, two scans: CUB's sort and scans launch several kernels each and count as one launch here
     *launches += 4;
-    e = cub::DeviceRadixSort::SortPairs(p, cub_bytes, keys, skeys, ids, sids, (int)nev, 0, 32, s);
-    if (e == cudaSuccess) e = launch(k_rd_gather, grid, kThreads, 0, s, skeys, sids, reinterpret_cast<const unsigned long long*>(dbytes),
-                                     reinterpret_cast<const unsigned long long*>(dsse), nev, acc, last);
+    e = cub::DeviceRadixSort::SortPairs(sc.cub, cub_bytes, keys, sc.skeys, ids, sc.sids, (int)nev, 0, 32, s);
+    if (e == cudaSuccess) e = launch(k_rd_gather, grid, kThreads, 0, s, sc.skeys, sc.sids, reinterpret_cast<const unsigned long long*>(dbytes),
+                                     reinterpret_cast<const unsigned long long*>(dsse), nev, sc.acc, sc.last);
     if (e == cudaSuccess) {
-      cub_bytes = rd_cub_bytes(nev);
-      e = cub::DeviceScan::InclusiveScan(p, cub_bytes, acc, sums, RdAccSum(), (int)nev, s);
+      cub_bytes = sc.cub_bytes;
+      e = cub::DeviceScan::InclusiveScan(sc.cub, cub_bytes, sc.acc, sc.sums, RdAccSum(), (int)nev, s);
     }
     if (e == cudaSuccess) {
-      cub_bytes = rd_cub_bytes(nev);
-      e = cub::DeviceScan::InclusiveSum(p, cub_bytes, last, points, (int)nev, s);
+      cub_bytes = sc.cub_bytes;
+      e = cub::DeviceScan::InclusiveSum(sc.cub, cub_bytes, sc.last, sc.points, (int)nev, s);
     }
   }
   if (e != cudaSuccess) return e;
   ++*launches;
-  return launch(k_rd_compact, grid, kThreads, 0, s, skeys, sums, points, nev, reinterpret_cast<const unsigned long long*>(base),
+  return launch(k_rd_compact, grid, kThreads, 0, s, sc.skeys, sc.sums, sc.points, nev, reinterpret_cast<const unsigned long long*>(base),
                 (unsigned long long)max_sse, pt_key, reinterpret_cast<unsigned long long*>(pt_bytes), reinterpret_cast<unsigned long long*>(pt_sse),
                 out);
 }
@@ -3278,18 +3279,28 @@ static size_t rdo_cub_bytes(uint32_t nev) {
   cub::DeviceScan::InclusiveScan(nullptr, scan, (const RdAcc*)nullptr, (RdAcc*)nullptr, RdAccSum(), (int)nev);
   return std::max(sort, scan);
 }
-size_t rdo_curve_scratch_bytes(uint32_t nev) { return 2 * rd_align((size_t)nev * sizeof(RdAcc)) + rd_align(rdo_cub_bytes(nev)); }
+struct RdoCurveScratch {
+  RdAcc *acc = nullptr, *sums = nullptr;
+  uint8_t* cub = nullptr;
+  size_t cub_bytes = 0;
+};
+static auto rdo_curve_layout(uint32_t nev, RdoCurveScratch& sc) {
+  sc.cub_bytes = rdo_cub_bytes(nev);
+  return layout_of(part(sc.acc, nev), part(sc.sums, nev), part(sc.cub, sc.cub_bytes));
+}
+size_t rdo_curve_scratch_bytes(uint32_t nev) {
+  RdoCurveScratch sc;
+  return rdo_curve_layout(nev, sc).bytes();
+}
 
 cudaError_t launch_rdo_curve(RdoEvent* ev, uint32_t* ids, uint32_t nev, const uint64_t* base, uint64_t max_bytes, uint64_t max_sse, void* scratch,
                              size_t scratch_bytes, uint32_t* rank, uint64_t* pt_bytes, uint64_t* pt_sse, RdoOut* out, cudaStream_t s, int sm_count,
                              uint64_t* launches) {
-  if (scratch_bytes < rdo_curve_scratch_bytes(nev) || nev > 0x7FFFFFFFu) return cudaErrorInvalidValue;
-  uint8_t* p = static_cast<uint8_t*>(scratch);
-  RdAcc* acc = reinterpret_cast<RdAcc*>(p);
-  p += rd_align((size_t)nev * sizeof(RdAcc));
-  RdAcc* sums = reinterpret_cast<RdAcc*>(p);
-  p += rd_align((size_t)nev * sizeof(RdAcc));
-  size_t cub_bytes = rdo_cub_bytes(nev);
+  RdoCurveScratch sc;
+  const auto lay = rdo_curve_layout(nev, sc);
+  if (scratch_bytes < lay.bytes() || nev > 0x7FFFFFFFu) return cudaErrorInvalidValue;
+  lay.place(scratch);
+  size_t cub_bytes = sc.cub_bytes;
   // best_within = 0 (none), first_within = all ones (none)
   cudaError_t e = cudaMemsetAsync(out, 0, sizeof(RdoOut), s);
   if (e == cudaSuccess) e = cudaMemsetAsync(&out->first_within, 0xFF, sizeof(uint32_t), s);
@@ -3297,17 +3308,18 @@ cudaError_t launch_rdo_curve(RdoEvent* ev, uint32_t* ids, uint32_t nev, const ui
   if (e == cudaSuccess && nev > 0) {
     // sort, gather, scan: CUB's sort and scan launch several kernels each and count as one launch here
     *launches += 3;
-    e = cub::DeviceMergeSort::StableSortPairs(p, cub_bytes, ev, ids, (int)nev, RdoRateDesc(), s);
-    if (e == cudaSuccess) e = launch(k_rdo_gather, grid, kThreads, 0, s, ev, ids, nev, acc, rank);
+    e = cub::DeviceMergeSort::StableSortPairs(sc.cub, cub_bytes, ev, ids, (int)nev, RdoRateDesc(), s);
+    if (e == cudaSuccess) e = launch(k_rdo_gather, grid, kThreads, 0, s, ev, ids, nev, sc.acc, rank);
     if (e == cudaSuccess) {
-      cub_bytes = rdo_cub_bytes(nev);
-      e = cub::DeviceScan::InclusiveScan(p, cub_bytes, acc, sums, RdAccSum(), (int)nev, s);
+      cub_bytes = sc.cub_bytes;
+      e = cub::DeviceScan::InclusiveScan(sc.cub, cub_bytes, sc.acc, sc.sums, RdAccSum(), (int)nev, s);
     }
   }
   if (e != cudaSuccess) return e;
   ++*launches;
-  return launch(k_rdo_points, grid, kThreads, 0, s, ev, sums, nev, reinterpret_cast<const unsigned long long*>(base), (unsigned long long)max_bytes,
-                (unsigned long long)max_sse, reinterpret_cast<unsigned long long*>(pt_bytes), reinterpret_cast<unsigned long long*>(pt_sse), out);
+  return launch(k_rdo_points, grid, kThreads, 0, s, ev, sc.sums, nev, reinterpret_cast<const unsigned long long*>(base),
+                (unsigned long long)max_bytes, (unsigned long long)max_sse, reinterpret_cast<unsigned long long*>(pt_bytes),
+                reinterpret_cast<unsigned long long*>(pt_sse), out);
 }
 
 cudaError_t launch_rdo_levels(const uint32_t* pass0, const uint32_t* ev_pass, const uint32_t* rank, uint32_t maxev, uint32_t nblocks,

@@ -6,9 +6,43 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <tuple>
+
 #include "../../include/pixlzr_b200.h"
 
 namespace pxz {
+
+// One device block cut into typed arrays.  A layout is the list of its arrays, each a pointer to set and an element count;
+// the same list gives the block's size (bytes()) and, once the block is allocated, every array's address (place()), so the
+// two cannot disagree.  Every array starts at a multiple of kLayoutAlign bytes from the base, as aligned as an allocation of
+// its own would be.
+constexpr size_t kLayoutAlign = 256;
+inline size_t layout_round(size_t bytes) { return (bytes + kLayoutAlign - 1) & ~(kLayoutAlign - 1); }
+template <class T>
+struct LayoutPart {
+  T** ptr;
+  size_t n;
+  size_t bytes() const { return layout_round(n * sizeof(T)); }
+  void place(uint8_t*& at) const {
+    *ptr = reinterpret_cast<T*>(at);
+    at += bytes();
+  }
+};
+template <class T>
+LayoutPart<T> part(T*& ptr, size_t n) { return {&ptr, n}; }
+template <class... T>
+struct Layout {
+  std::tuple<LayoutPart<T>...> parts;
+  size_t bytes() const {
+    return std::apply([](const auto&... p) { return (size_t{0} + ... + p.bytes()); }, parts);
+  }
+  void place(void* base) const {
+    uint8_t* at = static_cast<uint8_t*>(base);
+    std::apply([&](const auto&... p) { (p.place(at), ...); }, parts);
+  }
+};
+template <class... T>
+Layout<T...> layout_of(LayoutPart<T>... parts) { return {{parts...}}; }
 
 constexpr int kMaxLevel = 16;              // level exponents 0..16 get their own resample table
 constexpr int kLevelsPerClass = kMaxLevel + 1;

@@ -104,6 +104,14 @@ def test_edges_of_the_budget(ctx):
         dimg.shrink_to_size(bw, bh, N.METRIC_OKLAB_MAD, 10000, int(P.FilterType.Lanczos3), N.FLAG_AFTER_IDENTITY)
     assert e.value.status == N.E_ARG
     dimg.free()
+    # refused before anything runs, also on an RGB image that the call would widen to RGBA
+    rgb, rbw, rbh = IMAGES["ruscher"]()
+    drgb = ctx.image_upload(rgb)
+    launches = ctx.launch_count()
+    with pytest.raises(N.PixlzrError) as e:
+        drgb.shrink_to_size(rbw, rbh, N.METRIC_OKLAB_MAD, 10000, int(P.FilterType.Lanczos3), N.FLAG_AFTER_IDENTITY)
+    assert e.value.status == N.E_ARG and ctx.launch_count() == launches
+    drgb.free()
     batch = ctx.image_upload_batch(np.stack([img, img]))
     with pytest.raises(N.PixlzrError) as e:
         batch.shrink_to_size(bw, bh, N.METRIC_OKLAB_MAD, 10000, int(P.FilterType.Lanczos3))
